@@ -1,8 +1,12 @@
 #!/usr/bin/env python
 """bench.py -- ERP Mpx/s, entropy encode+decode of the LIC360 context-model path (BASELINE.json metric).
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--dump-outputs DIR]
   (N > 1: python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...)
+
+`--dump-outputs DIR`: after the timed steps, rank 0 writes what the last timed step returned to its caller as float32 .npy files:
+imp_stream.npy and code_stream.npy (the two bitstreams, one value per byte), code.npy and mask.npy (the decoded latent and its
+importance mask).  The inputs are seeded, so two builds run with the same arguments can be compared array for array.
 
 A step = one pass of the hot path over one synthetic 512x1024 ERP image per GPU (BASELINE.json configs[1], batch 1):
 importance stream + code stream ENCODE to the two bitstreams, then DECODE back to the latent, through the fused native
@@ -128,7 +132,7 @@ def chain_kernel_algorithmic_bytes():
 
 
 # ------------------------------------------------------------------------------------------------ CPU arm
-def cpu_arm(steps, warmup, sample_hw=(H, W), budget_s=900.0):
+def cpu_arm(steps, warmup, sample_hw=(H, W)):
     """CPU rendition of the same workload: one (8*h)x(8*w)-pixel ERP image worth of latent (default: the full 512x1024 image of
     configs[1], ~20 s per step on the GPU box's host cores), all host threads."""
     import numpy as np
@@ -140,22 +144,18 @@ def cpu_arm(steps, warmup, sample_hw=(H, W), budget_s=900.0):
     params = {'code': ops.make_entropy_params(48, 4, 3, 3, 2024, 'cpu'), 'imp': ops.make_entropy_params(1, 144, 49, None, 2025, 'cpu')}
     codec = cpu_codec.CpuCodecFast(cpu_codec.params_to_numpy(params))  # channel-last SIMD dot products, same streams (oracle/cpu_codec.py)
     px = (8 * h) * (8 * w) / 1e6
-    times, start = [], time.time()
-    for it in range(warmup + steps):
+    times = []
+    for _ in range(warmup + steps):
         t0 = time.time()
         bi, bc = codec.encode(q, mask, lv)
         code, m = codec.decode(bi, bc, h // 2, w // 2)
         times.append(time.time() - t0)
         assert np.array_equal(code, q * mask) and np.array_equal(m, mask)
-        # safety net for a slow / oversubscribed host: never run past the time box, report the steps that were really timed
-        if it >= warmup and time.time() - start + times[-1] > budget_s:
-            break
-    done = max(1, len(times) - warmup)
-    t = sum(times[-done:]) / done
+    t = sum(times[warmup:]) / steps
     from oracle import oracle as O
-    return {"value": px / t, "unit": "Mpx/s", "cores": os.cpu_count(), "kind": "port", "steps_timed": done,
+    return {"value": px / t, "unit": "Mpx/s", "cores": os.cpu_count(), "kind": "port", "steps_timed": steps,
             "sample": "%dx%d-pixel ERP latent (1,48,%d,%d)+(1,1,%d,%d), encode+decode, OpenMP channel-last fp32 conv + oracle tables + %s host coder, %.1f s/step"
-                      % (8 * h, 8 * w, h, w, h // 2, w // 2, "reference" if O.have_ref_coder() else "restated", t)}, t
+                      % (8 * h, 8 * w, h, w, h // 2, w // 2, "reference" if O.have_ref_coder() else "restated", t)}, t, (bi, bc, code, m)
 
 
 def workload_config(h=H, w=W):
@@ -171,6 +171,16 @@ def emit(line, real_stdout):
     os.write(real_stdout, (json.dumps(line) + "\n").encode())
 
 
+def dump_outputs(dst, imp_stream, code_stream, code, mask):
+    """the last timed step's results as float32 arrays: bitstreams one value per byte, decoded code and mask as returned"""
+    import numpy as np
+    os.makedirs(dst, exist_ok=True)
+    arrays = {"imp_stream": np.frombuffer(imp_stream, np.uint8), "code_stream": np.frombuffer(code_stream, np.uint8),
+              "code": np.asarray(code), "mask": np.asarray(mask)}
+    for name, a in arrays.items():
+        np.save(os.path.join(dst, name + ".npy"), a.astype(np.float32))
+
+
 def main():
     # keep stdout clean: libraries (NCCL prints its version banner to stdout) write to fd 1, which now points at stderr
     sys.stdout.flush()
@@ -183,7 +193,10 @@ def main():
     ap.add_argument("--impl", default="b200", choices=["b200", "reference"])
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-ref-ext", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the last timed step's outputs to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
@@ -201,9 +214,11 @@ def main():
         os.environ.setdefault("OMP_WAIT_POLICY", "passive")  # ~3000 short parallel regions per image: do not burn the cores between them
         # the SAME config and the same K / W as the b200 arm: one full 512x1024 image per step (about 20 s of CPU work per step on the
         # box's host cores; LIC360_BENCH_REF_SAMPLE=h,w shrinks the latent for a quick look, and says so in `config`)
-        steps, ref_warm = max(1, args.steps), max(0, args.warmup)
+        steps, ref_warm = args.steps, max(0, args.warmup)
         hw = tuple(int(v) for v in os.environ.get("LIC360_BENCH_REF_SAMPLE", "%d,%d" % (H, W)).split(","))
-        cb, t = cpu_arm(steps, ref_warm, hw)
+        cb, t, outs = cpu_arm(steps, ref_warm, hw)
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, *outs)
         line = {"impl": "reference", "metric": "ERP Mpx/s encode+decode (entropy path, model-idx 3 shape)", "value": cb["value"], "unit": "Mpx/s",
                 "n_gpus": args.gpus, "steps": cb["steps_timed"], "warmup": ref_warm, "ms_per_step": t * 1e3, "higher_is_better": True,
                 "scaling": "weak", "vs_baseline": None, "dtype": "f32", "data": "synthetic",
@@ -254,7 +269,7 @@ def main():
             if e2e:
                 code_h, mask_h = code.cpu(), mup.cpu()
             nbytes = (len(bi), len(bc))
-        return nbytes, timing, (code, mup)
+        return nbytes, timing, (code, mup, bi, bc)
 
     def timed(steps, e2e):
         barrier()
@@ -304,6 +319,8 @@ def main():
         sampler.stop_flag.set()
         sampler.join()
     ok = bool(torch.equal(outs[0], tq * tm)) and bool(torch.equal(outs[1], tm))
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, outs[2], outs[3], outs[0].cpu().numpy(), outs[1].cpu().numpy())
     run(1, True)
     ms_e2e, _, _, _, _ = timed(args.steps, True)
 
@@ -486,7 +503,7 @@ def main():
         line["clocks"] = sampler.summary()
     if world == 1 and not args.no_cpu_baseline:
         try:
-            line["cpu_baseline"], _ = cpu_arm(1, 0)
+            line["cpu_baseline"] = cpu_arm(1, 0)[0]
         except Exception as e:  # the CPU arm is a reported baseline; never let it take the bench line down
             line["cpu_baseline"] = {"value": None, "unit": "Mpx/s", "cores": os.cpu_count(), "kind": "port", "sample": "failed: %r" % (e,)}
     if world == 1 and not args.no_ref_ext:

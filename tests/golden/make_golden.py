@@ -1,16 +1,18 @@
 """Records outputs of the UNMODIFIED reference CUDA extension (oracle/_ref/lic360_ref*.so, built for sm_100 by
 oracle/Makefile.ref) on the B200 box for every case of tests/op_cases.py:
 
-    gpurun -- python tests/golden/make_golden.py        # writes gpurun_out/golden/ops_golden.npz
-    cp gpurun_out/golden/ops_golden.npz tests/golden/   # committed fixture
+    python tests/golden/make_golden.py                # writes golden_out/ops_golden_*.npz
+    cp golden_out/ops_golden_*.npz tests/golden/        # committed fixture
 
 Bit-exact-tier arrays larger than 16K elements are stored as their SHA-256 only; float-tier arrays larger than that are
 stored as a fixed strided subsample of 8192 elements (`<key>#sub`: flat[::size // 8192][:8192]) -- the full arrays are
-covered by the live comparison in tests/test_gpu_ops.py::test_vs_reference_extension.
+covered by the live comparison in tests/test_gpu_ops.py::test_vs_reference_extension.  The arrays are split over as many
+shards as keep each file below 1 MB (tests/util.py:ops_golden reads them back as one mapping).
 """
 import hashlib
 import os
 import sys
+import zlib
 
 import numpy as np
 
@@ -43,7 +45,15 @@ for case in CASES:
         else:
             out["%s/%s#sub" % (case.name, k)] = np.ascontiguousarray(v).reshape(-1)[::v.size // 8192][:8192].copy()
     print("recorded", case.name, sorted(res))
-dst = os.path.join(ROOT, "gpurun_out", "golden")
+dst = os.path.join(ROOT, "golden_out")
 os.makedirs(dst, exist_ok=True)
-np.savez_compressed(os.path.join(dst, "ops_golden.npz"), **out)
-print("wrote", os.path.join(dst, "ops_golden.npz"), len(out), "arrays")
+shards, size = [{}], 0
+for k, v in out.items():
+    z = len(zlib.compress(np.ascontiguousarray(v).tobytes())) + 512
+    if size + z > 900 * 1024 and shards[-1]:
+        shards.append({})
+        size = 0
+    shards[-1][k], size = v, size + z
+for i, s in enumerate(shards, 1):
+    np.savez_compressed(os.path.join(dst, "ops_golden_%d.npz" % i), **s)
+print("wrote", len(out), "arrays to", len(shards), "shards under", dst)

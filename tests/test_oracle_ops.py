@@ -1,8 +1,6 @@
 """CPU: pins the oracle (oracle/lic360_oracle.c) with the independent formulations the reference itself contains
 (SURVEY.md s8c): masked conv2d == CconvEc == CconvDc-wavefront, the documented index-plan example, adjointness of
 forward/backward pairs, inverse pairs, and table invariants the arithmetic coder asserts."""
-import os
-
 import numpy as np
 import pytest
 import torch
@@ -228,27 +226,23 @@ def test_config1_cpu_entropy_round_trip():
 
 
 # ------------------------------------------------------------------------------------------------ oracle vs golden
-GOLDEN_OPS = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "ops_golden.npz")
-
-
 def _golden_cases():
     from op_cases import CASES
-    if not os.path.exists(GOLDEN_OPS):
-        return []
-    files = set(np.load(GOLDEN_OPS).files)
+    from util import ops_golden
+    files = set(ops_golden())
     return [c for c in CASES if any(f.startswith(c.name + "/") for f in files)]
 
 
 @pytest.mark.parametrize("case", _golden_cases(), ids=[c.name for c in _golden_cases()])
 def test_oracle_against_reference_golden(case):
     """The oracle is pinned on the CPU, without a GPU: its output for every op case is compared with what the UNMODIFIED
-    reference CUDA extension produced for the same seeded inputs on a B200 (tests/golden/ops_golden.npz, make_golden.py).
+    reference CUDA extension produced for the same seeded inputs on a B200 (tests/golden/ops_golden_*.npz, make_golden.py).
     Tiers as in tests/test_gpu_ops.py: exact keys bit for bit (SHA-256 for the large ones), expf/erff-derived integers within one
     count on a tiny fraction (glibc vs libdevice), floats within the case's relative tolerance."""
     import hashlib
-    from util import rel_err
-    gold = np.load(GOLDEN_OPS)
-    keys = [k[len(case.name) + 1:] for k in gold.files if k.startswith(case.name + "/")]
+    from util import ops_golden, rel_err
+    gold = ops_golden()
+    keys = [k[len(case.name) + 1:] for k in gold if k.startswith(case.name + "/")]
     if case.levels_from_device:
         pytest.skip("needs the device's exp() levels as an input")
     exp = case.oracle()

@@ -1,8 +1,24 @@
 """Shared helpers for the parity tests."""
+import functools
+import glob
 import hashlib
+import os
 
 import numpy as np
 import torch
+
+OPS_GOLDEN = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "ops_golden_*.npz")
+
+
+@functools.lru_cache(maxsize=None)
+def ops_golden():
+    """Outputs of the reference extension for every op case, recorded on a B200 by tests/golden/make_golden.py:
+    {"<case>/<key>[#sha256|#sub]": array}, stored in shards (tests/golden/ops_golden_*.npz) that each stay below 1 MB."""
+    out = {}
+    for f in sorted(glob.glob(OPS_GOLDEN)):
+        with np.load(f) as z:
+            out.update({k: z[k] for k in z.files})
+    return out
 
 
 def rng(seed):
