@@ -457,7 +457,7 @@ static int run_ec_net(const NetDesc& n, cudaStream_t s) {
         ConvArgs a;
         int rc = conv_args(n, l, a);
         if (rc) return rc;
-        LIC360_CUDA(launch_cconv_ec(a, s));
+        LIC360_CUDA(launch_cconv_ec(a, s, false));  // the canonical P pass: the decoder reproduces these outputs bit for bit
     }
     return LIC360_OK;
 }

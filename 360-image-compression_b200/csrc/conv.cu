@@ -661,7 +661,7 @@ int fill_conv_args(ConvArgs& a, const float* x, const float* wp, const float* wq
     return 0;
 }
 
-cudaError_t launch_cconv_ec(const ConvArgs& a, cudaStream_t s) {
+cudaError_t launch_cconv_ec(const ConvArgs& a, cudaStream_t s, bool allow_mma) {
     static SmemAttr ec_attr;  // per device (ADVICE r1: a process-wide flag left cuda:1 at the 48 KB default)
     {
         cudaError_t e = ec_attr.ensure(cconv_ec_kernel, EC_SMEM_BYTES);
@@ -669,7 +669,9 @@ cudaError_t launch_cconv_ec(const ConvArgs& a, cudaStream_t s) {
     }
     const int ny = (a.nchunk + EC_CHUNKS - 1) / EC_CHUNKS, nxy = ((a.W + TW - 1) / TW) * ((a.H + TH - 1) / TH);
     cudaError_t e;
-    if (cconv_ec_mma_enabled()) {  // opt-in tensor-core form of the old-term pass (conv_mma.cu): NOT bit-identical to the decoder
+    // opt-in tensor-core form of the old-term pass (conv_mma.cu), per-op CconvEc only: it is NOT bit-identical to the decoder,
+    // so the codec (run_ec_net, allow_mma = false) never uses it and its streams do not depend on LIC360_EC_MMA
+    if (allow_mma && cconv_ec_mma_enabled()) {
         e = launch_cconv_ec_mma(a, s);
     } else {
         const int pair = (long long)nxy * ny * a.N > 2 * 148 ? 1 : 0;  // more than one wave of CTAs (2 per SM): balance them in pairs
@@ -765,7 +767,7 @@ extern "C" int lic360_cconv_ec_forward(const float* x_dev, const float* wp_dev, 
     ConvArgs a;
     LIC360_CHECK_ARG(fill_conv_args(a, x_dev, wp_dev, wq_dev, bias_dev, slope_dev, resid_dev, out_dev, N, Cin, H, W, Cout, G,
                                constrain, nsets) == 0, "bad shape / constrain");
-    LIC360_CUDA(launch_cconv_ec(a, as_stream(stream)));
+    LIC360_CUDA(launch_cconv_ec(a, as_stream(stream), true));
     return LIC360_OK;
 }
 

@@ -17,7 +17,8 @@
 // split leaves 1.2x, mask padding inside the 32-channel tile (~0.85) and issue overhead take the rest -- and the DECODER would have
 // to replay the same MMA sequence per output on its N = 4 wavefront tiles (half of every n8 tile wasted) to stay bit-identical,
 // which is slower than its SIMT kernels.  With this kernel enabled the encoder no longer matches the (SIMT) decoder bit for bit:
-// it is a measurement and parity (1e-5 vs the reference) vehicle, not a codec path.
+// it is a measurement and parity (1e-5 vs the reference) vehicle of the per-op CconvEc, not a codec path (the codec's run_ec_net
+// calls launch_cconv_ec with allow_mma = false).
 #include <cstdlib>
 #include "internal.cuh"
 #include "conv_dev.cuh"

@@ -16,7 +16,8 @@ struct StepDesc { int psum, start, len, pad; };
 
 int fill_conv_args(ConvArgs& a, const float* x, const float* wp, const float* wq, const float* bias, const float* slope,
                    const float* resid, float* out, int N, int Cin, int H, int W, int Cout, int G, int constrain, int nsets);
-cudaError_t launch_cconv_ec(const ConvArgs& a, cudaStream_t s);
+// allow_mma: the per-op CconvEc honours LIC360_EC_MMA; the codec passes false, its streams need the canonical P pass
+cudaError_t launch_cconv_ec(const ConvArgs& a, cudaStream_t s, bool allow_mma);
 // conv_mma.cu: opt-in (LIC360_EC_MMA=1) tensor-core form of the encoder's old-term pass, mma.sync TF32 with a 3-way split
 bool cconv_ec_mma_enabled();
 cudaError_t launch_cconv_ec_mma(const ConvArgs& a, cudaStream_t s);
