@@ -78,6 +78,16 @@ struct NetDesc {
     double t_host_coder = 0, t_gpu_wait = 0, t_done = 0;
     lic360_coder* coder = nullptr;
     char err[256] = {0};                // error text of a worker thread (set_error is thread-local)
+    double* bits_partial_dev = nullptr; // estimate: one partial sum per block of the bits kernel
+    int bits_blocks = 0;
+};
+
+constexpr int BITS_THREADS = 256;  // block size of the estimate's bits and sum kernels
+
+// device-side results of an estimate, copied back with one cudaMemcpyAsync; index = stream_id (0 code, 1 importance)
+struct EstimateTotals {
+    double bits[2];
+    unsigned long long err[2];
 };
 
 }  // namespace lic360
@@ -163,6 +173,9 @@ struct lic360_codec {
     float* mask192_dev = nullptr;       // scratch: Imp2mask output
     std::atomic<int> imp_ready{0};      // decode: importance levels of diagonals < imp_ready are in levels_dev
     std::atomic<int> abort_flag{0};     // decode: one of the two stream loops failed
+    lic360::EstimateTotals* est_dev = nullptr;   // estimate: totals and error keys of both streams
+    lic360::EstimateTotals* est_host = nullptr;  // pinned copy of est_dev
+    cudaEvent_t ev_est = nullptr;                // estimate: the importance stream's results are in est_dev
     double t_host_coder = 0, t_total = 0, t_gpu_wait = 0, t_imp = 0, t_gpu_steps = 0, t_gpu_steps_imp = 0;
 };
 
@@ -219,12 +232,8 @@ __global__ void gmm_rows_kernel(const float* __restrict__ y, const float* __rest
     }
     gmm_row(wv, dv, mv, o, 3, 8, 3.5f, 65536.f, 1e-6f, s2);
     const size_t pos = ((size_t)tc * H + th) * W + tw;
-    int sym = 0;
-    if (code) {  // NaN and anything outside [0, 8) become the out-of-range marker of the packed row
-        const float cv = code[pos];
-        sym = (cv >= 0.f && cv < 8.f) ? (int)cv : 8;
-    }
-    pack_gmm_row(o, sym, mask[pos] < 0.5f ? 0 : 1, rows + (size_t)row * 8);
+    const int sym = code ? code_symbol(code[pos]) : 0;  // NaN and anything outside [0, 8) become the out-of-range marker of the row
+    pack_gmm_row(o, sym, code_mask_bit(mask[pos]), rows + (size_t)row * 8);
 }
 
 // importance stream: y (1, 49, h, w) logits; one thread = one position in plan order (G = 1: step p = diagonal p)
@@ -255,8 +264,109 @@ __global__ void imp_rows_kernel(const float* __restrict__ y, const float* __rest
         dst[j - 1] = (uint16_t)(v & 0xFFFF);
         ovf[(j - 1) / 16] |= ((v >> 16) & 1u) << ((j - 1) % 16);
     }
-    dst[48] = levels ? (uint16_t)(int)levels[th * W + tw] : 0;
+    dst[48] = levels ? (uint16_t)imp_symbol(levels[th * W + tw]) : 0;
     dst[49] = (uint16_t)ovf[0]; dst[50] = (uint16_t)ovf[1]; dst[51] = (uint16_t)ovf[2];
+}
+
+// ---- rate estimate (lic360_codec_estimate): the ideal code length 16 - log2(T[s+1] - T[s]) bits of every symbol the encoder would
+// code, from the rows the two kernels above build (same row functions, same symbol and mask rules), without packing the rows or
+// running the host coder.  One thread per symbol, in any order.  A symbol's cost goes into its block's partial in a fixed tree order
+// and bits_sum_kernel adds the partials in a fixed order too, so a total depends on the inputs only (no floating-point atomics).
+// The first error in CODING order -- the row the host coder would stop at -- is kept as the smallest key (row << 32) | symbol;
+// symbol >= number of symbols: out of range, else: a zero-width bin.
+constexpr unsigned long long kNoError = ~0ull;
+
+// sum of v over the block in a fixed order (a shuffle tree per warp, then one over the warp sums); valid in thread 0
+__device__ __forceinline__ double block_sum_fixed(double v) {
+    __shared__ double warp_sum[BITS_THREADS / 32];
+#pragma unroll
+    for (int k = 16; k > 0; k >>= 1) v += __shfl_down_sync(0xffffffffu, v, k);
+    if ((threadIdx.x & 31) == 0) warp_sum[threadIdx.x >> 5] = v;
+    __syncthreads();
+    if (threadIdx.x < 32) {
+        v = threadIdx.x < BITS_THREADS / 32 ? warp_sum[threadIdx.x] : 0.0;
+#pragma unroll
+        for (int k = 16; k > 0; k >>= 1) v += __shfl_down_sync(0xffffffffu, v, k);
+    }
+    return v;
+}
+
+// cost of symbol s (0 <= s < N) of a row; false: zero-width bin, which the host coder refuses ("symbol has zero frequency")
+template <int N>
+__device__ __forceinline__ bool symbol_bits(const float* o, int s, double* bits) {
+    uint32_t lo, hi;
+    coded_bins<N>(o, s, &lo, &hi);
+    if (lo == hi) return false;
+    *bits = 16.0 - log2((double)hi - (double)lo);
+    return true;
+}
+
+// code stream: y as in gmm_rows_kernel; thread i = symbol (tc = i / HW, k = i % HW in plan order), bits in (G, H, W) layout
+__global__ void __launch_bounds__(BITS_THREADS) gmm_bits_kernel(const float* __restrict__ y, const float* __restrict__ code,
+                                const float* __restrict__ mask, const int32_t* __restrict__ idx, const StepDesc* __restrict__ steps,
+                                const int* __restrict__ row_off, float* __restrict__ bits, double* __restrict__ partial,
+                                unsigned long long* err, int G, int H, int W, float s2) {
+    const int HW = H * W;
+    const int i = blockIdx.x * blockDim.x + threadIdx.x;
+    double cost = 0.0;
+    if (i < G * HW) {
+        const int k = i % HW, tc = i / HW;
+        const int th = __ldg(idx + k), tw = __ldg(idx + k + HW);
+        const size_t pos = ((size_t)tc * H + th) * W + tw;
+        if (code_mask_bit(mask[pos])) {  // a position the encoder skips costs nothing, whatever its symbol
+            float wv[3], dv[3], mv[3], o[9];
+            const size_t net = (size_t)G * 3 * HW;
+            const size_t base = ((size_t)tc * 3 * H + th) * W + tw;
+#pragma unroll
+            for (int j = 0; j < 3; j++) {
+                wv[j] = y[base + (size_t)j * HW];
+                dv[j] = y[net + base + (size_t)j * HW];
+                mv[j] = y[2 * net + base + (size_t)j * HW];
+            }
+            gmm_row(wv, dv, mv, o, 3, 8, 3.5f, 65536.f, 1e-6f, s2);
+            const int s = code_symbol(code[pos]);
+            if (s > 7 || !symbol_bits<8>(o, s, &cost)) {
+                const int p = th + tw + tc;
+                const unsigned long long row = (unsigned)(__ldg(row_off + p) + k - steps[p].start);
+                atomicMin(err, (row << 32) | (unsigned)s);
+                cost = 0.0;
+            }
+        }
+        bits[pos] = (float)cost;
+    }
+    cost = block_sum_fixed(cost);
+    if (threadIdx.x == 0) partial[blockIdx.x] = cost;
+}
+
+// importance stream: y (1, 49, h, w) logits; thread k = position k of the plan = row k of the stream, bits in (h, w) layout
+__global__ void __launch_bounds__(BITS_THREADS) imp_bits_kernel(const float* __restrict__ y, const float* __restrict__ levels,
+                                const int32_t* __restrict__ idx, float* __restrict__ bits, double* __restrict__ partial,
+                                unsigned long long* err, int H, int W) {
+    const int HW = H * W;
+    const int k = blockIdx.x * blockDim.x + threadIdx.x;
+    double cost = 0.0;
+    if (k < HW) {
+        const int th = __ldg(idx + k), tw = __ldg(idx + k + HW);
+        float o[50];
+        for (int j = 0; j < 49; j++) o[1 + j] = y[((size_t)j * H + th) * W + tw];
+        entropy_row(o, 49, 65536.f);
+        const uint32_t s = imp_symbol(levels[th * W + tw]);
+        if (s >= 49 || !symbol_bits<49>(o, (int)s, &cost)) {
+            atomicMin(err, ((unsigned long long)k << 32) | s);
+            cost = 0.0;
+        }
+        bits[th * W + tw] = (float)cost;
+    }
+    cost = block_sum_fixed(cost);
+    if (threadIdx.x == 0) partial[blockIdx.x] = cost;
+}
+
+// one block: thread t adds partials t, t + BITS_THREADS, ... in index order, then the block's fixed tree
+__global__ void __launch_bounds__(BITS_THREADS) bits_sum_kernel(const double* __restrict__ partial, int n, double* __restrict__ total) {
+    double v = 0.0;
+    for (int i = threadIdx.x; i < n; i += BITS_THREADS) v += partial[i];
+    v = block_sum_fixed(v);
+    if (threadIdx.x == 0) *total = v;
 }
 
 // TileInput of the previous step read from mapped pinned memory (tile_input_cuda.cu:27-43) into both layouts of the
@@ -638,6 +748,8 @@ static int ctx_buffers(NetDesc& n) {
     LIC360_CUDA(cudaHostAlloc(&n.rows_host, (size_t)n.total_rows * n.row_bytes, cudaHostAllocDefault));
     LIC360_CUDA(cudaHostAlloc(&n.rows_step_host, (size_t)n.max_len * n.row_bytes, cudaHostAllocMapped));
     LIC360_CUDA(cudaHostAlloc(&n.syms_host, (size_t)n.max_len * sizeof(float), cudaHostAllocMapped));
+    n.bits_blocks = (n.G * n.H * n.W + BITS_THREADS - 1) / BITS_THREADS;
+    LIC360_CUDA(cudaMalloc(&n.bits_partial_dev, (size_t)n.bits_blocks * sizeof(double)));
     return LIC360_OK;
 }
 
@@ -645,6 +757,7 @@ static void ctx_free(NetDesc& n) {
     cudaFree(n.ctr_dev); cudaFree(n.done_dev); cudaFree(n.arrived_dev); cudaFree(n.sync_dev); cudaFree(n.go_dev); cudaFree(n.old_done_dev); cudaFree(n.scat_done_dev);
     cudaFreeHost(n.flag_host); cudaFreeHost(n.go_host);
     cudaFree(n.rows_dev); cudaFreeHost(n.rows_host); cudaFreeHost(n.rows_step_host); cudaFreeHost(n.syms_host);
+    cudaFree(n.bits_partial_dev);
     if (n.ev_fork) cudaEventDestroy(n.ev_fork);
     if (n.ev_join) cudaEventDestroy(n.ev_join);
     for (int i = 0; i < 6; i++) if (n.ev_prof[i]) cudaEventDestroy(n.ev_prof[i]);
@@ -673,6 +786,9 @@ lic360_codec* lic360_codec_create(int device, int H, int W) {
     if (ok) c->chain_cap = wf_chain_capacity(c->code.wf);
     ok = ok && cudaMalloc(&c->levels_dev, (size_t)(H / 2) * (W / 2) * sizeof(float)) == cudaSuccess;
     ok = ok && cudaMalloc(&c->mask192_dev, (size_t)192 * (H / 2) * (W / 2) * sizeof(float)) == cudaSuccess;
+    ok = ok && cudaMalloc(&c->est_dev, sizeof(EstimateTotals)) == cudaSuccess;
+    ok = ok && cudaHostAlloc(&c->est_host, sizeof(EstimateTotals), cudaHostAllocDefault) == cudaSuccess;
+    ok = ok && cudaEventCreateWithFlags(&c->ev_est, cudaEventDisableTiming) == cudaSuccess;
     if (!ok) {
         if (wf_ok) set_error("codec: allocation failed (%s)", cudaGetErrorString(cudaGetLastError()));  // else: wf_init's message
         lic360_codec_destroy(c);
@@ -688,6 +804,8 @@ void lic360_codec_destroy(lic360_codec* c) {
     wf_free(c->code.wf); wf_free(c->imp.wf);
     ctx_free(c->code); ctx_free(c->imp);
     cudaFree(c->levels_dev); cudaFree(c->mask192_dev);
+    cudaFree(c->est_dev); cudaFreeHost(c->est_host);
+    if (c->ev_est) cudaEventDestroy(c->ev_est);
     delete c;
 }
 
@@ -718,6 +836,23 @@ int lic360_codec_set_layer(lic360_codec* c, int stream_id, int layer, const floa
     return LIC360_OK;
 }
 
+// The network part of an encode, shared with the rate estimate: the input frame of one stream from the caller's tensors and the
+// stream's 12 layers, enqueued on its own CUDA stream; the outputs land in n.frame[12].
+//   importance stream (lic360_demo.py:173-189): Scale(-1, 2/47) of the levels
+//   code stream (lic360_demo.py:124-131): (code - 3.5) * mask, once for each of the three nets
+static int run_encoder_net(lic360_codec* c, bool is_code, const float* code_dev, const float* mask_dev, const float* imp_dev) {
+    NetDesc& n = is_code ? c->code : c->imp;
+    if (is_code) {
+        const int nel = n.G * n.H * n.W;
+        prep_code_kernel<<<stream_grid(nel, 256), 256, 0, n.stream>>>(code_dev, mask_dev, n.frame[0], nel, 3.5f);
+        LAUNCH_CHECK();
+    } else {
+        const int rc = lic360_scale(imp_dev, n.frame[0], n.H * n.W, -1.0f, (float)(2. / (48 - 1.)), n.stream);
+        if (rc) return rc;
+    }
+    return run_ec_net(n, n.stream);
+}
+
 int lic360_codec_encode(lic360_codec* c, const float* code_dev, const float* mask_dev, const float* imp_dev) {
     LIC360_CHECK_ARG(c && code_dev && mask_dev && imp_dev, "bad arguments");
     DeviceGuard guard(c->device);
@@ -729,14 +864,12 @@ int lic360_codec_encode(lic360_codec* c, const float* code_dev, const float* mas
     c->t_host_coder = 0; c->t_gpu_wait = 0; c->t_imp = 0; c->t_gpu_steps = 0; c->t_gpu_steps_imp = 0;
     // The two bitstreams are independent: both networks are enqueued on their own CUDA streams first, then the host
     // codes the (small) importance stream while the code-stream network is still running.
-    // ---- importance stream (lic360_demo.py:173-189): Scale(-1, 2/47) -> net -> rows of all symbols
+    // ---- importance stream: net -> rows of all symbols
     {
         NetDesc& n = c->imp;
         cudaStream_t s = n.stream;
         const int HW = n.H * n.W;
-        rc = lic360_scale(imp_dev, n.frame[0], HW, -1.0f, (float)(2. / (48 - 1.)), s);
-        if (rc) return rc;
-        rc = run_ec_net(n, s);
+        rc = run_encoder_net(c, false, code_dev, mask_dev, imp_dev);
         if (rc) return rc;
         imp_rows_kernel<<<(HW + 127) / 128, 128, 0, s>>>(n.frame[12], imp_dev, n.idx_dev, n.steps_dev, n.ctr_dev, n.rows_dev, n.H, n.W, 1);
         LAUNCH_CHECK();
@@ -749,9 +882,7 @@ int lic360_codec_encode(lic360_codec* c, const float* code_dev, const float* mas
         cudaStream_t s = n.stream;
         const auto tq0 = clk::now();
         const int nel = n.G * n.H * n.W;
-        prep_code_kernel<<<stream_grid(nel, 256), 256, 0, s>>>(code_dev, mask_dev, n.frame[0], nel, 3.5f);
-        LAUNCH_CHECK();
-        rc = run_ec_net(n, s);
+        rc = run_encoder_net(c, true, code_dev, mask_dev, imp_dev);
         if (rc) return rc;
         gmm_rows_kernel<<<(nel + 127) / 128, 128, 0, s>>>(n.frame[12], code_dev, mask_dev, n.idx_dev, n.steps_dev, n.row_off_dev,
                                                           n.ctr_dev, n.rows_dev, n.G, n.H, n.W, 1, (float)(1. / sqrt(2.0)));
@@ -785,6 +916,80 @@ int lic360_codec_encode(lic360_codec* c, const float* code_dev, const float* mas
         c->t_host_coder += ms_since(th);
     }
     c->t_total = ms_since(t0);
+    return LIC360_OK;
+}
+
+// the GPU work of an estimate on the codec's two streams; the code stream ends with the copy of both streams' results
+static int enqueue_estimate(lic360_codec* c, const float* code_dev, const float* mask_dev, const float* imp_dev, float* code_bits_dev,
+                            float* imp_bits_dev) {
+    EstimateTotals* r = c->est_dev;
+    {
+        NetDesc& n = c->imp;
+        cudaStream_t s = n.stream;
+        LIC360_CUDA(cudaMemsetAsync(&r->err[1], 0xFF, sizeof(r->err[1]), s));
+        int rc = run_encoder_net(c, false, code_dev, mask_dev, imp_dev);
+        if (rc) return rc;
+        imp_bits_kernel<<<n.bits_blocks, BITS_THREADS, 0, s>>>(n.frame[12], imp_dev, n.idx_dev, imp_bits_dev, n.bits_partial_dev,
+                                                               &r->err[1], n.H, n.W);
+        LAUNCH_CHECK();
+        bits_sum_kernel<<<1, BITS_THREADS, 0, s>>>(n.bits_partial_dev, n.bits_blocks, &r->bits[1]);
+        LAUNCH_CHECK();
+        LIC360_CUDA(cudaEventRecord(c->ev_est, s));
+    }
+    {
+        NetDesc& n = c->code;
+        cudaStream_t s = n.stream;
+        LIC360_CUDA(cudaMemsetAsync(&r->err[0], 0xFF, sizeof(r->err[0]), s));
+        int rc = run_encoder_net(c, true, code_dev, mask_dev, imp_dev);
+        if (rc) return rc;
+        gmm_bits_kernel<<<n.bits_blocks, BITS_THREADS, 0, s>>>(n.frame[12], code_dev, mask_dev, n.idx_dev, n.steps_dev, n.row_off_dev,
+                                                               code_bits_dev, n.bits_partial_dev, &r->err[0], n.G, n.H, n.W,
+                                                               (float)(1. / sqrt(2.0)));
+        LAUNCH_CHECK();
+        bits_sum_kernel<<<1, BITS_THREADS, 0, s>>>(n.bits_partial_dev, n.bits_blocks, &r->bits[0]);
+        LAUNCH_CHECK();
+        LIC360_CUDA(cudaStreamWaitEvent(s, c->ev_est, 0));
+        LIC360_CUDA(cudaMemcpyAsync(c->est_host, r, sizeof(EstimateTotals), cudaMemcpyDeviceToHost, s));
+    }
+    return LIC360_OK;
+}
+
+int lic360_codec_estimate(lic360_codec* c, const float* code_dev, const float* mask_dev, const float* imp_dev, float* code_bits_dev,
+                          float* imp_bits_dev, double* bits_host) {
+    LIC360_CHECK_ARG(c && code_dev && mask_dev && imp_dev && code_bits_dev && imp_bits_dev && bits_host, "bad arguments");
+    DeviceGuard guard(c->device);
+    LIC360_CUDA(guard.err);
+    int rc = check_params(c->code);
+    if (rc == LIC360_OK) rc = check_params(c->imp);
+    if (rc) return rc;
+    const auto t0 = clk::now();
+    c->t_host_coder = 0; c->t_gpu_wait = 0; c->t_imp = 0; c->t_gpu_steps = 0; c->t_gpu_steps_imp = 0;
+    rc = enqueue_estimate(c, code_dev, mask_dev, imp_dev, code_bits_dev, imp_bits_dev);
+    // both streams are drained on every path: the caller may reuse the inputs and the maps as soon as the call returns
+    const auto tw = clk::now();
+    const cudaError_t e_imp = cudaStreamSynchronize(c->imp.stream);
+    const cudaError_t e_code = cudaStreamSynchronize(c->code.stream);
+    c->t_gpu_wait = ms_since(tw);
+    c->t_total = ms_since(t0);
+    if (rc) return rc;
+    LIC360_CUDA(e_imp);
+    LIC360_CUDA(e_code);
+    // the errors encode reports, with its messages: the importance stream is coded (and checked) first
+    const EstimateTotals& r = *c->est_host;
+    if (r.err[1] != kNoError) {
+        const unsigned s = (unsigned)r.err[1];
+        if (s >= 49) set_error("coder: importance level %u out of range", s);
+        else set_error("coder: symbol has zero frequency");
+        return LIC360_ERR_CODER;
+    }
+    if (r.err[0] != kNoError) {
+        const int row = (int)(r.err[0] >> 32);
+        if ((unsigned)r.err[0] > 7) set_error("coder: symbol out of range in packed row %d", row);
+        else set_error("coder: symbol has zero frequency (row %d)", row);
+        return LIC360_ERR_CODER;
+    }
+    bits_host[0] = r.bits[0];
+    bits_host[1] = r.bits[1];
     return LIC360_OK;
 }
 

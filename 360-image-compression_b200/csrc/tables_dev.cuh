@@ -134,6 +134,31 @@ __device__ __forceinline__ void entropy_row49_warp(float v0, float v1, float* o,
     __syncwarp();
 }
 
+// The symbol and mask rules of the encoder, shared by the kernels that pack rows for the host coder and the ones that cost the
+// symbols without it (codec.cu), so the two cannot disagree on a fractional, negative or NaN input.
+// code stream: 0..7, anything else (NaN included) is the out-of-range marker 8
+__device__ __forceinline__ int code_symbol(float cv) { return (cv >= 0.f && cv < 8.f) ? (int)cv : 8; }
+// code stream: a position is coded unless its mask is below 0.5 (NaN is coded)
+__device__ __forceinline__ int code_mask_bit(float m) { return m < 0.5f ? 0 : 1; }
+// importance stream: the level as the packed row stores it (u16); 49 or more is out of range
+__device__ __forceinline__ uint32_t imp_symbol(float level) { return (uint16_t)(int)level; }
+
+// bins T[s], T[s+1] (0 <= s < N) of a row of N symbols as the host coder reads them back from the packed row: T[0] = 0 and
+// T[N] = 65536 are implied, the interior bins are the low 17 bits of (int)o[j] (16-bit word + overflow bit, pack_gmm_row /
+// imp_rows_kernel).  Selected in an unrolled loop, so a row held in registers is not indexed dynamically.
+template <int N>
+__device__ __forceinline__ void coded_bins(const float* o, int s, uint32_t* lo, uint32_t* hi) {
+    uint32_t a = 0u, b = 65536u;
+#pragma unroll
+    for (int j = 1; j < N; j++) {
+        const uint32_t v = (uint32_t)(int)o[j] & 0x1FFFFu;
+        if (j == s) a = v;
+        if (j == s + 1) b = v;
+    }
+    *lo = a;
+    *hi = b;
+}
+
 // packed code-stream row (coder_internal.h): 7 x u16 low words of T[1..7] + meta = sym | bad << 3 | mask << 8 | overflow bits << 9
 // bad: the symbol is outside 0..7 (sym >= 8 or negative); the host encoder reports it like the per-op path does ("symbol out
 // of range") instead of coding a wrapped, decodable but wrong symbol

@@ -79,6 +79,7 @@ SIGNATURES = {
     "lic360_codec_destroy": (None, [_P]),
     "lic360_codec_set_layer": (_I, [_P, _I, _I, _P, _P, _P]),
     "lic360_codec_encode": (_I, [_P, _P, _P, _P]),
+    "lic360_codec_estimate": (_I, [_P, _P, _P, _P, _P, _P, _P]),
     "lic360_codec_stream_size": (_L, [_P, _I]),
     "lic360_codec_stream_copy": (_L, [_P, _I, _P, _L]),
     "lic360_codec_decode": (_I, [_P, _P, _L, _P, _L, _P, _P]),

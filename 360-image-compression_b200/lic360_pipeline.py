@@ -137,6 +137,27 @@ class FusedCodec(object):
         check(LIB.lic360_codec_encode(self._h, code.data_ptr(), mask.data_ptr(), imp.data_ptr()))
         return self._stream_bytes(1), self._stream_bytes(0)
 
+    def estimate(self, code, mask, imap_quant):
+        """The rate of the latent `encode` would code, without the arithmetic coder: the same networks and integer CDF rows, and for
+        every coded symbol its ideal code length 16 - log2(T[s+1] - T[s]) bits (include/lic360_b200.h, lic360_codec_estimate).
+
+        Returns {'code_bits': float, 'imp_bits': float, 'code_map': (1,48,H,W), 'imp_map': (1,1,H/2,W/2)}: the totals of the code and
+        importance streams and the bits of every symbol as float32 tensors on the codec's device (0 where mask < 0.5).  The image
+        is 8H x 8W pixels, so its rate is (code_bits + imp_bits) / (64 H W) bits per pixel.  For each stream, with N coded symbols
+        and I its total, the bytes `encode` writes satisfy -(1 + u + N/8192) <= 8 * len(stream) - I <= 8 + N/8192, where u is the
+        number of pending underflow bits the coder drops at the end (a few at most in practice; derivation in
+        tests/test_rate_estimate.py).  Raises RuntimeError on the inputs `encode` refuses, with the same message."""
+        code = self._f32(code, (1, 48, self.H, self.W))
+        mask = self._f32(mask, (1, 48, self.H, self.W))
+        imp = self._f32(imap_quant, (1, 1, self.H // 2, self.W // 2))
+        code_map = torch.empty((1, 48, self.H, self.W), dtype=torch.float32, device=self.dev)
+        imp_map = torch.empty((1, 1, self.H // 2, self.W // 2), dtype=torch.float32, device=self.dev)
+        totals = (ctypes.c_double * 2)()
+        torch.cuda.current_stream(self.dev).synchronize()  # inputs were produced on torch's stream
+        check(LIB.lic360_codec_estimate(self._h, code.data_ptr(), mask.data_ptr(), imp.data_ptr(), code_map.data_ptr(),
+                                        imp_map.data_ptr(), totals))
+        return {'code_bits': totals[0], 'imp_bits': totals[1], 'code_map': code_map, 'imp_map': imp_map}
+
     def decode(self, imp_bytes, code_bytes, h=None, w=None, name=None):
         code = torch.empty((1, 48, self.H, self.W), dtype=torch.float32, device=self.dev)
         mask = torch.empty((1, 48, self.H, self.W), dtype=torch.float32, device=self.dev)

@@ -220,13 +220,25 @@ int lic360_codec_set_layer(lic360_codec* c, int stream_id, int layer, const floa
                            const float* slope_dev);
 /* code_dev (1,48,H,W) symbols 0..7, mask_dev (1,48,H,W) 0/1, imp_dev (1,1,H/2,W/2) importance levels 0..48 */
 int lic360_codec_encode(lic360_codec* c, const float* code_dev, const float* mask_dev, const float* imp_dev);
+/* Exact-table rate of one latent without arithmetic coding: runs the same two networks as lic360_codec_encode and, for
+ * every symbol the encoder would code, its ideal code length 16 - log2(T[s+1] - T[s]) bits from the same integer CDF row.
+ *   code_bits_dev (1,48,H,W) float32: bits of each code symbol; exactly 0 where mask < 0.5 (not coded)
+ *   imp_bits_dev  (1,1,H/2,W/2) float32: bits of each importance level
+ *   bits_host[0] = code stream total, bits_host[1] = importance stream total (stream_id order), summed in double in a fixed
+ *   order (the same inputs give the same totals on every call and every codec)
+ * Rejects exactly the inputs lic360_codec_encode rejects, with the same status and message.  A stream of N coded symbols and
+ * I = its total is len bytes long with -(1 + u + N/8192) <= 8*len - I <= 8 + N/8192, u = the coder's pending underflow bits at
+ * the end, which the terminator makes unnecessary (a few at most in practice; derivation in tests/test_rate_estimate.py). */
+int lic360_codec_estimate(lic360_codec* c, const float* code_dev, const float* mask_dev, const float* imp_dev,
+                          float* code_bits_dev, float* imp_bits_dev, double* bits_host);
 long lic360_codec_stream_size(lic360_codec* c, int stream_id);
 long lic360_codec_stream_copy(lic360_codec* c, int stream_id, uint8_t* out, long cap);
 /* -> code_out_dev (1,48,H,W) = symbols where mask == 1, else 0 (lic360_demo.py:236-237); mask_out_dev (1,48,H,W) */
 int lic360_codec_decode(lic360_codec* c, const uint8_t* imp_bytes, long n_imp, const uint8_t* code_bytes, long n_code,
                         float* code_out_dev, float* mask_out_dev);
-/* milliseconds of the last encode/decode call: [0] total, [1] host arithmetic coder, [2] waiting for the GPU,
- * [3] importance stream part of a decode, [4] CUDA-event time of all decode graph replays, [5] of the importance stream ones */
+/* milliseconds of the last encode/decode/estimate call: [0] total, [1] host arithmetic coder, [2] waiting for the GPU,
+ * [3] importance stream part of a decode, [4] CUDA-event time of all decode graph replays, [5] of the importance stream ones
+ * (an estimate fills [0] and [2] only) */
 int lic360_codec_last_timing(lic360_codec* c, double* out, int n);
 /* mode 0 (default): pipelined graph replay per wavefront step.  mode 1: the same kernels launched one by one on the codec
  * stream with CUDA events between them (the decode is serialized and slower; used by bench.py for the roofline block).
