@@ -42,8 +42,8 @@ struct NetDesc {
     bool act[12];
     float* wp[12] = {nullptr}; float* wq[12] = {nullptr}; float* bias[12] = {nullptr}; float* slope[12] = {nullptr};
     bool set[12] = {false};
-    float* frame[13] = {nullptr};  // frame[0] = network input, frame[i+1] = output of layer i (persistent in decode)
-    size_t frame_floats[13];
+    float* frame[13] = {nullptr};  // encoder: frame[0] = network input, frame[i+1] = output of layer i, for lic360_codec::batch_cap latents
+    size_t frame_floats[13];       // floats of one latent
     int32_t* idx_dev = nullptr;
     std::vector<int32_t> plan;
     std::vector<StepDesc> steps;
@@ -78,17 +78,31 @@ struct NetDesc {
     double t_host_coder = 0, t_gpu_wait = 0, t_done = 0;
     lic360_coder* coder = nullptr;
     char err[256] = {0};                // error text of a worker thread (set_error is thread-local)
-    double* bits_partial_dev = nullptr; // estimate: one partial sum per block of the bits kernel
-    int bits_blocks = 0;
+    double* bits_partial_dev = nullptr; // estimate: one partial sum per block of the bits kernel and latent
+    int* count_partial_dev = nullptr;   // estimate: coded symbols per block of the bits kernel and latent
+    int bits_blocks = 0;                // blocks of the bits kernel per latent
 };
 
 constexpr int BITS_THREADS = 256;  // block size of the estimate's bits and sum kernels
 
-// device-side results of an estimate, copied back with one cudaMemcpyAsync; index = stream_id (0 code, 1 importance)
+// device-side results of an estimate of K latents, copied back with one cudaMemcpyAsync: the totals, the first-error keys and the
+// coded-symbol counts, each indexed [stream_id * K + k] (stream_id 0 code, 1 importance)
 struct EstimateTotals {
-    double bits[2];
-    unsigned long long err[2];
+    double* bits;
+    unsigned long long* err;
+    long long* count;
 };
+inline size_t estimate_bytes(int K) { return (size_t)2 * K * (sizeof(double) + sizeof(unsigned long long) + sizeof(long long)); }
+inline EstimateTotals estimate_totals(void* base, int K) {
+    EstimateTotals r;
+    r.bits = static_cast<double*>(base);
+    r.err = reinterpret_cast<unsigned long long*>(r.bits + 2 * K);
+    r.count = reinterpret_cast<long long*>(r.err + 2 * K);
+    return r;
+}
+// a batch of K latents runs the code network with 3K images (grid.z of the conv kernels, at most 65535) and indexes its input frame
+// with int
+constexpr int kMaxBatch = 65535 / 3;
 
 }  // namespace lic360
 
@@ -173,8 +187,9 @@ struct lic360_codec {
     float* mask192_dev = nullptr;       // scratch: Imp2mask output
     std::atomic<int> imp_ready{0};      // decode: importance levels of diagonals < imp_ready are in levels_dev
     std::atomic<int> abort_flag{0};     // decode: one of the two stream loops failed
-    lic360::EstimateTotals* est_dev = nullptr;   // estimate: totals and error keys of both streams
-    lic360::EstimateTotals* est_host = nullptr;  // pinned copy of est_dev
+    int batch_cap = 0;                  // latents the encoder frames, the bits partials and est_dev / est_host hold (grown on demand)
+    void* est_dev = nullptr;            // estimate: totals, error keys and counts of both streams (EstimateTotals layout)
+    void* est_host = nullptr;           // pinned copy of est_dev
     cudaEvent_t ev_est = nullptr;                // estimate: the importance stream's results are in est_dev
     double t_host_coder = 0, t_total = 0, t_gpu_wait = 0, t_imp = 0, t_gpu_steps = 0, t_gpu_steps_imp = 0;
 };
@@ -188,7 +203,8 @@ static void codec_trace_set(unsigned long long* buf, int sel) {
 }
 
 // ------------------------------------------------------------------------------------------------ kernels
-// code stream encoder input: x = (code - 3.5) * mask replicated for the 3 nets (lic360_demo.py:130-131)
+// code stream encoder input: x = (code - 3.5) * mask replicated for the 3 nets (lic360_demo.py:130-131).  n = K latents x (48, H, W):
+// x is set-major, [net][k][48][H][W], the layout the conv kernels read with N = 3K images and 3 weight sets (image / K = set)
 __global__ void prep_code_kernel(const float* __restrict__ code, const float* __restrict__ mask, float* __restrict__ x,
                                  int n, float bias) {
     for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x) {
@@ -301,21 +317,30 @@ __device__ __forceinline__ bool symbol_bits(const float* o, int s, double* bits)
     return true;
 }
 
-// code stream: y as in gmm_rows_kernel; thread i = symbol (tc = i / HW, k = i % HW in plan order), bits in (G, H, W) layout
+// A batch: latent blockIdx.y of gridDim.y, each with the block partition, the partials and the error key of a single latent, so its
+// totals and map do not depend on the other latents.
+// code stream: y as in gmm_rows_kernel, [net][latent][G*3][H][W]; thread i = symbol (tc = i / HW, k = i % HW in plan order), bits
+// (optional) in (G, H, W) layout per latent; count: coded symbols (mask >= 0.5) per block
 __global__ void __launch_bounds__(BITS_THREADS) gmm_bits_kernel(const float* __restrict__ y, const float* __restrict__ code,
                                 const float* __restrict__ mask, const int32_t* __restrict__ idx, const StepDesc* __restrict__ steps,
                                 const int* __restrict__ row_off, float* __restrict__ bits, double* __restrict__ partial,
-                                unsigned long long* err, int G, int H, int W, float s2) {
+                                int* __restrict__ count, unsigned long long* err, int G, int H, int W, float s2) {
     const int HW = H * W;
+    const size_t lat = blockIdx.y, plane = (size_t)G * HW;  // one latent's symbols
+    y += lat * 3 * plane; code += lat * plane; mask += lat * plane; err += lat;
+    if (bits) bits += lat * plane;
+    partial += lat * gridDim.x; count += lat * gridDim.x;
     const int i = blockIdx.x * blockDim.x + threadIdx.x;
     double cost = 0.0;
+    int coded = 0;
     if (i < G * HW) {
         const int k = i % HW, tc = i / HW;
         const int th = __ldg(idx + k), tw = __ldg(idx + k + HW);
         const size_t pos = ((size_t)tc * H + th) * W + tw;
-        if (code_mask_bit(mask[pos])) {  // a position the encoder skips costs nothing, whatever its symbol
+        coded = code_mask_bit(mask[pos]);
+        if (coded) {  // a position the encoder skips costs nothing, whatever its symbol
             float wv[3], dv[3], mv[3], o[9];
-            const size_t net = (size_t)G * 3 * HW;
+            const size_t net = gridDim.y * 3 * plane;
             const size_t base = ((size_t)tc * 3 * H + th) * W + tw;
 #pragma unroll
             for (int j = 0; j < 3; j++) {
@@ -332,17 +357,23 @@ __global__ void __launch_bounds__(BITS_THREADS) gmm_bits_kernel(const float* __r
                 cost = 0.0;
             }
         }
-        bits[pos] = (float)cost;
+        if (bits) bits[pos] = (float)cost;
     }
+    coded = __syncthreads_count(coded);
     cost = block_sum_fixed(cost);
-    if (threadIdx.x == 0) partial[blockIdx.x] = cost;
+    if (threadIdx.x == 0) { partial[blockIdx.x] = cost; count[blockIdx.x] = coded; }
 }
 
-// importance stream: y (1, 49, h, w) logits; thread k = position k of the plan = row k of the stream, bits in (h, w) layout
+// importance stream: y (K, 49, h, w) logits; thread k = position k of the plan = row k of the stream, bits (optional) in (h, w) layout
+// per latent; every position is coded
 __global__ void __launch_bounds__(BITS_THREADS) imp_bits_kernel(const float* __restrict__ y, const float* __restrict__ levels,
                                 const int32_t* __restrict__ idx, float* __restrict__ bits, double* __restrict__ partial,
-                                unsigned long long* err, int H, int W) {
+                                int* __restrict__ count, unsigned long long* err, int H, int W) {
     const int HW = H * W;
+    const size_t lat = blockIdx.y;
+    y += lat * 49 * HW; levels += lat * HW; err += lat;
+    if (bits) bits += lat * HW;
+    partial += lat * gridDim.x; count += lat * gridDim.x;
     const int k = blockIdx.x * blockDim.x + threadIdx.x;
     double cost = 0.0;
     if (k < HW) {
@@ -355,18 +386,44 @@ __global__ void __launch_bounds__(BITS_THREADS) imp_bits_kernel(const float* __r
             atomicMin(err, ((unsigned long long)k << 32) | s);
             cost = 0.0;
         }
-        bits[th * W + tw] = (float)cost;
+        if (bits) bits[th * W + tw] = (float)cost;
     }
+    const int coded = __syncthreads_count(k < HW);
     cost = block_sum_fixed(cost);
-    if (threadIdx.x == 0) partial[blockIdx.x] = cost;
+    if (threadIdx.x == 0) { partial[blockIdx.x] = cost; count[blockIdx.x] = coded; }
 }
 
-// one block: thread t adds partials t, t + BITS_THREADS, ... in index order, then the block's fixed tree
-__global__ void __launch_bounds__(BITS_THREADS) bits_sum_kernel(const double* __restrict__ partial, int n, double* __restrict__ total) {
+// block b = latent b: thread t adds the latent's n partials t, t + BITS_THREADS, ... in index order, then the block's fixed tree; the
+// counts are integers, added in any order
+__global__ void __launch_bounds__(BITS_THREADS) bits_sum_kernel(const double* __restrict__ partial, const int* __restrict__ count, int n,
+                                                                double* __restrict__ total, long long* __restrict__ total_count) {
+    __shared__ unsigned long long coded;
+    partial += (size_t)blockIdx.x * n; count += (size_t)blockIdx.x * n;
+    if (threadIdx.x == 0) coded = 0;
     double v = 0.0;
-    for (int i = threadIdx.x; i < n; i += BITS_THREADS) v += partial[i];
-    v = block_sum_fixed(v);
-    if (threadIdx.x == 0) *total = v;
+    long long m = 0;
+    for (int i = threadIdx.x; i < n; i += BITS_THREADS) { v += partial[i]; m += count[i]; }
+    v = block_sum_fixed(v);  // its barrier orders the reset of `coded` before the adds
+    atomicAdd(&coded, (unsigned long long)m);
+    __syncthreads();
+    if (threadIdx.x == 0) { total[blockIdx.x] = v; total_count[blockIdx.x] = (long long)coded; }
+}
+
+// candidate j (blockIdx.y) of lic360_imp_levels_to_mask: level max(s - off, 0) of every cell, s = imp_symbol(level) the symbol encode
+// codes, and the (48, 2h, 2w) code mask the decoder derives from it (Imp2mask + Dtow)
+struct LevelOffsets { int k[32]; };
+__global__ void imp_levels_to_mask_kernel(const float* __restrict__ levels, int h, int w, LevelOffsets off, float* __restrict__ levels_out,
+                                          float* __restrict__ mask_out) {
+    const int j = blockIdx.y, k = off.k[j], hw = h * w, W = 2 * w, n = 48 * 4 * hw;
+    levels_out += (size_t)j * hw;
+    mask_out += (size_t)j * n;
+    for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x) {
+        const int tw = i % W, th = (i / W) % (2 * h), tc = i / (W * 2 * h);
+        const int cell = (th >> 1) * w + (tw >> 1);
+        const int lvl = max((int)imp_symbol(levels[cell]) - k, 0);
+        mask_out[i] = (float)code_mask_from_level(lvl, tc, th, tw);
+        if (i < hw) levels_out[i] = (float)max((int)imp_symbol(levels[i]) - k, 0);
+    }
 }
 
 // TileInput of the previous step read from mapped pinned memory (tile_input_cuda.cu:27-43) into both layouts of the
@@ -466,7 +523,7 @@ __global__ void gmm_rows_wf_kernel(const float* __restrict__ y, const float* __r
     if (live && j == 0) {
         fixup_row(o, 8, true);
         const int lvl = (int)(levels[(th >> 1) * (W >> 1) + (tw >> 1)] + 1e-5f);
-        pack_gmm_row(o, 0, (4 * tc + 2 * (th & 1) + (tw & 1)) < 4 * lvl ? 1 : 0, rows + (size_t)l * 8);
+        pack_gmm_row(o, 0, code_mask_from_level(lvl, tc, th, tw), rows + (size_t)l * 8);
     }
     rows_done(done, flag, step, G);
 }
@@ -508,7 +565,6 @@ static void net_init(NetDesc& n, int G, int cpg, int nlast, int nsets, int H, in
 }
 
 static int net_alloc(NetDesc& n) {
-    for (int i = 0; i < 13; i++) LIC360_CUDA(cudaMalloc(&n.frame[i], n.frame_floats[i] * sizeof(float)));
     const int H = n.H, W = n.W, G = n.G;
     std::vector<int32_t> idx(2 * (size_t)H * W);
     n.plan.resize(H + W);
@@ -550,11 +606,12 @@ static void layer_io(const NetDesc& n, int l, const float** x, const float** res
     *resid = (l >= 2 && l <= 10 && (l % 2) == 0) ? n.frame[l - 1] : nullptr;  // conv2 of block b = layer 2b+2
 }
 
-static int conv_args(const NetDesc& n, int l, ConvArgs& a) {
+// K latents: N = nsets * K images, set-major (image / K = weight set)
+static int conv_args(const NetDesc& n, int l, int K, ConvArgs& a) {
     const float *x, *r;
     float* out;
     layer_io(n, l, &x, &r, &out);
-    if (fill_conv_args(a, x, n.wp[l], n.wq[l], n.bias[l], n.act[l] ? n.slope[l] : nullptr, r, out, n.nsets, n.Cin[l], n.H, n.W,
+    if (fill_conv_args(a, x, n.wp[l], n.wq[l], n.bias[l], n.act[l] ? n.slope[l] : nullptr, r, out, n.nsets * K, n.Cin[l], n.H, n.W,
                        n.Cout[l], n.G, n.constrain[l], n.nsets)) {
         set_error("codec: bad layer geometry");
         return LIC360_ERR_ARG;
@@ -562,10 +619,10 @@ static int conv_args(const NetDesc& n, int l, ConvArgs& a) {
     return LIC360_OK;
 }
 
-static int run_ec_net(const NetDesc& n, cudaStream_t s) {
+static int run_ec_net(const NetDesc& n, int K, cudaStream_t s) {
     for (int l = 0; l < 12; l++) {
         ConvArgs a;
-        int rc = conv_args(n, l, a);
+        int rc = conv_args(n, l, K, a);
         if (rc) return rc;
         LIC360_CUDA(launch_cconv_ec(a, s, false));  // the canonical P pass: the decoder reproduces these outputs bit for bit
     }
@@ -749,7 +806,40 @@ static int ctx_buffers(NetDesc& n) {
     LIC360_CUDA(cudaHostAlloc(&n.rows_step_host, (size_t)n.max_len * n.row_bytes, cudaHostAllocMapped));
     LIC360_CUDA(cudaHostAlloc(&n.syms_host, (size_t)n.max_len * sizeof(float), cudaHostAllocMapped));
     n.bits_blocks = (n.G * n.H * n.W + BITS_THREADS - 1) / BITS_THREADS;
-    LIC360_CUDA(cudaMalloc(&n.bits_partial_dev, (size_t)n.bits_blocks * sizeof(double)));
+    return LIC360_OK;
+}
+
+// The buffers that scale with the number of latents an encode (1) or an estimate (K) runs at once: both networks' encoder frames, the
+// bits kernels' partials and the estimate's results.  They only grow; the old ones are kept unless every new one was allocated.
+static int batch_reserve(lic360_codec* c, int K) {
+    if (K <= c->batch_cap) return LIC360_OK;
+    struct Buf { void** slot; size_t bytes; bool pinned; };
+    std::vector<Buf> bufs;
+    for (NetDesc* n : {&c->code, &c->imp}) {
+        for (int i = 0; i < 13; i++) bufs.push_back({reinterpret_cast<void**>(&n->frame[i]), n->frame_floats[i] * K * sizeof(float), false});
+        bufs.push_back({reinterpret_cast<void**>(&n->bits_partial_dev), (size_t)n->bits_blocks * K * sizeof(double), false});
+        bufs.push_back({reinterpret_cast<void**>(&n->count_partial_dev), (size_t)n->bits_blocks * K * sizeof(int), false});
+    }
+    bufs.push_back({&c->est_dev, estimate_bytes(K), false});
+    bufs.push_back({&c->est_host, estimate_bytes(K), true});
+    // the old buffers may still be in use by work enqueued on the codec's streams
+    LIC360_CUDA(cudaStreamSynchronize(c->code.stream));
+    LIC360_CUDA(cudaStreamSynchronize(c->imp.stream));
+    std::vector<void*> fresh(bufs.size(), nullptr);
+    cudaError_t e = cudaSuccess;
+    for (size_t i = 0; i < bufs.size() && e == cudaSuccess; i++)
+        e = bufs[i].pinned ? cudaHostAlloc(&fresh[i], bufs[i].bytes, cudaHostAllocDefault) : cudaMalloc(&fresh[i], bufs[i].bytes);
+    for (size_t i = 0; i < bufs.size(); i++) {
+        void* old = e == cudaSuccess ? *bufs[i].slot : fresh[i];
+        if (bufs[i].pinned) cudaFreeHost(old); else cudaFree(old);
+        if (e == cudaSuccess) *bufs[i].slot = fresh[i];
+    }
+    if (e != cudaSuccess) {
+        cudaGetLastError();
+        set_error("codec: cannot allocate the buffers of %d latents (%s)", K, cudaGetErrorString(e));
+        return LIC360_ERR_CUDA;
+    }
+    c->batch_cap = K;
     return LIC360_OK;
 }
 
@@ -757,7 +847,7 @@ static void ctx_free(NetDesc& n) {
     cudaFree(n.ctr_dev); cudaFree(n.done_dev); cudaFree(n.arrived_dev); cudaFree(n.sync_dev); cudaFree(n.go_dev); cudaFree(n.old_done_dev); cudaFree(n.scat_done_dev);
     cudaFreeHost(n.flag_host); cudaFreeHost(n.go_host);
     cudaFree(n.rows_dev); cudaFreeHost(n.rows_host); cudaFreeHost(n.rows_step_host); cudaFreeHost(n.syms_host);
-    cudaFree(n.bits_partial_dev);
+    cudaFree(n.bits_partial_dev); cudaFree(n.count_partial_dev);
     if (n.ev_fork) cudaEventDestroy(n.ev_fork);
     if (n.ev_join) cudaEventDestroy(n.ev_join);
     for (int i = 0; i < 6; i++) if (n.ev_prof[i]) cudaEventDestroy(n.ev_prof[i]);
@@ -786,11 +876,10 @@ lic360_codec* lic360_codec_create(int device, int H, int W) {
     if (ok) c->chain_cap = wf_chain_capacity(c->code.wf);
     ok = ok && cudaMalloc(&c->levels_dev, (size_t)(H / 2) * (W / 2) * sizeof(float)) == cudaSuccess;
     ok = ok && cudaMalloc(&c->mask192_dev, (size_t)192 * (H / 2) * (W / 2) * sizeof(float)) == cudaSuccess;
-    ok = ok && cudaMalloc(&c->est_dev, sizeof(EstimateTotals)) == cudaSuccess;
-    ok = ok && cudaHostAlloc(&c->est_host, sizeof(EstimateTotals), cudaHostAllocDefault) == cudaSuccess;
     ok = ok && cudaEventCreateWithFlags(&c->ev_est, cudaEventDisableTiming) == cudaSuccess;
+    if (!ok && wf_ok) set_error("codec: allocation failed (%s)", cudaGetErrorString(cudaGetLastError()));  // else: wf_init's message
+    ok = ok && batch_reserve(c, 1) == LIC360_OK;  // (its own message)
     if (!ok) {
-        if (wf_ok) set_error("codec: allocation failed (%s)", cudaGetErrorString(cudaGetLastError()));  // else: wf_init's message
         lic360_codec_destroy(c);
         return nullptr;
     }
@@ -837,20 +926,22 @@ int lic360_codec_set_layer(lic360_codec* c, int stream_id, int layer, const floa
 }
 
 // The network part of an encode, shared with the rate estimate: the input frame of one stream from the caller's tensors and the
-// stream's 12 layers, enqueued on its own CUDA stream; the outputs land in n.frame[12].
+// stream's 12 layers, enqueued on its own CUDA stream; the outputs land in n.frame[12].  K latents (K <= c->batch_cap) run as one
+// batch of the same kernels: each latent's outputs are those of a run of that latent alone (the conv kernels compute every image
+// alike, whatever else is in the batch).
 //   importance stream (lic360_demo.py:173-189): Scale(-1, 2/47) of the levels
 //   code stream (lic360_demo.py:124-131): (code - 3.5) * mask, once for each of the three nets
-static int run_encoder_net(lic360_codec* c, bool is_code, const float* code_dev, const float* mask_dev, const float* imp_dev) {
+static int run_encoder_net(lic360_codec* c, bool is_code, int K, const float* code_dev, const float* mask_dev, const float* imp_dev) {
     NetDesc& n = is_code ? c->code : c->imp;
     if (is_code) {
-        const int nel = n.G * n.H * n.W;
+        const int nel = K * n.G * n.H * n.W;
         prep_code_kernel<<<stream_grid(nel, 256), 256, 0, n.stream>>>(code_dev, mask_dev, n.frame[0], nel, 3.5f);
         LAUNCH_CHECK();
     } else {
-        const int rc = lic360_scale(imp_dev, n.frame[0], n.H * n.W, -1.0f, (float)(2. / (48 - 1.)), n.stream);
+        const int rc = lic360_scale(imp_dev, n.frame[0], (size_t)K * n.H * n.W, -1.0f, (float)(2. / (48 - 1.)), n.stream);
         if (rc) return rc;
     }
-    return run_ec_net(n, n.stream);
+    return run_ec_net(n, K, n.stream);
 }
 
 int lic360_codec_encode(lic360_codec* c, const float* code_dev, const float* mask_dev, const float* imp_dev) {
@@ -869,7 +960,7 @@ int lic360_codec_encode(lic360_codec* c, const float* code_dev, const float* mas
         NetDesc& n = c->imp;
         cudaStream_t s = n.stream;
         const int HW = n.H * n.W;
-        rc = run_encoder_net(c, false, code_dev, mask_dev, imp_dev);
+        rc = run_encoder_net(c, false, 1, code_dev, mask_dev, imp_dev);
         if (rc) return rc;
         imp_rows_kernel<<<(HW + 127) / 128, 128, 0, s>>>(n.frame[12], imp_dev, n.idx_dev, n.steps_dev, n.ctr_dev, n.rows_dev, n.H, n.W, 1);
         LAUNCH_CHECK();
@@ -882,7 +973,7 @@ int lic360_codec_encode(lic360_codec* c, const float* code_dev, const float* mas
         cudaStream_t s = n.stream;
         const auto tq0 = clk::now();
         const int nel = n.G * n.H * n.W;
-        rc = run_encoder_net(c, true, code_dev, mask_dev, imp_dev);
+        rc = run_encoder_net(c, true, 1, code_dev, mask_dev, imp_dev);
         if (rc) return rc;
         gmm_rows_kernel<<<(nel + 127) / 128, 128, 0, s>>>(n.frame[12], code_dev, mask_dev, n.idx_dev, n.steps_dev, n.row_off_dev,
                                                           n.ctr_dev, n.rows_dev, n.G, n.H, n.W, 1, (float)(1. / sqrt(2.0)));
@@ -919,52 +1010,53 @@ int lic360_codec_encode(lic360_codec* c, const float* code_dev, const float* mas
     return LIC360_OK;
 }
 
-// the GPU work of an estimate on the codec's two streams; the code stream ends with the copy of both streams' results
-static int enqueue_estimate(lic360_codec* c, const float* code_dev, const float* mask_dev, const float* imp_dev, float* code_bits_dev,
-                            float* imp_bits_dev) {
-    EstimateTotals* r = c->est_dev;
+// the GPU work of an estimate of K latents on the codec's two streams; the code stream ends with the copy of both streams' results
+static int enqueue_estimate(lic360_codec* c, int K, const float* code_dev, const float* mask_dev, const float* imp_dev,
+                            float* code_bits_dev, float* imp_bits_dev) {
+    const EstimateTotals r = estimate_totals(c->est_dev, K);
     {
         NetDesc& n = c->imp;
         cudaStream_t s = n.stream;
-        LIC360_CUDA(cudaMemsetAsync(&r->err[1], 0xFF, sizeof(r->err[1]), s));
-        int rc = run_encoder_net(c, false, code_dev, mask_dev, imp_dev);
+        LIC360_CUDA(cudaMemsetAsync(r.err + K, 0xFF, K * sizeof(*r.err), s));
+        int rc = run_encoder_net(c, false, K, code_dev, mask_dev, imp_dev);
         if (rc) return rc;
-        imp_bits_kernel<<<n.bits_blocks, BITS_THREADS, 0, s>>>(n.frame[12], imp_dev, n.idx_dev, imp_bits_dev, n.bits_partial_dev,
-                                                               &r->err[1], n.H, n.W);
+        imp_bits_kernel<<<dim3(n.bits_blocks, K), BITS_THREADS, 0, s>>>(n.frame[12], imp_dev, n.idx_dev, imp_bits_dev, n.bits_partial_dev,
+                                                                        n.count_partial_dev, r.err + K, n.H, n.W);
         LAUNCH_CHECK();
-        bits_sum_kernel<<<1, BITS_THREADS, 0, s>>>(n.bits_partial_dev, n.bits_blocks, &r->bits[1]);
+        bits_sum_kernel<<<K, BITS_THREADS, 0, s>>>(n.bits_partial_dev, n.count_partial_dev, n.bits_blocks, r.bits + K, r.count + K);
         LAUNCH_CHECK();
         LIC360_CUDA(cudaEventRecord(c->ev_est, s));
     }
     {
         NetDesc& n = c->code;
         cudaStream_t s = n.stream;
-        LIC360_CUDA(cudaMemsetAsync(&r->err[0], 0xFF, sizeof(r->err[0]), s));
-        int rc = run_encoder_net(c, true, code_dev, mask_dev, imp_dev);
+        LIC360_CUDA(cudaMemsetAsync(r.err, 0xFF, K * sizeof(*r.err), s));
+        int rc = run_encoder_net(c, true, K, code_dev, mask_dev, imp_dev);
         if (rc) return rc;
-        gmm_bits_kernel<<<n.bits_blocks, BITS_THREADS, 0, s>>>(n.frame[12], code_dev, mask_dev, n.idx_dev, n.steps_dev, n.row_off_dev,
-                                                               code_bits_dev, n.bits_partial_dev, &r->err[0], n.G, n.H, n.W,
-                                                               (float)(1. / sqrt(2.0)));
+        gmm_bits_kernel<<<dim3(n.bits_blocks, K), BITS_THREADS, 0, s>>>(n.frame[12], code_dev, mask_dev, n.idx_dev, n.steps_dev,
+                                                                        n.row_off_dev, code_bits_dev, n.bits_partial_dev,
+                                                                        n.count_partial_dev, r.err, n.G, n.H, n.W, (float)(1. / sqrt(2.0)));
         LAUNCH_CHECK();
-        bits_sum_kernel<<<1, BITS_THREADS, 0, s>>>(n.bits_partial_dev, n.bits_blocks, &r->bits[0]);
+        bits_sum_kernel<<<K, BITS_THREADS, 0, s>>>(n.bits_partial_dev, n.count_partial_dev, n.bits_blocks, r.bits, r.count);
         LAUNCH_CHECK();
         LIC360_CUDA(cudaStreamWaitEvent(s, c->ev_est, 0));
-        LIC360_CUDA(cudaMemcpyAsync(c->est_host, r, sizeof(EstimateTotals), cudaMemcpyDeviceToHost, s));
+        LIC360_CUDA(cudaMemcpyAsync(c->est_host, c->est_dev, estimate_bytes(K), cudaMemcpyDeviceToHost, s));
     }
     return LIC360_OK;
 }
 
-int lic360_codec_estimate(lic360_codec* c, const float* code_dev, const float* mask_dev, const float* imp_dev, float* code_bits_dev,
-                          float* imp_bits_dev, double* bits_host) {
-    LIC360_CHECK_ARG(c && code_dev && mask_dev && imp_dev && code_bits_dev && imp_bits_dev && bits_host, "bad arguments");
+// lic360_codec_estimate (K = 1, latent_suffix false) and lic360_codec_estimate_batch; the maps may be NULL
+static int estimate_latents(lic360_codec* c, int K, const float* code_dev, const float* mask_dev, const float* imp_dev,
+                            float* code_bits_dev, float* imp_bits_dev, double* bits_host, long long* counts_host, bool latent_suffix) {
     DeviceGuard guard(c->device);
     LIC360_CUDA(guard.err);
     int rc = check_params(c->code);
     if (rc == LIC360_OK) rc = check_params(c->imp);
+    if (rc == LIC360_OK) rc = batch_reserve(c, K);
     if (rc) return rc;
     const auto t0 = clk::now();
     c->t_host_coder = 0; c->t_gpu_wait = 0; c->t_imp = 0; c->t_gpu_steps = 0; c->t_gpu_steps_imp = 0;
-    rc = enqueue_estimate(c, code_dev, mask_dev, imp_dev, code_bits_dev, imp_bits_dev);
+    rc = enqueue_estimate(c, K, code_dev, mask_dev, imp_dev, code_bits_dev, imp_bits_dev);
     // both streams are drained on every path: the caller may reuse the inputs and the maps as soon as the call returns
     const auto tw = clk::now();
     const cudaError_t e_imp = cudaStreamSynchronize(c->imp.stream);
@@ -974,22 +1066,63 @@ int lic360_codec_estimate(lic360_codec* c, const float* code_dev, const float* m
     if (rc) return rc;
     LIC360_CUDA(e_imp);
     LIC360_CUDA(e_code);
-    // the errors encode reports, with its messages: the importance stream is coded (and checked) first
-    const EstimateTotals& r = *c->est_host;
-    if (r.err[1] != kNoError) {
-        const unsigned s = (unsigned)r.err[1];
-        if (s >= 49) set_error("coder: importance level %u out of range", s);
-        else set_error("coder: symbol has zero frequency");
+    // the errors encode reports for the first bad latent, with its messages: the importance stream is coded (and checked) first
+    const EstimateTotals r = estimate_totals(c->est_host, K);
+    for (int k = 0; k < K; k++) {
+        char msg[96], suffix[32] = "";
+        if (latent_suffix) snprintf(suffix, sizeof(suffix), " (latent %d)", k);
+        if (r.err[K + k] != kNoError) {
+            const unsigned s = (unsigned)r.err[K + k];
+            if (s >= 49) snprintf(msg, sizeof(msg), "coder: importance level %u out of range", s);
+            else snprintf(msg, sizeof(msg), "coder: symbol has zero frequency");
+        } else if (r.err[k] != kNoError) {
+            const int row = (int)(r.err[k] >> 32);
+            if ((unsigned)r.err[k] > 7) snprintf(msg, sizeof(msg), "coder: symbol out of range in packed row %d", row);
+            else snprintf(msg, sizeof(msg), "coder: symbol has zero frequency (row %d)", row);
+        } else {
+            continue;
+        }
+        set_error("%s%s", msg, suffix);
         return LIC360_ERR_CODER;
     }
-    if (r.err[0] != kNoError) {
-        const int row = (int)(r.err[0] >> 32);
-        if ((unsigned)r.err[0] > 7) set_error("coder: symbol out of range in packed row %d", row);
-        else set_error("coder: symbol has zero frequency (row %d)", row);
-        return LIC360_ERR_CODER;
+    for (int k = 0; k < K; k++)
+        for (int sid = 0; sid < 2; sid++) {
+            bits_host[2 * k + sid] = r.bits[sid * K + k];
+            if (counts_host) counts_host[2 * k + sid] = r.count[sid * K + k];
+        }
+    return LIC360_OK;
+}
+
+int lic360_codec_estimate(lic360_codec* c, const float* code_dev, const float* mask_dev, const float* imp_dev, float* code_bits_dev,
+                          float* imp_bits_dev, double* bits_host) {
+    LIC360_CHECK_ARG(c && code_dev && mask_dev && imp_dev && code_bits_dev && imp_bits_dev && bits_host, "bad arguments");
+    return estimate_latents(c, 1, code_dev, mask_dev, imp_dev, code_bits_dev, imp_bits_dev, bits_host, nullptr, false);
+}
+
+int lic360_codec_estimate_batch(lic360_codec* c, int K, const float* code_dev, const float* mask_dev, const float* imp_dev,
+                                float* code_bits_dev, float* imp_bits_dev, double* bits_host, long long* counts_host) {
+    LIC360_CHECK_ARG(K >= 1, "K must be at least 1");
+    LIC360_CHECK_ARG(c && code_dev && mask_dev && imp_dev && bits_host && counts_host, "bad arguments");
+    LIC360_CHECK_ARG(K <= kMaxBatch && (long long)3 * K * c->code.G * c->H * c->W <= 0x7fffffffLL,
+                     "K exceeds the launch limits of a batch (3K conv images, 3 * K * 48 * H * W input floats)");
+    return estimate_latents(c, K, code_dev, mask_dev, imp_dev, code_bits_dev, imp_bits_dev, bits_host, counts_host, true);
+}
+
+int lic360_imp_levels_to_mask(const float* levels_dev, int h, int w, const int* offsets_host, int K, float* levels_out_dev,
+                              float* mask_out_dev, void* stream) {
+    LIC360_CHECK_ARG(K >= 1, "K must be at least 1");
+    LIC360_CHECK_ARG(levels_dev && offsets_host && levels_out_dev && mask_out_dev, "bad arguments");
+    LIC360_CHECK_ARG(h > 0 && w > 0 && (long long)48 * 4 * h * w <= 0x7fffffffLL, "bad importance map size");
+    for (int j = 0; j < K; j++) LIC360_CHECK_ARG(offsets_host[j] >= 0, "offsets must not be negative");
+    const int n = 48 * 4 * h * w;
+    for (int j0 = 0; j0 < K; j0 += 32) {  // 32 candidates per launch (the offsets travel as a kernel parameter)
+        LevelOffsets off;
+        const int nj = std::min(32, K - j0);
+        for (int j = 0; j < nj; j++) off.k[j] = offsets_host[j0 + j];
+        imp_levels_to_mask_kernel<<<dim3(std::max(1, stream_grid(n, 256) / nj), nj), 256, 0, as_stream(stream)>>>(
+            levels_dev, h, w, off, levels_out_dev + (size_t)j0 * h * w, mask_out_dev + (size_t)j0 * n);
+        LAUNCH_CHECK();
     }
-    bits_host[0] = r.bits[0];
-    bits_host[1] = r.bits[1];
     return LIC360_OK;
 }
 

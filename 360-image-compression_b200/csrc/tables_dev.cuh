@@ -142,6 +142,11 @@ __device__ __forceinline__ int code_symbol(float cv) { return (cv >= 0.f && cv <
 __device__ __forceinline__ int code_mask_bit(float m) { return m < 0.5f ? 0 : 1; }
 // importance stream: the level as the packed row stores it (u16); 49 or more is out of range
 __device__ __forceinline__ uint32_t imp_symbol(float level) { return (uint16_t)(int)level; }
+// the mask bit of code symbol (tc, th, tw) that the decoder derives from the integer importance level lvl of its 2x2 cell:
+// Imp2mask (channel c of 192 kept iff c < 4 * lvl) and Dtow (c = 4 tc + 2 (th % 2) + tw % 2) in one expression
+__device__ __forceinline__ int code_mask_from_level(int lvl, int tc, int th, int tw) {
+    return (4 * tc + 2 * (th & 1) + (tw & 1)) < 4 * lvl ? 1 : 0;
+}
 
 // bins T[s], T[s+1] (0 <= s < N) of a row of N symbols as the host coder reads them back from the packed row: T[0] = 0 and
 // T[N] = 65536 are implied, the interior bins are the low 17 bits of (int)o[j] (16-bit word + overflow bit, pack_gmm_row /

@@ -873,7 +873,7 @@ __device__ __noinline__ void wf_chain4_rows(const WfNetDev& net, const WfRows& r
         if (live && j == 0) {
             fixup_row(o, 8, true);
             const int lvl = (int)(__ldcg(rows.levels + (th >> 1) * (W >> 1) + (tw >> 1)) + 1e-5f);  // written by the other stream's kernels
-            pack_gmm_row(o, 0, (4 * tc + 2 * (th & 1) + (tw & 1)) < 4 * lvl ? 1 : 0, rows.rows + (size_t)li * 8, rows.tagged ? psum % 15 + 1 : 0);
+            pack_gmm_row(o, 0, code_mask_from_level(lvl, tc, th, tw), rows.rows + (size_t)li * 8, rows.tagged ? psum % 15 + 1 : 0);
         }
     }
     if (rows.tagged) {  // self-validating rows: no fence, no flag; the host decodes row i as soon as row i carries this step's tag

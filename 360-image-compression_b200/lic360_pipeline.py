@@ -8,13 +8,14 @@ EntDecoder), packaged as one object so that bench.py and the tests drive exactly
 repo's mirror or the reference extension.
 """
 import ctypes
+import math
 import os
 import tempfile
 
 import torch
 
 import lic360_codec_ops as ops
-from lic360._lib import LIB, check
+from lic360._lib import LIB, check, cstream
 
 LAYER_KEYS = ['net.0'] + ['net.%d.conv%d' % (b, c) for b in range(1, 6) for c in (1, 2)] + ['net.6']
 
@@ -26,6 +27,65 @@ def make_codec_params(device, seed=2024):
         'code': ops.make_entropy_params(48, 4, 3, 3, seed, device),
         'imp': ops.make_entropy_params(1, 144, 49, None, seed + 1, device),
     }
+
+
+def levels_to_mask(imap_quant, offsets):
+    """Candidate importance maps for rate control and the code masks the decoder derives from them (lic360_imp_levels_to_mask).
+
+    imap_quant: (1,1,h,w) float32 CUDA tensor of importance levels as `encode` reads them (s = int(level), the symbol it codes);
+    offsets: K integers >= 0.  Returns (levels, masks) on the input's device: levels (K,1,h,w) = max(s - offsets[j], 0) and masks
+    (K,48,2h,2w), channel c at (y, x) = 1 iff 4c + 2 (y % 2) + x % 2 < 4 * level(y/2, x/2).  `encode(code, masks[j:j+1],
+    levels[j:j+1])` gives streams that decode to exactly masks[j]."""
+    if not (isinstance(imap_quant, torch.Tensor) and imap_quant.is_cuda and imap_quant.dtype == torch.float32
+            and imap_quant.dim() == 4 and tuple(imap_quant.shape[:2]) == (1, 1)):
+        raise RuntimeError("levels_to_mask: expected a (1,1,h,w) float32 CUDA tensor")
+    offs = [int(k) for k in offsets]
+    K, (h, w) = len(offs), imap_quant.shape[2:]
+    dev = imap_quant.device
+    levels = torch.empty((K, 1, h, w), dtype=torch.float32, device=dev)
+    masks = torch.empty((K, 48, 2 * h, 2 * w), dtype=torch.float32, device=dev)
+    with torch.cuda.device(dev):
+        lv = imap_quant.contiguous()
+        check(LIB.lic360_imp_levels_to_mask(lv.data_ptr(), h, w, (ctypes.c_int * max(K, 1))(*offs), K, levels.data_ptr(),
+                                            masks.data_ptr(), cstream(lv)))
+    return levels, masks
+
+
+BUDGET_OFFSETS = tuple(range(0, 49, 8))  # first stage of encode_to_budget's search
+
+
+def stream_bytes_bound(bits, symbols):
+    """Most bytes a stream of `symbols` coded symbols with exact-table total `bits` can take: 8 len <= I + 8 + N/8192 (derived in
+    tests/test_rate_estimate.py); the 1e-6 absorbs the rounding of the double total."""
+    return int(math.floor((bits + 8 + symbols / 8192.0) / 8 + 1e-6))
+
+
+def budget_bound(est):
+    """bytes both streams of an estimate (a dict of FusedCodec.estimate_batch) can take at most"""
+    return stream_bytes_bound(est['imp_bits'], est['imp_symbols']) + stream_bytes_bound(est['code_bits'], est['code_symbols'])
+
+
+def select_budget_offset(estimate, max_bytes):
+    """The level offset encode_to_budget codes: `estimate(offsets)` returns one estimate dict per offset; an offset fits when its
+    budget_bound is at most max_bytes.  Stage 1 evaluates offsets 0, 8, ..., 48; if the smallest that fits, k1, is not 0, stage 2
+    evaluates the seven offsets k1 - 7 .. k1 - 1.  The answer is the smallest evaluated offset that fits; the rate is not assumed to
+    fall monotonically with the offset.  Returns (offset, {offset: bound in bytes} of every offset evaluated); RuntimeError if no
+    offset of stage 1 fits."""
+    bounds = {}
+
+    def run(offsets):
+        offsets = list(offsets)
+        for k, est in zip(offsets, estimate(offsets)):
+            bounds[k] = budget_bound(est)
+
+    run(BUDGET_OFFSETS)
+    fit = [k for k in BUDGET_OFFSETS if bounds[k] <= max_bytes]
+    if not fit:
+        raise RuntimeError("encode_to_budget: no level offset up to %d fits %d bytes (bound at offset %d: %d bytes)"
+                           % (BUDGET_OFFSETS[-1], max_bytes, BUDGET_OFFSETS[-1], bounds[BUDGET_OFFSETS[-1]]))
+    if fit[0] > 0:
+        run(range(fit[0] - 7, fit[0]))
+    return min(k for k, b in bounds.items() if b <= max_bytes), bounds
 
 
 class PerOpCodec(object):
@@ -157,6 +217,61 @@ class FusedCodec(object):
         check(LIB.lic360_codec_estimate(self._h, code.data_ptr(), mask.data_ptr(), imp.data_ptr(), code_map.data_ptr(),
                                         imp_map.data_ptr(), totals))
         return {'code_bits': totals[0], 'imp_bits': totals[1], 'code_map': code_map, 'imp_map': imp_map}
+
+    def estimate_batch(self, code, mask, imap_quant, maps=True):
+        """`estimate` of K latents in one pass (lic360_codec_estimate_batch): code, mask (K,48,H,W), imap_quant (K,1,H/2,W/2).
+
+        Returns one dict per latent with estimate()'s keys plus 'code_symbols' and 'imp_symbols', the numbers of coded symbols
+        (mask >= 0.5, and every importance position).  Latent k's totals and maps are bit-identical to estimate() of that latent
+        alone.  The maps are views into (K,...) tensors, or None with maps=False.  A latent encode would refuse raises encode's
+        message followed by ' (latent k)', for the first such k."""
+        K = int(code.shape[0]) if code.dim() == 4 else -1
+        code = self._f32(code, (K, 48, self.H, self.W))
+        mask = self._f32(mask, (K, 48, self.H, self.W))
+        imp = self._f32(imap_quant, (K, 1, self.H // 2, self.W // 2))
+        code_map = imp_map = None
+        if maps:
+            code_map = torch.empty((K, 48, self.H, self.W), dtype=torch.float32, device=self.dev)
+            imp_map = torch.empty((K, 1, self.H // 2, self.W // 2), dtype=torch.float32, device=self.dev)
+        totals = (ctypes.c_double * max(2 * K, 1))()
+        counts = (ctypes.c_longlong * max(2 * K, 1))()
+        torch.cuda.current_stream(self.dev).synchronize()  # inputs were produced on torch's stream
+        check(LIB.lic360_codec_estimate_batch(self._h, K, code.data_ptr(), mask.data_ptr(), imp.data_ptr(),
+                                              None if code_map is None else code_map.data_ptr(),
+                                              None if imp_map is None else imp_map.data_ptr(), totals, counts))
+        return [{'code_bits': totals[2 * k], 'imp_bits': totals[2 * k + 1], 'code_symbols': counts[2 * k],
+                 'imp_symbols': counts[2 * k + 1], 'code_map': None if code_map is None else code_map[k:k + 1],
+                 'imp_map': None if imp_map is None else imp_map[k:k + 1]} for k in range(K)]
+
+    def encode_to_budget(self, code, imap_quant, max_bytes):
+        """Encode the latent in at most max_bytes bytes (both streams) by lowering its importance levels: candidate k codes the
+        levels max(s - k, 0) with the mask the decoder derives from them (levels_to_mask), so the result always decodes.  The
+        offset comes from select_budget_offset on batched exact-table estimates (two estimate_batch calls, 7 latents each at
+        most), where a candidate fits when the proven upper bound of its stream lengths (stream_bytes_bound) is at most max_bytes;
+        then one encode of the chosen candidate.
+
+        Returns {'imp_bytes', 'code_bytes', 'offset', 'levels' (1,1,H/2,W/2), 'mask' (1,48,H,W), 'bound': bytes bound of the
+        chosen offset, 'bounds': {offset: bound} of every offset evaluated}.  RuntimeError when no offset fits, and when the
+        encoded streams exceed max_bytes (the bound would be broken: never returned silently)."""
+        code = self._f32(code, (1, 48, self.H, self.W))
+        imp = self._f32(imap_quant, (1, 1, self.H // 2, self.W // 2))
+        max_bytes = int(max_bytes)
+        cands = {}
+
+        def estimate(offsets):
+            levels, masks = levels_to_mask(imp, offsets)
+            for j, k in enumerate(offsets):
+                cands[k] = (levels[j:j + 1], masks[j:j + 1])
+            return self.estimate_batch(code.expand(len(offsets), -1, -1, -1), masks, levels, maps=False)
+
+        offset, bounds = select_budget_offset(estimate, max_bytes)
+        levels, mask = cands[offset]
+        imp_bytes, code_bytes = self.encode(code, mask, levels)
+        if len(imp_bytes) + len(code_bytes) > max_bytes:
+            raise RuntimeError("encode_to_budget: offset %d encoded to %d bytes, above its bound of %d and the budget of %d bytes"
+                               % (offset, len(imp_bytes) + len(code_bytes), bounds[offset], max_bytes))
+        return {'imp_bytes': imp_bytes, 'code_bytes': code_bytes, 'offset': offset, 'levels': levels, 'mask': mask,
+                'bound': bounds[offset], 'bounds': bounds}
 
     def decode(self, imp_bytes, code_bytes, h=None, w=None, name=None):
         code = torch.empty((1, 48, self.H, self.W), dtype=torch.float32, device=self.dev)

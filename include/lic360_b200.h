@@ -231,6 +231,26 @@ int lic360_codec_encode(lic360_codec* c, const float* code_dev, const float* mas
  * the end, which the terminator makes unnecessary (a few at most in practice; derivation in tests/test_rate_estimate.py). */
 int lic360_codec_estimate(lic360_codec* c, const float* code_dev, const float* mask_dev, const float* imp_dev,
                           float* code_bits_dev, float* imp_bits_dev, double* bits_host);
+/* lic360_codec_estimate of K latents of the codec's size in one pass: both networks run once at batch K (the code network as 3K
+ * images over its 3 weight sets), the bits kernels once with the latent in blockIdx.y.  Latent k's totals and map are bit-identical
+ * to lic360_codec_estimate of that latent alone (same block partition, same fixed-order sums, no floating-point atomics).
+ *   code_dev, mask_dev (K,48,H,W), imp_dev (K,1,H/2,W/2): the inputs of K encodes, stacked
+ *   code_bits_dev (K,48,H,W), imp_bits_dev (K,1,H/2,W/2): the maps; either may be NULL (not written; the totals still are)
+ *   bits_host[2k + stream_id]: totals of latent k; counts_host[2k + stream_id]: its coded symbols, counted on the device (code
+ *   stream: positions with mask >= 0.5; importance stream: every position)
+ * The encoder buffers grow to the largest K seen and are freed by lic360_codec_destroy.  A bad latent fails the call with the status
+ * and message lic360_codec_encode gives for it, followed by " (latent k)", for the lowest such k.  K < 1, or K beyond the launch
+ * limits (3K <= 65535 and 3 * K * 48 * H * W < 2^31), is an argument error. */
+int lic360_codec_estimate_batch(lic360_codec* c, int K, const float* code_dev, const float* mask_dev, const float* imp_dev,
+                                float* code_bits_dev, float* imp_bits_dev, double* bits_host, long long* counts_host);
+/* Candidate importance maps and the code masks the decoder derives from them, for rate control.  levels_dev (h,w) are importance
+ * levels as lic360_codec_encode reads them: s = the symbol it codes for a level ((int) of it).  For each offsets_host[j] >= 0:
+ *   levels_out_dev[j] (K,1,h,w) = max(s - offsets_host[j], 0)
+ *   mask_out_dev[j]  (K,48,2h,2w) = the decoder's mask of that level, Imp2mask + Dtow in one pass: channel c at (y, x) is 1 iff
+ *                                   4c + 2 (y % 2) + x % 2 < 4 * level(y/2, x/2)
+ * Encoding a pair (levels_out[j], mask_out[j]) gives streams that decode to exactly that mask.  Enqueued on `stream`. */
+int lic360_imp_levels_to_mask(const float* levels_dev, int h, int w, const int* offsets_host, int K, float* levels_out_dev,
+                              float* mask_out_dev, void* stream);
 long lic360_codec_stream_size(lic360_codec* c, int stream_id);
 long lic360_codec_stream_copy(lic360_codec* c, int stream_id, uint8_t* out, long cap);
 /* -> code_out_dev (1,48,H,W) = symbols where mask == 1, else 0 (lic360_demo.py:236-237); mask_out_dev (1,48,H,W) */
