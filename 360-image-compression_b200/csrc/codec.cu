@@ -1598,4 +1598,21 @@ int lic360_codec_kernel_times(lic360_codec* c, int stream_id, double* out, int n
     return LIC360_OK;
 }
 
+int lic360_codec_engine_info(lic360_codec* c, int stream_id, int* out, int n) {
+    LIC360_CHECK_ARG(c && out && (stream_id == 0 || stream_id == 1), "bad arguments");
+    const NetDesc& d = stream_id == 0 ? c->code : c->imp;
+    const WfEngine& e = d.wf;
+    int tail_rounds = 0;
+    if (e.chain4 && n > 12) {
+        std::vector<int32_t> idx(2 * (size_t)d.H * d.W), plan(d.H + d.W);
+        lic360_code_contex(d.H, d.W, idx.data(), plan.data());
+        tail_rounds = wf_tail_rounds(e, idx.data(), d.steps.data());
+    }
+    const int v[13] = {e.chain1 ? 2 : e.chain4 ? 1 : 0, e.chain1 && e.c1_dsm, e.cluster, e.chain_threads, (int)e.chain_smem, e.max_len,
+                       e.chain1 ? e.c1_lenp : 0, e.chain1 ? e.c1_kpc : 0, e.chain_tasks, e.old4 ? 4 : e.old2 ? 2 : 1, e.parts4,
+                       e.dev.parts, tail_rounds};
+    for (int i = 0; i < n && i < 13; i++) out[i] = v[i];
+    return LIC360_OK;
+}
+
 }  // extern "C"

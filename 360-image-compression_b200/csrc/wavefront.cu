@@ -767,22 +767,33 @@ __device__ __noinline__ float4 wf_r_layer0_c1(const WfNetDev& net, int n, int d,
 // clusters in wf_chain4_rows -- the tail then runs from shared-memory weights like the chain itself.
 struct WfTailPlan { int i0, nloc, tc_lo, nrows, lpg; };
 
-__device__ __forceinline__ WfTailPlan wf_tail_plan(const WfNetDev& net, int rank, int nc, int psum1, int smem_rows) {
+// step s1 = step psum1 of the index plan idx (H * W positions); also evaluated on the host (wf_tail_rounds)
+__host__ __device__ __forceinline__ WfTailPlan wf_tail_plan_of(const int32_t* idx, int HW, StepDesc s1, int rank, int nc, int psum1,
+                                                               int smem_rows) {
+#ifdef __CUDA_ARCH__
+#define WF_IDX(k) __ldg(idx + (k))
+#else
+#define WF_IDX(k) idx[k]
+#endif
     WfTailPlan t = {0, 0, 0, 0, 1};
-    if (psum1 >= net.nsteps) return t;
-    const StepDesc s1 = net.steps[psum1];
     const int per = (s1.len + nc - 1) / nc;
     t.i0 = min(s1.len, rank * per);
     const int i1 = min(s1.len, t.i0 + per);
     t.nloc = i1 - t.i0;
     if (t.nloc > 0) {  // plan order is diagonal-major: the chunk's output groups are a contiguous range
-        const int HW = net.H * net.W, ka = s1.start + t.i0, kb = s1.start + i1 - 1;
-        const int tc_hi = psum1 - __ldg(net.idx + ka) - __ldg(net.idx + ka + HW);
-        t.tc_lo = psum1 - __ldg(net.idx + kb) - __ldg(net.idx + kb + HW);
+        const int ka = s1.start + t.i0, kb = s1.start + i1 - 1;
+        const int tc_hi = psum1 - WF_IDX(ka) - WF_IDX(ka + HW);
+        t.tc_lo = psum1 - WF_IDX(kb) - WF_IDX(kb + HW);
         t.nrows = tc_hi - t.tc_lo + 1;
         t.lpg = max(1, min(WF_LAYERS - 1, smem_rows / t.nrows));
     }
+#undef WF_IDX
     return t;
+}
+
+__device__ __forceinline__ WfTailPlan wf_tail_plan(const WfNetDev& net, int rank, int nc, int psum1, int smem_rows) {
+    if (psum1 >= net.nsteps) return WfTailPlan{0, 0, 0, 0, 1};
+    return wf_tail_plan_of(net.idx, net.H * net.W, net.steps[psum1], rank, nc, psum1, smem_rows);
 }
 
 // cp.async of the R rows [tc_lo, tc_lo + nrows) of layers l0 .. l0 + nl - 1 into the dynamic shared memory, issued by threads t0, t0 + 1, ..
@@ -1627,6 +1638,17 @@ int wf_init(WfEngine& e, int G, int cpg, int nlast, int nsets, int H, int W, con
     int want = G > 1 ? 8 : 16;
     if (const char* s = getenv("LIC360_WF_CLUSTER")) want = std::max(1, std::min(16, atoi(s)));
     if (const char* s = getenv(G > 1 ? "LIC360_WF_CLUSTER_CODE" : "LIC360_WF_CLUSTER_IMP")) want = std::max(1, std::min(16, atoi(s)));
+    // the one limit of every chain kernel's dynamic shared memory: the per-block opt-in maximum (227 KB on B200) minus the largest
+    // static shared memory of the three kernels
+    int dev = 0, optin = 0;
+    LIC360_CUDA(cudaGetDevice(&dev));
+    LIC360_CUDA(cudaDeviceGetAttribute(&optin, cudaDevAttrMaxSharedMemoryPerBlockOptin, dev));
+    size_t static_max = 0;
+    cudaFuncAttributes fa;
+    LIC360_CUDA(cudaFuncGetAttributes(&fa, wf_chain_kernel<384>)); static_max = std::max(static_max, fa.sharedSizeBytes);
+    LIC360_CUDA(cudaFuncGetAttributes(&fa, wf_chain4_kernel)); static_max = std::max(static_max, fa.sharedSizeBytes);
+    LIC360_CUDA(cudaFuncGetAttributes(&fa, wf_chain1_kernel)); static_max = std::max(static_max, fa.sharedSizeBytes);
+    const size_t cap = (size_t)optin - static_max;
     for (e.cluster = want;; e.cluster = 8) {
         int tasks_max = 0;
         for (int l = 0; l < WF_LAYERS; l++) {
@@ -1636,6 +1658,7 @@ int wf_init(WfEngine& e, int G, int cpg, int nlast, int nsets, int H, int W, con
         // a kernel row of an item (5 activations + 20 weight vectors) is kept in registers: at most 384 threads per CTA
         // (168 registers each); CTAs with more tasks loop
         e.chain_threads = std::min(384, std::max(128, ((tasks_max + 31) / 32) * 32));
+        e.chain_tasks = tasks_max;
         e.chain_smem = (size_t)tasks_max * sizeof(float4);
         e.chain4 = G > 1 && G <= 64;
         for (int l = 0; l < WF_LAYERS; l++) e.chain4 = e.chain4 && n.L[l].cpg4 == 1 && (l == 0 || n.L[l].cin_g == 4);
@@ -1652,13 +1675,12 @@ int wf_init(WfEngine& e, int G, int cpg, int nlast, int nsets, int H, int W, con
             const size_t tile = (size_t)(e.c1_lenp + 4) * (e.c1_cmax + 4) * sizeof(float);            // one activation tile
             const size_t parts = (size_t)e.c1_kpc * ((e.c1_cmax + CB - 1) / CB) * e.c1_lenp * sizeof(float4);
             const bool logits_fit = (size_t)e.c1_lenp * 52 * sizeof(float) <= wbuf1;                 // they reuse weight buffer 0
-            const size_t cap = 226 * 1024;  // 227 KB per CTA minus the kernel's static shared memory
             e.c1_dsm = logits_fit && 2 * wbuf1 + 2 * tile + parts <= cap;   // activations exchanged through distributed shared memory
             const size_t sm = 2 * wbuf1 + (e.c1_dsm ? 2 : 1) * tile + parts;
             if (logits_fit && sm <= cap) { e.chain_smem = sm; e.chain_threads = 384; }
             else e.chain1 = false;  // too large for shared memory: the generic chain kernel handles it
         }
-        if (e.chain_smem > 200 * 1024) { set_error("wavefront engine: slab too large for the chain kernel"); return LIC360_ERR_ARG; }
+        if (e.chain_smem > cap) { set_error("wavefront engine: slab too large for the chain kernel"); return LIC360_ERR_ARG; }
         // The old-term kernel of the next step runs concurrently (programmatic dependent launch): claim the whole shared
         // memory of the SM so that none of its CTAs lands next to a chain CTA and steals its issue slots.
         if (!getenv("LIC360_WF_SHARE_SM")) e.chain_smem = std::max(e.chain_smem, (size_t)196 * 1024);
@@ -1699,6 +1721,18 @@ int wf_chain_capacity(const WfEngine& e) {
     int nclusters = 0;
     if (cudaOccupancyMaxActiveClusters(&nclusters, wf_chain4_kernel, &cfg) != cudaSuccess) { cudaGetLastError(); return 1; }
     return std::max(1, nclusters / e.dev.nsets);
+}
+
+int wf_tail_rounds(const WfEngine& e, const int32_t* idx, const StepDesc* steps) {
+    if (!e.chain4) return 0;
+    const int smem_rows = (int)(e.chain_smem / (WF_ROW_F4 * sizeof(float4)));  // as wf_launch_chain passes it
+    int rounds = 0;
+    for (int p = 1; p < e.dev.nsteps; p++)
+        for (int rank = 0; rank < e.cluster; rank++) {
+            const WfTailPlan t = wf_tail_plan_of(idx, e.dev.H * e.dev.W, steps[p], rank, e.cluster, p, smem_rows);
+            if (t.nloc > 0) rounds = std::max(rounds, (WF_LAYERS - 1 + t.lpg - 1) / t.lpg);
+        }
+    return rounds;
 }
 
 const void* wf_old_kernel_ptr() { return reinterpret_cast<const void*>(&wf_old_kernel); }

@@ -90,6 +90,7 @@ struct WfEngine {
     int C[WF_LAYERS + 1];
     int max_len = 0, cpg4_max = 0, nblk_max = 0, nqb_max = 0;
     int cluster = 1, chain_threads = 0;
+    int chain_tasks = 0;  // wf_chain_kernel: (item, block) tasks of one CTA in the longest step's most expensive layer
     bool chain4 = false;  // every chained layer has 4 channels per group: the staged-weight chain kernel applies
     bool chain1 = false;  // single-group net: the output-chunk-split chain kernel applies
     bool c1_dsm = false;  // chain1: both activation tiles fit, layers exchange activations through distributed shared memory
@@ -104,6 +105,9 @@ int wf_init(WfEngine& e, int G, int cpg, int nlast, int nsets, int H, int W, con
 void wf_set_layer(WfEngine& e, int l, const float* wp, const float* wq, const float* bias, const float* slope);
 void wf_free(WfEngine& e);
 int wf_chain_capacity(const WfEngine& e);  // decodes whose code-stream chains may be in flight together on the device
+// wf_chain4_kernel's R tail: the most rounds in which a CTA stages its weight rows, over all steps (0: not a chain4 engine).
+// idx, steps: the host copies of the index plan and the step list the engine was created with
+int wf_tail_rounds(const WfEngine& e, const int32_t* idx, const StepDesc* steps);
 const void* wf_old_kernel_ptr();
 const void* wf_old2_kernel_ptr();  // to give the old-term kernel node its own (lowest) priority in the step graph
 cudaError_t wf_clear(const WfEngine& e, cudaStream_t s);                    // zero every frame (start of a decode)

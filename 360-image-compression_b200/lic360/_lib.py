@@ -88,6 +88,7 @@ SIGNATURES = {
     "lic360_codec_last_timing": (_I, [_P, _P, _I]),
     "lic360_codec_set_mode": (_I, [_P, _I]),
     "lic360_codec_kernel_times": (_I, [_P, _I, _P, _I]),
+    "lic360_codec_engine_info": (_I, [_P, _I, _P, _I]),
 }
 
 for _name, (_res, _args) in SIGNATURES.items():

@@ -292,6 +292,14 @@ class FusedCodec(object):
         check(LIB.lic360_codec_kernel_times(self._h, stream_id, out, 5))
         return {'old_ms': out[0], 'prev_ms': out[1], 'chain_ms': out[2], 'scatter_rows_ms': out[3], 'steps': int(out[4])}
 
+    def engine_info(self, stream_id=0):
+        """The decoder's kernel choices for one stream (0 = code, 1 = importance), fixed at creation (lic360_codec_engine_info)."""
+        out = (ctypes.c_int * 13)()
+        check(LIB.lic360_codec_engine_info(self._h, stream_id, out, 13))
+        return {'chain': ('generic', 'chain4', 'chain1')[out[0]], 'dsm': bool(out[1]), 'cluster': out[2], 'chain_threads': out[3],
+                'chain_smem': out[4], 'max_len': out[5], 'c1_lenp': out[6], 'c1_kpc': out[7], 'chain_tasks': out[8],
+                'old_positions_per_lane': out[9], 'parts4': out[10], 'parts': out[11], 'tail_rounds': out[12]}
+
     def last_timing(self):
         out = (ctypes.c_double * 6)()
         LIB.lic360_codec_last_timing(self._h, out, 6)

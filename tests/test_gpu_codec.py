@@ -285,7 +285,7 @@ def test_fused_codec_low_latency_mode_several_decodes_at_once(ncodec):
 
 @pytest.mark.parametrize("switch", ["LIC360_WF_OLD1", "LIC360_WF_OLD2", "LIC360_WF_ROWS_KERNEL", "LIC360_WF_PREV_KERNEL", "LIC360_WF_R0_KERNEL",
                                     "LIC360_WF_ROWS_FLAGS", "LIC360_WF_SHARE_SM", "LIC360_WF_NO_OVERLAP", "LIC360_WF_OLD_SPLIT=3",
-                                    "LIC360_WF_LAUNCH_AHEAD", "LIC360_EC_RQ_GENERIC"])
+                                    "LIC360_WF_LAUNCH_AHEAD", "LIC360_EC_RQ_GENERIC", "LIC360_WF_CLUSTER=4"])
 def test_fused_codec_alternate_kernel_paths(monkeypatch, switch):
     """Every kernel the default pipeline replaced is still selectable by an environment switch (DESIGN.md s8) and is the reference
     point of an A/B number in DESIGN.md: each must still produce the same bytes and the same symbols as the default path."""
