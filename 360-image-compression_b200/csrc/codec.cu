@@ -62,9 +62,10 @@ struct NetDesc {
     int* done_dev = nullptr;            // CTA counter of the rows kernel
     int* arrived_dev = nullptr;         // CTA counter of the scatter kernel (the last CTA advances ctr_dev)
     int* sync_dev = nullptr;            // code stream: monotone cross-cluster counter of the chain kernel's rows phase
-    int* flag_host = nullptr;           // mapped pinned: step + 1 once the rows of a step are in rows_step_host
-    int nflags = 1;                     // host flags the rows producer raises (one per CTA of the fused code-stream chain)
-    int* go_host = nullptr;             // mapped pinned: the stream may run step p once this is >= p (launch-ahead / persistent decode)
+    int* flag_host = nullptr;           // mapped pinned, importance stream: step + 1 once the rows of a step are in rows_step_host;
+                                        // code stream: one per chain CTA, negative when that CTA gave up waiting for the other clusters
+    int nflags = 1;                     // code stream: chain CTAs, each with its own host flag
+    int* go_host = nullptr;             // mapped pinned: the stream may run step p once this is >= p (persistent decode)
     int* go_dev = nullptr;              // persistent decode: CTA 0's republished go / abort decision
     int* old_done_dev = nullptr;        // persistent decode: old-term sums of steps < this are complete
     int* scat_done_dev = nullptr;       // persistent decode, one per net: symbols of steps < this are in the net's input frame
@@ -74,7 +75,6 @@ struct NetDesc {
     float* syms_host = nullptr;         // mapped pinned: decoded symbols of one step
     std::vector<float> step_wait_us, step_decode_us, step_levels_us;  // debug timeline (LIC360_WF_TRACE_FILE): host time per step waiting for rows / decoding
     int row_bytes = 16;                 // packed row size (16 B code stream, 128 B importance stream)
-    bool tagged = false;                // decode: the step's rows carry a publication tag and are validated row by row (no fence + flag)
     double t_host_coder = 0, t_gpu_wait = 0, t_done = 0;
     lic360_coder* coder = nullptr;
     char err[256] = {0};                // error text of a worker thread (set_error is thread-local)
@@ -485,49 +485,6 @@ __device__ __forceinline__ void rows_done(int* done, volatile int* flag, int ste
     }
 }
 
-// decoder: CDF rows of the slab of step *ctr from the engine's last frame (group-major channel-last, 3 nets x G x 3).
-// 8 lanes per symbol: lane j computes bin j (the 21 erff of a row are the critical path of this latency-bound kernel),
-// lane 0 gathers the bins, runs the monotonic fix-up and stores the packed 16-byte row.
-// The mask bit of a symbol comes straight from the decoded importance level of its 2x2 cell (Imp2mask + Dtow fused:
-// mask_up[g][h][w] = (4g + 2(h%2) + (w%2)) < 4*level[h/2][w/2], imp2mask_cuda.cu:25-38, dtow_cuda.cu:38-56), so the code
-// stream only needs the importance diagonals that are already decoded and the two streams decode concurrently.
-__global__ void gmm_rows_wf_kernel(const float* __restrict__ y, const float* __restrict__ levels, const int32_t* __restrict__ idx,
-                                   const StepDesc* __restrict__ steps, const int* __restrict__ ctr, uint16_t* __restrict__ rows,
-                                   int G, int H, int W, int Dp, int Hp, float s2, int* done, int* flag) {
-    const int step = *ctr;
-    if (threadIdx.x == 0) WF_TRACE_MIN(G, step, WF_TR_ROWS0);
-    const StepDesc d = steps[step];
-    const int gt = blockIdx.x * blockDim.x + threadIdx.x;
-    const int l = gt >> 3, j = gt & 7;
-    const bool live = l < d.len;
-    float bin = 0.f;
-    int th = 0, tw = 0, tc = 0;
-    if (live) {
-        const int HW = H * W;
-        th = __ldg(idx + d.start + l); tw = __ldg(idx + d.start + l + HW);
-        tc = d.psum - th - tw;
-        float wv[3], dv[3], mv[3];
-#pragma unroll
-        for (int i = 0; i < 3; i++) {
-            wv[i] = y[wf_fc_index(Dp, Hp, G, 3, 0, th + tw, tc, th) + i];
-            dv[i] = y[wf_fc_index(Dp, Hp, G, 3, 1, th + tw, tc, th) + i];
-            mv[i] = y[wf_fc_index(Dp, Hp, G, 3, 2, th + tw, tc, th) + i];
-        }
-        gmm_prep(wv, dv, 3, 1e-6f);
-        if (j >= 1) bin = gmm_bin_value(wv, dv, mv, j, 3, 3.5f, 65536.f, s2);
-    }
-    float o[9];
-    o[0] = 0.f; o[8] = 65536.f;
-#pragma unroll
-    for (int k = 1; k < 8; k++) o[k] = __shfl_sync(0xffffffffu, bin, (threadIdx.x & 24) + k);
-    if (live && j == 0) {
-        fixup_row(o, 8, true);
-        const int lvl = (int)(levels[(th >> 1) * (W >> 1) + (tw >> 1)] + 1e-5f);
-        pack_gmm_row(o, 0, code_mask_from_level(lvl, tc, th, tw), rows + (size_t)l * 8);
-    }
-    rows_done(done, flag, step, G);
-}
-
 // decoder, importance stream: CDF row of every position of the step's diagonal from the 49 logits of the engine's last frame.
 // One WARP per symbol (the step has <= min(H, W) symbols and sits on the critical path of BOTH streams, so it is latency that
 // counts): lanes hold logits i and i + 32, the softmax denominator is accumulated in index order by every lane from shared memory
@@ -636,8 +593,9 @@ static int check_params(const NetDesc& n) {
 }
 
 // the kernels of one decode step.  side == s (serialized / profile mode): everything in stream order, the old terms of
-// the NEXT step last.  side != s (graph capture): the old terms run on a parallel low-priority branch; either way the
-// host is released by the flag that the rows kernel raises, so the bulk of the arithmetic also overlaps the host coder.
+// the NEXT step last.  side != s (graph capture): the old terms run beside the chain as its programmatic dependent; either way the
+// host is released by the step's rows (published row by row in the code stream, by a flag in the importance stream), so the bulk
+// of the arithmetic also overlaps the host coder.
 // ev != nullptr: profile mode, events bracket the kernel classes (everything on `s`).
 #define WF_DEBUG_SYNC(what)                                                                               \
     do {                                                                                                \
@@ -663,61 +621,48 @@ static int launch_step(lic360_codec* c, NetDesc& n, bool is_code, cudaStream_t s
     WF_DEBUG_SYNC("scatter kernel");
     const bool fork = side != s;  // graph capture: overlap the old terms of the next step with the chain (see below)
     if (ev) LIC360_CUDA(cudaEventRecord(ev[1], s));
-    const bool fused_rows = (is_code ? n.wf.chain4 : n.wf.chain1) && !getenv("LIC360_WF_ROWS_KERNEL");
-    if (!(fused_rows && n.wf.r0_inline)) {  // else the chain kernel evaluates them in its prologue
+    // wf_chain4_kernel (code stream) and wf_chain1_kernel evaluate layer 0's previous-wavefront terms in their prologue and emit the
+    // step's CDF rows themselves; the generic chain kernel (importance stream, long diagonals) needs a launch for each
+    const bool fused = n.wf.chain4 || n.wf.chain1;
+    if (!fused) {
         LIC360_CUDA(wf_launch_prev(n.wf, 0, 0, 1, s));  // layer 0 only: its taps read the symbols scattered a moment ago
         WF_DEBUG_SYNC("previous-wavefront kernel (layer 0)");
     }
     if (ev) LIC360_CUDA(cudaEventRecord(ev[2], s));
-    // the chain; for the code stream it also emits the CDF rows of the step and raises the host flag
     WfRows rows;
-    memset(&rows, 0, sizeof(rows));
-    if (fused_rows) {
-        rows.rows = n.rows_step_host; rows.levels = c->levels_dev; rows.done = n.done_dev; rows.flag = n.flag_host;
-        rows.sync = n.sync_dev; rows.s2 = (float)(1. / sqrt(2.0)); rows.enabled = 1;
-    }
-    // code stream: the chain kernel also leaves the previous-wavefront terms of the next step behind (no launch, no side branch)
-    n.nflags = fused_rows && is_code ? n.wf.dev.nsets * n.wf.cluster : 1;
-    if (n.nflags > 64) { set_error("codec: %d chain CTAs exceed the 64 host flags", n.nflags); return LIC360_ERR_ARG; }
-    const bool rtail = fused_rows && is_code && n.wf.chain4 && !getenv("LIC360_WF_PREV_KERNEL");
-    rows.rtail = rtail ? 1 : 0;
-    // code stream: every 16-byte row is published by its own tag (step % 15 + 1 in the meta word; 0 = never written); the host decodes row i as soon as
-    // it has arrived -- no system fence and no flag write behind the rows, and the PCIe flight of the later rows overlaps the decoding
-    n.tagged = fused_rows && is_code && n.wf.chain4 && !getenv("LIC360_WF_ROWS_FLAGS");
-    rows.tagged = n.tagged ? 1 : 0;
-    LIC360_CUDA(wf_launch_chain(n.wf, s, fused_rows ? &rows : nullptr));
+    rows.rows = n.rows_step_host; rows.levels = c->levels_dev; rows.flag = n.flag_host; rows.sync = n.sync_dev;
+    rows.s2 = (float)(1. / sqrt(2.0));
+    LIC360_CUDA(wf_launch_chain(n.wf, s, rows));
     WF_DEBUG_SYNC("chain kernel");
     if (ev) LIC360_CUDA(cudaEventRecord(ev[3], s));
     // The old terms of step p+1 only read wavefronts <= p-1: they are launched right behind the chain kernel as its
     // PROGRAMMATIC dependent -- they start once every chain CTA is resident (so the chain's clusters got their SMs first)
-    // and fill the SMs the chain leaves idle.  Whatever still needs the chain's RESULTS (a separate rows kernel, the
-    // previous-wavefront kernel of the next step) waits for the chain's completion on the side stream; when the chain kernel
-    // does all of that itself (rtail) there is no side branch at all.
+    // and fill the SMs the chain leaves idle.  In the importance stream, whatever still needs the chain's RESULTS (the rows
+    // kernel of the generic chain, the previous-wavefront kernel of the next step) waits for the chain's completion on the side
+    // stream.  The code stream's chain kernel also leaves the previous-wavefront terms of the next step behind: no side branch.
     cudaStream_t rs = s;  // stream of the kernels behind the chain
     if (fork) {
         LIC360_CUDA(cudaEventRecord(n.ev_fork, s));
         LIC360_CUDA(wf_launch_old(n.wf, 1, s, true));
-        if (!rtail) {
+        if (!is_code) {
             LIC360_CUDA(cudaStreamWaitEvent(side, n.ev_fork, 0));
             rs = side;
         }
     }
-    if (fused_rows) {
-    } else if (is_code)
-        gmm_rows_wf_kernel<<<(n.max_len * 8 + 127) / 128, 128, 0, rs>>>(n.wf.fc[12], c->levels_dev, n.idx_dev,
-                                                 n.steps_dev, n.ctr_dev, n.rows_step_host, n.G, n.H, n.W, w.Dp, w.Hp,
-                                                 (float)(1. / sqrt(2.0)), n.done_dev, n.flag_host);
-    else
+    if (!fused) {
         imp_rows_wf_kernel<<<std::max(1, std::min(4, (n.max_len + IMP_ROWS_WARPS - 1) / IMP_ROWS_WARPS)), 32 * IMP_ROWS_WARPS, 0, rs>>>(n.wf.fc[12], n.idx_dev, n.steps_dev, n.ctr_dev, n.rows_step_host, n.H, n.W, w.Dp, w.Hp,
                                                  n.done_dev, n.flag_host);
-    if (!fused_rows) LAUNCH_CHECK();
-    WF_DEBUG_SYNC("rows kernel");
-    // previous-wavefront terms of layers 1..11 for step p+1 (the activations of wavefront p are final): behind the rows
-    // kernel, i.e. underneath the host decoder instead of on the critical path
-    if (!rtail) LIC360_CUDA(wf_launch_prev(n.wf, 1, 1, WF_LAYERS, rs));
-    WF_DEBUG_SYNC("previous-wavefront kernel (layers 1..11 of the next step)");
+        LAUNCH_CHECK();
+        WF_DEBUG_SYNC("rows kernel");
+    }
+    if (!is_code) {
+        // previous-wavefront terms of layers 1..11 for step p+1 (the activations of wavefront p are final): behind the rows,
+        // i.e. underneath the host decoder instead of on the critical path
+        LIC360_CUDA(wf_launch_prev(n.wf, 1, 1, WF_LAYERS, rs));
+        WF_DEBUG_SYNC("previous-wavefront kernel (layers 1..11 of the next step)");
+    }
     if (ev) LIC360_CUDA(cudaEventRecord(ev[4], s));
-    if (fork && rtail) {
+    if (fork && is_code) {
         // the old-term kernel is only a PROGRAMMATIC dependent of the chain: give the end of the step a full edge from the chain too
         LIC360_CUDA(cudaStreamWaitEvent(s, n.ev_fork, 0));
     } else if (fork) {
@@ -738,14 +683,13 @@ static int build_step_graph(lic360_codec* c, NetDesc& n, bool is_code) {
     cudaGraph_t g;
     const long long l0 = g_launches;
     LIC360_CUDA(cudaStreamBeginCapture(s, cudaStreamCaptureModeThreadLocal));
-    const bool overlap = getenv("LIC360_WF_NO_OVERLAP") == nullptr;  // (graph build time: not on a hot path)
-    const int rc = launch_step(c, n, is_code, s, overlap ? n.side : s, nullptr);
+    const int rc = launch_step(c, n, is_code, s, n.side, nullptr);
     cudaError_t e = cudaStreamEndCapture(s, &g);
     n.graph_nodes = (int)(g_launches - l0);
     g_launches = l0;  // captured, not launched: replays are counted in decode_stream
     if (rc != LIC360_OK) { if (e == cudaSuccess) cudaGraphDestroy(g); return rc; }
     LIC360_CUDA(e);
-    {   // kernel-node priorities: old-term kernel lowest, everything on the critical path highest
+    {   // kernel-node priorities: the importance stream's old-term kernel lowest, everything else at its stream's level
         int prio_lo = 0, prio_hi = 0;
         cudaDeviceGetStreamPriorityRange(&prio_lo, &prio_hi);
         size_t nn = 0;
@@ -759,10 +703,11 @@ static int build_step_graph(lic360_codec* c, NetDesc& n, bool is_code) {
             if (cudaGraphKernelNodeGetParams(nodes[i], &kp) != cudaSuccess) continue;
             cudaKernelNodeAttrValue v;
             memset(&v, 0, sizeof(v));
-            // code stream: critical kernels highest, its old-term kernel lowest; the importance stream has slack (it only has
-            // to stay ahead of the code stream): one level below the code stream's critical kernels, old terms lowest
+            // code stream: every kernel highest -- its old-term kernel, wf_old4_kernel, is not singled out here; the importance
+            // stream has slack (it only has to stay ahead of the code stream): one level below, its old-term kernel
+            // (wf_old_kernel) lowest
             const int hi = is_code ? prio_hi : std::min(prio_lo, prio_hi + 2);
-            v.priority = (kp.func == wf_old_kernel_ptr() || kp.func == wf_old2_kernel_ptr()) ? prio_lo : hi;
+            v.priority = kp.func == wf_old_kernel_ptr() ? prio_lo : hi;
             cudaGraphKernelNodeSetAttribute(nodes[i], cudaKernelNodeAttributePriority, &v);
         }
         cudaGetLastError();
@@ -873,7 +818,10 @@ lic360_codec* lic360_codec_create(int device, int H, int W) {
     ok = ok && wf_init(c->code.wf, 48, 4, 3, 3, H, W, c->code.idx_dev, c->code.steps_dev, c->code.ctr_dev, c->code.nsteps, c->code.max_len) == LIC360_OK;
     ok = ok && wf_init(c->imp.wf, 1, 144, 49, 1, H / 2, W / 2, c->imp.idx_dev, c->imp.steps_dev, c->imp.ctr_dev, c->imp.nsteps, c->imp.max_len) == LIC360_OK;
     const bool wf_ok = ok || !pre_ok;
-    if (ok) c->chain_cap = wf_chain_capacity(c->code.wf);
+    if (ok) {
+        c->chain_cap = wf_chain_capacity(c->code.wf);
+        c->code.nflags = c->code.wf.dev.nsets * c->code.wf.cluster;  // at most 3 x 16 of the 64 flags
+    }
     ok = ok && cudaMalloc(&c->levels_dev, (size_t)(H / 2) * (W / 2) * sizeof(float)) == cudaSuccess;
     ok = ok && cudaMalloc(&c->mask192_dev, (size_t)192 * (H / 2) * (W / 2) * sizeof(float)) == cudaSuccess;
     ok = ok && cudaEventCreateWithFlags(&c->ev_est, cudaEventDisableTiming) == cudaSuccess;
@@ -1136,45 +1084,11 @@ long lic360_codec_stream_copy(lic360_codec* c, int stream_id, uint8_t* out, long
     return lic360_coder_get_bytes(stream_id ? c->imp.coder : c->code.coder, out, cap);
 }
 
-// cuStreamWaitValue32 through the runtime's driver entry point lookup (no link-time dependency on libcuda)
-typedef CUresult (*StreamWaitValue32Fn)(CUstream, CUdeviceptr, cuuint32_t, unsigned int);
-static StreamWaitValue32Fn stream_wait_value_fn() {
-    static StreamWaitValue32Fn fn = nullptr;
-    static bool tried = false;
-    if (!tried) {
-        tried = true;
-        void* p = nullptr;
-        cudaDriverEntryPointQueryResult q;
-        if (getenv("LIC360_WF_LAUNCH_AHEAD") &&
-            cudaGetDriverEntryPoint("cuStreamWaitValue32", &p, cudaEnableDefault, &q) == cudaSuccess && q == cudaDriverEntryPointSuccess)
-            fn = reinterpret_cast<StreamWaitValue32Fn>(p);
-        else
-            cudaGetLastError();
-    }
-    return fn;
-}
-
-// releases a stream that may be parked on its go flag, whatever way decode_stream is left (a parked stream never drains)
-struct GoRelease {
-    int* go;
-    ~GoRelease() { __atomic_store_n(go, 0x7fffffff, __ATOMIC_RELEASE); }
-};
-
-// wait for the rows of step p without synchronising the stream (a later kernel of the step graph may still be running)
+// importance stream: wait for the rows of step p without synchronising the stream (a later kernel of the step graph may still be
+// running).  An acquire load: the rows the device wrote before raising the flag are read (non-atomically) by the coder right after.
 static int wait_rows(lic360_codec* c, NetDesc& n, int p) {
-    const int* f = n.flag_host;
     const auto t0 = clk::now();
-    const int nf = n.nflags;
-    bool dev_abort = false;
-    // acquire loads: the rows the device wrote before raising a flag are read (non-atomically) by the coder right after
-    auto ready = [&]() {
-        for (int i = 0; i < nf; i++) {
-            const int v = __atomic_load_n(f + i, __ATOMIC_ACQUIRE);
-            if (v < 0) { dev_abort = true; return true; }
-            if (v != p + 1) return false;
-        }
-        return true;
-    };
+    auto ready = [&]() { return __atomic_load_n(n.flag_host, __ATOMIC_ACQUIRE) == p + 1; };
     for (unsigned spins = 1; !ready(); spins++) {
         if ((spins & 0x3FFF) == 0) {
             if (c->abort_flag.load()) { set_error("codec: aborted (the other stream failed)"); return LIC360_ERR_CUDA; }
@@ -1192,14 +1106,11 @@ static int wait_rows(lic360_codec* c, NetDesc& n, int p) {
 #endif
         if ((spins & 0x7F) == 0) sched_yield();  // several ranks / images per box: do not starve the other polling threads
     }
-    if (dev_abort) {
-        set_error("codec: step %d: a chain cluster gave up waiting for the other nets' clusters (too many decodes in flight on this device?)", p);
-        return LIC360_ERR_CUDA;
-    }
     return LIC360_OK;
 }
 
-// called by the tagged row decoder every few thousand polls of a row that has not arrived: the same give-up conditions as wait_rows
+// code stream: called by the tagged row decoder every few thousand polls of a row that has not arrived.  The give-up conditions of
+// wait_rows, and a negative flag: a chain CTA gave up waiting for the other nets' clusters
 struct StallCtx { lic360_codec* c; NetDesc* n; int p; clk::time_point t0; };
 static int rows_stalled(void* vp) {
     StallCtx* x = static_cast<StallCtx*>(vp);
@@ -1285,17 +1196,13 @@ static int decode_stream_persistent(lic360_codec* c, NetDesc& n) {
     LIC360_CUDA(cudaStreamWaitEvent(side, n.ev_fork, 0));
     LIC360_CUDA(wf_launch_old(n.wf, 0, side, false, 0, n.old_done_dev, n.scat_done_dev));  // old terms of step 0 (all zero; keeps the protocol uniform)
     WfRows rows;
-    memset(&rows, 0, sizeof(rows));
-    rows.rows = n.rows_step_host; rows.levels = c->levels_dev; rows.done = n.done_dev; rows.flag = n.flag_host;
-    rows.sync = n.sync_dev; rows.s2 = (float)(1. / sqrt(2.0)); rows.enabled = 1; rows.rtail = 1; rows.tagged = 1;
-    n.tagged = true;
-    n.nflags = n.wf.dev.nsets * n.wf.cluster;
-    if (n.nflags > 64) { set_error("codec: %d chain CTAs exceed the 64 host flags", n.nflags); return LIC360_ERR_ARG; }
+    rows.rows = n.rows_step_host; rows.levels = c->levels_dev; rows.flag = n.flag_host; rows.sync = n.sync_dev;
+    rows.s2 = (float)(1. / sqrt(2.0));
     WfPersist ps;
     memset(&ps, 0, sizeof(ps));
     ps.syms = n.syms_host; ps.go_host = n.go_host; ps.go_dev = n.go_dev; ps.old_done = n.old_done_dev; ps.ctr = n.ctr_dev; ps.scat_done = n.scat_done_dev;
     ps.bias = -3.5f; ps.scale = 1.0f;
-    LIC360_CUDA(wf_launch_chain(n.wf, s, &rows, &ps));
+    LIC360_CUDA(wf_launch_chain(n.wf, s, rows, &ps));
     int rc = LIC360_OK;
     for (int p = 0; p < n.nsteps; p++) {
         auto tw = clk::now();
@@ -1331,30 +1238,12 @@ static int decode_stream_persistent(lic360_codec* c, NetDesc& n) {
 // The wavefront loop of one bitstream.  is_code: before step p the importance levels of every 2x2 cell the slab touches
 // must be decoded (cells on importance diagonals <= min(p, H+W-2)/2): the loop waits on c->imp_ready, which the
 // importance loop (running concurrently on another host thread and CUDA stream) publishes.
-static bool persistent_ok(const lic360_codec* c, const NetDesc& n) {
-    return c->mode == 2 && n.wf.chain4 && n.wf.r0_inline && n.wf.old2 && !getenv("LIC360_WF_ROWS_KERNEL") && !getenv("LIC360_WF_PREV_KERNEL");
-}
-
 static int decode_stream(lic360_codec* c, NetDesc& n, bool is_code) {
-    if (is_code && persistent_ok(c, n)) return decode_stream_persistent(c, n);
+    if (is_code && c->mode == 2) return decode_stream_persistent(c, n);
     cudaStream_t s = n.stream;
     int rc = LIC360_OK;
     for (int i = 0; i < 64; i++) n.flag_host[i] = 0;
     memset(n.rows_step_host, 0, (size_t)n.max_len * n.row_bytes);  // publication tags of a previous decode must not match step 0
-    // Launch-ahead (experiment, LIC360_WF_LAUNCH_AHEAD=1; measured ~1 ms SLOWER per 512x1024 decode than launching each step's
-    // graph when its symbols are ready, so it is off by default): while the GPU works on step p the host already enqueues
-    // [wait until *go >= p+1][graph of step p+1]; once the symbols of step p are decoded (and, for the code stream, the importance
-    // levels step p+1 needs are there) one store to the mapped flag lets the stream's front end start the step.  The wait is a
-    // stream memory operation (no kernel spins); GoRelease un-parks the stream on every exit path.
-    StreamWaitValue32Fn wait_value = c->mode != 1 ? stream_wait_value_fn() : nullptr;
-    CUdeviceptr go_dev = 0;
-    if (wait_value) {
-        void* dp = nullptr;
-        if (cudaHostGetDevicePointer(&dp, n.go_host, 0) != cudaSuccess) { cudaGetLastError(); wait_value = nullptr; }
-        go_dev = (CUdeviceptr)(uintptr_t)dp;
-    }
-    __atomic_store_n(n.go_host, 0, __ATOMIC_RELEASE);
-    GoRelease go_release{n.go_host};
     n.t_host_coder = 0; n.t_gpu_wait = 0;
     const bool trace_file = getenv("LIC360_WF_TRACE_FILE") != nullptr;
     n.step_wait_us.clear(); n.step_decode_us.clear(); n.step_levels_us.clear();
@@ -1366,32 +1255,18 @@ static int decode_stream(lic360_codec* c, NetDesc& n, bool is_code) {
     LIC360_CUDA(wf_launch_old(n.wf, 1, s));  // old terms of step 0 = counter (-1) + 1 (all zero, but it keeps the schedule uniform)
     if (getenv("LIC360_DEBUG_SYNC")) LIC360_CUDA(cudaStreamSynchronize(s));
     for (int i = 0; i < 5; i++) n.t_kernel[i] = 0;
-    bool ahead = false;  // the graph of the current step is already enqueued (behind its go flag)
     for (int p = 0; p < n.nsteps; p++) {
         auto tw = clk::now();
+        if (is_code) { rc = wait_levels(c, n, p); if (rc) return rc; }
         if (c->mode != 1) {
-            if (!ahead) {
-                if (is_code) { rc = wait_levels(c, n, p); if (rc) return rc; }
-                if (trace_file && is_code) n.step_levels_us.push_back((float)(ms_since(tw) * 1e3));
-                LIC360_CUDA(cudaGraphLaunch(n.graph, s));
-                g_launches += n.graph_nodes;
-            }
-            ahead = false;
-            if (wait_value && p + 1 < n.nsteps) {
-                if (wait_value(s, go_dev, (cuuint32_t)(p + 1), 0 /* CU_STREAM_WAIT_VALUE_GEQ */) == CUDA_SUCCESS) {
-                    LIC360_CUDA(cudaGraphLaunch(n.graph, s));
-                    g_launches += n.graph_nodes;
-                    ahead = true;
-                } else {
-                    wait_value = nullptr;  // not supported here: plain launch per step
-                }
-            }
-            if (!n.tagged) {
+            if (trace_file && is_code) n.step_levels_us.push_back((float)(ms_since(tw) * 1e3));
+            LIC360_CUDA(cudaGraphLaunch(n.graph, s));
+            g_launches += n.graph_nodes;
+            if (!is_code) {
                 rc = wait_rows(c, n, p);
                 if (rc) return rc;
             }
         } else {
-            if (is_code) { rc = wait_levels(c, n, p); if (rc) return rc; }
             rc = launch_step(c, n, is_code, s, s, n.ev_prof);
             if (rc) return rc;
             LIC360_CUDA(cudaStreamSynchronize(s));
@@ -1403,7 +1278,7 @@ static int decode_stream(lic360_codec* c, NetDesc& n, bool is_code) {
         if (!is_code) c->imp_ready.store(p, std::memory_order_release);  // the scatter of this step wrote diagonal p-1
         auto th = clk::now();
         const int len = n.steps[p].len;
-        if (is_code && n.tagged) {
+        if (is_code) {
             StallCtx sc{c, &n, p, clk::now()};
             // time until the first row is there = waiting for the GPU; the rest of the call decodes while the later rows arrive
             for (unsigned spins = 1; ((__atomic_load_n(n.rows_step_host + 7, __ATOMIC_ACQUIRE) >> 4) & 15) != (unsigned)(p % 15 + 1); spins++) {
@@ -1417,16 +1292,11 @@ static int decode_stream(lic360_codec* c, NetDesc& n, bool is_code) {
             th = clk::now();
             rc = coder_decode_packed_gmm_tagged(n.coder, n.rows_step_host, len, n.syms_host, p % 15 + 1, rows_stalled, &sc);
         } else {
-            rc = is_code ? coder_decode_packed_gmm(n.coder, n.rows_step_host, len, n.syms_host)
-                         : coder_decode_packed_imp(n.coder, n.rows_step_host, len, n.syms_host);
+            rc = coder_decode_packed_imp(n.coder, n.rows_step_host, len, n.syms_host);
         }
         n.t_host_coder += ms_since(th);
-        if (trace_file && is_code && n.tagged) n.step_decode_us.push_back((float)(ms_since(th) * 1e3));
+        if (trace_file && is_code) n.step_decode_us.push_back((float)(ms_since(th) * 1e3));
         if (rc) return rc;
-        if (ahead) {
-            if (is_code) { rc = wait_levels(c, n, p + 1); if (rc) return rc; }
-            __atomic_store_n(n.go_host, p + 1, __ATOMIC_RELEASE);  // symbols of step p are in syms_host: step p+1 may run
-        }
     }
     rc = final_scatter(c, n, is_code);
     if (rc) return rc;
@@ -1469,10 +1339,10 @@ int lic360_codec_decode(lic360_codec* c, const uint8_t* imp_bytes, long n_imp, c
     // device -- runs inside the slot: a thread that blocks in the driver while ANOTHER decode's persistent kernel waits for its host
     // would stall that decode's importance-stream launches (observed as a 20 s "levels" time-out under a 7-thread stress).
     std::unique_ptr<ChainSlot> slot;
-    if (c->mode != 1) slot.reset(new ChainSlot(c->device, c->chain_cap, persistent_ok(c, c->code) ? c->chain_cap : 1));
+    if (c->mode != 1) slot.reset(new ChainSlot(c->device, c->chain_cap, c->mode == 2 ? c->chain_cap : 1));
     if (c->mode != 1) {  // both step graphs exist before the second host thread starts (the persistent code stream needs none)
         rc = build_step_graph(c, c->imp, false);
-        if (rc == LIC360_OK && !persistent_ok(c, c->code)) rc = build_step_graph(c, c->code, true);
+        if (rc == LIC360_OK && c->mode != 2) rc = build_step_graph(c, c->code, true);
         if (rc) return rc;
     }
     lic360_coder_start_decoder_mem(c->imp.coder, imp_bytes, n_imp);
@@ -1609,7 +1479,7 @@ int lic360_codec_engine_info(lic360_codec* c, int stream_id, int* out, int n) {
         tail_rounds = wf_tail_rounds(e, idx.data(), d.steps.data());
     }
     const int v[13] = {e.chain1 ? 2 : e.chain4 ? 1 : 0, e.chain1 && e.c1_dsm, e.cluster, e.chain_threads, (int)e.chain_smem, e.max_len,
-                       e.chain1 ? e.c1_lenp : 0, e.chain1 ? e.c1_kpc : 0, e.chain_tasks, e.old4 ? 4 : e.old2 ? 2 : 1, e.parts4,
+                       e.chain1 ? e.c1_lenp : 0, e.chain1 ? e.c1_kpc : 0, e.chain_tasks, e.old4 ? 4 : 1, e.parts4,
                        e.dev.parts, tail_rounds};
     for (int i = 0; i < n && i < 13; i++) out[i] = v[i];
     return LIC360_OK;

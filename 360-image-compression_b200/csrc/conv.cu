@@ -682,8 +682,7 @@ cudaError_t launch_cconv_ec(const ConvArgs& a, cudaStream_t s, bool allow_mma) {
     }
     if (e != cudaSuccess) return e;
     const int nqb = (a.cin_g + CB - 1) / CB;
-    const bool rq_tile_off = getenv("LIC360_EC_RQ_GENERIC") != nullptr;
-    if (a.cin_g == 4 && a.cpg4 == 1 && a.G >= 8 && a.W % 4 == 0 && (reinterpret_cast<uintptr_t>(a.x) & 15) == 0 && !rq_tile_off) {
+    if (a.cin_g == 4 && a.cpg4 == 1 && a.G >= 8 && a.W % 4 == 0 && (reinterpret_cast<uintptr_t>(a.x) & 15) == 0) {
         static SmemAttr rqt_attr;
         e = rqt_attr.ensure(cconv_ec_rq_tile_kernel, RQ4_SMEM_BYTES);
         if (e != cudaSuccess) return e;

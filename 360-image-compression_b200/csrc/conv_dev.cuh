@@ -95,68 +95,12 @@ __device__ __forceinline__ void dc_stage_fma(const float* band, const float4* ws
     }
 }
 
-
-// Two adjacent positions of one diagonal per lane (skewed band, row = kh + kw, BW columns; bw points at the cell of the lane's
-// FIRST position for tap (0, 0) and is 8-byte aligned).  Position i reads band cell [row][kh + i], so one row serves both
-// positions with the cells kh_min .. kh_max + 1: they are fetched as aligned float2 (19 loads per channel instead of 50 scalar
-// ones for the two positions) and each broadcast weight vector is used for 8 FMAs instead of 4.  The old-term kernel is bound by
-// shared-memory wavefronts (a broadcast LDS.128 costs 2, profiles/), not by the FMA pipe: this is where its time goes.
-// Per-accumulator FMA order = the canonical (kh, kw) order of dc_taps_fma.
-template <int BW, int NS>
-__device__ __forceinline__ void dc_taps_fma2(const float* bw, const float4* wrow, float4& u0, float4& u1) {
-    float cell[9][6];
-#pragma unroll
-    for (int r = 0; r < 9; r++) {
-        if (r >= NS) continue;
-        const int khmin = r > 4 ? r - 4 : 0, khmax = r < 4 ? r : 4;
-#pragma unroll
-        for (int m = 0; m < 6; m += 2) {
-            if (m + 1 < khmin || m > khmax + 1) continue;
-            const float2 v = *reinterpret_cast<const float2*>(bw + r * BW + m);
-            cell[r][m] = v.x;
-            cell[r][m + 1] = v.y;
-        }
-    }
-#pragma unroll
-    for (int kh = 0; kh < 5; kh++) {
-#pragma unroll
-        for (int kw = 0; kw < 5; kw++) {
-            if (kh + kw >= NS) continue;
-            const float4 w4 = wrow[kh * 5 + kw];
-            fma4(u0, cell[kh + kw][kh], w4);
-            fma4(u1, cell[kh + kw][kh + 1], w4);
-        }
-    }
-}
-
-template <int BW, int CHS>
-__device__ __forceinline__ void dc_stage_fma2(const float* band, const float4* wsm, int nc, int lane, int chan0, int cin_g, int tc,
-                                              float4& u0, float4& u1) {
-    for (int ch = 0; ch < nc; ch++) {
-        const float* bw = band + ch * CHS + 2 * lane;
-        const float4* wrow = wsm + ch * TAPS;
-        const int bound = tc + 3 - (chan0 + ch) / cin_g;  // warp-uniform
-        if (bound >= 9) { dc_taps_fma2<BW, 9>(bw, wrow, u0, u1); continue; }
-        switch (bound) {
-            case 8: dc_taps_fma2<BW, 8>(bw, wrow, u0, u1); break;
-            case 7: dc_taps_fma2<BW, 7>(bw, wrow, u0, u1); break;
-            case 6: dc_taps_fma2<BW, 6>(bw, wrow, u0, u1); break;
-            case 5: dc_taps_fma2<BW, 5>(bw, wrow, u0, u1); break;
-            case 4: dc_taps_fma2<BW, 4>(bw, wrow, u0, u1); break;
-            case 3: dc_taps_fma2<BW, 3>(bw, wrow, u0, u1); break;
-            case 2: dc_taps_fma2<BW, 2>(bw, wrow, u0, u1); break;
-            case 1: dc_taps_fma2<BW, 1>(bw, wrow, u0, u1); break;
-            default: break;
-        }
-    }
-}
-
 // Four adjacent positions of one diagonal per lane: 16 lanes cover 64 positions, and the other half-warp works on the NEXT diagonal
 // of the same band (its band rows are one further down, its weight vectors belong to the next lower output group).  bw points at the
 // 16-byte aligned cell of the lane's FIRST position for tap (0, 0); position i reads band cell [row][kh + i], so a row serves the four
-// positions with the cells kh_min .. kh_max + 3: at most two aligned float4 (16 loads per channel for 400 FMAs; the two-position form
-// needs 19 float2 for 200).  A weight vector is one LDS.128 with ONE ADDRESS PER HALF-WARP -- the cost of a broadcast, 2 wavefronts
-// (tools/lds_probe.cu) -- and feeds 16 FMAs instead of 8.  Per-accumulator FMA order = the canonical (kh, kw) order of dc_taps_fma.
+// positions with the cells kh_min .. kh_max + 3: at most two aligned float4 (16 loads per channel for 400 FMAs).  A weight vector is
+// one LDS.128 with ONE ADDRESS PER HALF-WARP -- the cost of a broadcast, 2 wavefronts (tools/lds_probe.cu) -- and feeds 16 FMAs.
+// Per-accumulator FMA order = the canonical (kh, kw) order of dc_taps_fma.
 template <int BW, int NS>
 __device__ __forceinline__ void dc_taps_fma4(const float* bw, const float4* wrow, float4 (&u)[4]) {
     float cell[9][8];

@@ -105,11 +105,11 @@ __device__ __forceinline__ WfTile wf_tile(const WfNetDev& net, int dp, int l0 = 
 constexpr int WF_OLD_WARPS = 4;  // warps per CTA; warp w walks the canonical blocks w, w+4, ... that have old terms
 
 __global__ void __launch_bounds__(32 * WF_OLD_WARPS) wf_old_kernel(const __grid_constant__ WfNetDev net,
-                                                                  const __grid_constant__ WfMaps maps, int dp, int l0) {
+                                                                  const __grid_constant__ WfMaps maps, int dp) {
     extern __shared__ unsigned char wf_raw[];
     // grid = ((layer, net), chunk, (diagonal, part)): CTAs are dispatched x-fastest, so the tiles of the LARGEST output
     // groups (most old terms) of every layer start first and the light ones fill the tail
-    const WfTile t = wf_tile(net, dp, l0, true);
+    const WfTile t = wf_tile(net, dp, 0, true);
     if (!t.ok) return;  // CTA-uniform
     if (threadIdx.x == 0 && threadIdx.y == 0) WF_TRACE_MIN(net.G, t.psum - dp, WF_TR_OLD0);
     const WfLayerDev& L = net.L[t.l];
@@ -166,111 +166,9 @@ __global__ void __launch_bounds__(32 * WF_OLD_WARPS) wf_old_kernel(const __grid_
     if (threadIdx.x == 0 && threadIdx.y == 0) WF_TRACE_MAX(net.G, t.psum - dp, WF_TR_OLD1);
 }
 
-// ------------------------------------------------------------------------------------------------ old terms, 2 positions / lane
-// Same tile decomposition as wf_old_kernel but a CTA covers 64 consecutive positions of the diagonal and every lane owns two
-// ADJACENT ones (dc_taps_fma2): the tile starts at the even position below hmin so that the float2 band reads are aligned, the
-// TMA box is {72 h, 9 d, 2 c} starting at the multiple of 4 below (tile start - 2).  Two channels per stage: the same bytes,
-// MACs and shared memory per stage (hence the same 6 CTAs per SM) as the one-position kernel's 4-channel stage over 32
-// positions, with 176 instead of 300 shared-memory load wavefronts.
-constexpr int WF2_STAGE = 2;
-constexpr int WF2_BOX_W = 72;
-constexpr int WF2_BAND = 9 * WF2_BOX_W;
-constexpr int WF2_BAND_BYTES = WF2_STAGE * WF2_BAND * 4;
-constexpr int WF2_STAGE_BYTES = ((WF2_BAND_BYTES + WF2_STAGE * TAPS * 16 + 127) / 128) * 128;
-
-__global__ void __launch_bounds__(32 * WF_OLD_WARPS) wf_old2_kernel(const __grid_constant__ WfNetDev net,
-                                                                   const __grid_constant__ WfMaps maps, int dp, int l0, int parts2, int psum_x,
-                                                                   const int* __restrict__ scat_done) {
-    extern __shared__ unsigned char wf_raw[];
-    // grid = ((layer, net), chunk, (diagonal, part)), x fastest: the heaviest output groups of every layer start first
-    const int bx = blockIdx.z, bz = blockIdx.x;
-    const int l = l0 + bz / net.nsets, n = bz % net.nsets, kc = blockIdx.y;
-    const int psum = psum_x >= 0 ? psum_x : *net.ctr + dp;  // explicit step: persistent decode (the host paces the steps)
-    if (kc >= net.L[l].cpg4 || psum >= net.nsteps) return;
-    const int la = max(0, psum - net.G + 1), lb = min(psum, net.H + net.W - 2);
-    const int d = la + bx / parts2;
-    if (d > lb) return;
-    const int hmin = max(0, d - net.W + 1), hmax = min(net.H - 1, d);
-    const int hb = (hmin & ~1) + (bx % parts2) * 64;   // even: the lane's pair (hb + 2 lane, hb + 2 lane + 1) is float2-aligned
-    if (hb > hmax) return;                             // CTA-uniform
-    const int tc = psum - d;
-    if (threadIdx.x == 0 && threadIdx.y == 0) WF_TRACE_MIN(net.G, psum - dp, WF_TR_OLD0);
-    if (scat_done && l == 0) {
-        // persistent decode: this launch was enqueued right behind the host's go for step psum - 1; layer 0 reads the symbols of steps
-        // <= psum - 2, which the chain kernel scatters at the top of step psum - 1 -- normally long done, but not ordered by any stream
-        if (threadIdx.x == 0 && threadIdx.y == 0) {
-            unsigned long long t0 = 0, t1 = 0;
-            for (unsigned spins = 1; reinterpret_cast<const volatile int*>(scat_done)[n] < psum - 1; spins++)
-                if ((spins & 0xFFF) == 0) {
-                    asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t1));
-                    if (t0 == 0) t0 = t1;
-                    else if (t1 - t0 > 5000000000ull) break;
-                }
-            __threadfence();
-        }
-        __syncthreads();
-    }
-    const WfLayerDev& L = net.L[l];
-    const unsigned raw_s = (unsigned)__cvta_generic_to_shared(wf_raw);
-    unsigned char* base = wf_raw + ((128u - (raw_s & 127u)) & 127u);                            // 128-B aligned
-    float4* part = reinterpret_cast<float4*>(base + (size_t)WF_OLD_WARPS * WF2_STAGE_BYTES);   // [nblk][64]
-    unsigned long long* bars = reinterpret_cast<unsigned long long*>(part + L.nblk * 64);      // [WF_OLD_WARPS]
-    const int lane = threadIdx.x, seg = threadIdx.y;
-    float* band = reinterpret_cast<float*>(base + (size_t)seg * WF2_STAGE_BYTES);
-    float4* wsm = reinterpret_cast<float4*>(band + WF2_STAGE * WF2_BAND);
-    const unsigned band_s = (unsigned)__cvta_generic_to_shared(band);
-    const unsigned wsm_s = band_s + WF2_BAND_BYTES;
-    const int h0 = (hb - 2 + WF_HSHIFT) & ~3;          // aligned box start, in frame columns (row h = column h + WF_HSHIFT)
-    const float* bandl = band + (hb - 2 + WF_HSHIFT - h0);   // 0 or 2 floats in
-    const unsigned bar = (unsigned)__cvta_generic_to_shared(bars + seg);
-    if (lane == 0) {
-        mbar_init(bar, 1);
-        asm volatile("fence.mbarrier_init.release.cluster;\n" ::: "memory");
-    }
-    __syncthreads();
-    const int Cin = L.Cin;
-    const int lim = min(Cin, (tc + 3) * L.cin_g);  // old terms: g_in <= tc + 2
-    const int nact = (lim + CB - 1) / CB;          // canonical blocks that have old terms
-    const int chunk = tc * L.cpg4 + kc;
-    unsigned phase = 0;
-    for (int j = seg; j < nact; j += WF_OLD_WARPS) {
-        float4 u0 = make_float4(0.f, 0.f, 0.f, 0.f), u1 = u0;
-        const int cb = min(CB, Cin - j * CB);
-        const float4* wp4 = reinterpret_cast<const float4*>(L.wp) + (((size_t)n * L.nchunk + chunk) * Cin + j * CB) * TAPS;
-        for (int c0 = 0; c0 < cb && j * CB + c0 < lim; c0 += WF2_STAGE) {
-            const int nc = min(WF2_STAGE, cb - c0);
-            __syncwarp();  // every lane is done with the previous stage
-            if (lane == 0) {
-                mbar_expect_tx(bar, WF2_BAND_BYTES + nc * TAPS * 16);
-                tma_load_3d(band_s, &maps.tm[l], h0, d - 4, n * Cin + j * CB + c0, bar);
-                bulk_load(wsm_s, wp4 + c0 * TAPS, nc * TAPS * 16, bar);
-            }
-            mbar_wait(bar, phase);
-            phase ^= 1;
-            dc_stage_fma2<WF2_BOX_W, WF2_BAND>(bandl, wsm, nc, lane, j * CB + c0, L.cin_g, tc, u0, u1);
-        }
-        part[j * 64 + 2 * lane] = u0;
-        part[j * 64 + 2 * lane + 1] = u1;
-    }
-    __syncthreads();
-    // the block sums in canonical order: warp 0 finishes the even positions, warp 1 the odd ones
-    if (seg < 2) {
-        const int pos = 2 * lane + seg, h = hb + pos;
-        if (h >= hmin && h <= hmax) {
-            float4 P = make_float4(0.f, 0.f, 0.f, 0.f);
-            for (int j = 0; j < nact; j++) {  // blocks without old terms add nothing (the encoder skips them too)
-                const float4 v = part[j * 64 + pos];
-                P.x = P.x + v.x; P.y = P.y + v.y; P.z = P.z + v.z; P.w = P.w + v.w;
-            }
-            L.pbuf[psum & 1][(((size_t)n * L.cpg4 + kc) * net.D + d) * net.HS + h] = P;
-        }
-    }
-    if (threadIdx.x == 0 && threadIdx.y == 0) WF_TRACE_MAX(net.G, psum - dp, WF_TR_OLD1);
-}
-
 // ------------------------------------------------------------------------------------------------ old terms, 4 positions / lane
-// The old-term kernels are bound by shared-memory load wavefronts, and the two-position form spends 50 of its 88 per channel on the 25
-// weight vectors.  Here a warp takes TWO neighbouring diagonals of the slab -- output groups tc and tc - 1 -- 64 positions each:
+// The old-term kernels are bound by shared-memory load wavefronts, and a two-positions-per-lane form spends 50 of its 88 per channel on
+// the 25 weight vectors.  Here a warp takes TWO neighbouring diagonals of the slab -- output groups tc and tc - 1 -- 64 positions each:
 // 16 lanes per diagonal, four adjacent positions per lane (dc_taps_fma4).  Both diagonals read the SAME input channels around the same
 // rows, one diagonal apart: one TMA box {72 h, 10 d, 2 c} serves both (the second half-warp's band rows are one further down), and
 // each half-warp reads its own group's weight vector with a single LDS.128 (two addresses per instruction cost what a broadcast
@@ -286,13 +184,13 @@ constexpr int WF4_W_BYTES = WF4_STAGE * TAPS * 16;  // weight vectors of one hal
 constexpr int WF4_STAGE_BYTES = ((WF4_BAND_BYTES + 2 * WF4_W_BYTES + 127) / 128) * 128;
 
 __global__ void __launch_bounds__(32 * WF_OLD_WARPS) wf_old4_kernel(const __grid_constant__ WfNetDev net,
-                                                                   const __grid_constant__ WfMaps maps, int dp, int l0, int parts4, int psum_x,
+                                                                   const __grid_constant__ WfMaps maps, int dp, int parts4, int psum_x,
                                                                    const int* __restrict__ scat_done) {
     extern __shared__ unsigned char wf_raw[];
     // grid = ((layer, net), 1, (diagonal pair, part)), x fastest: the heaviest output groups of every layer start first
     const int bx = blockIdx.z, bz = blockIdx.x;
-    const int l = l0 + bz / net.nsets, n = bz % net.nsets;
-    const int psum = psum_x >= 0 ? psum_x : *net.ctr + dp;
+    const int l = bz / net.nsets, n = bz % net.nsets;
+    const int psum = psum_x >= 0 ? psum_x : *net.ctr + dp;  // explicit step: persistent decode (the host paces the steps)
     if (psum >= net.nsteps) return;
     const int la = max(0, psum - net.G + 1), lb = min(psum, net.H + net.W - 2);
     const int dA = la + 2 * (bx / parts4);  // half-warp 0: diagonal dA, group tcA; half-warp 1: diagonal dA + 1, group tcA - 1
@@ -304,7 +202,9 @@ __global__ void __launch_bounds__(32 * WF_OLD_WARPS) wf_old4_kernel(const __grid
     if (hb > max(hmaxA, hmaxB)) return;                // CTA-uniform
     const int tcA = psum - dA;
     if (threadIdx.x == 0 && threadIdx.y == 0) WF_TRACE_MIN(net.G, psum - dp, WF_TR_OLD0);
-    if (scat_done && l == 0) {  // persistent decode: see wf_old2_kernel
+    if (scat_done && l == 0) {
+        // persistent decode: this launch was enqueued right behind the host's go for step psum - 1; layer 0 reads the symbols of steps
+        // <= psum - 2, which the chain kernel scatters at the top of step psum - 1 -- normally long done, but not ordered by any stream
         if (threadIdx.x == 0 && threadIdx.y == 0) {
             unsigned long long t0 = 0, t1 = 0;
             for (unsigned spins = 1; reinterpret_cast<const volatile int*>(scat_done)[n] < psum - 1; spins++)
@@ -821,7 +721,7 @@ __device__ __noinline__ void wf_chain4_rows(const WfNetDev& net, const WfRows& r
     __threadfence();
     __syncthreads();
     // the layer loop is done with the weight buffers: warps 1.. fill them with the R rows of the tail while thread 0 meets the other clusters
-    if (rows.rtail && tail.nloc > 0) wf_tail_stage(net, n, tail, 1, min(tail.lpg, WF_LAYERS - 1), tid, 32, nt - 32);
+    if (tail.nloc > 0) wf_tail_stage(net, n, tail, 1, min(tail.lpg, WF_LAYERS - 1), tid, 32, nt - 32);
     if (tid == 0) {
         atomicAdd(rows.sync, 1);
         const int target = (psum + 1) * (int)gridDim.x;
@@ -884,22 +784,11 @@ __device__ __noinline__ void wf_chain4_rows(const WfNetDev& net, const WfRows& r
         if (live && j == 0) {
             fixup_row(o, 8, true);
             const int lvl = (int)(__ldcg(rows.levels + (th >> 1) * (W >> 1) + (tw >> 1)) + 1e-5f);  // written by the other stream's kernels
-            pack_gmm_row(o, 0, code_mask_from_level(lvl, tc, th, tw), rows.rows + (size_t)li * 8, rows.tagged ? psum % 15 + 1 : 0);
+            pack_gmm_row(o, 0, code_mask_from_level(lvl, tc, th, tw), rows.rows + (size_t)li * 8, psum % 15 + 1);
         }
     }
-    if (rows.tagged) {  // self-validating rows: no fence, no flag; the host decodes row i as soon as row i carries this step's tag
-        if (tid == 0) WF_TRACE_MAX(net.G, psum, WF_TR_ROWS1);
-        return;
-    }
-    // every CTA raises its own host flag once its rows are on their way (the host waits for all of them): no second
-    // device-wide counter round and no second system fence between the last row and the flag
-    __threadfence_system();
-    __syncthreads();
-    if (tid == 0) {
-        __threadfence_system();  // thread 0's own fence between the barrier and the flag (as rows_done() in codec.cu)
-        reinterpret_cast<volatile int*>(rows.flag)[blockIdx.x] = psum + 1;
-        WF_TRACE_MAX(net.G, psum, WF_TR_ROWS1);
-    }
+    // self-validating rows: no fence, no flag; the host decodes row i as soon as row i carries this step's tag
+    if (tid == 0) WF_TRACE_MAX(net.G, psum, WF_TR_ROWS1);
 }
 
 // Previous-wavefront terms R of step psum1 = p + 1, layers 1..11, evaluated by the chain kernel of step p right behind its CDF
@@ -1092,7 +981,7 @@ __device__ __noinline__ bool wf_chain4_step_begin(const WfNetDev& net, const WfP
 }
 
 __global__ void __launch_bounds__(384, 1) wf_chain4_kernel(const __grid_constant__ WfNetDev net, int nc, int rows_cap,
-                                                         const __grid_constant__ WfRows rows, int r0_inline,
+                                                         const __grid_constant__ WfRows rows,
                                                          const __grid_constant__ WfPersist persist, int smem_rows) {
     extern __shared__ float4 wf_wsm[];  // [2][rows_cap][WF_ROW_F4]
     const int tid = threadIdx.x, nt = blockDim.x;
@@ -1133,8 +1022,8 @@ __global__ void __launch_bounds__(384, 1) wf_chain4_kernel(const __grid_constant
         if (!wf_chain4_step_begin(net, persist, step, n, rank, nc, tid, nt)) return;
         if (threadIdx.x == 0) WF_TRACE_MIN(net.G, sd.psum, WF_TR_CHAIN0);
     }
-    // no launch computed layer 0's R for this step
-    if (has0 && r0_inline) pre.rr = persist.enabled ? wf_r_layer0_c1<true>(net, n, d0, h0, tc0) : wf_r_layer0_c1<false>(net, n, d0, h0, tc0);
+    // layer 0's previous-wavefront terms read the symbols of step p - 1: evaluated here, not a step ahead like the other layers'
+    if (has0) pre.rr = persist.enabled ? wf_r_layer0_c1<true>(net, n, d0, h0, tc0) : wf_r_layer0_c1<false>(net, n, d0, h0, tc0);
     // debug timeline (LIC360_WF_TRACE=1): ns spent by thread 0 of CTA 0 in the phases of every layer, accumulated behind the step slots
     const bool phase_trace = g_wf_trace && g_wf_trace_sel == 0 && blockIdx.x == 0 && tid == 0;
     unsigned long long tph = 0;
@@ -1167,7 +1056,7 @@ __global__ void __launch_bounds__(384, 1) wf_chain4_kernel(const __grid_constant
                 d = h + __ldg(net.idx + k + HW);
                 tc = sd.psum - d;
                 wf_chain4_prefetch(net, L, n, par, d, h, tc, p);
-                if (l == 0 && r0_inline) p.rr = persist.enabled ? wf_r_layer0_c1<true>(net, n, d, h, tc) : wf_r_layer0_c1<false>(net, n, d, h, tc);
+                if (l == 0) p.rr = persist.enabled ? wf_r_layer0_c1<true>(net, n, d, h, tc) : wf_r_layer0_c1<false>(net, n, d, h, tc);
             }
             float4 u = make_float4(0.f, 0.f, 0.f, 0.f);
             if (L.has_q) {
@@ -1243,11 +1132,9 @@ __global__ void __launch_bounds__(384, 1) wf_chain4_kernel(const __grid_constant
         phase(l, 3);
     }
     if (threadIdx.x == 0) WF_TRACE_MAX(net.G, sd.psum, WF_TR_CHAIN1);
-    if (rows.enabled) {
-        const WfTailPlan tail = wf_tail_plan(net, rank, nc, sd.psum + 1, smem_rows);
-        wf_chain4_rows(net, rows, sd.psum, sd.start, sd.len, tid, nt, n, tail);
-        if (rows.rtail) wf_chain4_rtail(net, n, sd.psum + 1, tid, nt, tail);
-    }
+    const WfTailPlan tail = wf_tail_plan(net, rank, nc, sd.psum + 1, smem_rows);
+    wf_chain4_rows(net, rows, sd.psum, sd.start, sd.len, tid, nt, n, tail);
+    wf_chain4_rtail(net, n, sd.psum + 1, tid, nt, tail);
     if (persist.enabled) {  // the next step prefetches the R sums the tail just stored (other CTAs of the cluster) before its go
         if (nc > 1) cg::this_cluster().sync();
         else __syncthreads();
@@ -1268,7 +1155,7 @@ __global__ void __launch_bounds__(384, 1) wf_chain4_kernel(const __grid_constant
 // activation reads (row stride cin_g + 4) feeds kpc independent accumulator chains, weights are broadcasts.
 constexpr int C1_KB = 3;  // chunks a warp accumulates together
 __global__ void __launch_bounds__(384, 1) wf_chain1_kernel(const __grid_constant__ WfNetDev net, int nc, int kpc, int lenp,
-                                                         int cmax, WfRows rows, int r0_inline, int dsm) {
+                                                         int cmax, WfRows rows, int dsm) {
     extern __shared__ float4 wf_sm1[];
     __shared__ unsigned long long wbar_mem;  // mbarrier of the weight staging
     cg::cluster_group cluster = cg::this_cluster();
@@ -1341,7 +1228,7 @@ __global__ void __launch_bounds__(384, 1) wf_chain1_kernel(const __grid_constant
         pre.pr = __ldg(L.pbuf[par] + (((size_t)n * L.cpg4 + kc) * net.D + d) * net.HS + h);
         // layer 0 reads the symbols the scatter kernel wrote a moment ago: its previous-wavefront terms are evaluated here instead
         // of by one more launch in front of the chain
-        if (l == 0 && r0_inline) pre.rr = wf_r_layer0_c1(net, n, d, h, 0, kc);
+        if (l == 0) pre.rr = wf_r_layer0_c1(net, n, d, h, 0, kc);
         else pre.rr = __ldg(L.rbuf[par] + (((size_t)n * L.cpg4 + kc) * net.D + d) * net.HS + h);
         const size_t fc = wf_fc_index(net.Dp, net.Hp, 1, L.cout_g, n, d, 0, h) + kc * 4;
 #pragma unroll
@@ -1431,7 +1318,7 @@ __global__ void __launch_bounds__(384, 1) wf_chain1_kernel(const __grid_constant
             WfPre p = pre;
             if (it != tid) {  // further slots (more items than threads): nothing was prefetched
                 p.pr = __ldg(L.pbuf[par] + (((size_t)n * L.cpg4 + kc) * net.D + d) * net.HS + h);
-                if (l == 0 && r0_inline) p.rr = wf_r_layer0_c1(net, n, d, h, 0, kc);
+                if (l == 0) p.rr = wf_r_layer0_c1(net, n, d, h, 0, kc);
                 else p.rr = __ldg(L.rbuf[par] + (((size_t)n * L.cpg4 + kc) * net.D + d) * net.HS + h);
                 const size_t fcr = wf_fc_index(net.Dp, net.Hp, 1, L.cout_g, n, d, 0, h) + kc * 4;
 #pragma unroll
@@ -1470,7 +1357,7 @@ __global__ void __launch_bounds__(384, 1) wf_chain1_kernel(const __grid_constant
                     *reinterpret_cast<float4*>(dst) = v4;
                 }
             }
-            if (rows.enabled && l == WF_LAYERS - 1) {  // logits of the CDF rows, gathered in CTA 0
+            if (l == WF_LAYERS - 1) {  // logits of the CDF rows, gathered in CTA 0
                 float* yd = ylog + (size_t)pos * 52 + kc * 4;
                 if (nc > 1) yd = cluster.map_shared_rank(yd, 0);
 #pragma unroll
@@ -1498,7 +1385,6 @@ __global__ void __launch_bounds__(384, 1) wf_chain1_kernel(const __grid_constant
         phase(l, 3);
     }
     if (tid == 0) WF_TRACE_MAX(net.G, sd.psum, WF_TR_CHAIN1);
-    if (!rows.enabled) return;
     // CDF rows of the step (EntropyTable over the 49 logits of every position): the last layer's epilogues stored the logits into
     // CTA 0's shared memory; one warp per symbol, then the host flag -- no further launch on the critical path of the stream
     if (nc > 1) cluster.sync();
@@ -1556,7 +1442,19 @@ int wf_init(WfEngine& e, int G, int cpg, int nlast, int nsets, int H, int W, con
         e.cpg4_max = std::max(e.cpg4_max, L.cpg4); e.nblk_max = std::max(e.nblk_max, L.nblk); e.nqb_max = std::max(e.nqb_max, L.nqb);
         pb += 4 * (size_t)nsets * L.cpg4 * n.D * n.HS;  // P and R, two step parities each
     }
-    if (e.nblk_max > 32 || e.nqb_max > 32) { set_error("wavefront engine: too many channels"); return LIC360_ERR_ARG; }
+    if (e.nblk_max > 32) { set_error("wavefront engine: too many channels"); return LIC360_ERR_ARG; }
+    // wf_prev_kernel runs one warp per canonical 16-channel block of a group's input channels, at most 10
+    if (e.nqb_max > 10) { set_error("wavefront engine: more than 160 input channels per group"); return LIC360_ERR_ARG; }
+    // a many-group net runs wf_chain4_kernel and wf_old4_kernel: at most 64 groups, one output chunk (<= 4 channels) per group
+    // in every layer, 4 input channels per group in every layer after the first
+    e.chain4 = G > 1 && G <= 64;
+    for (int l = 0; l < WF_LAYERS; l++) e.chain4 = e.chain4 && n.L[l].cpg4 == 1 && (l == 0 || n.L[l].cin_g == 4);
+    if (G > 1 && !e.chain4) {
+        set_error("wavefront engine: a many-group net needs at most 64 groups, at most 4 output channels per group and 4 input "
+                  "channels per group after the first layer");
+        return LIC360_ERR_ARG;
+    }
+    e.old4 = G > 1;
     for (int i = 0; i <= WF_LAYERS; i++) {
         e.fc_floats[i] = (size_t)nsets * n.Dp * (G + 2 * WF_GPAD) * n.Hp * (e.C[i] / G);
         LIC360_CUDA(cudaMalloc(&e.fc[i], e.fc_floats[i] * sizeof(float)));
@@ -1584,16 +1482,12 @@ int wf_init(WfEngine& e, int G, int cpg, int nlast, int nsets, int H, int W, con
     for (int l = 0; l < WF_LAYERS; l++) {
         const cuuint64_t dims[3] = {(cuuint64_t)n.HS, (cuuint64_t)n.D, (cuuint64_t)nsets * e.C[l]};
         const cuuint64_t strides[2] = {(cuuint64_t)n.HS * 4, (cuuint64_t)n.D * n.HS * 4};
-        const cuuint32_t box[3] = {WF_BOX_W, 9, WF_STAGE}, box2[3] = {WF2_BOX_W, 9, WF2_STAGE};
+        const cuuint32_t box[3] = {WF_BOX_W, 9, WF_STAGE};
         const cuuint32_t estr[3] = {1, 1, 1};
         CUresult r = enc(&e.maps.tm[l], CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 3, e.fp[l], dims, strides, box, estr,
                          CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_L2_128B,
                          CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
         if (r != CUDA_SUCCESS) { set_error("wavefront engine: cuTensorMapEncodeTiled failed (%d) for layer %d", (int)r, l); return LIC360_ERR_CUDA; }
-        r = enc(&e.maps2.tm[l], CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 3, e.fp[l], dims, strides, box2, estr,
-                CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_L2_128B,
-                CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-        if (r != CUDA_SUCCESS) { set_error("wavefront engine: cuTensorMapEncodeTiled (72-wide box) failed (%d) for layer %d", (int)r, l); return LIC360_ERR_CUDA; }
         const cuuint32_t box4[3] = {WF4_BOX_W, WF4_ROWS, WF4_STAGE};
         r = enc(&e.maps4.tm[l], CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 3, e.fp[l], dims, strides, box4, estr,
                 CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_L2_128B,
@@ -1602,15 +1496,9 @@ int wf_init(WfEngine& e, int G, int cpg, int nlast, int nsets, int H, int W, con
     }
     // launch shapes
     e.old_smem = 128 + (size_t)WF_OLD_WARPS * WF_STAGE_BYTES + (size_t)e.nblk_max * 32 * sizeof(float4) + (size_t)WF_OLD_WARPS * 8;
-    // two positions per lane for the many-group nets (LIC360_WF_OLD1=1: the one-position kernel).  The single-group net keeps the
+    // four positions per lane, two diagonals per warp for the many-group nets (e.old4).  The single-group net keeps the
     // one-position kernel: its diagonals are short (half-empty warps) and its old-term launch is latency-, not throughput-critical
     // (twice as many TMA round trips per warp made the importance stream gate the code stream at 2048x4096).
-    e.old2 = G > 1 && getenv("LIC360_WF_OLD1") == nullptr;
-    // a diagonal with an odd first row starts its tile one position early; only when H > W can such a diagonal have full length
-    e.parts2 = (std::min(H, W) + (H > W ? 1 : 0) + 63) / 64;
-    e.old2_smem = 128 + (size_t)WF_OLD_WARPS * WF2_STAGE_BYTES + (size_t)e.nblk_max * 64 * sizeof(float4) + (size_t)WF_OLD_WARPS * 8;
-    // four positions per lane, two diagonals per warp: nets with one output chunk per group (LIC360_WF_OLD2=1: the two-position kernel)
-    e.old4 = e.old2 && e.cpg4_max == 1 && getenv("LIC360_WF_OLD2") == nullptr;
     e.parts4 = 1;
     for (int d = 0; d < n.D; d++) {  // a diagonal's tile starts at the multiple of 4 below its first row
         const int hmin = std::max(0, d - W + 1), hmax = std::min(H - 1, d);
@@ -1622,11 +1510,9 @@ int wf_init(WfEngine& e, int G, int cpg, int nlast, int nsets, int H, int W, con
     e.prev_smem = ((size_t)e.prev_wcap + (size_t)e.nqb_max * 32) * sizeof(float4);
     // the attribute is per kernel AND per device, not per engine: only ever raise it (two engines with different channel counts
     // share it), and remember it for every device separately (SmemAttr, common.cuh)
-    static SmemAttr prev_attr_a, prev_attr_b, old_attr, old2_attr, old4_attr, chain_attr_g, chain_attr_4, chain_attr_1;
-    LIC360_CUDA(prev_attr_a.ensure(wf_prev_kernel<320>, e.prev_smem));
-    LIC360_CUDA(prev_attr_b.ensure(wf_prev_kernel<1024>, e.prev_smem));
+    static SmemAttr prev_attr, old_attr, old4_attr, chain_attr_g, chain_attr_4, chain_attr_1;
+    LIC360_CUDA(prev_attr.ensure(wf_prev_kernel<320>, e.prev_smem));
     LIC360_CUDA(old_attr.ensure(wf_old_kernel, e.old_smem));
-    LIC360_CUDA(old2_attr.ensure(wf_old2_kernel, e.old2_smem));
     LIC360_CUDA(old4_attr.ensure(wf_old4_kernel, e.old4_smem));
     // chain kernels: one cluster per net.  16 CTAs (non-portable size, opt-in) when the device can co-schedule them,
     // else the portable maximum of 8.
@@ -1636,7 +1522,6 @@ int wf_init(WfEngine& e, int G, int cpg, int nlast, int nsets, int H, int W, con
     // many-group nets (3 clusters, old-term kernel running beside them): 8 CTAs each measured best; the single-group net
     // has one cluster and splits output chunks: 16
     int want = G > 1 ? 8 : 16;
-    if (const char* s = getenv("LIC360_WF_CLUSTER")) want = std::max(1, std::min(16, atoi(s)));
     if (const char* s = getenv(G > 1 ? "LIC360_WF_CLUSTER_CODE" : "LIC360_WF_CLUSTER_IMP")) want = std::max(1, std::min(16, atoi(s)));
     // the one limit of every chain kernel's dynamic shared memory: the per-block opt-in maximum (227 KB on B200) minus the largest
     // static shared memory of the three kernels
@@ -1660,13 +1545,9 @@ int wf_init(WfEngine& e, int G, int cpg, int nlast, int nsets, int H, int W, con
         e.chain_threads = std::min(384, std::max(128, ((tasks_max + 31) / 32) * 32));
         e.chain_tasks = tasks_max;
         e.chain_smem = (size_t)tasks_max * sizeof(float4);
-        e.chain4 = G > 1 && G <= 64;
-        for (int l = 0; l < WF_LAYERS; l++) e.chain4 = e.chain4 && n.L[l].cpg4 == 1 && (l == 0 || n.L[l].cin_g == 4);
         e.chain1 = G == 1;
         e.c1_cmax = 4;
         for (int l = 1; l < WF_LAYERS; l++) { e.chain1 = e.chain1 && (n.L[l].cin_g & 3) == 0; e.c1_cmax = std::max(e.c1_cmax, n.L[l].cin_g); }
-        if (getenv("LIC360_WF_GENERIC_CHAIN")) e.chain4 = e.chain1 = false;
-        e.r0_inline = ((e.chain4 && n.L[0].cpg4 == 1) || e.chain1) && n.L[0].cin_g == 1 && !getenv("LIC360_WF_R0_KERNEL");
         if (e.chain4) e.chain_smem = (size_t)2 * G * WF_ROW_F4 * sizeof(float4);
         if (e.chain1) {
             e.c1_kpc = (e.cpg4_max + e.cluster - 1) / e.cluster;
@@ -1683,7 +1564,7 @@ int wf_init(WfEngine& e, int G, int cpg, int nlast, int nsets, int H, int W, con
         if (e.chain_smem > cap) { set_error("wavefront engine: slab too large for the chain kernel"); return LIC360_ERR_ARG; }
         // The old-term kernel of the next step runs concurrently (programmatic dependent launch): claim the whole shared
         // memory of the SM so that none of its CTAs lands next to a chain CTA and steals its issue slots.
-        if (!getenv("LIC360_WF_SHARE_SM")) e.chain_smem = std::max(e.chain_smem, (size_t)196 * 1024);
+        e.chain_smem = std::max(e.chain_smem, (size_t)196 * 1024);
         LIC360_CUDA(chain_attr_g.ensure(wf_chain_kernel<384>, e.chain_smem));
         LIC360_CUDA(chain_attr_4.ensure(wf_chain4_kernel, e.chain_smem));
         LIC360_CUDA(chain_attr_1.ensure(wf_chain1_kernel, e.chain_smem));
@@ -1736,7 +1617,6 @@ int wf_tail_rounds(const WfEngine& e, const int32_t* idx, const StepDesc* steps)
 }
 
 const void* wf_old_kernel_ptr() { return reinterpret_cast<const void*>(&wf_old_kernel); }
-const void* wf_old2_kernel_ptr() { return reinterpret_cast<const void*>(&wf_old2_kernel); }
 
 void wf_set_layer(WfEngine& e, int l, const float* wp, const float* wq, const float* bias, const float* slope) {
     WfLayerDev& L = e.dev.L[l];
@@ -1765,32 +1645,24 @@ __global__ void wf_old_done_kernel(int* done, int value) {
 }
 
 cudaError_t wf_launch_old(const WfEngine& e, int dp, cudaStream_t s, bool programmatic, int psum, int* done, const int* scat_done) {
+    if (psum >= 0 && !e.old4) return cudaErrorInvalidValue;  // explicit steps: many-group engines only
     const WfNetDev& n = e.dev;
     cudaLaunchConfig_t cfg;
     memset(&cfg, 0, sizeof(cfg));
+    cfg.gridDim = e.old4 ? dim3(WF_LAYERS * n.nsets, 1, ((n.ndiag + 1) / 2) * e.parts4)
+                         : dim3(WF_LAYERS * n.nsets, e.cpg4_max, n.ndiag * n.parts);
     cfg.blockDim = dim3(32, WF_OLD_WARPS);
-    cfg.dynamicSmemBytes = e.old4 ? e.old4_smem : e.old2 ? e.old2_smem : e.old_smem;
+    cfg.dynamicSmemBytes = e.old4 ? e.old4_smem : e.old_smem;
     cfg.stream = s;
     cudaLaunchAttribute attr[1];
     attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;  // start once the previous kernel's CTAs have all
     attr[0].val.programmaticStreamSerializationAllowed = 1;          // executed griddepcontrol.launch_dependents
     cfg.attrs = attr;
-    // LIC360_WF_OLD_SPLIT=k (experiment): k launches over layer ranges, so that the grid drains k times per step and a
-    // cluster launch of the other bitstream's chain, which needs whole SMs, gets a window
-    const int split_env = getenv("LIC360_WF_OLD_SPLIT") ? std::max(1, std::min(WF_LAYERS, atoi(getenv("LIC360_WF_OLD_SPLIT")))) : 1;
-    const int split = n.G > 1 ? split_env : 1;
-    for (int k = 0; k < split; k++) {
-        const int l0 = k * WF_LAYERS / split, l1 = (k + 1) * WF_LAYERS / split;
-        cfg.gridDim = e.old4 ? dim3((l1 - l0) * n.nsets, 1, ((n.ndiag + 1) / 2) * e.parts4)
-                             : dim3((l1 - l0) * n.nsets, e.cpg4_max, n.ndiag * (e.old2 ? e.parts2 : n.parts));
-        cfg.numAttrs = programmatic && k == 0 ? 1 : 0;
-        g_launches++;
-        if (psum >= 0 && !e.old2) return cudaErrorInvalidValue;  // explicit steps: many-group engines only
-        const cudaError_t err = e.old4   ? cudaLaunchKernelEx(&cfg, wf_old4_kernel, n, e.maps4, dp, l0, e.parts4, psum, scat_done)
-                                : e.old2 ? cudaLaunchKernelEx(&cfg, wf_old2_kernel, n, e.maps2, dp, l0, e.parts2, psum, scat_done)
-                                         : cudaLaunchKernelEx(&cfg, wf_old_kernel, n, e.maps, dp, l0);
-        if (err != cudaSuccess) return err;
-    }
+    cfg.numAttrs = programmatic ? 1 : 0;
+    g_launches++;
+    const cudaError_t err = e.old4 ? cudaLaunchKernelEx(&cfg, wf_old4_kernel, n, e.maps4, dp, e.parts4, psum, scat_done)
+                                   : cudaLaunchKernelEx(&cfg, wf_old_kernel, n, e.maps, dp);
+    if (err != cudaSuccess) return err;
     if (done) {
         wf_old_done_kernel<<<1, 1, 0, s>>>(done, psum + 1);
         g_launches++;
@@ -1804,20 +1676,16 @@ cudaError_t wf_launch_prev(const WfEngine& e, int dp, int l0, int l1, cudaStream
     int cpg4 = 0, nqb = 0;
     for (int l = l0; l < l1; l++) { cpg4 = std::max(cpg4, n.L[l].cpg4); nqb = std::max(nqb, n.L[l].nqb); }
     dim3 grid(n.ndiag * n.parts, cpg4, (l1 - l0) * n.nsets), block(32, nqb);
-    if (e.nqb_max <= 10) wf_prev_kernel<320><<<grid, block, e.prev_smem, s>>>(n, e.prev_wcap, dp, l0);
-    else wf_prev_kernel<1024><<<grid, block, e.prev_smem, s>>>(n, e.prev_wcap, dp, l0);
+    wf_prev_kernel<320><<<grid, block, e.prev_smem, s>>>(n, e.prev_wcap, dp, l0);  // nqb <= 10 (wf_init)
     g_launches++;
     return cudaGetLastError();
 }
 
-cudaError_t wf_launch_chain(const WfEngine& e, cudaStream_t s, const WfRows* rows, const WfPersist* persist) {
-    WfRows r;
-    memset(&r, 0, sizeof(r));
-    if (rows && (e.chain4 || e.chain1)) r = *rows;
+cudaError_t wf_launch_chain(const WfEngine& e, cudaStream_t s, const WfRows& rows, const WfPersist* persist) {
     WfPersist ps;
     memset(&ps, 0, sizeof(ps));
     if (persist) {
-        if (!e.chain4 || !r.enabled || !r.rtail || !e.r0_inline) return cudaErrorInvalidValue;  // the persistent loop assumes the fully fused step
+        if (!e.chain4) return cudaErrorInvalidValue;
         ps = *persist;
         ps.enabled = 1;
     }
@@ -1834,9 +1702,8 @@ cudaError_t wf_launch_chain(const WfEngine& e, cudaStream_t s, const WfRows* row
     cfg.attrs = attr;
     cfg.numAttrs = e.cluster > 1 ? 1 : 0;
     g_launches++;
-    if (e.chain4) return cudaLaunchKernelEx(&cfg, wf_chain4_kernel, n, e.cluster, n.G, r, (int)(e.r0_inline && r.enabled), ps,
-                                            (int)(e.chain_smem / (WF_ROW_F4 * sizeof(float4))));
-    if (e.chain1) return cudaLaunchKernelEx(&cfg, wf_chain1_kernel, n, e.cluster, e.c1_kpc, e.c1_lenp, e.c1_cmax, r, (int)(e.r0_inline && r.enabled), (int)e.c1_dsm);
+    if (e.chain4) return cudaLaunchKernelEx(&cfg, wf_chain4_kernel, n, e.cluster, n.G, rows, ps, (int)(e.chain_smem / (WF_ROW_F4 * sizeof(float4))));
+    if (e.chain1) return cudaLaunchKernelEx(&cfg, wf_chain1_kernel, n, e.cluster, e.c1_kpc, e.c1_lenp, e.c1_cmax, rows, (int)e.c1_dsm);
     return cudaLaunchKernelEx(&cfg, wf_chain_kernel<384>, n, e.cluster);
 }
 

@@ -41,17 +41,16 @@ struct WfNetDev {
     int nsets, G, H, W, D, HS, Dp, Hp, nsteps, parts, ndiag, pad;
 };
 
-// code stream: the CDF rows of the step are produced at the end of the chain kernel (no extra launch on the critical path)
+// The CDF rows of the step are produced at the end of wf_chain4_kernel and wf_chain1_kernel (no extra launch on the critical path).
+// wf_chain4_kernel (code stream) publishes every row by its tag step % 15 + 1, with no system fence + flag behind the rows: the host
+// validates row by row; it also evaluates the previous-wavefront terms of the NEXT step (layers 1..11) behind the rows.
+// wf_chain1_kernel (importance stream) raises the flag once its rows are written.
 struct WfRows {
     uint16_t* rows;       // mapped pinned: packed rows of the step
     const float* levels;  // decoded importance levels (mask bit = Imp2mask + Dtow of the symbol's 2x2 cell)
-    int* done;            // CTA counter of the rows phase
-    int* flag;            // mapped pinned: step + 1 once the rows are written
+    int* flag;            // mapped pinned: step + 1 once the rows are written (wf_chain1_kernel); -(step + 1): a wf_chain4_kernel CTA gave up
     int* sync;            // monotone counter: all nets have finished layer 11 of step p when it reaches (p + 1) * gridDim.x
     float s2;
-    int enabled;
-    int rtail;            // the chain kernel also evaluates the previous-wavefront terms of the NEXT step (layers 1..11) behind the rows
-    int tagged;           // rows carry the publication tag step % 15 + 1 and are NOT followed by a system fence + flag: the host validates row by row
 };
 
 // Low-latency ("persistent") decode of the many-group stream: ONE launch of the chain kernel walks all wavefront steps; between steps it
@@ -74,12 +73,8 @@ struct WfMaps { CUtensorMap tm[WF_LAYERS]; };  // FP input frame of every layer,
 struct WfEngine {
     WfNetDev dev;
     WfMaps maps;
-    WfMaps maps2;         // box {72 h, 9 d, 2 c} of the two-positions-per-lane old-term kernel
-    bool old2 = false;    // use it (many-group nets; LIC360_WF_OLD1=1 switches back)
-    int parts2 = 1;       // 64-position parts per diagonal
-    size_t old2_smem = 0;
     WfMaps maps4;         // box {72 h, 10 d, 2 c} of the four-positions-per-lane, two-diagonals-per-warp old-term kernel
-    bool old4 = false;    // use it (many-group nets with one output chunk per group; LIC360_WF_OLD2=1 switches back)
+    bool old4 = false;    // many-group net: wf_old4_kernel (else wf_old_kernel)
     int parts4 = 1;
     size_t old4_smem = 0;
     float* fp[WF_LAYERS + 1] = {nullptr};
@@ -91,10 +86,10 @@ struct WfEngine {
     int max_len = 0, cpg4_max = 0, nblk_max = 0, nqb_max = 0;
     int cluster = 1, chain_threads = 0;
     int chain_tasks = 0;  // wf_chain_kernel: (item, block) tasks of one CTA in the longest step's most expensive layer
-    bool chain4 = false;  // every chained layer has 4 channels per group: the staged-weight chain kernel applies
+    // chain4 and chain1 also produce the step's CDF rows and compute layer 0's previous-wavefront terms themselves (no launch for them)
+    bool chain4 = false;  // many-group net (every chained layer has 4 channels per group): the staged-weight chain kernel
     bool chain1 = false;  // single-group net: the output-chunk-split chain kernel applies
     bool c1_dsm = false;  // chain1: both activation tiles fit, layers exchange activations through distributed shared memory
-    bool r0_inline = false;  // the chain kernel computes layer 0's previous-wavefront terms itself (no launch for them)
     int c1_kpc = 0, c1_lenp = 0, c1_cmax = 0, prev_wcap = 0;
     size_t old_smem = 0, prev_smem = 0, chain_smem = 0;
 };
@@ -108,8 +103,7 @@ int wf_chain_capacity(const WfEngine& e);  // decodes whose code-stream chains m
 // wf_chain4_kernel's R tail: the most rounds in which a CTA stages its weight rows, over all steps (0: not a chain4 engine).
 // idx, steps: the host copies of the index plan and the step list the engine was created with
 int wf_tail_rounds(const WfEngine& e, const int32_t* idx, const StepDesc* steps);
-const void* wf_old_kernel_ptr();
-const void* wf_old2_kernel_ptr();  // to give the old-term kernel node its own (lowest) priority in the step graph
+const void* wf_old_kernel_ptr();  // to give the importance stream's old-term kernel node its own (lowest) priority in the step graph
 cudaError_t wf_clear(const WfEngine& e, cudaStream_t s);                    // zero every frame (start of a decode)
 // P of step *ctr + dp, all layers.  programmatic: launch as a programmatic dependent of the previous kernel in the stream
 // psum >= 0: explicit step (persistent decode: the host knows it), else *ctr + dp.  done != nullptr: a one-thread kernel behind the launch
@@ -119,8 +113,9 @@ cudaError_t wf_launch_old(const WfEngine& e, int dp, cudaStream_t s, bool progra
 // R of step *ctr + dp for layers [l0, l1): layer 0 at dp = 0 right after the scatter (it reads the symbols just decoded),
 // layers 1..11 at dp = 1 right after the chain (underneath the host decoder)
 cudaError_t wf_launch_prev(const WfEngine& e, int dp, int l0, int l1, cudaStream_t s);
-// the 12-layer chain of step *ctr; persist != nullptr (chain4 engines only): all steps in one launch, paced by the host through persist->go_host
-cudaError_t wf_launch_chain(const WfEngine& e, cudaStream_t s, const WfRows* rows = nullptr, const WfPersist* persist = nullptr);
+// the 12-layer chain of step *ctr; rows: where chain4 and chain1 put the step's CDF rows (the generic chain kernel ignores them);
+// persist != nullptr (chain4 engines only): all steps in one launch, paced by the host through persist->go_host
+cudaError_t wf_launch_chain(const WfEngine& e, cudaStream_t s, const WfRows& rows, const WfPersist* persist = nullptr);
 
 // first channel of group g at (d, h); cpg = channels per group of that frame.  The group axis carries WF_GPAD zero
 // groups on each side: a tap of the R / Q terms may select group -5 .. G+3, which then reads zeros instead of needing a test.

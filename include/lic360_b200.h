@@ -274,14 +274,14 @@ int lic360_codec_set_mode(lic360_codec* c, int mode);
  * kernel, [2] the 12-layer chain kernel, [3] scatter + CDF-row kernels, and [4] the number of steps, for one stream */
 int lic360_codec_kernel_times(lic360_codec* c, int stream_id, double* out, int n);
 /* the decoder's kernel choices for one stream (0 = code, 1 = importance), fixed when the codec is created (they depend on the
- * latent size and the LIC360_WF_* switches read then); read-only.  out[0 .. n-1], at most 13 values:
+ * latent size; DESIGN.md s8 lists the overrides of the cluster size [2]); read-only.  out[0 .. n-1], at most 13 values:
  *   [0] chain kernel: 0 wf_chain_kernel (generic), 1 wf_chain4_kernel, 2 wf_chain1_kernel
  *   [1] wf_chain1_kernel exchanges activations through distributed shared memory (1) or reloads its tile every layer (0)
  *   [2] CTAs per cluster  [3] chain threads per CTA  [4] chain dynamic shared memory, bytes, as launched
  *   [5] longest wavefront step (positions)  [6] wf_chain1_kernel's padded step length lenp  [7] its output chunks per CTA
  *       ([6], [7]: 0 for the other chain kernels)
  *   [8] wf_chain_kernel's tasks per CTA in the longest step (its thread loop takes a second round when [8] > [3])
- *   [9] old-term kernel positions per lane (4, 2 or 1)  [10] parts4  [11] parts: 64- and 32-position tiles per diagonal
+ *   [9] old-term kernel positions per lane (4 or 1)  [10] parts4  [11] parts: 64- and 32-position tiles per diagonal
  *   [12] wf_chain4_kernel: most rounds in which a CTA's R tail stages its weight rows (0 for the other chain kernels) */
 int lic360_codec_engine_info(lic360_codec* c, int stream_id, int* out, int n);
 

@@ -15,7 +15,7 @@ def run_smoke():
 
     dev = "cuda:0"
     l0 = lic360.launch_count()
-    # 1. FIRST (so that the wavefront-engine kernels -- wf_old2_kernel, wf_chain4_kernel, wf_chain1_kernel -- are inside the
+    # 1. FIRST (so that the wavefront-engine kernels -- wf_old4_kernel, wf_chain4_kernel, wf_chain1_kernel -- are inside the
     # driver's launch window): the product path, the fused native codec, both streams, encode -> bitstreams -> decode == input
     import lic360_pipeline as pl
     q2, mask2, lv2 = synthetic_latent(8, H=16, W=32)

@@ -34,8 +34,7 @@ def _assert_bits(got, want, what):
 
 # ---- per-op layers --------------------------------------------------------------------------------------------------
 # name: (N, nsets, G, cin_g, cout_g, H, W, constrain, act, options); options: "resid" (EC residual through
-# lic360_cconv_ec_forward), "misaligned" (x at a 4-byte, not 16-byte, offset), "generic" (LIC360_EC_RQ_GENERIC=1),
-# "nodc" (EC only)
+# lic360_cconv_ec_forward), "misaligned" (x at a 4-byte, not 16-byte, offset), "nodc" (EC only)
 CASES = {
     "g48_first_24x72": (3, 3, 48, 1, 4, 24, 72, 5, True, ""),              # P over 3 blocks of Cin, rq<0>, no pairing
     "g48_hidden_64x128": (3, 3, 48, 4, 4, 64, 128, 6, True, "resid"),      # tile pairing, rq_tile
@@ -57,8 +56,6 @@ CASES = {
     "g6_1x7": (1, 1, 6, 4, 4, 1, 7, 6, True, ""),                          # degenerate frames
     "g6_5x1": (1, 1, 6, 4, 4, 5, 1, 6, True, ""),
     "g48_hidden_40x72": (3, 3, 48, 4, 4, 40, 72, 6, True, ""),             # DC: multi-part diagonals
-    "g48_hidden_generic": (3, 3, 48, 4, 4, 64, 128, 6, True, "generic nodc"),  # rq_tile switched off
-    "g10_hidden_generic": (1, 1, 10, 4, 4, 13, 36, 6, True, "generic nodc"),
 }
 
 
@@ -128,9 +125,7 @@ def _run_dc(name):
 
 
 @pytest.mark.parametrize("name", list(CASES))
-def test_cconv_ec_is_canonical(monkeypatch, name):
-    if "generic" in CASES[name][-1]:
-        monkeypatch.setenv("LIC360_EC_RQ_GENERIC", "1")
+def test_cconv_ec_is_canonical(name):
     _assert_bits(_run_ec(name), _layer_case(name)[-1], "CconvEc " + name)
 
 

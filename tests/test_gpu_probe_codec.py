@@ -55,20 +55,6 @@ def test_fused_codec_writes_the_expected_streams(name, H, W):
     assert _decode_ok(fused, want2, q2, mask2)
 
 
-@pytest.mark.parametrize("switch", ["LIC360_WF_ROWS_KERNEL", "LIC360_WF_ROWS_FLAGS", "LIC360_WF_GENERIC_CHAIN"])
-def test_alternate_row_producers_and_chain_decode_the_expected_streams(monkeypatch, switch):
-    import lic360_pipeline as pl
-    H, W = 24, 72
-    monkeypatch.setenv(switch, "1")
-    if switch == "LIC360_WF_GENERIC_CHAIN":
-        monkeypatch.setenv("LIC360_WF_CLUSTER", "8")
-    for name in pn.PROBES:
-        _, (q, mask, lv), want = _case(name, H, W, 100 + H + W)
-        fused = pl.FusedCodec(_torch_params(name), H=H, W=W)
-        assert fused.encode(t(q, DEV), t(mask, DEV), t(lv, DEV)) == want, name
-        assert _decode_ok(fused, want, q, mask), name
-
-
 def test_out_of_range_symbol_is_a_coder_error():
     """No table the fix-up emits has an empty bin (test_ref64), so a symbol the coder cannot code is one outside 0..7:
     both paths refuse it and return no stream."""
