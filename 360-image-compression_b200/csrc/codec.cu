@@ -20,12 +20,14 @@
 #include <atomic>
 #include <chrono>
 #include <condition_variable>
+#include <deque>
 #include <functional>
 #include <cstring>
 #include <memory>
 #include <mutex>
 #include <string>
 #include <sched.h>
+#include <system_error>
 #include <thread>
 #include <cmath>
 #include <vector>
@@ -175,12 +177,75 @@ struct StreamWorker {
         if (th.joinable()) th.join();
     }
 };
+
+// the host coding of a batch encode: persistent workers per codec (not a std::thread per call), each with its own coder, started
+// on demand and joined when the codec is destroyed.  Jobs start in the order they were posted.
+constexpr int kMaxCoderWorkers = 16;
+struct CoderPool {
+    std::vector<std::thread> th;
+    std::vector<lic360_coder*> coders;  // coders[i] belongs to th[i]
+    std::mutex m;
+    std::condition_variable cv, idle;
+    std::deque<std::function<void(lic360_coder*)>> jobs;
+    int running = 0;
+    bool quit = false;
+    void loop(lic360_coder* coder) {
+        std::unique_lock<std::mutex> lk(m);
+        for (;;) {
+            cv.wait(lk, [&] { return quit || !jobs.empty(); });
+            if (quit) return;
+            std::function<void(lic360_coder*)> j = std::move(jobs.front());
+            jobs.pop_front();
+            running++;
+            lk.unlock();
+            j(coder);
+            lk.lock();
+            if (--running == 0 && jobs.empty()) idle.notify_all();
+        }
+    }
+    // at least n workers, or as many as the system lets us start; returns the number of workers
+    int grow(int n) {
+        while ((int)th.size() < n) {
+            lic360_coder* coder = lic360_coder_create("", 3.5f);
+            try {
+                th.emplace_back([this, coder] { loop(coder); });
+            } catch (const std::system_error&) {
+                lic360_coder_destroy(coder);
+                break;
+            }
+            coders.push_back(coder);
+        }
+        return (int)th.size();
+    }
+    void post(std::function<void(lic360_coder*)> j) {
+        { std::lock_guard<std::mutex> lk(m); jobs.push_back(std::move(j)); }
+        cv.notify_one();
+    }
+    void wait() {  // until every posted job has finished
+        std::unique_lock<std::mutex> lk(m);
+        idle.wait(lk, [&] { return jobs.empty() && running == 0; });
+    }
+    ~CoderPool() {
+        { std::lock_guard<std::mutex> lk(m); quit = true; }
+        cv.notify_all();
+        for (std::thread& t : th) t.join();
+        for (lic360_coder* coder : coders) lic360_coder_destroy(coder);
+    }
+};
+
+// one stream of a batch encode: its bytes, or the status and message of the coder that refused it
+struct EncodedStream {
+    std::vector<uint8_t> bytes;
+    int rc = 0;
+    std::string err;
+};
 }  // namespace lic360
 
 struct lic360_codec {
     int device = 0, H = 0, W = 0;
     int chain_cap = 1;                  // concurrent decodes the device can hold (wf_chain_capacity)
     lic360::StreamWorker imp_worker;
+    lic360::CoderPool coder_pool;       // encode_batch: codes the 2K streams
     int mode = 0;                       // 0: pipelined graph replay, 1: serialized launches with per-kernel event timing
     NetDesc code, imp;
     float* levels_dev = nullptr;        // decoded importance levels (1,1,H/2,W/2), filled diagonal by diagonal
@@ -191,6 +256,10 @@ struct lic360_codec {
     void* est_dev = nullptr;            // estimate: totals, error keys and counts of both streams (EstimateTotals layout)
     void* est_host = nullptr;           // pinned copy of est_dev
     cudaEvent_t ev_est = nullptr;                // estimate: the importance stream's results are in est_dev
+    int rows_cap = 1;                   // latents the encoder's row buffers (rows_dev / rows_host of both streams) hold (grown on demand)
+    int enc_k = 0;                      // latents of the last successful encode / encode_batch (0 after a failure or a decode)
+    bool enc_pooled = false;            // the last encode coded on the pool: its streams are in enc_out, else in the two coders
+    std::vector<lic360::EncodedStream> enc_out;  // [2k + stream_id]
     double t_host_coder = 0, t_total = 0, t_gpu_wait = 0, t_imp = 0, t_gpu_steps = 0, t_gpu_steps_imp = 0;
 };
 
@@ -215,6 +284,8 @@ __global__ void prep_code_kernel(const float* __restrict__ code, const float* __
 
 // y: (3, G*3, H, W) outputs of [weight_net, delta_net, mean_net]; one thread = one symbol (tc, k) in plan order.
 // all_steps != 0: encoder, every symbol, row index = coding order; else: decoder, the slab of steps[*ctr].
+// The encoder's batch: latent blockIdx.y of gridDim.y, y as the bits kernels read it, [net][latent][G*3][H][W]; code, mask and rows
+// (G*H*W rows of 8 u16, the stream's total_rows) offset per latent.
 __global__ void gmm_rows_kernel(const float* __restrict__ y, const float* __restrict__ code, const float* __restrict__ mask,
                                 const int32_t* __restrict__ idx, const StepDesc* __restrict__ steps,
                                 const int* __restrict__ row_off, const int* __restrict__ ctr, uint16_t* __restrict__ rows,
@@ -222,6 +293,8 @@ __global__ void gmm_rows_kernel(const float* __restrict__ y, const float* __rest
     const int HW = H * W;
     int th, tw, tc, row;
     if (all_steps) {
+        const size_t lat = blockIdx.y, plane = (size_t)G * HW;
+        y += lat * 3 * plane; code += lat * plane; mask += lat * plane; rows += lat * plane * 8;
         const int i = blockIdx.x * blockDim.x + threadIdx.x;
         if (i >= G * HW) return;
         const int k = i % HW;
@@ -238,7 +311,7 @@ __global__ void gmm_rows_kernel(const float* __restrict__ y, const float* __rest
         row = l;
     }
     float wv[3], dv[3], mv[3], o[9];
-    const size_t net = (size_t)G * 3 * HW;
+    const size_t net = (size_t)gridDim.y * G * 3 * HW;
     const size_t base = ((size_t)tc * 3 * H + th) * W + tw;
 #pragma unroll
     for (int i = 0; i < 3; i++) {
@@ -253,12 +326,15 @@ __global__ void gmm_rows_kernel(const float* __restrict__ y, const float* __rest
 }
 
 // importance stream: y (1, 49, h, w) logits; one thread = one position in plan order (G = 1: step p = diagonal p)
+// The encoder's batch: latent blockIdx.y, y (K, 49, h, w), levels and rows (h*w rows of 64 u16) offset per latent.
 __global__ void imp_rows_kernel(const float* __restrict__ y, const float* __restrict__ levels, const int32_t* __restrict__ idx,
                                 const StepDesc* __restrict__ steps, const int* __restrict__ ctr, uint16_t* __restrict__ rows,
                                 int H, int W, int all_steps) {
     const int HW = H * W;
     int k, row;
     if (all_steps) {
+        const size_t lat = blockIdx.y;
+        y += lat * 49 * HW; levels += lat * HW; rows += lat * HW * 64;
         k = blockIdx.x * blockDim.x + threadIdx.x;
         if (k >= HW) return;
         row = k;
@@ -754,19 +830,9 @@ static int ctx_buffers(NetDesc& n) {
     return LIC360_OK;
 }
 
-// The buffers that scale with the number of latents an encode (1) or an estimate (K) runs at once: both networks' encoder frames, the
-// bits kernels' partials and the estimate's results.  They only grow; the old ones are kept unless every new one was allocated.
-static int batch_reserve(lic360_codec* c, int K) {
-    if (K <= c->batch_cap) return LIC360_OK;
-    struct Buf { void** slot; size_t bytes; bool pinned; };
-    std::vector<Buf> bufs;
-    for (NetDesc* n : {&c->code, &c->imp}) {
-        for (int i = 0; i < 13; i++) bufs.push_back({reinterpret_cast<void**>(&n->frame[i]), n->frame_floats[i] * K * sizeof(float), false});
-        bufs.push_back({reinterpret_cast<void**>(&n->bits_partial_dev), (size_t)n->bits_blocks * K * sizeof(double), false});
-        bufs.push_back({reinterpret_cast<void**>(&n->count_partial_dev), (size_t)n->bits_blocks * K * sizeof(int), false});
-    }
-    bufs.push_back({&c->est_dev, estimate_bytes(K), false});
-    bufs.push_back({&c->est_host, estimate_bytes(K), true});
+// Replaces every buffer of `bufs` with one of its new size, or none of them: the old ones are kept unless every new one was allocated.
+struct GrowBuf { void** slot; size_t bytes; bool pinned; };
+static int grow_buffers(lic360_codec* c, const std::vector<GrowBuf>& bufs, int K) {
     // the old buffers may still be in use by work enqueued on the codec's streams
     LIC360_CUDA(cudaStreamSynchronize(c->code.stream));
     LIC360_CUDA(cudaStreamSynchronize(c->imp.stream));
@@ -784,8 +850,39 @@ static int batch_reserve(lic360_codec* c, int K) {
         set_error("codec: cannot allocate the buffers of %d latents (%s)", K, cudaGetErrorString(e));
         return LIC360_ERR_CUDA;
     }
-    c->batch_cap = K;
     return LIC360_OK;
+}
+
+// The buffers that scale with the number of latents an encode or an estimate runs at once: both networks' encoder frames, the bits
+// kernels' partials and the estimate's results.  They only grow.
+static int batch_reserve(lic360_codec* c, int K) {
+    if (K <= c->batch_cap) return LIC360_OK;
+    std::vector<GrowBuf> bufs;
+    for (NetDesc* n : {&c->code, &c->imp}) {
+        for (int i = 0; i < 13; i++) bufs.push_back({reinterpret_cast<void**>(&n->frame[i]), n->frame_floats[i] * K * sizeof(float), false});
+        bufs.push_back({reinterpret_cast<void**>(&n->bits_partial_dev), (size_t)n->bits_blocks * K * sizeof(double), false});
+        bufs.push_back({reinterpret_cast<void**>(&n->count_partial_dev), (size_t)n->bits_blocks * K * sizeof(int), false});
+    }
+    bufs.push_back({&c->est_dev, estimate_bytes(K), false});
+    bufs.push_back({&c->est_host, estimate_bytes(K), true});
+    const int rc = grow_buffers(c, bufs, K);
+    if (rc == LIC360_OK) c->batch_cap = K;
+    return rc;
+}
+
+// The encoder's CDF rows of K latents, on the device and in pinned host memory, for both streams.  Only an encode grows them (an
+// estimate packs no rows), and they only grow.
+static int rows_reserve(lic360_codec* c, int K) {
+    if (K <= c->rows_cap) return LIC360_OK;
+    std::vector<GrowBuf> bufs;
+    for (NetDesc* n : {&c->code, &c->imp}) {
+        const size_t bytes = (size_t)n->total_rows * n->row_bytes * K;
+        bufs.push_back({reinterpret_cast<void**>(&n->rows_dev), bytes, false});
+        bufs.push_back({reinterpret_cast<void**>(&n->rows_host), bytes, true});
+    }
+    const int rc = grow_buffers(c, bufs, K);
+    if (rc == LIC360_OK) c->rows_cap = K;
+    return rc;
 }
 
 static void ctx_free(NetDesc& n) {
@@ -892,15 +989,9 @@ static int run_encoder_net(lic360_codec* c, bool is_code, int K, const float* co
     return run_ec_net(n, K, n.stream);
 }
 
-int lic360_codec_encode(lic360_codec* c, const float* code_dev, const float* mask_dev, const float* imp_dev) {
-    LIC360_CHECK_ARG(c && code_dev && mask_dev && imp_dev, "bad arguments");
-    DeviceGuard guard(c->device);
-    LIC360_CUDA(guard.err);
-    int rc = check_params(c->code);
-    if (rc == LIC360_OK) rc = check_params(c->imp);
-    if (rc) return rc;
-    const auto t0 = clk::now();
-    c->t_host_coder = 0; c->t_gpu_wait = 0; c->t_imp = 0; c->t_gpu_steps = 0; c->t_gpu_steps_imp = 0;
+// the GPU work of an encode of K latents on the codec's two streams: both networks at batch K, the CDF rows of every latent in coding
+// order (latent k's rows at k * total_rows) and their copy to the host, one per stream
+static int enqueue_encode(lic360_codec* c, int K, const float* code_dev, const float* mask_dev, const float* imp_dev, clk::time_point t0) {
     // The two bitstreams are independent: both networks are enqueued on their own CUDA streams first, then the host
     // codes the (small) importance stream while the code-stream network is still running.
     // ---- importance stream: net -> rows of all symbols
@@ -908,11 +999,11 @@ int lic360_codec_encode(lic360_codec* c, const float* code_dev, const float* mas
         NetDesc& n = c->imp;
         cudaStream_t s = n.stream;
         const int HW = n.H * n.W;
-        rc = run_encoder_net(c, false, 1, code_dev, mask_dev, imp_dev);
+        int rc = run_encoder_net(c, false, K, code_dev, mask_dev, imp_dev);
         if (rc) return rc;
-        imp_rows_kernel<<<(HW + 127) / 128, 128, 0, s>>>(n.frame[12], imp_dev, n.idx_dev, n.steps_dev, n.ctr_dev, n.rows_dev, n.H, n.W, 1);
+        imp_rows_kernel<<<dim3((HW + 127) / 128, K), 128, 0, s>>>(n.frame[12], imp_dev, n.idx_dev, n.steps_dev, n.ctr_dev, n.rows_dev, n.H, n.W, 1);
         LAUNCH_CHECK();
-        LIC360_CUDA(cudaMemcpyAsync(n.rows_host, n.rows_dev, (size_t)n.total_rows * 128, cudaMemcpyDeviceToHost, s));
+        LIC360_CUDA(cudaMemcpyAsync(n.rows_host, n.rows_dev, (size_t)K * n.total_rows * 128, cudaMemcpyDeviceToHost, s));
         c->t_gpu_steps_imp = ms_since(t0);  // host time spent enqueueing the importance-stream work
     }
     // ---- code stream (lic360_demo.py:124-141)
@@ -921,14 +1012,21 @@ int lic360_codec_encode(lic360_codec* c, const float* code_dev, const float* mas
         cudaStream_t s = n.stream;
         const auto tq0 = clk::now();
         const int nel = n.G * n.H * n.W;
-        rc = run_encoder_net(c, true, 1, code_dev, mask_dev, imp_dev);
+        int rc = run_encoder_net(c, true, K, code_dev, mask_dev, imp_dev);
         if (rc) return rc;
-        gmm_rows_kernel<<<(nel + 127) / 128, 128, 0, s>>>(n.frame[12], code_dev, mask_dev, n.idx_dev, n.steps_dev, n.row_off_dev,
-                                                          n.ctr_dev, n.rows_dev, n.G, n.H, n.W, 1, (float)(1. / sqrt(2.0)));
+        gmm_rows_kernel<<<dim3((nel + 127) / 128, K), 128, 0, s>>>(n.frame[12], code_dev, mask_dev, n.idx_dev, n.steps_dev, n.row_off_dev,
+                                                                   n.ctr_dev, n.rows_dev, n.G, n.H, n.W, 1, (float)(1. / sqrt(2.0)));
         LAUNCH_CHECK();
-        LIC360_CUDA(cudaMemcpyAsync(n.rows_host, n.rows_dev, (size_t)n.total_rows * 16, cudaMemcpyDeviceToHost, s));
+        LIC360_CUDA(cudaMemcpyAsync(n.rows_host, n.rows_dev, (size_t)K * n.total_rows * 16, cudaMemcpyDeviceToHost, s));
         c->t_gpu_steps = ms_since(tq0);  // host time spent enqueueing the code-stream work
     }
+    return LIC360_OK;
+}
+
+// one latent on the calling thread, into the codec's own two coders: the importance stream as soon as its rows are on the host, then
+// the code stream
+static int code_on_caller(lic360_codec* c, clk::time_point t0) {
+    int rc;
     {
         NetDesc& n = c->imp;
         auto tw = clk::now();
@@ -954,8 +1052,119 @@ int lic360_codec_encode(lic360_codec* c, const float* code_dev, const float* mas
         if (lic360_coder_finish_mem(n.coder) < 0) return LIC360_ERR_CODER;
         c->t_host_coder += ms_since(th);
     }
-    c->t_total = ms_since(t0);
     return LIC360_OK;
+}
+
+// a job of the coder pool: stream sid of one latent from its rows into `out`
+static void code_stream_job(lic360_coder* coder, const uint16_t* rows, int nrows, int sid, EncodedStream* out) {
+    lic360_coder_start_encoder_mem(coder);
+    int rc = sid ? coder_encode_packed_imp(coder, rows, nrows) : coder_encode_packed_gmm(coder, rows, nrows);
+    if (rc == LIC360_OK && lic360_coder_finish_mem(coder) < 0) rc = LIC360_ERR_CODER;
+    out->rc = rc;
+    if (rc) {
+        out->err = lic360_last_error();  // the message is thread-local
+        out->bytes.clear();
+        return;
+    }
+    long nb = 0;
+    const uint8_t* b = coder_bytes(coder, &nb);
+    out->bytes.assign(b, b + nb);
+}
+
+// K > 1 latents on the coder pool: the K importance streams as soon as their rows are on the host (the code network may still be
+// running), then the K code streams.  Both CUDA streams are drained on every path.
+static int code_on_pool(lic360_codec* c, int K) {
+    const unsigned hw = std::thread::hardware_concurrency();
+    const int want = std::min(std::min(K, kMaxCoderWorkers), std::max(1, (int)hw));
+    if (c->coder_pool.grow(want) == 0) {
+        cudaStreamSynchronize(c->imp.stream); cudaStreamSynchronize(c->code.stream);
+        set_error("codec: cannot start a coder thread");
+        return LIC360_ERR_CODER;
+    }
+    c->enc_out.resize(2 * (size_t)K);
+    c->enc_pooled = true;
+    auto post_stream = [&](NetDesc& n, int sid) {
+        const size_t row_u16 = (size_t)n.total_rows * n.row_bytes / 2;
+        for (int k = 0; k < K; k++) {
+            const uint16_t* rows = n.rows_host + k * row_u16;
+            EncodedStream* out = &c->enc_out[2 * (size_t)k + sid];
+            const int nrows = n.total_rows;
+            c->coder_pool.post([=](lic360_coder* coder) { code_stream_job(coder, rows, nrows, sid, out); });
+        }
+    };
+    auto tw = clk::now();
+    const cudaError_t e_imp = cudaStreamSynchronize(c->imp.stream);
+    c->t_gpu_wait += ms_since(tw);
+    const auto th = clk::now();
+    if (e_imp == cudaSuccess) post_stream(c->imp, 1);
+    tw = clk::now();
+    const cudaError_t e_code = cudaStreamSynchronize(c->code.stream);
+    c->t_gpu_wait += ms_since(tw);
+    if (e_imp == cudaSuccess && e_code == cudaSuccess) post_stream(c->code, 0);
+    c->coder_pool.wait();
+    c->t_host_coder = ms_since(th);
+    int rc = LIC360_OK;
+    if (e_imp != cudaSuccess || e_code != cudaSuccess) {
+        set_error("codec: the batch encode's GPU work failed -> %s", cudaGetErrorString(e_imp != cudaSuccess ? e_imp : e_code));
+        rc = LIC360_ERR_CUDA;
+    }
+    // the error encode reports for the first bad latent alone, whichever worker finished first; within a latent the importance
+    // stream's (encode codes it first)
+    for (int k = 0; k < K && rc == LIC360_OK; k++)
+        for (int sid : {1, 0}) {
+            const EncodedStream& r = c->enc_out[2 * (size_t)k + sid];
+            if (r.rc == LIC360_OK) continue;
+            set_error("%s (latent %d)", r.err.c_str(), k);
+            rc = r.rc;
+            break;
+        }
+    if (rc)
+        for (EncodedStream& e : c->enc_out) e.bytes.clear();
+    return rc;
+}
+
+// lic360_codec_encode (K = 1, latent_suffix false) and lic360_codec_encode_batch.  K = 1 codes on the calling thread into the codec's
+// two coders, K > 1 on the coder pool.
+static int encode_latents(lic360_codec* c, int K, const float* code_dev, const float* mask_dev, const float* imp_dev, bool latent_suffix) {
+    DeviceGuard guard(c->device);
+    LIC360_CUDA(guard.err);
+    c->enc_k = 0;
+    c->enc_pooled = false;
+    int rc = check_params(c->code);
+    if (rc == LIC360_OK) rc = check_params(c->imp);
+    if (rc == LIC360_OK) rc = batch_reserve(c, K);
+    if (rc == LIC360_OK) rc = rows_reserve(c, K);
+    if (rc) return rc;
+    const auto t0 = clk::now();
+    c->t_host_coder = 0; c->t_gpu_wait = 0; c->t_imp = 0; c->t_gpu_steps = 0; c->t_gpu_steps_imp = 0;
+    rc = enqueue_encode(c, K, code_dev, mask_dev, imp_dev, t0);
+    if (rc && K > 1) { cudaStreamSynchronize(c->imp.stream); cudaStreamSynchronize(c->code.stream); }
+    if (rc) return rc;
+    if (K == 1) {
+        rc = code_on_caller(c, t0);
+        if (rc && latent_suffix) {
+            const std::string msg = lic360_last_error();
+            set_error("%s (latent 0)", msg.c_str());
+        }
+    } else {
+        rc = code_on_pool(c, K);
+    }
+    c->t_total = ms_since(t0);
+    if (rc == LIC360_OK) c->enc_k = K;
+    return rc;
+}
+
+int lic360_codec_encode(lic360_codec* c, const float* code_dev, const float* mask_dev, const float* imp_dev) {
+    LIC360_CHECK_ARG(c && code_dev && mask_dev && imp_dev, "bad arguments");
+    return encode_latents(c, 1, code_dev, mask_dev, imp_dev, false);
+}
+
+int lic360_codec_encode_batch(lic360_codec* c, int K, const float* code_dev, const float* mask_dev, const float* imp_dev) {
+    LIC360_CHECK_ARG(K >= 1, "K must be at least 1");
+    LIC360_CHECK_ARG(c && code_dev && mask_dev && imp_dev, "bad arguments");
+    LIC360_CHECK_ARG(K <= kMaxBatch && (long long)3 * K * c->code.G * c->H * c->W <= 0x7fffffffLL,
+                     "K exceeds the launch limits of a batch (3K conv images, 3 * K * 48 * H * W input floats)");
+    return encode_latents(c, K, code_dev, mask_dev, imp_dev, true);
 }
 
 // the GPU work of an estimate of K latents on the codec's two streams; the code stream ends with the copy of both streams' results
@@ -1074,14 +1283,44 @@ int lic360_imp_levels_to_mask(const float* levels_dev, int h, int w, const int* 
     return LIC360_OK;
 }
 
+// stream stream_id of latent k of the last encode: in enc_out after a batch coded on the pool, else (k = 0) in the codec's coders
+static const uint8_t* encoded_stream(lic360_codec* c, int k, int stream_id, long* n) {
+    if (c->enc_pooled) {
+        const std::vector<uint8_t>& b = c->enc_out[2 * (size_t)k + (stream_id ? 1 : 0)].bytes;
+        *n = (long)b.size();
+        return b.data();
+    }
+    return coder_bytes(stream_id ? c->imp.coder : c->code.coder, n);
+}
+
+static long copy_stream(lic360_codec* c, int k, int stream_id, uint8_t* out, long cap) {
+    long n = 0;
+    const uint8_t* b = encoded_stream(c, k, stream_id, &n);
+    if (out && cap > 0) memcpy(out, b, (size_t)std::min(n, cap));
+    return n;
+}
+
 long lic360_codec_stream_size(lic360_codec* c, int stream_id) {
     long n = 0;
-    coder_bytes(stream_id ? c->imp.coder : c->code.coder, &n);
+    encoded_stream(c, 0, stream_id, &n);
     return n;
 }
 
 long lic360_codec_stream_copy(lic360_codec* c, int stream_id, uint8_t* out, long cap) {
-    return lic360_coder_get_bytes(stream_id ? c->imp.coder : c->code.coder, out, cap);
+    return copy_stream(c, 0, stream_id, out, cap);
+}
+
+long lic360_codec_batch_stream_size(lic360_codec* c, int k, int stream_id) {
+    return lic360_codec_batch_stream_copy(c, k, stream_id, nullptr, 0);
+}
+
+long lic360_codec_batch_stream_copy(lic360_codec* c, int k, int stream_id, uint8_t* out, long cap) {
+    if (!c || (stream_id != 0 && stream_id != 1)) { set_error("codec: bad arguments to a batch stream accessor"); return -1; }
+    if (k < 0 || k >= c->enc_k) {
+        set_error("codec: latent %d is not in the last encode (%d latents)", k, c->enc_k);
+        return -1;
+    }
+    return copy_stream(c, k, stream_id, out, cap);
 }
 
 // importance stream: wait for the rows of step p without synchronising the stream (a later kernel of the step graph may still be
@@ -1317,6 +1556,7 @@ int lic360_codec_decode(lic360_codec* c, const uint8_t* imp_bytes, long n_imp, c
     if (rc) return rc;
     const auto t0 = clk::now();
     c->t_host_coder = 0; c->t_gpu_wait = 0; c->t_gpu_steps = 0; c->t_gpu_steps_imp = 0; c->t_imp = 0;
+    c->enc_k = 0;  // the streams of the last encode are no longer returned by the batch accessors
     c->imp_ready.store(0);
     c->abort_flag.store(0);
     // debug timeline of the code stream (LIC360_WF_TRACE=1): %globaltimer stamps per step, summarised on stderr

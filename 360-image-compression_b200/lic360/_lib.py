@@ -81,6 +81,9 @@ SIGNATURES = {
     "lic360_codec_encode": (_I, [_P, _P, _P, _P]),
     "lic360_codec_estimate": (_I, [_P, _P, _P, _P, _P, _P, _P]),
     "lic360_codec_estimate_batch": (_I, [_P, _I, _P, _P, _P, _P, _P, _P, _P]),
+    "lic360_codec_encode_batch": (_I, [_P, _I, _P, _P, _P]),
+    "lic360_codec_batch_stream_size": (_L, [_P, _I, _I]),
+    "lic360_codec_batch_stream_copy": (_L, [_P, _I, _I, _P, _L]),
     "lic360_imp_levels_to_mask": (_I, [_P, _I, _I, _P, _I, _P, _P, _P]),
     "lic360_codec_stream_size": (_L, [_P, _I]),
     "lic360_codec_stream_copy": (_L, [_P, _I, _P, _L]),

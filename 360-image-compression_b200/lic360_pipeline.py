@@ -197,6 +197,29 @@ class FusedCodec(object):
         check(LIB.lic360_codec_encode(self._h, code.data_ptr(), mask.data_ptr(), imp.data_ptr()))
         return self._stream_bytes(1), self._stream_bytes(0)
 
+    def _batch_stream_bytes(self, k, sid):
+        n = LIB.lic360_codec_batch_stream_size(self._h, k, sid)
+        if n < 0:
+            check(1)
+        buf = (ctypes.c_uint8 * max(n, 1))()
+        LIB.lic360_codec_batch_stream_copy(self._h, k, sid, buf, n)
+        return bytes(buf[:n])
+
+    def encode_batch(self, code, mask, imap_quant):
+        """`encode` of K latents in one pass (lic360_codec_encode_batch): code, mask (K,48,H,W), imap_quant (K,1,H/2,W/2).
+
+        Both networks run once at batch K; the host codes the 2K streams on the codec's worker threads, the importance streams while
+        the code network still runs.  Returns K pairs (imp_bytes, code_bytes), in the order `encode` returns them; pair k is
+        byte-identical to encode() of latent k alone.  A latent encode would refuse raises encode's message followed by
+        ' (latent k)', for the first such k."""
+        K = int(code.shape[0]) if code.dim() == 4 else -1
+        code = self._f32(code, (K, 48, self.H, self.W))
+        mask = self._f32(mask, (K, 48, self.H, self.W))
+        imp = self._f32(imap_quant, (K, 1, self.H // 2, self.W // 2))
+        torch.cuda.current_stream(self.dev).synchronize()  # inputs were produced on torch's stream
+        check(LIB.lic360_codec_encode_batch(self._h, K, code.data_ptr(), mask.data_ptr(), imp.data_ptr()))
+        return [(self._batch_stream_bytes(k, 1), self._batch_stream_bytes(k, 0)) for k in range(K)]
+
     def estimate(self, code, mask, imap_quant):
         """The rate of the latent `encode` would code, without the arithmetic coder: the same networks and integer CDF rows, and for
         every coded symbol its ideal code length 16 - log2(T[s+1] - T[s]) bits (include/lic360_b200.h, lic360_codec_estimate).

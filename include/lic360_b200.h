@@ -243,6 +243,28 @@ int lic360_codec_estimate(lic360_codec* c, const float* code_dev, const float* m
  * limits (3K <= 65535 and 3 * K * 48 * H * W < 2^31), is an argument error. */
 int lic360_codec_estimate_batch(lic360_codec* c, int K, const float* code_dev, const float* mask_dev, const float* imp_dev,
                                 float* code_bits_dev, float* imp_bits_dev, double* bits_host, long long* counts_host);
+/* lic360_codec_encode of K latents of the codec's size in one pass: both networks run once at batch K, as in
+ * lic360_codec_estimate_batch, the row kernels once with the latent in blockIdx.y, and each stream's rows come back with one copy.
+ * The host codes the K importance streams as soon as their rows are on the host, while the code network still runs, then the K
+ * code streams.  Latent k's two streams are byte-identical to lic360_codec_encode of that latent alone.
+ *   code_dev, mask_dev (K,48,H,W), imp_dev (K,1,H/2,W/2): the inputs of K encodes, stacked
+ * Workers: K = 1 codes on the calling thread, exactly as lic360_codec_encode.  K > 1 codes the 2K streams on a pool of persistent
+ * host threads owned by the codec, each with its own coder: min(K, hardware threads, 16) workers, started on demand the first time a
+ * batch needs them and joined by lic360_codec_destroy.
+ * Results: latent k's streams stay in codec-owned buffers until the next encode, encode_batch or decode on this codec; read them
+ * with lic360_codec_batch_stream_size / _copy.  lic360_codec_stream_size / _copy return latent 0's.
+ * Buffers: the encoder frames grow as in lic360_codec_estimate_batch; the CDF-row buffers of both streams (device and pinned host)
+ * grow to the largest K an encode has seen (an estimate does not grow them).  A failed allocation keeps the old buffers.
+ * Errors: a bad latent fails the whole call with the status and message lic360_codec_encode gives for it, followed by " (latent k)",
+ * for the lowest such k; within a latent the importance stream's error comes first.  A failed call returns no streams.  K < 1, or
+ * K beyond the launch limits of lic360_codec_estimate_batch, is an argument error.
+ * lic360_codec_last_timing after a batch: [0] wall time of the call, [1] wall time of the host-coding phase (from the importance
+ * rows' arrival to the last stream coded), [2] time the calling thread waited for the GPU. */
+int lic360_codec_encode_batch(lic360_codec* c, int K, const float* code_dev, const float* mask_dev, const float* imp_dev);
+/* bytes of stream stream_id (0 code, 1 importance) of latent k of the last encode or encode_batch; the copy writes at most cap of
+ * them to out and returns the stream's size.  -1 (and a message) when k is not a latent of the last successful encode. */
+long lic360_codec_batch_stream_size(lic360_codec* c, int k, int stream_id);
+long lic360_codec_batch_stream_copy(lic360_codec* c, int k, int stream_id, uint8_t* out, long cap);
 /* Candidate importance maps and the code masks the decoder derives from them, for rate control.  levels_dev (h,w) are importance
  * levels as lic360_codec_encode reads them: s = the symbol it codes for a level ((int) of it).  For each offsets_host[j] >= 0:
  *   levels_out_dev[j] (K,1,h,w) = max(s - offsets_host[j], 0)
@@ -258,7 +280,7 @@ int lic360_codec_decode(lic360_codec* c, const uint8_t* imp_bytes, long n_imp, c
                         float* code_out_dev, float* mask_out_dev);
 /* milliseconds of the last encode/decode/estimate call: [0] total, [1] host arithmetic coder, [2] waiting for the GPU,
  * [3] importance stream part of a decode, [4] CUDA-event time of all decode graph replays, [5] of the importance stream ones
- * (an estimate fills [0] and [2] only) */
+ * (an estimate fills [0] and [2] only; an encode_batch of K > 1 fills [1] with the wall time of its host-coding phase) */
 int lic360_codec_last_timing(lic360_codec* c, double* out, int n);
 /* mode 0 (default): pipelined graph replay per wavefront step.  mode 1: the same kernels launched one by one on the codec
  * stream with CUDA events between them (the decode is serialized and slower; used by bench.py for the roofline block).
