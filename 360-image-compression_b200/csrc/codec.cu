@@ -47,7 +47,6 @@ struct NetDesc {
     float* frame[13] = {nullptr};  // encoder: frame[0] = network input, frame[i+1] = output of layer i, for lic360_codec::batch_cap latents
     size_t frame_floats[13];       // floats of one latent
     int32_t* idx_dev = nullptr;
-    std::vector<int32_t> plan;
     std::vector<StepDesc> steps;
     std::vector<int> row_off;  // first row of each step in coding order
     StepDesc* steps_dev = nullptr;
@@ -77,9 +76,8 @@ struct NetDesc {
     float* syms_host = nullptr;         // mapped pinned: decoded symbols of one step
     std::vector<float> step_wait_us, step_decode_us, step_levels_us;  // debug timeline (LIC360_WF_TRACE_FILE): host time per step waiting for rows / decoding
     int row_bytes = 16;                 // packed row size (16 B code stream, 128 B importance stream)
-    double t_host_coder = 0, t_gpu_wait = 0, t_done = 0;
+    double t_host_coder = 0, t_gpu_wait = 0;
     lic360_coder* coder = nullptr;
-    char err[256] = {0};                // error text of a worker thread (set_error is thread-local)
     double* bits_partial_dev = nullptr; // estimate: one partial sum per block of the bits kernel and latent
     int* count_partial_dev = nullptr;   // estimate: coded symbols per block of the bits kernel and latent
     int bits_blocks = 0;                // blocks of the bits kernel per latent
@@ -258,8 +256,7 @@ struct lic360_codec {
     cudaEvent_t ev_est = nullptr;                // estimate: the importance stream's results are in est_dev
     int rows_cap = 1;                   // latents the encoder's row buffers (rows_dev / rows_host of both streams) hold (grown on demand)
     int enc_k = 0;                      // latents of the last successful encode / encode_batch (0 after a failure or a decode)
-    bool enc_pooled = false;            // the last encode coded on the pool: its streams are in enc_out, else in the two coders
-    std::vector<lic360::EncodedStream> enc_out;  // [2k + stream_id]
+    std::vector<lic360::EncodedStream> enc_out = std::vector<lic360::EncodedStream>(2);  // [2k + stream_id]: the streams of the last encode (empty after a failed one)
     double t_host_coder = 0, t_total = 0, t_gpu_wait = 0, t_imp = 0, t_gpu_steps = 0, t_gpu_steps_imp = 0;
 };
 
@@ -269,6 +266,79 @@ WF_TRACE_DECL
 static void codec_trace_set(unsigned long long* buf, int sel) {
     cudaMemcpyToSymbol(g_wf_trace, &buf, sizeof(buf));
     cudaMemcpyToSymbol(g_wf_trace_sel, &sel, sizeof(sel));
+}
+
+// Debug timeline of a decode (LIC360_WF_TRACE=1: the code stream, 2: the importance stream): %globaltimer stamps in the WF_TR_SLOTS
+// slots of every step, then the per-layer phase sums of the traced stream's chain kernel
+struct DecodeTrace {
+    unsigned long long* dev = nullptr;  // nullptr: no trace
+    int sel = 0;                        // 0: code stream, 1: importance stream
+    int steps = 0;                      // steps with slots
+};
+
+static int decode_trace_begin(lic360_codec* c, DecodeTrace& t) {
+    const char* env = getenv("LIC360_WF_TRACE");
+    if (!env) return LIC360_OK;
+    t.sel = atoi(env) == 2 ? 1 : 0;
+    t.steps = (t.sel ? c->imp : c->code).nsteps + 2;
+    std::vector<unsigned long long> init((size_t)t.steps * WF_TR_SLOTS + 64, 0ull);  // + per-layer phase sums of the chain
+    for (int p = 0; p < t.steps; p++)
+        for (int k = 0; k < WF_TR_SLOTS; k++)
+            init[(size_t)p * WF_TR_SLOTS + k] = (k == WF_TR_CHAIN1 || k == WF_TR_ROWS1 || k == WF_TR_OLD1 || k == WF_TR_TAIL1) ? 0ull : ~0ull;
+    LIC360_CUDA(cudaMalloc(&t.dev, init.size() * 8));
+    LIC360_CUDA(cudaMemcpy(t.dev, init.data(), init.size() * 8, cudaMemcpyHostToDevice));
+    wf_trace_set(t.dev, t.sel);
+    codec_trace_set(t.dev, t.sel);
+    return LIC360_OK;
+}
+
+// after a decode: the trace's summary on stderr, and one line per step in the CSV file LIC360_WF_TRACE_FILE names
+static void decode_trace_report(lic360_codec* c, DecodeTrace& t) {
+    if (!t.dev) return;
+    const NetDesc& net = t.sel ? c->imp : c->code;
+    std::vector<unsigned long long> tr((size_t)t.steps * WF_TR_SLOTS + 64);
+    cudaMemcpy(tr.data(), t.dev, tr.size() * 8, cudaMemcpyDeviceToHost);
+    wf_trace_set(nullptr, 0);
+    codec_trace_set(nullptr, 0);
+    cudaFree(t.dev);
+    t.dev = nullptr;
+    const char* names[WF_TR_SLOTS] = {"scatter start", "prev start", "chain start", "chain end", "rows start", "rows flag", "old start", "old end", "R tail start", "R tail end"};
+    for (int w0 = 0; w0 < 2; w0++) {  // two windows: while the importance stream still runs / after it finished
+        const int pa = t.sel ? (w0 == 0 ? 10 : 50) : (w0 == 0 ? 20 : 140), pb = t.sel ? (w0 == 0 ? 45 : 90) : (w0 == 0 ? 80 : 220);
+        double acc[WF_TR_SLOTS] = {0}, period = 0;
+        int cnt = 0;
+        for (int p = pa; p < pb && p + 1 < net.nsteps; p++) {
+            const unsigned long long* r = &tr[(size_t)p * WF_TR_SLOTS];
+            for (int k = 0; k < WF_TR_SLOTS; k++) acc[k] += (double)(long long)(r[k] - r[0]) * 1e-3;
+            period += (double)(long long)(tr[(size_t)(p + 1) * WF_TR_SLOTS] - r[0]) * 1e-3;
+            cnt++;
+        }
+        fprintf(stderr, "lic360 trace, %s-stream steps %d..%d: period %.1f us;", t.sel ? "importance" : "code", pa, pb, period / cnt);
+        for (int k = 1; k < WF_TR_SLOTS; k++) fprintf(stderr, " %s +%.1f;", names[k], acc[k] / cnt);
+        fprintf(stderr, "\n");
+    }
+    if (const char* fn = getenv("LIC360_WF_TRACE_FILE")) {  // per-step dump: step, slab length, us relative to the step's slot 0, period
+        if (FILE* f = fopen(fn, "w")) {
+            fprintf(f, "step,len,prev_start,chain_start,chain_end,rows_start,rows_last,old_start,old_end,tail_start,tail_end,period,host_wait_us,host_decode_us,levels_wait_us\n");
+            for (int p = 0; p + 1 < net.nsteps; p++) {
+                const unsigned long long* r = &tr[(size_t)p * WF_TR_SLOTS];
+                fprintf(f, "%d,%d", p, net.steps[p].len);
+                for (int k = 1; k < WF_TR_SLOTS; k++) fprintf(f, ",%.1f", (double)(long long)(r[k] - r[0]) * 1e-3);
+                fprintf(f, ",%.1f", (double)(long long)(tr[(size_t)(p + 1) * WF_TR_SLOTS] - r[0]) * 1e-3);
+                fprintf(f, ",%.1f,%.1f,%.1f\n", (size_t)p < net.step_wait_us.size() ? net.step_wait_us[p] : 0.f,
+                        (size_t)p < net.step_decode_us.size() ? net.step_decode_us[p] : 0.f,
+                        (size_t)p < net.step_levels_us.size() ? net.step_levels_us[p] : 0.f);
+            }
+            fclose(f);
+        }
+    }
+    fprintf(stderr, "%s", t.sel ? "lic360 trace, G=1 chain, CTA 0, us per layer [weight staging | Q product | epilogue + DSMEM stores | prefetch + cluster barrier]:"
+                                : "lic360 trace, code-stream chain, CTA 0 thread 0, us per layer [weight staging issue | item: 25 loads, 100 FMA4, stores | prefetch issue + weights landed | cluster barrier]:");
+    for (int l = 0; l < 12; l++) {
+        fprintf(stderr, " L%d", l);
+        for (int ph = 0; ph < 4; ph++) fprintf(stderr, "%c%.2f", ph ? '|' : ' ', (double)tr[(size_t)t.steps * WF_TR_SLOTS + l * 4 + ph] * 1e-3 / net.nsteps);
+    }
+    fprintf(stderr, "\n");
 }
 
 // ------------------------------------------------------------------------------------------------ kernels
@@ -282,35 +352,20 @@ __global__ void prep_code_kernel(const float* __restrict__ code, const float* __
     }
 }
 
-// y: (3, G*3, H, W) outputs of [weight_net, delta_net, mean_net]; one thread = one symbol (tc, k) in plan order.
-// all_steps != 0: encoder, every symbol, row index = coding order; else: decoder, the slab of steps[*ctr].
-// The encoder's batch: latent blockIdx.y of gridDim.y, y as the bits kernels read it, [net][latent][G*3][H][W]; code, mask and rows
-// (G*H*W rows of 8 u16, the stream's total_rows) offset per latent.
-__global__ void gmm_rows_kernel(const float* __restrict__ y, const float* __restrict__ code, const float* __restrict__ mask,
-                                const int32_t* __restrict__ idx, const StepDesc* __restrict__ steps,
-                                const int* __restrict__ row_off, const int* __restrict__ ctr, uint16_t* __restrict__ rows,
-                                int G, int H, int W, int all_steps, float s2) {
+// The encoder's kernels run a batch of latents: latent blockIdx.y of gridDim.y.  The helpers below give each stream's batch layout, network
+// outputs and CDF row once, for the row kernels (which pack the rows for the host coder) and the bits kernels (the rate estimate).
+// code stream: y [net][latent][G*3][H][W], the outputs of [weight_net, delta_net, mean_net]; code, mask and the rest (G, H, W) per latent.
+// Moves y to the block's latent and returns the offset of its symbols.
+__device__ __forceinline__ size_t gmm_latent(const float* __restrict__& y, int G, int HW) {
+    const size_t lat = blockIdx.y, plane = (size_t)G * HW;
+    y += lat * 3 * plane;
+    return lat * plane;
+}
+
+// code stream: the CDF row o[9] of symbol (tc, th, tw) from its 3x3 network outputs (y as gmm_latent left it)
+__device__ __forceinline__ void gmm_symbol_row(const float* y, int G, int H, int W, int tc, int th, int tw, float s2, float* o) {
     const int HW = H * W;
-    int th, tw, tc, row;
-    if (all_steps) {
-        const size_t lat = blockIdx.y, plane = (size_t)G * HW;
-        y += lat * 3 * plane; code += lat * plane; mask += lat * plane; rows += lat * plane * 8;
-        const int i = blockIdx.x * blockDim.x + threadIdx.x;
-        if (i >= G * HW) return;
-        const int k = i % HW;
-        tc = i / HW;
-        th = __ldg(idx + k); tw = __ldg(idx + k + HW);
-        const int p = th + tw + tc;
-        row = __ldg(row_off + p) + k - steps[p].start;
-    } else {
-        const StepDesc d = steps[*ctr];
-        const int l = blockIdx.x * blockDim.x + threadIdx.x;
-        if (l >= d.len) return;
-        th = __ldg(idx + d.start + l); tw = __ldg(idx + d.start + l + HW);
-        tc = d.psum - th - tw;
-        row = l;
-    }
-    float wv[3], dv[3], mv[3], o[9];
+    float wv[3], dv[3], mv[3];
     const size_t net = (size_t)gridDim.y * G * 3 * HW;
     const size_t base = ((size_t)tc * 3 * H + th) * W + tw;
 #pragma unroll
@@ -320,43 +375,68 @@ __global__ void gmm_rows_kernel(const float* __restrict__ y, const float* __rest
         mv[i] = y[2 * net + base + (size_t)i * HW];
     }
     gmm_row(wv, dv, mv, o, 3, 8, 3.5f, 65536.f, 1e-6f, s2);
-    const size_t pos = ((size_t)tc * H + th) * W + tw;
-    const int sym = code ? code_symbol(code[pos]) : 0;  // NaN and anything outside [0, 8) become the out-of-range marker of the row
-    pack_gmm_row(o, sym, code_mask_bit(mask[pos]), rows + (size_t)row * 8);
 }
 
-// importance stream: y (1, 49, h, w) logits; one thread = one position in plan order (G = 1: step p = diagonal p)
-// The encoder's batch: latent blockIdx.y, y (K, 49, h, w), levels and rows (h*w rows of 64 u16) offset per latent.
-__global__ void imp_rows_kernel(const float* __restrict__ y, const float* __restrict__ levels, const int32_t* __restrict__ idx,
-                                const StepDesc* __restrict__ steps, const int* __restrict__ ctr, uint16_t* __restrict__ rows,
-                                int H, int W, int all_steps) {
-    const int HW = H * W;
-    int k, row;
-    if (all_steps) {
-        const size_t lat = blockIdx.y;
-        y += lat * 49 * HW; levels += lat * HW; rows += lat * HW * 64;
-        k = blockIdx.x * blockDim.x + threadIdx.x;
-        if (k >= HW) return;
-        row = k;
-    } else {
-        const StepDesc d = steps[*ctr];
-        const int l = blockIdx.x * blockDim.x + threadIdx.x;
-        if (l >= d.len) return;
-        k = d.start + l;
-        row = l;
-    }
-    const int th = __ldg(idx + k), tw = __ldg(idx + k + HW);
-    float o[50];
+// code stream: the row of plan position k of group tc in coding order (its step is th + tw + tc)
+__device__ __forceinline__ int gmm_coding_row(const int* row_off, const StepDesc* steps, int k, int tc, int th, int tw) {
+    const int p = th + tw + tc;
+    return __ldg(row_off + p) + k - steps[p].start;
+}
+
+// importance stream: y [latent][49][h][w] logits, the levels and the rest (h, w) per latent.  Moves y to the block's latent and
+// returns the offset of its cells.
+__device__ __forceinline__ size_t imp_latent(const float* __restrict__& y, int HW) {
+    const size_t lat = blockIdx.y;
+    y += lat * 49 * HW;
+    return lat * HW;
+}
+
+// importance stream: the CDF row o[1..49] of cell (th, tw) from its 49 logits (y as imp_latent left it)
+__device__ __forceinline__ void imp_symbol_row(const float* y, int H, int W, int th, int tw, float* o) {
     for (int i = 0; i < 49; i++) o[1 + i] = y[((size_t)i * H + th) * W + tw];
     entropy_row(o, 49, 65536.f);
-    uint16_t* dst = rows + (size_t)row * 64;
+}
+
+// code stream: one thread = one symbol (tc = i / HW, k = i % HW in plan order); its packed row (8 u16) at its coding-order row
+__global__ void gmm_rows_kernel(const float* __restrict__ y, const float* __restrict__ code, const float* __restrict__ mask,
+                                const int32_t* __restrict__ idx, const StepDesc* __restrict__ steps,
+                                const int* __restrict__ row_off, uint16_t* __restrict__ rows, int G, int H, int W, float s2) {
+    const int HW = H * W;
+    const size_t lat = gmm_latent(y, G, HW);
+    code += lat; mask += lat; rows += lat * 8;
+    const int i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= G * HW) return;
+    const int k = i % HW, tc = i / HW;
+    const int th = __ldg(idx + k), tw = __ldg(idx + k + HW);
+    rows += (size_t)gmm_coding_row(row_off, steps, k, tc, th, tw) * 8;
+    const size_t pos = ((size_t)tc * H + th) * W + tw;
+    // NaN and anything outside [0, 8) become the out-of-range marker of the row.  Symbol and mask bit are read before the row is built:
+    // it keeps the kernel at 32 registers.
+    const int sym = code_symbol(code[pos]), maskbit = code_mask_bit(mask[pos]);
+    float o[9];
+    gmm_symbol_row(y, G, H, W, tc, th, tw, s2, o);
+    pack_gmm_row(o, sym, maskbit, rows);
+}
+
+// importance stream: one thread = one position k of the plan = row k of the stream (64 u16)
+__global__ void imp_rows_kernel(const float* __restrict__ y, const float* __restrict__ levels, const int32_t* __restrict__ idx,
+                                uint16_t* __restrict__ rows, int H, int W) {
+    const int HW = H * W;
+    const size_t lat = imp_latent(y, HW);
+    levels += lat; rows += lat * 64;
+    const int k = blockIdx.x * blockDim.x + threadIdx.x;
+    if (k >= HW) return;
+    const int th = __ldg(idx + k), tw = __ldg(idx + k + HW);
+    float o[50];
+    imp_symbol_row(y, H, W, th, tw, o);
+    uint16_t* dst = rows + (size_t)k * 64;
     uint32_t ovf[3] = {0, 0, 0};
     for (int j = 1; j <= 48; j++) {
         const uint32_t v = (uint32_t)(int)o[j];
         dst[j - 1] = (uint16_t)(v & 0xFFFF);
         ovf[(j - 1) / 16] |= ((v >> 16) & 1u) << ((j - 1) % 16);
     }
-    dst[48] = levels ? (uint16_t)imp_symbol(levels[th * W + tw]) : 0;
+    dst[48] = (uint16_t)imp_symbol(levels[th * W + tw]);
     dst[49] = (uint16_t)ovf[0]; dst[50] = (uint16_t)ovf[1]; dst[51] = (uint16_t)ovf[2];
 }
 
@@ -395,17 +475,17 @@ __device__ __forceinline__ bool symbol_bits(const float* o, int s, double* bits)
 
 // A batch: latent blockIdx.y of gridDim.y, each with the block partition, the partials and the error key of a single latent, so its
 // totals and map do not depend on the other latents.
-// code stream: y as in gmm_rows_kernel, [net][latent][G*3][H][W]; thread i = symbol (tc = i / HW, k = i % HW in plan order), bits
-// (optional) in (G, H, W) layout per latent; count: coded symbols (mask >= 0.5) per block
+// code stream: thread i = symbol (tc = i / HW, k = i % HW in plan order), bits (optional) in (G, H, W) layout per latent; count: coded
+// symbols (mask >= 0.5) per block
 __global__ void __launch_bounds__(BITS_THREADS) gmm_bits_kernel(const float* __restrict__ y, const float* __restrict__ code,
                                 const float* __restrict__ mask, const int32_t* __restrict__ idx, const StepDesc* __restrict__ steps,
                                 const int* __restrict__ row_off, float* __restrict__ bits, double* __restrict__ partial,
                                 int* __restrict__ count, unsigned long long* err, int G, int H, int W, float s2) {
     const int HW = H * W;
-    const size_t lat = blockIdx.y, plane = (size_t)G * HW;  // one latent's symbols
-    y += lat * 3 * plane; code += lat * plane; mask += lat * plane; err += lat;
-    if (bits) bits += lat * plane;
-    partial += lat * gridDim.x; count += lat * gridDim.x;
+    const size_t lat = gmm_latent(y, G, HW);
+    code += lat; mask += lat; err += blockIdx.y;
+    if (bits) bits += lat;
+    partial += (size_t)blockIdx.y * gridDim.x; count += (size_t)blockIdx.y * gridDim.x;
     const int i = blockIdx.x * blockDim.x + threadIdx.x;
     double cost = 0.0;
     int coded = 0;
@@ -415,20 +495,11 @@ __global__ void __launch_bounds__(BITS_THREADS) gmm_bits_kernel(const float* __r
         const size_t pos = ((size_t)tc * H + th) * W + tw;
         coded = code_mask_bit(mask[pos]);
         if (coded) {  // a position the encoder skips costs nothing, whatever its symbol
-            float wv[3], dv[3], mv[3], o[9];
-            const size_t net = gridDim.y * 3 * plane;
-            const size_t base = ((size_t)tc * 3 * H + th) * W + tw;
-#pragma unroll
-            for (int j = 0; j < 3; j++) {
-                wv[j] = y[base + (size_t)j * HW];
-                dv[j] = y[net + base + (size_t)j * HW];
-                mv[j] = y[2 * net + base + (size_t)j * HW];
-            }
-            gmm_row(wv, dv, mv, o, 3, 8, 3.5f, 65536.f, 1e-6f, s2);
+            float o[9];
+            gmm_symbol_row(y, G, H, W, tc, th, tw, s2, o);
             const int s = code_symbol(code[pos]);
             if (s > 7 || !symbol_bits<8>(o, s, &cost)) {
-                const int p = th + tw + tc;
-                const unsigned long long row = (unsigned)(__ldg(row_off + p) + k - steps[p].start);
+                const unsigned long long row = (unsigned)gmm_coding_row(row_off, steps, k, tc, th, tw);
                 atomicMin(err, (row << 32) | (unsigned)s);
                 cost = 0.0;
             }
@@ -440,23 +511,22 @@ __global__ void __launch_bounds__(BITS_THREADS) gmm_bits_kernel(const float* __r
     if (threadIdx.x == 0) { partial[blockIdx.x] = cost; count[blockIdx.x] = coded; }
 }
 
-// importance stream: y (K, 49, h, w) logits; thread k = position k of the plan = row k of the stream, bits (optional) in (h, w) layout
-// per latent; every position is coded
+// importance stream: thread k = position k of the plan = row k of the stream, bits (optional) in (h, w) layout per latent; every
+// position is coded
 __global__ void __launch_bounds__(BITS_THREADS) imp_bits_kernel(const float* __restrict__ y, const float* __restrict__ levels,
                                 const int32_t* __restrict__ idx, float* __restrict__ bits, double* __restrict__ partial,
                                 int* __restrict__ count, unsigned long long* err, int H, int W) {
     const int HW = H * W;
-    const size_t lat = blockIdx.y;
-    y += lat * 49 * HW; levels += lat * HW; err += lat;
-    if (bits) bits += lat * HW;
-    partial += lat * gridDim.x; count += lat * gridDim.x;
+    const size_t lat = imp_latent(y, HW);
+    levels += lat; err += blockIdx.y;
+    if (bits) bits += lat;
+    partial += (size_t)blockIdx.y * gridDim.x; count += (size_t)blockIdx.y * gridDim.x;
     const int k = blockIdx.x * blockDim.x + threadIdx.x;
     double cost = 0.0;
     if (k < HW) {
         const int th = __ldg(idx + k), tw = __ldg(idx + k + HW);
         float o[50];
-        for (int j = 0; j < 49; j++) o[1 + j] = y[((size_t)j * H + th) * W + tw];
-        entropy_row(o, 49, 65536.f);
+        imp_symbol_row(y, H, W, th, tw, o);
         const uint32_t s = imp_symbol(levels[th * W + tw]);
         if (s >= 49 || !symbol_bits<49>(o, (int)s, &cost)) {
             atomicMin(err, ((unsigned long long)k << 32) | s);
@@ -599,9 +669,8 @@ static void net_init(NetDesc& n, int G, int cpg, int nlast, int nsets, int H, in
 
 static int net_alloc(NetDesc& n) {
     const int H = n.H, W = n.W, G = n.G;
-    std::vector<int32_t> idx(2 * (size_t)H * W);
-    n.plan.resize(H + W);
-    lic360_code_contex(H, W, idx.data(), n.plan.data());
+    std::vector<int32_t> idx(2 * (size_t)H * W), plan(H + W);
+    lic360_code_contex(H, W, idx.data(), plan.data());
     LIC360_CUDA(cudaMalloc(&n.idx_dev, idx.size() * sizeof(int32_t)));
     LIC360_CUDA(cudaMemcpy(n.idx_dev, idx.data(), idx.size() * sizeof(int32_t), cudaMemcpyHostToDevice));
     n.nsteps = H + W + G - 2;
@@ -610,7 +679,7 @@ static int net_alloc(NetDesc& n) {
     int off = 0;
     for (int p = 0; p < n.nsteps; p++) {
         int s, l;
-        slab_of(n.plan.data(), H, W, G, p, &s, &l);
+        slab_of(plan.data(), H, W, G, p, &s, &l);
         n.steps[p] = {p, s, l, 0};
         n.row_off[p] = off;
         off += l;
@@ -668,6 +737,46 @@ static int check_params(const NetDesc& n) {
     return LIC360_OK;
 }
 
+// s2 of gmm_row: 1 / sqrt(2)
+static const float kGmmS2 = (float)(1. / sqrt(2.0));
+// importance stream network input: Scale(-1, 2/47) of the levels (lic360_demo.py:173-189)
+static const float kImpScale = (float)(2. / (48 - 1.));
+
+// TileInput of a decoded symbol into the stream's network input: scale * symbol + bias, once for each of its rep nets
+struct TileIn { float bias, scale; int rep; };
+static TileIn tile_input(bool is_code) { return is_code ? TileIn{-3.5f, 1.0f, 3} : TileIn{-1.0f, kImpScale, 1}; }
+
+// LIC360_DEBUG_SYNC: synchronise after every kernel of a serialized (mode 1) decode step, and after the set-up of every decode
+static bool debug_sync() {
+    static const bool on = getenv("LIC360_DEBUG_SYNC") != nullptr;
+    return on;
+}
+
+// the error paths that leave work on both CUDA streams: wait for it, so that the caller may reuse its buffers once the call returns
+static void drain(lic360_codec* c) {
+    cudaStreamSynchronize(c->code.stream);
+    cudaStreamSynchronize(c->imp.stream);
+}
+
+// where the chain kernels of a decode step put its CDF rows
+static WfRows wf_rows(lic360_codec* c, NetDesc& n) {
+    WfRows rows;
+    rows.rows = n.rows_step_host; rows.levels = c->levels_dev; rows.flag = n.flag_host; rows.sync = n.sync_dev;
+    rows.s2 = kGmmS2;
+    return rows;
+}
+
+// the symbols of the previous step into the network input (TileInput); the importance stream also keeps them as the decoded levels
+static int launch_scatter(lic360_codec* c, NetDesc& n, bool is_code, cudaStream_t s) {
+    const WfNetDev& w = n.wf.dev;
+    const TileIn t = tile_input(is_code);
+    scatter_prev_kernel<<<(n.max_len + 127) / 128, 128, 0, s>>>(n.syms_host, n.wf.fp[0], n.wf.fc[0], n.idx_dev, n.steps_dev, n.ctr_dev,
+                                                              n.arrived_dev, n.G, n.H, n.W, w.D, w.HS, w.Dp, w.Hp, t.bias, t.scale, t.rep,
+                                                              is_code ? nullptr : c->levels_dev);
+    LAUNCH_CHECK();
+    return LIC360_OK;
+}
+
 // the kernels of one decode step.  side == s (serialized / profile mode): everything in stream order, the old terms of
 // the NEXT step last.  side != s (graph capture): the old terms run beside the chain as its programmatic dependent; either way the
 // host is released by the step's rows (published row by row in the code stream, by a flag in the importance stream), so the bulk
@@ -683,17 +792,10 @@ static int check_params(const NetDesc& n) {
 
 static int launch_step(lic360_codec* c, NetDesc& n, bool is_code, cudaStream_t s, cudaStream_t side, cudaEvent_t* ev) {
     const WfNetDev& w = n.wf.dev;
-    static const bool dbg_env = getenv("LIC360_DEBUG_SYNC") != nullptr;
-    const bool dbg = dbg_env && ev != nullptr;  // only in the serialized mode
-    const int tgrid = (n.max_len + 127) / 128;
+    const bool dbg = debug_sync() && ev != nullptr;  // only in the serialized mode
     if (ev) LIC360_CUDA(cudaEventRecord(ev[0], s));
-    if (is_code)
-        scatter_prev_kernel<<<tgrid, 128, 0, s>>>(n.syms_host, n.wf.fp[0], n.wf.fc[0], n.idx_dev, n.steps_dev, n.ctr_dev, n.arrived_dev, n.G, n.H, n.W,
-                                                  w.D, w.HS, w.Dp, w.Hp, -3.5f, 1.0f, 3, nullptr);
-    else
-        scatter_prev_kernel<<<tgrid, 128, 0, s>>>(n.syms_host, n.wf.fp[0], n.wf.fc[0], n.idx_dev, n.steps_dev, n.ctr_dev, n.arrived_dev, 1, n.H, n.W,
-                                                  w.D, w.HS, w.Dp, w.Hp, -1.0f, (float)(2. / (48 - 1.)), 1, c->levels_dev);
-    LAUNCH_CHECK();
+    const int rc = launch_scatter(c, n, is_code, s);
+    if (rc) return rc;
     WF_DEBUG_SYNC("scatter kernel");
     const bool fork = side != s;  // graph capture: overlap the old terms of the next step with the chain (see below)
     if (ev) LIC360_CUDA(cudaEventRecord(ev[1], s));
@@ -705,10 +807,7 @@ static int launch_step(lic360_codec* c, NetDesc& n, bool is_code, cudaStream_t s
         WF_DEBUG_SYNC("previous-wavefront kernel (layer 0)");
     }
     if (ev) LIC360_CUDA(cudaEventRecord(ev[2], s));
-    WfRows rows;
-    rows.rows = n.rows_step_host; rows.levels = c->levels_dev; rows.flag = n.flag_host; rows.sync = n.sync_dev;
-    rows.s2 = (float)(1. / sqrt(2.0));
-    LIC360_CUDA(wf_launch_chain(n.wf, s, rows));
+    LIC360_CUDA(wf_launch_chain(n.wf, s, wf_rows(c, n)));
     WF_DEBUG_SYNC("chain kernel");
     if (ev) LIC360_CUDA(cudaEventRecord(ev[3], s));
     // The old terms of step p+1 only read wavefronts <= p-1: they are launched right behind the chain kernel as its
@@ -983,7 +1082,7 @@ static int run_encoder_net(lic360_codec* c, bool is_code, int K, const float* co
         prep_code_kernel<<<stream_grid(nel, 256), 256, 0, n.stream>>>(code_dev, mask_dev, n.frame[0], nel, 3.5f);
         LAUNCH_CHECK();
     } else {
-        const int rc = lic360_scale(imp_dev, n.frame[0], (size_t)K * n.H * n.W, -1.0f, (float)(2. / (48 - 1.)), n.stream);
+        const int rc = lic360_scale(imp_dev, n.frame[0], (size_t)K * n.H * n.W, -1.0f, kImpScale, n.stream);
         if (rc) return rc;
     }
     return run_ec_net(n, K, n.stream);
@@ -1001,7 +1100,7 @@ static int enqueue_encode(lic360_codec* c, int K, const float* code_dev, const f
         const int HW = n.H * n.W;
         int rc = run_encoder_net(c, false, K, code_dev, mask_dev, imp_dev);
         if (rc) return rc;
-        imp_rows_kernel<<<dim3((HW + 127) / 128, K), 128, 0, s>>>(n.frame[12], imp_dev, n.idx_dev, n.steps_dev, n.ctr_dev, n.rows_dev, n.H, n.W, 1);
+        imp_rows_kernel<<<dim3((HW + 127) / 128, K), 128, 0, s>>>(n.frame[12], imp_dev, n.idx_dev, n.rows_dev, n.H, n.W);
         LAUNCH_CHECK();
         LIC360_CUDA(cudaMemcpyAsync(n.rows_host, n.rows_dev, (size_t)K * n.total_rows * 128, cudaMemcpyDeviceToHost, s));
         c->t_gpu_steps_imp = ms_since(t0);  // host time spent enqueueing the importance-stream work
@@ -1015,7 +1114,7 @@ static int enqueue_encode(lic360_codec* c, int K, const float* code_dev, const f
         int rc = run_encoder_net(c, true, K, code_dev, mask_dev, imp_dev);
         if (rc) return rc;
         gmm_rows_kernel<<<dim3((nel + 127) / 128, K), 128, 0, s>>>(n.frame[12], code_dev, mask_dev, n.idx_dev, n.steps_dev, n.row_off_dev,
-                                                                   n.ctr_dev, n.rows_dev, n.G, n.H, n.W, 1, (float)(1. / sqrt(2.0)));
+                                                                   n.rows_dev, n.G, n.H, n.W, kGmmS2);
         LAUNCH_CHECK();
         LIC360_CUDA(cudaMemcpyAsync(n.rows_host, n.rows_dev, (size_t)K * n.total_rows * 16, cudaMemcpyDeviceToHost, s));
         c->t_gpu_steps = ms_since(tq0);  // host time spent enqueueing the code-stream work
@@ -1023,39 +1122,7 @@ static int enqueue_encode(lic360_codec* c, int K, const float* code_dev, const f
     return LIC360_OK;
 }
 
-// one latent on the calling thread, into the codec's own two coders: the importance stream as soon as its rows are on the host, then
-// the code stream
-static int code_on_caller(lic360_codec* c, clk::time_point t0) {
-    int rc;
-    {
-        NetDesc& n = c->imp;
-        auto tw = clk::now();
-        LIC360_CUDA(cudaStreamSynchronize(n.stream));
-        c->t_gpu_wait += ms_since(tw);
-        auto th = clk::now();
-        lic360_coder_start_encoder_mem(n.coder);
-        rc = coder_encode_packed_imp(n.coder, n.rows_host, n.total_rows);
-        if (rc) return rc;
-        if (lic360_coder_finish_mem(n.coder) < 0) return LIC360_ERR_CODER;
-        c->t_host_coder += ms_since(th);
-        c->t_imp = ms_since(t0);
-    }
-    {
-        NetDesc& n = c->code;
-        auto tw = clk::now();
-        LIC360_CUDA(cudaStreamSynchronize(n.stream));
-        c->t_gpu_wait += ms_since(tw);
-        auto th = clk::now();
-        lic360_coder_start_encoder_mem(n.coder);
-        rc = coder_encode_packed_gmm(n.coder, n.rows_host, n.total_rows);
-        if (rc) return rc;
-        if (lic360_coder_finish_mem(n.coder) < 0) return LIC360_ERR_CODER;
-        c->t_host_coder += ms_since(th);
-    }
-    return LIC360_OK;
-}
-
-// a job of the coder pool: stream sid of one latent from its rows into `out`
+// one stream of one latent from its rows into `out`, with `coder`
 static void code_stream_job(lic360_coder* coder, const uint16_t* rows, int nrows, int sid, EncodedStream* out) {
     lic360_coder_start_encoder_mem(coder);
     int rc = sid ? coder_encode_packed_imp(coder, rows, nrows) : coder_encode_packed_gmm(coder, rows, nrows);
@@ -1071,50 +1138,64 @@ static void code_stream_job(lic360_coder* coder, const uint16_t* rows, int nrows
     out->bytes.assign(b, b + nb);
 }
 
-// K > 1 latents on the coder pool: the K importance streams as soon as their rows are on the host (the code network may still be
-// running), then the K code streams.  Both CUDA streams are drained on every path.
-static int code_on_pool(lic360_codec* c, int K) {
-    const unsigned hw = std::thread::hardware_concurrency();
-    const int want = std::min(std::min(K, kMaxCoderWorkers), std::max(1, (int)hw));
-    if (c->coder_pool.grow(want) == 0) {
-        cudaStreamSynchronize(c->imp.stream); cudaStreamSynchronize(c->code.stream);
-        set_error("codec: cannot start a coder thread");
-        return LIC360_ERR_CODER;
+// appends " (latent k)" to the message of the calling thread's last error
+static void add_latent_suffix(int k) {
+    const std::string msg = lic360_last_error();
+    set_error("%s (latent %d)", msg.c_str(), k);
+}
+
+// The host coding of an encode of K latents, every stream into enc_out: the K importance streams as soon as their rows are on the host
+// (the code network may still be running), then the K code streams.  K = 1 codes on the calling thread with the codec's two coders,
+// K > 1 on the coder pool.  Both CUDA streams are drained on every path.
+static int code_streams(lic360_codec* c, int K, bool latent_suffix, clk::time_point t0) {
+    const bool pooled = K > 1;
+    if (pooled) {
+        const unsigned hw = std::thread::hardware_concurrency();
+        if (c->coder_pool.grow(std::min(std::min(K, kMaxCoderWorkers), std::max(1, (int)hw))) == 0) {
+            drain(c);
+            set_error("codec: cannot start a coder thread");
+            return LIC360_ERR_CODER;
+        }
     }
     c->enc_out.resize(2 * (size_t)K);
-    c->enc_pooled = true;
-    auto post_stream = [&](NetDesc& n, int sid) {
+    auto code_stream = [&](NetDesc& n, int sid) {
         const size_t row_u16 = (size_t)n.total_rows * n.row_bytes / 2;
         for (int k = 0; k < K; k++) {
             const uint16_t* rows = n.rows_host + k * row_u16;
             EncodedStream* out = &c->enc_out[2 * (size_t)k + sid];
             const int nrows = n.total_rows;
-            c->coder_pool.post([=](lic360_coder* coder) { code_stream_job(coder, rows, nrows, sid, out); });
+            if (pooled) c->coder_pool.post([=](lic360_coder* coder) { code_stream_job(coder, rows, nrows, sid, out); });
+            else code_stream_job(n.coder, rows, nrows, sid, out);
         }
     };
     auto tw = clk::now();
     const cudaError_t e_imp = cudaStreamSynchronize(c->imp.stream);
     c->t_gpu_wait += ms_since(tw);
     const auto th = clk::now();
-    if (e_imp == cudaSuccess) post_stream(c->imp, 1);
+    if (e_imp == cudaSuccess) code_stream(c->imp, 1);
+    const double t_imp_coder = ms_since(th);
+    if (!pooled) c->t_imp = ms_since(t0);
     tw = clk::now();
     const cudaError_t e_code = cudaStreamSynchronize(c->code.stream);
     c->t_gpu_wait += ms_since(tw);
-    if (e_imp == cudaSuccess && e_code == cudaSuccess) post_stream(c->code, 0);
-    c->coder_pool.wait();
-    c->t_host_coder = ms_since(th);
+    const auto tc = clk::now();
+    if (e_imp == cudaSuccess && e_code == cudaSuccess) code_stream(c->code, 0);
+    if (pooled) c->coder_pool.wait();
+    // K = 1: the coder's time; K > 1: the wall time of the coding phase
+    c->t_host_coder = pooled ? ms_since(th) : t_imp_coder + ms_since(tc);
     int rc = LIC360_OK;
     if (e_imp != cudaSuccess || e_code != cudaSuccess) {
         set_error("codec: the batch encode's GPU work failed -> %s", cudaGetErrorString(e_imp != cudaSuccess ? e_imp : e_code));
         rc = LIC360_ERR_CUDA;
     }
-    // the error encode reports for the first bad latent alone, whichever worker finished first; within a latent the importance
+    // the error encode reports for the lowest bad latent alone, whichever worker finished first; within a latent the importance
     // stream's (encode codes it first)
     for (int k = 0; k < K && rc == LIC360_OK; k++)
         for (int sid : {1, 0}) {
             const EncodedStream& r = c->enc_out[2 * (size_t)k + sid];
             if (r.rc == LIC360_OK) continue;
-            set_error("%s (latent %d)", r.err.c_str(), k);
+            set_error("%s", r.err.c_str());
+            if (latent_suffix) add_latent_suffix(k);
             rc = r.rc;
             break;
         }
@@ -1123,36 +1204,38 @@ static int code_on_pool(lic360_codec* c, int K) {
     return rc;
 }
 
-// lic360_codec_encode (K = 1, latent_suffix false) and lic360_codec_encode_batch.  K = 1 codes on the calling thread into the codec's
-// two coders, K > 1 on the coder pool.
-static int encode_latents(lic360_codec* c, int K, const float* code_dev, const float* mask_dev, const float* imp_dev, bool latent_suffix) {
-    DeviceGuard guard(c->device);
+// the start of an encode or an estimate of K latents on the codec's device (guard): both networks have their parameters, the buffers
+// that scale with K hold K latents, and the timing of the last call is reset
+static int begin_latents(lic360_codec* c, const DeviceGuard& guard, int K) {
     LIC360_CUDA(guard.err);
-    c->enc_k = 0;
-    c->enc_pooled = false;
     int rc = check_params(c->code);
     if (rc == LIC360_OK) rc = check_params(c->imp);
     if (rc == LIC360_OK) rc = batch_reserve(c, K);
+    if (rc) return rc;
+    c->t_host_coder = 0; c->t_gpu_wait = 0; c->t_imp = 0; c->t_gpu_steps = 0; c->t_gpu_steps_imp = 0;
+    return LIC360_OK;
+}
+
+// lic360_codec_encode (K = 1, latent_suffix false) and lic360_codec_encode_batch
+static int encode_latents(lic360_codec* c, int K, const float* code_dev, const float* mask_dev, const float* imp_dev, bool latent_suffix) {
+    DeviceGuard guard(c->device);
+    c->enc_k = 0;
+    int rc = begin_latents(c, guard, K);
     if (rc == LIC360_OK) rc = rows_reserve(c, K);
     if (rc) return rc;
     const auto t0 = clk::now();
-    c->t_host_coder = 0; c->t_gpu_wait = 0; c->t_imp = 0; c->t_gpu_steps = 0; c->t_gpu_steps_imp = 0;
     rc = enqueue_encode(c, K, code_dev, mask_dev, imp_dev, t0);
-    if (rc && K > 1) { cudaStreamSynchronize(c->imp.stream); cudaStreamSynchronize(c->code.stream); }
-    if (rc) return rc;
-    if (K == 1) {
-        rc = code_on_caller(c, t0);
-        if (rc && latent_suffix) {
-            const std::string msg = lic360_last_error();
-            set_error("%s (latent 0)", msg.c_str());
-        }
-    } else {
-        rc = code_on_pool(c, K);
-    }
+    if (rc) { drain(c); return rc; }
+    rc = code_streams(c, K, latent_suffix, t0);
     c->t_total = ms_since(t0);
     if (rc == LIC360_OK) c->enc_k = K;
     return rc;
 }
+
+// K within the launch limits of a batch
+#define LIC360_CHECK_BATCH(c, K)                                                                                \
+    LIC360_CHECK_ARG(K <= kMaxBatch && (long long)3 * K * (c)->code.G * (c)->H * (c)->W <= 0x7fffffffLL,       \
+                     "K exceeds the launch limits of a batch (3K conv images, 3 * K * 48 * H * W input floats)")
 
 int lic360_codec_encode(lic360_codec* c, const float* code_dev, const float* mask_dev, const float* imp_dev) {
     LIC360_CHECK_ARG(c && code_dev && mask_dev && imp_dev, "bad arguments");
@@ -1162,8 +1245,7 @@ int lic360_codec_encode(lic360_codec* c, const float* code_dev, const float* mas
 int lic360_codec_encode_batch(lic360_codec* c, int K, const float* code_dev, const float* mask_dev, const float* imp_dev) {
     LIC360_CHECK_ARG(K >= 1, "K must be at least 1");
     LIC360_CHECK_ARG(c && code_dev && mask_dev && imp_dev, "bad arguments");
-    LIC360_CHECK_ARG(K <= kMaxBatch && (long long)3 * K * c->code.G * c->H * c->W <= 0x7fffffffLL,
-                     "K exceeds the launch limits of a batch (3K conv images, 3 * K * 48 * H * W input floats)");
+    LIC360_CHECK_BATCH(c, K);
     return encode_latents(c, K, code_dev, mask_dev, imp_dev, true);
 }
 
@@ -1192,7 +1274,7 @@ static int enqueue_estimate(lic360_codec* c, int K, const float* code_dev, const
         if (rc) return rc;
         gmm_bits_kernel<<<dim3(n.bits_blocks, K), BITS_THREADS, 0, s>>>(n.frame[12], code_dev, mask_dev, n.idx_dev, n.steps_dev,
                                                                         n.row_off_dev, code_bits_dev, n.bits_partial_dev,
-                                                                        n.count_partial_dev, r.err, n.G, n.H, n.W, (float)(1. / sqrt(2.0)));
+                                                                        n.count_partial_dev, r.err, n.G, n.H, n.W, kGmmS2);
         LAUNCH_CHECK();
         bits_sum_kernel<<<K, BITS_THREADS, 0, s>>>(n.bits_partial_dev, n.count_partial_dev, n.bits_blocks, r.bits, r.count);
         LAUNCH_CHECK();
@@ -1206,13 +1288,9 @@ static int enqueue_estimate(lic360_codec* c, int K, const float* code_dev, const
 static int estimate_latents(lic360_codec* c, int K, const float* code_dev, const float* mask_dev, const float* imp_dev,
                             float* code_bits_dev, float* imp_bits_dev, double* bits_host, long long* counts_host, bool latent_suffix) {
     DeviceGuard guard(c->device);
-    LIC360_CUDA(guard.err);
-    int rc = check_params(c->code);
-    if (rc == LIC360_OK) rc = check_params(c->imp);
-    if (rc == LIC360_OK) rc = batch_reserve(c, K);
+    int rc = begin_latents(c, guard, K);
     if (rc) return rc;
     const auto t0 = clk::now();
-    c->t_host_coder = 0; c->t_gpu_wait = 0; c->t_imp = 0; c->t_gpu_steps = 0; c->t_gpu_steps_imp = 0;
     rc = enqueue_estimate(c, K, code_dev, mask_dev, imp_dev, code_bits_dev, imp_bits_dev);
     // both streams are drained on every path: the caller may reuse the inputs and the maps as soon as the call returns
     const auto tw = clk::now();
@@ -1223,25 +1301,16 @@ static int estimate_latents(lic360_codec* c, int K, const float* code_dev, const
     if (rc) return rc;
     LIC360_CUDA(e_imp);
     LIC360_CUDA(e_code);
-    // the errors encode reports for the first bad latent, with its messages: the importance stream is coded (and checked) first
+    // the error encode reports for the first bad latent, with its message: the importance stream is coded (and checked) first
     const EstimateTotals r = estimate_totals(c->est_host, K);
-    for (int k = 0; k < K; k++) {
-        char msg[96], suffix[32] = "";
-        if (latent_suffix) snprintf(suffix, sizeof(suffix), " (latent %d)", k);
-        if (r.err[K + k] != kNoError) {
-            const unsigned s = (unsigned)r.err[K + k];
-            if (s >= 49) snprintf(msg, sizeof(msg), "coder: importance level %u out of range", s);
-            else snprintf(msg, sizeof(msg), "coder: symbol has zero frequency");
-        } else if (r.err[k] != kNoError) {
-            const int row = (int)(r.err[k] >> 32);
-            if ((unsigned)r.err[k] > 7) snprintf(msg, sizeof(msg), "coder: symbol out of range in packed row %d", row);
-            else snprintf(msg, sizeof(msg), "coder: symbol has zero frequency (row %d)", row);
-        } else {
-            continue;
+    for (int k = 0; k < K; k++)
+        for (int sid : {1, 0}) {
+            const unsigned long long e = r.err[sid * K + k];
+            if (e == kNoError) continue;
+            coder_row_error(sid, (int)(e >> 32), (unsigned)e);
+            if (latent_suffix) add_latent_suffix(k);
+            return LIC360_ERR_CODER;
         }
-        set_error("%s%s", msg, suffix);
-        return LIC360_ERR_CODER;
-    }
     for (int k = 0; k < K; k++)
         for (int sid = 0; sid < 2; sid++) {
             bits_host[2 * k + sid] = r.bits[sid * K + k];
@@ -1260,8 +1329,7 @@ int lic360_codec_estimate_batch(lic360_codec* c, int K, const float* code_dev, c
                                 float* code_bits_dev, float* imp_bits_dev, double* bits_host, long long* counts_host) {
     LIC360_CHECK_ARG(K >= 1, "K must be at least 1");
     LIC360_CHECK_ARG(c && code_dev && mask_dev && imp_dev && bits_host && counts_host, "bad arguments");
-    LIC360_CHECK_ARG(K <= kMaxBatch && (long long)3 * K * c->code.G * c->H * c->W <= 0x7fffffffLL,
-                     "K exceeds the launch limits of a batch (3K conv images, 3 * K * 48 * H * W input floats)");
+    LIC360_CHECK_BATCH(c, K);
     return estimate_latents(c, K, code_dev, mask_dev, imp_dev, code_bits_dev, imp_bits_dev, bits_host, counts_host, true);
 }
 
@@ -1283,27 +1351,16 @@ int lic360_imp_levels_to_mask(const float* levels_dev, int h, int w, const int* 
     return LIC360_OK;
 }
 
-// stream stream_id of latent k of the last encode: in enc_out after a batch coded on the pool, else (k = 0) in the codec's coders
-static const uint8_t* encoded_stream(lic360_codec* c, int k, int stream_id, long* n) {
-    if (c->enc_pooled) {
-        const std::vector<uint8_t>& b = c->enc_out[2 * (size_t)k + (stream_id ? 1 : 0)].bytes;
-        *n = (long)b.size();
-        return b.data();
-    }
-    return coder_bytes(stream_id ? c->imp.coder : c->code.coder, n);
-}
-
+// stream stream_id of latent k of the last encode (none before the first encode and after a failed one)
 static long copy_stream(lic360_codec* c, int k, int stream_id, uint8_t* out, long cap) {
-    long n = 0;
-    const uint8_t* b = encoded_stream(c, k, stream_id, &n);
-    if (out && cap > 0) memcpy(out, b, (size_t)std::min(n, cap));
+    const std::vector<uint8_t>& b = c->enc_out[2 * (size_t)k + (stream_id ? 1 : 0)].bytes;
+    const long n = (long)b.size();
+    if (out && cap > 0) memcpy(out, b.data(), (size_t)std::min(n, cap));
     return n;
 }
 
 long lic360_codec_stream_size(lic360_codec* c, int stream_id) {
-    long n = 0;
-    encoded_stream(c, 0, stream_id, &n);
-    return n;
+    return copy_stream(c, 0, stream_id, nullptr, 0);
 }
 
 long lic360_codec_stream_copy(lic360_codec* c, int stream_id, uint8_t* out, long cap) {
@@ -1367,18 +1424,19 @@ static int rows_stalled(void* vp) {
     return 0;
 }
 
-static int final_scatter(lic360_codec* c, NetDesc& n, bool is_code) {
-    // scatter the symbols of the last step (the final TileInput of lic360_demo.py:236,285)
-    const WfNetDev& w = n.wf.dev;
-    const int tgrid = (n.max_len + 127) / 128;
-    cudaStream_t s = n.stream;
-    if (is_code)
-        scatter_prev_kernel<<<tgrid, 128, 0, s>>>(n.syms_host, n.wf.fp[0], n.wf.fc[0], n.idx_dev, n.steps_dev, n.ctr_dev, n.arrived_dev, n.G, n.H, n.W,
-                                                  w.D, w.HS, w.Dp, w.Hp, -3.5f, 1.0f, 3, nullptr);
-    else
-        scatter_prev_kernel<<<tgrid, 128, 0, s>>>(n.syms_host, n.wf.fp[0], n.wf.fc[0], n.idx_dev, n.steps_dev, n.ctr_dev, n.arrived_dev, 1, n.H, n.W,
-                                                  w.D, w.HS, w.Dp, w.Hp, -1.0f, (float)(2. / (48 - 1.)), 1, c->levels_dev);
-    LAUNCH_CHECK();
+// code stream: spin until the first row of step sc.p carries its tag (the time until then is waiting for the GPU; the coder decodes the
+// later rows as they arrive)
+static int wait_first_row(StallCtx& sc) {
+    const uint16_t* meta = sc.n->rows_step_host + 7;
+    for (unsigned spins = 1; ((__atomic_load_n(meta, __ATOMIC_ACQUIRE) >> 4) & 15) != (unsigned)wf_row_tag(sc.p); spins++) {
+#if defined(__x86_64__)
+        __builtin_ia32_pause();
+#endif
+        if ((spins & 0x3FFF) == 0) {
+            const int rc = rows_stalled(&sc);
+            if (rc) return rc;
+        }
+    }
     return LIC360_OK;
 }
 
@@ -1412,37 +1470,43 @@ struct PersistStop {  // every exit path: the chain kernel stops at its next ste
 // old-term kernel on the low-priority side stream, (3) decodes the rows as they arrive.  Against the graph replay per step this
 // takes the graph launch, the scatter kernel and the chain kernel's prologue off the critical path; the price is that the chain's 24
 // SMs stay occupied for the whole decode (fine for one image at a time, the wrong trade with several in flight).
-static int decode_stream_persistent(lic360_codec* c, NetDesc& n) {
-    cudaStream_t s = n.stream, side = n.side;
+// The state every decode of a stream starts from: host flags and publication tags, timers, the trace vectors, the engine's frames and
+// the device counters (enqueued on the stream's CUDA stream)
+static int decode_reset(NetDesc& n) {
+    cudaStream_t s = n.stream;
     for (int i = 0; i < 64; i++) n.flag_host[i] = 0;
-    memset(n.rows_step_host, 0, (size_t)n.max_len * n.row_bytes);
-    memset(n.syms_host, 0, (size_t)n.max_len * sizeof(float));  // tag 0 = not published
-    __atomic_store_n(n.go_host, -1, __ATOMIC_RELEASE);
-    PersistStop stop{n.go_host};
+    memset(n.rows_step_host, 0, (size_t)n.max_len * n.row_bytes);  // publication tags of a previous decode must not match step 0
     n.t_host_coder = 0; n.t_gpu_wait = 0;
-    const bool trace_file = getenv("LIC360_WF_TRACE_FILE") != nullptr;
-    n.step_wait_us.clear(); n.step_decode_us.clear(); n.step_levels_us.clear();
     for (int i = 0; i < 5; i++) n.t_kernel[i] = 0;
+    n.step_wait_us.clear(); n.step_decode_us.clear(); n.step_levels_us.clear();
     LIC360_CUDA(wf_clear(n.wf, s));
-    LIC360_CUDA(cudaMemsetAsync(n.ctr_dev, 0xFF, sizeof(int), s));
+    LIC360_CUDA(cudaMemsetAsync(n.ctr_dev, 0xFF, sizeof(int), s));  // -1: the scatter kernel of step p makes it p
     LIC360_CUDA(cudaMemsetAsync(n.done_dev, 0, sizeof(int), s));
     LIC360_CUDA(cudaMemsetAsync(n.arrived_dev, 0, sizeof(int), s));
     LIC360_CUDA(cudaMemsetAsync(n.sync_dev, 0, sizeof(int), s));
+    return LIC360_OK;
+}
+
+static int decode_stream_persistent(lic360_codec* c, NetDesc& n) {
+    cudaStream_t s = n.stream, side = n.side;
+    int rc = decode_reset(n);
+    if (rc) return rc;
+    memset(n.syms_host, 0, (size_t)n.max_len * sizeof(float));  // tag 0 = not published
+    __atomic_store_n(n.go_host, -1, __ATOMIC_RELEASE);
+    PersistStop stop{n.go_host};
+    const bool trace_file = getenv("LIC360_WF_TRACE_FILE") != nullptr;
     LIC360_CUDA(cudaMemsetAsync(n.go_dev, 0xFF, sizeof(int), s));
     LIC360_CUDA(cudaMemsetAsync(n.old_done_dev, 0, sizeof(int), s));
     LIC360_CUDA(cudaMemsetAsync(n.scat_done_dev, 0, 4 * sizeof(int), s));
     LIC360_CUDA(cudaEventRecord(n.ev_fork, s));
     LIC360_CUDA(cudaStreamWaitEvent(side, n.ev_fork, 0));
     LIC360_CUDA(wf_launch_old(n.wf, 0, side, false, 0, n.old_done_dev, n.scat_done_dev));  // old terms of step 0 (all zero; keeps the protocol uniform)
-    WfRows rows;
-    rows.rows = n.rows_step_host; rows.levels = c->levels_dev; rows.flag = n.flag_host; rows.sync = n.sync_dev;
-    rows.s2 = (float)(1. / sqrt(2.0));
     WfPersist ps;
     memset(&ps, 0, sizeof(ps));
     ps.syms = n.syms_host; ps.go_host = n.go_host; ps.go_dev = n.go_dev; ps.old_done = n.old_done_dev; ps.ctr = n.ctr_dev; ps.scat_done = n.scat_done_dev;
-    ps.bias = -3.5f; ps.scale = 1.0f;
-    LIC360_CUDA(wf_launch_chain(n.wf, s, rows, &ps));
-    int rc = LIC360_OK;
+    const TileIn t = tile_input(true);
+    ps.bias = t.bias; ps.scale = t.scale;
+    LIC360_CUDA(wf_launch_chain(n.wf, s, wf_rows(c, n), &ps));
     for (int p = 0; p < n.nsteps; p++) {
         auto tw = clk::now();
         rc = wait_levels(c, n, p);
@@ -1453,17 +1517,13 @@ static int decode_stream_persistent(lic360_codec* c, NetDesc& n) {
         // the critical path (the GPU is busy with step p for the next ~60 us)
         if (p + 1 < n.nsteps) LIC360_CUDA(wf_launch_old(n.wf, 0, side, false, p + 1, n.old_done_dev, n.scat_done_dev));
         StallCtx sc{c, &n, p, clk::now()};
-        for (unsigned spins = 1; ((__atomic_load_n(n.rows_step_host + 7, __ATOMIC_ACQUIRE) >> 4) & 15) != (unsigned)(p % 15 + 1); spins++) {
-#if defined(__x86_64__)
-            __builtin_ia32_pause();
-#endif
-            if ((spins & 0x3FFF) == 0) { rc = rows_stalled(&sc); if (rc) return rc; }
-        }
+        rc = wait_first_row(sc);
+        if (rc) return rc;
         n.t_gpu_wait += ms_since(tw);
         if (trace_file) n.step_wait_us.push_back((float)(ms_since(tw) * 1e3));
         auto th = clk::now();
-        rc = coder_decode_packed_gmm_tagged(n.coder, n.rows_step_host, n.steps[p].len, n.syms_host, p % 15 + 1, rows_stalled, &sc,
-                                            p + 1 < n.nsteps ? (unsigned)(p % 15 + 1) : 0u);  // symbol words tagged too: the chain kernel polls
+        rc = coder_decode_packed_gmm_tagged(n.coder, n.rows_step_host, n.steps[p].len, n.syms_host, wf_row_tag(p), rows_stalled, &sc,
+                                            p + 1 < n.nsteps ? (unsigned)wf_row_tag(p) : 0u);  // symbol words tagged too: the chain kernel polls
                                             // them one by one (not the last step's: the final scatter reads plain floats)
         n.t_host_coder += ms_since(th);
         if (trace_file) n.step_decode_us.push_back((float)(ms_since(th) * 1e3));
@@ -1471,7 +1531,8 @@ static int decode_stream_persistent(lic360_codec* c, NetDesc& n) {
     }
     LIC360_CUDA(cudaEventRecord(n.ev_join, side));
     LIC360_CUDA(cudaStreamWaitEvent(s, n.ev_join, 0));
-    return final_scatter(c, n, true);  // behind the chain kernel in stream order; the device step counter is nsteps - 1
+    // the final TileInput of lic360_demo.py:236: behind the chain kernel in stream order; the device step counter is nsteps - 1
+    return launch_scatter(c, n, true, s);
 }
 
 // The wavefront loop of one bitstream.  is_code: before step p the importance levels of every 2x2 cell the slab touches
@@ -1480,20 +1541,11 @@ static int decode_stream_persistent(lic360_codec* c, NetDesc& n) {
 static int decode_stream(lic360_codec* c, NetDesc& n, bool is_code) {
     if (is_code && c->mode == 2) return decode_stream_persistent(c, n);
     cudaStream_t s = n.stream;
-    int rc = LIC360_OK;
-    for (int i = 0; i < 64; i++) n.flag_host[i] = 0;
-    memset(n.rows_step_host, 0, (size_t)n.max_len * n.row_bytes);  // publication tags of a previous decode must not match step 0
-    n.t_host_coder = 0; n.t_gpu_wait = 0;
+    int rc = decode_reset(n);
+    if (rc) return rc;
     const bool trace_file = getenv("LIC360_WF_TRACE_FILE") != nullptr;
-    n.step_wait_us.clear(); n.step_decode_us.clear(); n.step_levels_us.clear();
-    LIC360_CUDA(wf_clear(n.wf, s));
-    LIC360_CUDA(cudaMemsetAsync(n.ctr_dev, 0xFF, sizeof(int), s));  // -1: the scatter kernel of step p makes it p
-    LIC360_CUDA(cudaMemsetAsync(n.done_dev, 0, sizeof(int), s));
-    LIC360_CUDA(cudaMemsetAsync(n.arrived_dev, 0, sizeof(int), s));
-    LIC360_CUDA(cudaMemsetAsync(n.sync_dev, 0, sizeof(int), s));
     LIC360_CUDA(wf_launch_old(n.wf, 1, s));  // old terms of step 0 = counter (-1) + 1 (all zero, but it keeps the schedule uniform)
-    if (getenv("LIC360_DEBUG_SYNC")) LIC360_CUDA(cudaStreamSynchronize(s));
-    for (int i = 0; i < 5; i++) n.t_kernel[i] = 0;
+    if (debug_sync()) LIC360_CUDA(cudaStreamSynchronize(s));
     for (int p = 0; p < n.nsteps; p++) {
         auto tw = clk::now();
         if (is_code) { rc = wait_levels(c, n, p); if (rc) return rc; }
@@ -1519,17 +1571,12 @@ static int decode_stream(lic360_codec* c, NetDesc& n, bool is_code) {
         const int len = n.steps[p].len;
         if (is_code) {
             StallCtx sc{c, &n, p, clk::now()};
-            // time until the first row is there = waiting for the GPU; the rest of the call decodes while the later rows arrive
-            for (unsigned spins = 1; ((__atomic_load_n(n.rows_step_host + 7, __ATOMIC_ACQUIRE) >> 4) & 15) != (unsigned)(p % 15 + 1); spins++) {
-#if defined(__x86_64__)
-                __builtin_ia32_pause();
-#endif
-                if ((spins & 0x3FFF) == 0) { rc = rows_stalled(&sc); if (rc) return rc; }
-            }
+            rc = wait_first_row(sc);
+            if (rc) return rc;
             n.t_gpu_wait += ms_since(th);
             if (trace_file) n.step_wait_us.push_back((float)(ms_since(tw) * 1e3));
             th = clk::now();
-            rc = coder_decode_packed_gmm_tagged(n.coder, n.rows_step_host, len, n.syms_host, p % 15 + 1, rows_stalled, &sc);
+            rc = coder_decode_packed_gmm_tagged(n.coder, n.rows_step_host, len, n.syms_host, wf_row_tag(p), rows_stalled, &sc);
         } else {
             rc = coder_decode_packed_imp(n.coder, n.rows_step_host, len, n.syms_host);
         }
@@ -1537,7 +1584,7 @@ static int decode_stream(lic360_codec* c, NetDesc& n, bool is_code) {
         if (trace_file && is_code) n.step_decode_us.push_back((float)(ms_since(th) * 1e3));
         if (rc) return rc;
     }
-    rc = final_scatter(c, n, is_code);
+    rc = launch_scatter(c, n, is_code, s);  // the symbols of the last step (the final TileInput of lic360_demo.py:236,285)
     if (rc) return rc;
     if (!is_code) {
         LIC360_CUDA(cudaStreamSynchronize(s));
@@ -1559,21 +1606,9 @@ int lic360_codec_decode(lic360_codec* c, const uint8_t* imp_bytes, long n_imp, c
     c->enc_k = 0;  // the streams of the last encode are no longer returned by the batch accessors
     c->imp_ready.store(0);
     c->abort_flag.store(0);
-    // debug timeline of the code stream (LIC360_WF_TRACE=1): %globaltimer stamps per step, summarised on stderr
-    unsigned long long* trace_dev = nullptr;
-    const int tr_sel = getenv("LIC360_WF_TRACE") && atoi(getenv("LIC360_WF_TRACE")) == 2 ? 1 : 0;  // 2: trace the importance stream
-    const NetDesc& tr_net = tr_sel ? c->imp : c->code;
-    const int tr_steps = tr_net.nsteps + 2;
-    if (getenv("LIC360_WF_TRACE")) {
-        std::vector<unsigned long long> init((size_t)tr_steps * WF_TR_SLOTS + 64, 0ull);  // + per-layer phase sums of the G = 1 chain
-        for (int p = 0; p < tr_steps; p++)
-            for (int k = 0; k < WF_TR_SLOTS; k++)
-                init[(size_t)p * WF_TR_SLOTS + k] = (k == WF_TR_CHAIN1 || k == WF_TR_ROWS1 || k == WF_TR_OLD1 || k == WF_TR_TAIL1) ? 0ull : ~0ull;
-        LIC360_CUDA(cudaMalloc(&trace_dev, init.size() * 8));
-        LIC360_CUDA(cudaMemcpy(trace_dev, init.data(), init.size() * 8, cudaMemcpyHostToDevice));
-        wf_trace_set(trace_dev, tr_sel);
-        codec_trace_set(trace_dev, tr_sel);
-    }
+    DecodeTrace trace;
+    rc = decode_trace_begin(c, trace);
+    if (rc) return rc;
     // Admission first: a decode queues here when the device already runs as many decodes as it can hold, and a low-latency decode takes
     // the device for itself.  Everything below -- graph capture and instantiation included, which may allocate and therefore wait for the
     // device -- runs inside the slot: a thread that blocks in the driver while ANOTHER decode's persistent kernel waits for its host
@@ -1590,12 +1625,12 @@ int lic360_codec_decode(lic360_codec* c, const uint8_t* imp_bytes, long n_imp, c
     // ---- importance stream (lic360_demo.py:272-290) and code stream (:220-238), concurrently in the pipelined mode: the
     // code stream only reads importance levels that are already decoded (decode_stream).  Serialized in profile mode.
     int rc_imp = LIC360_OK;
-    c->imp.err[0] = 0;
+    char imp_err[256] = {0};  // error text of the importance loop's thread (set_error is thread-local)
     auto imp_loop = [&]() {
         cudaSetDevice(c->device);
         rc_imp = decode_stream(c, c->imp, false);
         if (rc_imp) {
-            snprintf(c->imp.err, sizeof(c->imp.err), "%s", lic360_last_error());
+            snprintf(imp_err, sizeof(imp_err), "%s", lic360_last_error());
             c->abort_flag.store(1);
         }
         c->t_imp = ms_since(t0);
@@ -1607,17 +1642,17 @@ int lic360_codec_decode(lic360_codec* c, const uint8_t* imp_bytes, long n_imp, c
         if (rc) { code_err = lic360_last_error(); c->abort_flag.store(1); }
         c->imp_worker.wait();
         // both failed: the stream that failed FIRST carries the cause, the other one only reports the abort it was told about
-        if (rc && rc_imp && strstr(c->imp.err, "aborted (the other stream failed)")) {
+        if (rc && rc_imp && strstr(imp_err, "aborted (the other stream failed)")) {
             set_error("%s", code_err.c_str());
-            cudaStreamSynchronize(c->code.stream); cudaStreamSynchronize(c->imp.stream);
+            drain(c);
             return rc;
         }
     } else {
         imp_loop();
         if (rc_imp == LIC360_OK) rc = decode_stream(c, c->code, true);
     }
-    if (rc_imp) { set_error("%s", c->imp.err); cudaStreamSynchronize(c->code.stream); cudaStreamSynchronize(c->imp.stream); return rc_imp; }
-    if (rc) { cudaStreamSynchronize(c->code.stream); cudaStreamSynchronize(c->imp.stream); return rc; }
+    if (rc_imp) { set_error("%s", imp_err); drain(c); return rc_imp; }
+    if (rc) { drain(c); return rc; }
     // ---- outputs: mask_up = Dtow(Imp2mask(levels)) (lic360_demo.py:285-290), code = frame + 3.5 * mask (:236-237)
     cudaStream_t s = c->code.stream;
     rc = lic360_imp2mask(c->levels_dev, c->mask192_dev, 1, 192, c->imp.H, c->imp.W, 48, s);
@@ -1629,59 +1664,7 @@ int lic360_codec_decode(lic360_codec* c, const uint8_t* imp_bytes, long n_imp, c
                                                              c->code.wf.dev.Dp, c->code.wf.dev.Hp, 3.5f);
     LAUNCH_CHECK();
     LIC360_CUDA(cudaStreamSynchronize(s));
-    if (trace_dev) {
-        std::vector<unsigned long long> tr((size_t)tr_steps * WF_TR_SLOTS + 64);
-        cudaMemcpy(tr.data(), trace_dev, tr.size() * 8, cudaMemcpyDeviceToHost);
-        wf_trace_set(nullptr, 0);
-        codec_trace_set(nullptr, 0);
-        cudaFree(trace_dev);
-        const char* names[WF_TR_SLOTS] = {"scatter start", "prev start", "chain start", "chain end", "rows start", "rows flag", "old start", "old end", "R tail start", "R tail end"};
-        for (int w0 = 0; w0 < 2; w0++) {  // two windows: while the importance stream still runs / after it finished
-            const int pa = tr_sel ? (w0 == 0 ? 10 : 50) : (w0 == 0 ? 20 : 140), pb = tr_sel ? (w0 == 0 ? 45 : 90) : (w0 == 0 ? 80 : 220);
-            double acc[WF_TR_SLOTS] = {0}, period = 0;
-            int cnt = 0;
-            for (int p = pa; p < pb && p + 1 < tr_net.nsteps; p++) {
-                const unsigned long long* r = &tr[(size_t)p * WF_TR_SLOTS];
-                for (int k = 0; k < WF_TR_SLOTS; k++) acc[k] += (double)(long long)(r[k] - r[0]) * 1e-3;
-                period += (double)(long long)(tr[(size_t)(p + 1) * WF_TR_SLOTS] - r[0]) * 1e-3;
-                cnt++;
-            }
-            fprintf(stderr, "lic360 trace, %s-stream steps %d..%d: period %.1f us;", tr_sel ? "importance" : "code", pa, pb, period / cnt);
-            for (int k = 1; k < WF_TR_SLOTS; k++) fprintf(stderr, " %s +%.1f;", names[k], acc[k] / cnt);
-            fprintf(stderr, "\n");
-        }
-        if (const char* fn = getenv("LIC360_WF_TRACE_FILE")) {  // per-step dump: step, slab length, us relative to the step's slot 0, period
-            if (FILE* f = fopen(fn, "w")) {
-                fprintf(f, "step,len,prev_start,chain_start,chain_end,rows_start,rows_last,old_start,old_end,tail_start,tail_end,period,host_wait_us,host_decode_us,levels_wait_us\n");
-                for (int p = 0; p + 1 < tr_net.nsteps; p++) {
-                    const unsigned long long* r = &tr[(size_t)p * WF_TR_SLOTS];
-                    fprintf(f, "%d,%d", p, tr_net.steps[p].len);
-                    for (int k = 1; k < WF_TR_SLOTS; k++) fprintf(f, ",%.1f", (double)(long long)(r[k] - r[0]) * 1e-3);
-                    fprintf(f, ",%.1f", (double)(long long)(tr[(size_t)(p + 1) * WF_TR_SLOTS] - r[0]) * 1e-3);
-                    fprintf(f, ",%.1f,%.1f,%.1f\n", (size_t)p < tr_net.step_wait_us.size() ? tr_net.step_wait_us[p] : 0.f,
-                            (size_t)p < tr_net.step_decode_us.size() ? tr_net.step_decode_us[p] : 0.f,
-                            (size_t)p < tr_net.step_levels_us.size() ? tr_net.step_levels_us[p] : 0.f);
-                }
-                fclose(f);
-            }
-        }
-        if (!tr_sel) {
-            fprintf(stderr, "lic360 trace, code-stream chain, CTA 0 thread 0, us per layer [weight staging issue | item: 25 loads, 100 FMA4, stores | prefetch issue + weights landed | cluster barrier]:");
-            for (int l = 0; l < 12; l++) {
-                fprintf(stderr, " L%d", l);
-                for (int ph = 0; ph < 4; ph++) fprintf(stderr, "%c%.2f", ph ? '|' : ' ', (double)tr[(size_t)tr_steps * WF_TR_SLOTS + l * 4 + ph] * 1e-3 / tr_net.nsteps);
-            }
-            fprintf(stderr, "\n");
-        }
-        if (tr_sel) {
-            fprintf(stderr, "lic360 trace, G=1 chain, CTA 0, us per layer [weight staging | Q product | epilogue + DSMEM stores | prefetch + cluster barrier]:");
-            for (int l = 0; l < 12; l++) {
-                fprintf(stderr, " L%d", l);
-                for (int ph = 0; ph < 4; ph++) fprintf(stderr, "%c%.2f", ph ? '|' : ' ', (double)tr[(size_t)tr_steps * WF_TR_SLOTS + l * 4 + ph] * 1e-3 / tr_net.nsteps);
-            }
-            fprintf(stderr, "\n");
-        }
-    }
+    decode_trace_report(c, trace);
     c->t_host_coder = c->code.t_host_coder + c->imp.t_host_coder;
     c->t_gpu_wait = c->code.t_gpu_wait;
     c->t_total = ms_since(t0);

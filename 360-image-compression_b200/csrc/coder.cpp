@@ -146,6 +146,14 @@ inline int ac_update(lic360_coder* c, uint32_t sym_low, uint32_t sym_high, uint3
 // ---- packed-row fast paths of the fused pipeline (codec.cu); see coder_internal.h for the row formats ----------
 namespace lic360 {
 
+int coder_row_error(int stream_id, int row, unsigned sym) {
+    if (stream_id == 0 && sym > 7) set_error("coder: symbol out of range in packed row %d", row);
+    else if (stream_id == 0) set_error("coder: symbol has zero frequency (row %d)", row);
+    else if (sym >= 49) set_error("coder: importance level %u out of range", sym);
+    else set_error("coder: symbol has zero frequency");
+    return LIC360_ERR_CODER;
+}
+
 static inline uint32_t gmm_bin(const uint16_t* r, int j) {  // j in 0..8
     if (j == 0) return 0;
     if (j == 8) return 65536;
@@ -229,9 +237,9 @@ int coder_encode_packed_gmm(lic360_coder* c, const uint16_t* rows, int nrows) {
         for (int i = 0; i < nrows; i++) {
             const uint16_t* r = rows + (size_t)i * 8;
             if (!((r[7] >> 8) & 1)) continue;  // mask < 0.5: not coded (coder.cpp:79)
-            if (r[7] & 8) { set_error("coder: symbol out of range in packed row %d", i); return LIC360_ERR_CODER; }
+            if (r[7] & 8) return coder_row_error(0, i, 8);
             const int s = r[7] & 7;
-            if (!e.update(gmm_bin(r, s), gmm_bin(r, s + 1))) { set_error("coder: symbol has zero frequency (row %d)", i); return LIC360_ERR_CODER; }
+            if (!e.update(gmm_bin(r, s), gmm_bin(r, s + 1))) return coder_row_error(0, i, s);
         }
         return LIC360_OK;
     });
@@ -352,8 +360,10 @@ int coder_encode_packed_imp(lic360_coder* c, const uint16_t* rows, int nrows) {
     for (int i = 0; i < nrows; i++) {
         const uint16_t* r = rows + (size_t)i * 64;
         const int s = r[48];
-        if (s >= 49) { set_error("coder: importance level %d out of range", s); return LIC360_ERR_CODER; }
-        int rc = ac_update<false>(c, imp_bin(r, s), imp_bin(r, s + 1), 65536);
+        if (s >= 49) return coder_row_error(1, i, s);
+        const uint32_t lo = imp_bin(r, s), hi = imp_bin(r, s + 1);
+        if (lo == hi) return coder_row_error(1, i, s);
+        int rc = ac_update<false>(c, lo, hi, 65536);
         if (rc) return rc;
     }
     return LIC360_OK;

@@ -784,7 +784,7 @@ __device__ __noinline__ void wf_chain4_rows(const WfNetDev& net, const WfRows& r
         if (live && j == 0) {
             fixup_row(o, 8, true);
             const int lvl = (int)(__ldcg(rows.levels + (th >> 1) * (W >> 1) + (tw >> 1)) + 1e-5f);  // written by the other stream's kernels
-            pack_gmm_row(o, 0, code_mask_from_level(lvl, tc, th, tw), rows.rows + (size_t)li * 8, psum % 15 + 1);
+            pack_gmm_row(o, 0, code_mask_from_level(lvl, tc, th, tw), rows.rows + (size_t)li * 8, wf_row_tag(psum));
         }
     }
     // self-validating rows: no fence, no flag; the host decodes row i as soon as row i carries this step's tag
@@ -948,7 +948,7 @@ __device__ __noinline__ bool wf_chain4_step_begin(const WfNetDev& net, const WfP
     } else if (tid >= 32 && p > 0) {
         const StepDesc d = net.steps[p - 1];
         const int HW = net.H * net.W, nw = nt - 32;
-        const unsigned tag = (unsigned)((p - 1) % 15 + 1);
+        const unsigned tag = (unsigned)wf_row_tag(p - 1);
         float* fp0 = const_cast<float*>(net.L[0].xp);
         float* fc0 = const_cast<float*>(net.L[0].xc);
         const unsigned* words = reinterpret_cast<const unsigned*>(ps.syms);

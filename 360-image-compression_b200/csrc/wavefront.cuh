@@ -42,9 +42,12 @@ struct WfNetDev {
 };
 
 // The CDF rows of the step are produced at the end of wf_chain4_kernel and wf_chain1_kernel (no extra launch on the critical path).
-// wf_chain4_kernel (code stream) publishes every row by its tag step % 15 + 1, with no system fence + flag behind the rows: the host
+// wf_chain4_kernel (code stream) publishes every row by its tag wf_row_tag(step), with no system fence + flag behind the rows: the host
 // validates row by row; it also evaluates the previous-wavefront terms of the NEXT step (layers 1..11) behind the rows.
 // wf_chain1_kernel (importance stream) raises the flag once its rows are written.
+// The tag of a step is never 0 (the value of a row nobody has written) and differs from the previous step's.  The persistent decode
+// tags the decoded symbol words of a step with it too.
+__host__ __device__ __forceinline__ int wf_row_tag(int step) { return step % 15 + 1; }
 struct WfRows {
     uint16_t* rows;       // mapped pinned: packed rows of the step
     const float* levels;  // decoded importance levels (mask bit = Imp2mask + Dtow of the symbol's 2x2 cell)

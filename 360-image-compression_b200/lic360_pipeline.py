@@ -183,6 +183,15 @@ class FusedCodec(object):
             raise RuntimeError("FusedCodec: expected shape %s, got %s" % (shape, tuple(t.shape)))
         return t.contiguous()
 
+    def _latents(self, K, code, mask, imap_quant):
+        """K latents as the native calls read them: code, mask (K,48,H,W) and imap_quant (K,1,H/2,W/2), float32 and contiguous on the
+        codec's device (mask None: not checked, returned as None), once torch's stream has produced them."""
+        code = self._f32(code, (K, 48, self.H, self.W))
+        mask = None if mask is None else self._f32(mask, (K, 48, self.H, self.W))
+        imp = self._f32(imap_quant, (K, 1, self.H // 2, self.W // 2))
+        torch.cuda.current_stream(self.dev).synchronize()
+        return code, mask, imp
+
     def _stream_bytes(self, sid):
         n = LIB.lic360_codec_stream_size(self._h, sid)
         buf = (ctypes.c_uint8 * max(n, 1))()
@@ -190,10 +199,7 @@ class FusedCodec(object):
         return bytes(buf[:n])
 
     def encode(self, code, mask, imap_quant, name=None):
-        code = self._f32(code, (1, 48, self.H, self.W))
-        mask = self._f32(mask, (1, 48, self.H, self.W))
-        imp = self._f32(imap_quant, (1, 1, self.H // 2, self.W // 2))
-        torch.cuda.current_stream(self.dev).synchronize()  # inputs were produced on torch's stream
+        code, mask, imp = self._latents(1, code, mask, imap_quant)
         check(LIB.lic360_codec_encode(self._h, code.data_ptr(), mask.data_ptr(), imp.data_ptr()))
         return self._stream_bytes(1), self._stream_bytes(0)
 
@@ -213,10 +219,7 @@ class FusedCodec(object):
         byte-identical to encode() of latent k alone.  A latent encode would refuse raises encode's message followed by
         ' (latent k)', for the first such k."""
         K = int(code.shape[0]) if code.dim() == 4 else -1
-        code = self._f32(code, (K, 48, self.H, self.W))
-        mask = self._f32(mask, (K, 48, self.H, self.W))
-        imp = self._f32(imap_quant, (K, 1, self.H // 2, self.W // 2))
-        torch.cuda.current_stream(self.dev).synchronize()  # inputs were produced on torch's stream
+        code, mask, imp = self._latents(K, code, mask, imap_quant)
         check(LIB.lic360_codec_encode_batch(self._h, K, code.data_ptr(), mask.data_ptr(), imp.data_ptr()))
         return [(self._batch_stream_bytes(k, 1), self._batch_stream_bytes(k, 0)) for k in range(K)]
 
@@ -230,13 +233,10 @@ class FusedCodec(object):
         and I its total, the bytes `encode` writes satisfy -(1 + u + N/8192) <= 8 * len(stream) - I <= 8 + N/8192, where u is the
         number of pending underflow bits the coder drops at the end (a few at most in practice; derivation in
         tests/test_rate_estimate.py).  Raises RuntimeError on the inputs `encode` refuses, with the same message."""
-        code = self._f32(code, (1, 48, self.H, self.W))
-        mask = self._f32(mask, (1, 48, self.H, self.W))
-        imp = self._f32(imap_quant, (1, 1, self.H // 2, self.W // 2))
+        code, mask, imp = self._latents(1, code, mask, imap_quant)
         code_map = torch.empty((1, 48, self.H, self.W), dtype=torch.float32, device=self.dev)
         imp_map = torch.empty((1, 1, self.H // 2, self.W // 2), dtype=torch.float32, device=self.dev)
         totals = (ctypes.c_double * 2)()
-        torch.cuda.current_stream(self.dev).synchronize()  # inputs were produced on torch's stream
         check(LIB.lic360_codec_estimate(self._h, code.data_ptr(), mask.data_ptr(), imp.data_ptr(), code_map.data_ptr(),
                                         imp_map.data_ptr(), totals))
         return {'code_bits': totals[0], 'imp_bits': totals[1], 'code_map': code_map, 'imp_map': imp_map}
@@ -249,16 +249,13 @@ class FusedCodec(object):
         alone.  The maps are views into (K,...) tensors, or None with maps=False.  A latent encode would refuse raises encode's
         message followed by ' (latent k)', for the first such k."""
         K = int(code.shape[0]) if code.dim() == 4 else -1
-        code = self._f32(code, (K, 48, self.H, self.W))
-        mask = self._f32(mask, (K, 48, self.H, self.W))
-        imp = self._f32(imap_quant, (K, 1, self.H // 2, self.W // 2))
+        code, mask, imp = self._latents(K, code, mask, imap_quant)
         code_map = imp_map = None
         if maps:
             code_map = torch.empty((K, 48, self.H, self.W), dtype=torch.float32, device=self.dev)
             imp_map = torch.empty((K, 1, self.H // 2, self.W // 2), dtype=torch.float32, device=self.dev)
         totals = (ctypes.c_double * max(2 * K, 1))()
         counts = (ctypes.c_longlong * max(2 * K, 1))()
-        torch.cuda.current_stream(self.dev).synchronize()  # inputs were produced on torch's stream
         check(LIB.lic360_codec_estimate_batch(self._h, K, code.data_ptr(), mask.data_ptr(), imp.data_ptr(),
                                               None if code_map is None else code_map.data_ptr(),
                                               None if imp_map is None else imp_map.data_ptr(), totals, counts))
@@ -276,8 +273,7 @@ class FusedCodec(object):
         Returns {'imp_bytes', 'code_bytes', 'offset', 'levels' (1,1,H/2,W/2), 'mask' (1,48,H,W), 'bound': bytes bound of the
         chosen offset, 'bounds': {offset: bound} of every offset evaluated}.  RuntimeError when no offset fits, and when the
         encoded streams exceed max_bytes (the bound would be broken: never returned silently)."""
-        code = self._f32(code, (1, 48, self.H, self.W))
-        imp = self._f32(imap_quant, (1, 1, self.H // 2, self.W // 2))
+        code, _, imp = self._latents(1, code, None, imap_quant)
         max_bytes = int(max_bytes)
         cands = {}
 
