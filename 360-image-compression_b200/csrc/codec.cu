@@ -555,20 +555,26 @@ __global__ void __launch_bounds__(BITS_THREADS) bits_sum_kernel(const double* __
     if (threadIdx.x == 0) { total[blockIdx.x] = v; total_count[blockIdx.x] = (long long)coded; }
 }
 
-// candidate j (blockIdx.y) of lic360_imp_levels_to_mask: level max(s - off, 0) of every cell, s = imp_symbol(level) the symbol encode
-// codes, and the (48, 2h, 2w) code mask the decoder derives from it (Imp2mask + Dtow)
+// level of one cell in candidate t: max(s - max(t - P, 0), 0), s = imp_symbol(level) the symbol encode codes, P = protect[cell] clamped
+// to [0, 48] (0 without a protection map, where this is max(s - t, 0))
+__device__ __forceinline__ int candidate_level(const float* __restrict__ levels, const int32_t* __restrict__ protect, int cell, int t) {
+    const int drop = protect ? max(t - min(max(protect[cell], 0), 48), 0) : t;
+    return max((int)imp_symbol(levels[cell]) - drop, 0);
+}
+
+// candidate j (blockIdx.y) of lic360_imp_levels_to_mask_protected: the candidate level of every cell (candidate_level) and the
+// (48, 2h, 2w) code mask the decoder derives from it (Imp2mask + Dtow)
 struct LevelOffsets { int k[32]; };
-__global__ void imp_levels_to_mask_kernel(const float* __restrict__ levels, int h, int w, LevelOffsets off, float* __restrict__ levels_out,
-                                          float* __restrict__ mask_out) {
+__global__ void imp_levels_to_mask_kernel(const float* __restrict__ levels, const int32_t* __restrict__ protect, int h, int w,
+                                          LevelOffsets off, float* __restrict__ levels_out, float* __restrict__ mask_out) {
     const int j = blockIdx.y, k = off.k[j], hw = h * w, W = 2 * w, n = 48 * 4 * hw;
     levels_out += (size_t)j * hw;
     mask_out += (size_t)j * n;
     for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x) {
         const int tw = i % W, th = (i / W) % (2 * h), tc = i / (W * 2 * h);
         const int cell = (th >> 1) * w + (tw >> 1);
-        const int lvl = max((int)imp_symbol(levels[cell]) - k, 0);
-        mask_out[i] = (float)code_mask_from_level(lvl, tc, th, tw);
-        if (i < hw) levels_out[i] = (float)max((int)imp_symbol(levels[i]) - k, 0);
+        mask_out[i] = (float)code_mask_from_level(candidate_level(levels, protect, cell, k), tc, th, tw);
+        if (i < hw) levels_out[i] = (float)candidate_level(levels, protect, i, k);
     }
 }
 
@@ -1335,6 +1341,11 @@ int lic360_codec_estimate_batch(lic360_codec* c, int K, const float* code_dev, c
 
 int lic360_imp_levels_to_mask(const float* levels_dev, int h, int w, const int* offsets_host, int K, float* levels_out_dev,
                               float* mask_out_dev, void* stream) {
+    return lic360_imp_levels_to_mask_protected(levels_dev, h, w, offsets_host, K, nullptr, levels_out_dev, mask_out_dev, stream);
+}
+
+int lic360_imp_levels_to_mask_protected(const float* levels_dev, int h, int w, const int* offsets_host, int K, const int32_t* protect_dev,
+                                        float* levels_out_dev, float* mask_out_dev, void* stream) {
     LIC360_CHECK_ARG(K >= 1, "K must be at least 1");
     LIC360_CHECK_ARG(levels_dev && offsets_host && levels_out_dev && mask_out_dev, "bad arguments");
     LIC360_CHECK_ARG(h > 0 && w > 0 && (long long)48 * 4 * h * w <= 0x7fffffffLL, "bad importance map size");
@@ -1345,7 +1356,7 @@ int lic360_imp_levels_to_mask(const float* levels_dev, int h, int w, const int* 
         const int nj = std::min(32, K - j0);
         for (int j = 0; j < nj; j++) off.k[j] = offsets_host[j0 + j];
         imp_levels_to_mask_kernel<<<dim3(std::max(1, stream_grid(n, 256) / nj), nj), 256, 0, as_stream(stream)>>>(
-            levels_dev, h, w, off, levels_out_dev + (size_t)j0 * h * w, mask_out_dev + (size_t)j0 * n);
+            levels_dev, protect_dev, h, w, off, levels_out_dev + (size_t)j0 * h * w, mask_out_dev + (size_t)j0 * n);
         LAUNCH_CHECK();
     }
     return LIC360_OK;

@@ -369,14 +369,19 @@ class Dtow(BaseOpModule):
         return F_.FwdBwd.apply(self.op, False, x)
 
 
+# the 14 viewport directions of MultiProject (MultiProject.py:24-34), longitude theta and latitude phi in units of pi
+VIEWPORT_THETAS = (-0.5, 0, 0.5, 1, -0.5, 0, 0.5, 1, -0.5, 0, 0.5, 1, 0, 0)
+VIEWPORT_PHIS = (0, 0, 0, 0, 0.25, 0.25, 0.25, 0.25, -0.25, -0.25, -0.25, -0.25, 0.5, -0.5)
+
+
 class MultiProject(BaseOpModule):
     """MultiProject.py:24-34 (SURVEY s8f-2): the 14 viewports (theta, phi in units of pi) of an ERP batch, (N,C,H,W) ->
     (14*N, C, h, w) viewport-major; backward scatters the viewport gradients back with the bilinear weights."""
 
     def __init__(self, h, w, fov=0.6, near=False, device_id=0, time_flag=False):
         super(MultiProject, self).__init__(device_id)
-        self.thetas = [-0.5, 0, 0.5, 1, -0.5, 0, 0.5, 1, -0.5, 0, 0.5, 1, 0, 0]
-        self.phis = [0, 0, 0, 0, 0.25, 0.25, 0.25, 0.25, -0.25, -0.25, -0.25, -0.25, 0.5, -0.5]
+        self.thetas = list(VIEWPORT_THETAS)
+        self.phis = list(VIEWPORT_PHIS)
         self.op = {gid: lic360.ProjectsOp(int(h), int(w), self.thetas, self.phis, fov, near, gid, time_flag) for gid in self.device_list}
 
     def forward(self, x):

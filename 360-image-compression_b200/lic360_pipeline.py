@@ -29,13 +29,29 @@ def make_codec_params(device, seed=2024):
     }
 
 
-def levels_to_mask(imap_quant, offsets):
-    """Candidate importance maps for rate control and the code masks the decoder derives from them (lic360_imp_levels_to_mask).
+def _protect_map(protect, imap_quant):
+    """protect as lic360_imp_levels_to_mask_protected reads it: a (1,1,h,w) integer tensor on imap_quant's device with values in
+    [0, 48], converted to contiguous int32"""
+    if not (isinstance(protect, torch.Tensor) and protect.device == imap_quant.device and not protect.dtype.is_floating_point
+            and not protect.dtype.is_complex and protect.dtype != torch.bool and tuple(protect.shape) == tuple(imap_quant.shape)):
+        raise RuntimeError("levels_to_mask: protect must be a (1,1,h,w) integer tensor on %s, like the importance map"
+                           % imap_quant.device)
+    p = protect.to(torch.int32).contiguous()
+    lo, hi = int(p.min()), int(p.max())
+    if lo < 0 or hi > 48:
+        raise RuntimeError("levels_to_mask: protect values must lie in [0, 48] (got %d .. %d)" % (lo, hi))
+    return p
+
+
+def levels_to_mask(imap_quant, offsets, protect=None):
+    """Candidate importance maps for rate control and the code masks the decoder derives from them (lic360_imp_levels_to_mask,
+    lic360_imp_levels_to_mask_protected).
 
     imap_quant: (1,1,h,w) float32 CUDA tensor of importance levels as `encode` reads them (s = int(level), the symbol it codes);
-    offsets: K integers >= 0.  Returns (levels, masks) on the input's device: levels (K,1,h,w) = max(s - offsets[j], 0) and masks
-    (K,48,2h,2w), channel c at (y, x) = 1 iff 4c + 2 (y % 2) + x % 2 < 4 * level(y/2, x/2).  `encode(code, masks[j:j+1],
-    levels[j:j+1])` gives streams that decode to exactly masks[j]."""
+    offsets: K integers t >= 0; protect: None, or a (1,1,h,w) integer tensor on the same device with values P in [0, 48].
+    Returns (levels, masks) on the input's device: levels (K,1,h,w) = max(s - max(t - P, 0), 0) for t = offsets[j] (P = 0 without
+    a map: max(s - t, 0)) and masks (K,48,2h,2w), channel c at (y, x) = 1 iff 4c + 2 (y % 2) + x % 2 < 4 * level(y/2, x/2).
+    A cell keeps its level until t > P.  `encode(code, masks[j:j+1], levels[j:j+1])` gives streams that decode to exactly masks[j]."""
     if not (isinstance(imap_quant, torch.Tensor) and imap_quant.is_cuda and imap_quant.dtype == torch.float32
             and imap_quant.dim() == 4 and tuple(imap_quant.shape[:2]) == (1, 1)):
         raise RuntimeError("levels_to_mask: expected a (1,1,h,w) float32 CUDA tensor")
@@ -46,12 +62,74 @@ def levels_to_mask(imap_quant, offsets):
     masks = torch.empty((K, 48, 2 * h, 2 * w), dtype=torch.float32, device=dev)
     with torch.cuda.device(dev):
         lv = imap_quant.contiguous()
-        check(LIB.lic360_imp_levels_to_mask(lv.data_ptr(), h, w, (ctypes.c_int * max(K, 1))(*offs), K, levels.data_ptr(),
-                                            masks.data_ptr(), cstream(lv)))
+        offs_c = (ctypes.c_int * max(K, 1))(*offs)
+        if protect is None:
+            check(LIB.lic360_imp_levels_to_mask(lv.data_ptr(), h, w, offs_c, K, levels.data_ptr(), masks.data_ptr(), cstream(lv)))
+        else:
+            p = _protect_map(protect, imap_quant)
+            check(LIB.lic360_imp_levels_to_mask_protected(lv.data_ptr(), h, w, offs_c, K, p.data_ptr(), levels.data_ptr(),
+                                                          masks.data_ptr(), cstream(lv)))
     return levels, masks
 
 
-BUDGET_OFFSETS = tuple(range(0, 49, 8))  # first stage of encode_to_budget's search
+def latitude_protection(h, w, levels, device=None):
+    """Protection map (1,1,h,w) int32 for encode_to_budget / levels_to_mask that follows ERP's cos-latitude area weight: row i gets
+    round(levels * cos(phi_i)), phi_i = pi/2 - pi (i + 0.5) / h its centre latitude.  The equator rows keep their levels longest,
+    the polar rows, which ERP oversamples by 1 / cos(phi), are lowered first.  levels: integer in [0, 48]; device: any torch
+    device (CPU included).  Combine maps with torch.maximum."""
+    levels = _preset_levels(levels)
+    phi = math.pi / 2 - math.pi * (torch.arange(h, dtype=torch.float64) + 0.5) / h
+    rows = torch.round(levels * torch.cos(phi)).to(torch.int32)
+    return rows.view(1, 1, h, 1).expand(1, 1, h, w).contiguous().to(device)
+
+
+def viewport_protection(h, w, views, levels, fov=0.6, device=None):
+    """Protection map (1,1,h,w) int32 for encode_to_budget / levels_to_mask: `levels` on the cells the chosen viewports see, 0
+    elsewhere.  views: indices into MultiProject's 14 viewports (lic360_operator._modules.VIEWPORT_THETAS / VIEWPORT_PHIS; 1 is the
+    front view, 12 and 13 the poles); fov: the viewports' field of view in units of pi (MultiProject's default); device: a CUDA
+    device (default: the current one).  Combine maps with torch.maximum, e.g. with latitude_protection.
+
+    A cell is in the footprint iff it carries a non-zero bilinear weight for at least one pixel of a chosen viewport, rendered by
+    lic360.ProjectsOp (the projection MultiProject's viewport metrics use) from the h x w grid at n x n pixels: one forward, then
+    one backward whose gradient is 1 on the chosen viewports and 0 elsewhere; the footprint is where the scattered weight is > 0.
+
+    Why n leaves no holes: neighbouring viewport pixels are at most p = 2 tan(a) / (n - 1) apart on the sphere, a = fov * pi / 2
+    (at the viewport's centre; rectilinear pixels get denser towards its edges), and a pixel's bilinear taps cover the two cells
+    on either side of it along each axis.  So every cell inside the viewport is hit where p is below two cells, 2 pi / h along a
+    column and 4 pi cos(phi) / w along a row at latitude phi.  n = 2w meets this away from the poles (for the default fov up to
+    |phi| of 83 degrees); where a chosen viewport comes closer to a pole, the cells of the rows there narrow with cos(phi), and
+    the first row, 2 pi sin(pi / h) / w wide, is the narrowest: n is raised to meet the bound at the highest latitude the viewport
+    reaches, capped at that row, with a factor 1.25 for the uneven directions of the pixel grid around the pole.  That costs
+    O(h w) pixels per side for the polar and the +-0.25 viewports (about 720 at h, w = 64, 128), and 2w for the equator ones."""
+    from lic360 import ProjectsOp
+    from lic360_operator._modules import VIEWPORT_PHIS, VIEWPORT_THETAS
+    levels = _preset_levels(levels)
+    views = [int(v) for v in views]
+    if not views or not all(0 <= v < len(VIEWPORT_THETAS) for v in views):
+        raise RuntimeError("viewport_protection: views must be a non-empty list of indices in [0, %d)" % len(VIEWPORT_THETAS))
+    if not 0 < fov < 1:
+        raise RuntimeError("viewport_protection: fov must lie in (0, 1) (units of pi)")
+    device = torch.device('cuda') if device is None else torch.device(device)
+    if device.type != 'cuda':
+        raise RuntimeError("viewport_protection: the footprint is computed on a CUDA device (got %s)" % device)
+    if device.index is None:
+        device = torch.device('cuda', torch.cuda.current_device())
+    a = fov * math.pi / 2
+    reach = max(abs(VIEWPORT_PHIS[v]) for v in views) * math.pi + math.atan(math.sqrt(2) * math.tan(a))  # the corners' latitude
+    lat = min(reach, math.pi / 2 - math.pi / h)
+    n = max(2 * w, math.ceil(1.25 * math.tan(a) * max(w / (2 * math.pi * math.cos(lat)), h / math.pi)) + 1)
+    op = ProjectsOp(n, n, VIEWPORT_THETAS, VIEWPORT_PHIS, fov, False, device.index)
+    op.forward(torch.zeros((1, 1, h, w), dtype=torch.float32, device=device))
+    top = torch.zeros((len(VIEWPORT_THETAS), 1, n, n), dtype=torch.float32, device=device)
+    top[views] = 1
+    weight = op.backward(top)[0]
+    return (weight > 0).to(torch.int32) * levels
+
+
+def _preset_levels(levels):
+    if int(levels) != levels or not 0 <= levels <= 48:
+        raise RuntimeError("protection levels must be an integer in [0, 48] (got %r)" % (levels,))
+    return int(levels)
 
 
 def stream_bytes_bound(bits, symbols):
@@ -65,12 +143,13 @@ def budget_bound(est):
     return stream_bytes_bound(est['imp_bits'], est['imp_symbols']) + stream_bytes_bound(est['code_bits'], est['code_symbols'])
 
 
-def select_budget_offset(estimate, max_bytes):
+def select_budget_offset(estimate, max_bytes, max_offset=48):
     """The level offset encode_to_budget codes: `estimate(offsets)` returns one estimate dict per offset; an offset fits when its
-    budget_bound is at most max_bytes.  Stage 1 evaluates offsets 0, 8, ..., 48; if the smallest that fits, k1, is not 0, stage 2
-    evaluates the seven offsets k1 - 7 .. k1 - 1.  The answer is the smallest evaluated offset that fits; the rate is not assumed to
-    fall monotonically with the offset.  Returns (offset, {offset: bound in bytes} of every offset evaluated); RuntimeError if no
-    offset of stage 1 fits."""
+    budget_bound is at most max_bytes.  Stage 1 evaluates offsets 0, 8, 16, ... up to max_offset, and max_offset itself when it
+    is not on that grid; if the smallest that fits, k1, is not 0, stage 2 evaluates the offsets strictly between the stage-1
+    offset before k1 and k1 (the seven offsets k1 - 7 .. k1 - 1 on the grid).  The answer is the smallest evaluated offset that
+    fits; the rate is not assumed to fall monotonically with the offset.  Returns (offset, {offset: bound in bytes} of every
+    offset evaluated); RuntimeError if no offset of stage 1 fits."""
     bounds = {}
 
     def run(offsets):
@@ -78,13 +157,15 @@ def select_budget_offset(estimate, max_bytes):
         for k, est in zip(offsets, estimate(offsets)):
             bounds[k] = budget_bound(est)
 
-    run(BUDGET_OFFSETS)
-    fit = [k for k in BUDGET_OFFSETS if bounds[k] <= max_bytes]
+    stage1 = list(range(0, max_offset + 1, 8)) + ([max_offset] if max_offset % 8 else [])
+    run(stage1)
+    fit = [j for j, k in enumerate(stage1) if bounds[k] <= max_bytes]
     if not fit:
         raise RuntimeError("encode_to_budget: no level offset up to %d fits %d bytes (bound at offset %d: %d bytes)"
-                           % (BUDGET_OFFSETS[-1], max_bytes, BUDGET_OFFSETS[-1], bounds[BUDGET_OFFSETS[-1]]))
-    if fit[0] > 0:
-        run(range(fit[0] - 7, fit[0]))
+                           % (max_offset, max_bytes, max_offset, bounds[max_offset]))
+    j = fit[0]
+    if j > 0 and stage1[j] - stage1[j - 1] > 1:
+        run(range(stage1[j - 1] + 1, stage1[j]))
     return min(k for k, b in bounds.items() if b <= max_bytes), bounds
 
 
@@ -263,27 +344,35 @@ class FusedCodec(object):
                  'imp_symbols': counts[2 * k + 1], 'code_map': None if code_map is None else code_map[k:k + 1],
                  'imp_map': None if imp_map is None else imp_map[k:k + 1]} for k in range(K)]
 
-    def encode_to_budget(self, code, imap_quant, max_bytes):
+    def encode_to_budget(self, code, imap_quant, max_bytes, protect=None):
         """Encode the latent in at most max_bytes bytes (both streams) by lowering its importance levels: candidate k codes the
         levels max(s - k, 0) with the mask the decoder derives from them (levels_to_mask), so the result always decodes.  The
         offset comes from select_budget_offset on batched exact-table estimates (two estimate_batch calls, 7 latents each at
-        most), where a candidate fits when the proven upper bound of its stream lengths (stream_bytes_bound) is at most max_bytes;
-        then one encode of the chosen candidate.
+        most without protect), where a candidate fits when the proven upper bound of its stream lengths (stream_bytes_bound) is
+        at most max_bytes; then one encode of the chosen candidate.
+
+        protect: None, or a (1,1,H/2,W/2) integer map P in [0, 48] on the codec's device (latitude_protection,
+        viewport_protection, or their torch.maximum): candidate k then lowers each cell by max(k - P, 0), so a region keeps its
+        levels while the others are lowered, and the offsets run up to 48 + max P, where every level is 0.  The streams are
+        ordinary streams; decode needs no map.
 
         Returns {'imp_bytes', 'code_bytes', 'offset', 'levels' (1,1,H/2,W/2), 'mask' (1,48,H,W), 'bound': bytes bound of the
         chosen offset, 'bounds': {offset: bound} of every offset evaluated}.  RuntimeError when no offset fits, and when the
         encoded streams exceed max_bytes (the bound would be broken: never returned silently)."""
         code, _, imp = self._latents(1, code, None, imap_quant)
         max_bytes = int(max_bytes)
+        if protect is not None:
+            protect = _protect_map(protect, imp)
+        max_offset = 48 if protect is None else 48 + int(protect.max())
         cands = {}
 
         def estimate(offsets):
-            levels, masks = levels_to_mask(imp, offsets)
+            levels, masks = levels_to_mask(imp, offsets, protect)
             for j, k in enumerate(offsets):
                 cands[k] = (levels[j:j + 1], masks[j:j + 1])
             return self.estimate_batch(code.expand(len(offsets), -1, -1, -1), masks, levels, maps=False)
 
-        offset, bounds = select_budget_offset(estimate, max_bytes)
+        offset, bounds = select_budget_offset(estimate, max_bytes, max_offset)
         levels, mask = cands[offset]
         imp_bytes, code_bytes = self.encode(code, mask, levels)
         if len(imp_bytes) + len(code_bytes) > max_bytes:

@@ -270,9 +270,18 @@ long lic360_codec_batch_stream_copy(lic360_codec* c, int k, int stream_id, uint8
  *   levels_out_dev[j] (K,1,h,w) = max(s - offsets_host[j], 0)
  *   mask_out_dev[j]  (K,48,2h,2w) = the decoder's mask of that level, Imp2mask + Dtow in one pass: channel c at (y, x) is 1 iff
  *                                   4c + 2 (y % 2) + x % 2 < 4 * level(y/2, x/2)
- * Encoding a pair (levels_out[j], mask_out[j]) gives streams that decode to exactly that mask.  Enqueued on `stream`. */
+ * Encoding a pair (levels_out[j], mask_out[j]) gives streams that decode to exactly that mask.  Enqueued on `stream`.
+ * The case protect_dev = NULL of lic360_imp_levels_to_mask_protected. */
 int lic360_imp_levels_to_mask(const float* levels_dev, int h, int w, const int* offsets_host, int K, float* levels_out_dev,
                               float* mask_out_dev, void* stream);
+/* lic360_imp_levels_to_mask with a protection map: protect_dev (h,w) int32 per importance cell, or NULL.  Candidate t = offsets_host[j]
+ * lowers a cell with protection P = min(max(protect_dev[cell], 0), 48) by max(t - P, 0):
+ *   levels_out_dev[j] = max(s - max(t - P, 0), 0),  mask_out_dev[j] = the decoder's mask of that level, as above
+ * all in integer arithmetic; the outputs are integers stored as float.  A cell keeps its level until t > P, so the masks are nested
+ * in t and every level is 0 at t = 48 + max P.  NULL (or a map of zeros) gives the levels max(s - t, 0) of lic360_imp_levels_to_mask,
+ * bit for bit.  Same argument checks and messages as lic360_imp_levels_to_mask. */
+int lic360_imp_levels_to_mask_protected(const float* levels_dev, int h, int w, const int* offsets_host, int K, const int32_t* protect_dev,
+                                        float* levels_out_dev, float* mask_out_dev, void* stream);
 long lic360_codec_stream_size(lic360_codec* c, int stream_id);
 long lic360_codec_stream_copy(lic360_codec* c, int stream_id, uint8_t* out, long cap);
 /* -> code_out_dev (1,48,H,W) = symbols where mask == 1, else 0 (lic360_demo.py:236-237); mask_out_dev (1,48,H,W) */
