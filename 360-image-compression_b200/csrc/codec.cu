@@ -254,6 +254,8 @@ struct lic360_codec {
     void* est_dev = nullptr;            // estimate: totals, error keys and counts of both streams (EstimateTotals layout)
     void* est_host = nullptr;           // pinned copy of est_dev
     cudaEvent_t ev_est = nullptr;                // estimate: the importance stream's results are in est_dev
+    int2* cand_dev = nullptr;           // estimate_candidates: the (source latent, offset) table, batch_cap entries
+    float* cand_levels_dev = nullptr;   // estimate_candidates: the candidates' levels (batch_cap,1,H/2,W/2), the importance net's input
     int rows_cap = 1;                   // latents the encoder's row buffers (rows_dev / rows_host of both streams) hold (grown on demand)
     int enc_k = 0;                      // latents of the last successful encode / encode_batch (0 after a failure or a decode)
     std::vector<lic360::EncodedStream> enc_out = std::vector<lic360::EncodedStream>(2);  // [2k + stream_id]: the streams of the last encode (empty after a failed one)
@@ -350,6 +352,52 @@ __global__ void prep_code_kernel(const float* __restrict__ code, const float* __
         const float v = (code[i] - bias) * mask[i];
         x[i] = v; x[i + n] = v; x[i + 2 * n] = v;
     }
+}
+
+// level of one cell in candidate t: max(s - max(t - P, 0), 0), s = imp_symbol(level) the symbol encode codes, P = protect[cell] clamped
+// to [0, 48] (0 without a protection map, where this is max(s - t, 0))
+__device__ __forceinline__ int candidate_level(const float* __restrict__ levels, const int32_t* __restrict__ protect, int cell, int t) {
+    const int drop = protect ? max(t - min(max(protect[cell], 0), 48), 0) : t;
+    return max((int)imp_symbol(levels[cell]) - drop, 0);
+}
+
+// Candidates of lic360_codec_estimate_candidates: candidate j (the batch's latent j) is source latent tab[j].x lowered by offset
+// tab[j].y (candidate_level), with the levels, code and protection map of that source; the mask bit of a code symbol is
+// code_mask_from_level of its cell's candidate level, the bit lic360_imp_levels_to_mask_protected stores.
+struct Candidates {
+    const int2* tab;
+    const float* levels;     // (S,1,h,w) source levels
+    const int32_t* protect;  // (S,1,h,w) or NULL
+};
+
+// the mask bit of code symbol (tc, th, tw) of an H x W latent in the candidate of source src and offset t
+__device__ __forceinline__ int candidate_mask_bit(const Candidates& cd, int src, int t, int tc, int th, int tw, int H, int W) {
+    const size_t cells = (size_t)src * (H >> 1) * (W >> 1);
+    const int lvl = candidate_level(cd.levels + cells, cd.protect ? cd.protect + cells : nullptr, (th >> 1) * (W >> 1) + (tw >> 1), t);
+    return code_mask_from_level(lvl, tc, th, tw);
+}
+
+// prep_code_kernel of J candidates: x = (code - 3.5) * mask with the source's code and the candidate's mask bit as a float, the
+// arithmetic prep_code_kernel does on a materialised candidate.  n = J x (48, H, W), same set-major layout.
+__global__ void prep_candidate_code_kernel(const float* __restrict__ code, Candidates cd, float* __restrict__ x, int n, int G, int H,
+                                           int W, float bias) {
+    const int plane = G * H * W;
+    for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x) {
+        const int j = i / plane, p = i - j * plane;
+        const int2 e = cd.tab[j];
+        const int tw = p % W, th = (p / W) % H, tc = p / (W * H);
+        const float v = (code[(size_t)e.x * plane + p] - bias) * (float)candidate_mask_bit(cd, e.x, e.y, tc, th, tw, H, W);
+        x[i] = v; x[i + n] = v; x[i + 2 * n] = v;
+    }
+}
+
+// the candidate levels (J,1,h,w) as float, candidate j in blockIdx.y: the importance network's input and the levels its bits kernel reads
+__global__ void candidate_levels_kernel(Candidates cd, int hw, float* __restrict__ out) {
+    const int2 e = cd.tab[blockIdx.y];
+    const size_t cells = (size_t)e.x * hw;
+    out += (size_t)blockIdx.y * hw;
+    for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < hw; i += gridDim.x * blockDim.x)
+        out[i] = (float)candidate_level(cd.levels + cells, cd.protect ? cd.protect + cells : nullptr, i, e.y);
 }
 
 // The encoder's kernels run a batch of latents: latent blockIdx.y of gridDim.y.  The helpers below give each stream's batch layout, network
@@ -476,14 +524,24 @@ __device__ __forceinline__ bool symbol_bits(const float* o, int s, double* bits)
 // A batch: latent blockIdx.y of gridDim.y, each with the block partition, the partials and the error key of a single latent, so its
 // totals and map do not depend on the other latents.
 // code stream: thread i = symbol (tc = i / HW, k = i % HW in plan order), bits (optional) in (G, H, W) layout per latent; count: coded
-// symbols (mask >= 0.5) per block
+// symbols (mask >= 0.5) per block.  CAND: latent blockIdx.y is candidate blockIdx.y of `cd`, its code read from its source latent and
+// its mask bit derived from the candidate level (candidate_mask_bit); `mask` is not read.
+template <bool CAND>
 __global__ void __launch_bounds__(BITS_THREADS) gmm_bits_kernel(const float* __restrict__ y, const float* __restrict__ code,
-                                const float* __restrict__ mask, const int32_t* __restrict__ idx, const StepDesc* __restrict__ steps,
-                                const int* __restrict__ row_off, float* __restrict__ bits, double* __restrict__ partial,
-                                int* __restrict__ count, unsigned long long* err, int G, int H, int W, float s2) {
+                                const float* __restrict__ mask, Candidates cd, const int32_t* __restrict__ idx,
+                                const StepDesc* __restrict__ steps, const int* __restrict__ row_off, float* __restrict__ bits,
+                                double* __restrict__ partial, int* __restrict__ count, unsigned long long* err, int G, int H, int W,
+                                float s2) {
     const int HW = H * W;
     const size_t lat = gmm_latent(y, G, HW);
-    code += lat; mask += lat; err += blockIdx.y;
+    int2 cand = make_int2(0, 0);
+    if constexpr (CAND) {
+        cand = cd.tab[blockIdx.y];
+        code += (size_t)cand.x * G * HW;
+    } else {
+        code += lat; mask += lat;
+    }
+    err += blockIdx.y;
     if (bits) bits += lat;
     partial += (size_t)blockIdx.y * gridDim.x; count += (size_t)blockIdx.y * gridDim.x;
     const int i = blockIdx.x * blockDim.x + threadIdx.x;
@@ -493,7 +551,8 @@ __global__ void __launch_bounds__(BITS_THREADS) gmm_bits_kernel(const float* __r
         const int k = i % HW, tc = i / HW;
         const int th = __ldg(idx + k), tw = __ldg(idx + k + HW);
         const size_t pos = ((size_t)tc * H + th) * W + tw;
-        coded = code_mask_bit(mask[pos]);
+        if constexpr (CAND) coded = candidate_mask_bit(cd, cand.x, cand.y, tc, th, tw, H, W);
+        else coded = code_mask_bit(mask[pos]);
         if (coded) {  // a position the encoder skips costs nothing, whatever its symbol
             float o[9];
             gmm_symbol_row(y, G, H, W, tc, th, tw, s2, o);
@@ -555,19 +614,14 @@ __global__ void __launch_bounds__(BITS_THREADS) bits_sum_kernel(const double* __
     if (threadIdx.x == 0) { total[blockIdx.x] = v; total_count[blockIdx.x] = (long long)coded; }
 }
 
-// level of one cell in candidate t: max(s - max(t - P, 0), 0), s = imp_symbol(level) the symbol encode codes, P = protect[cell] clamped
-// to [0, 48] (0 without a protection map, where this is max(s - t, 0))
-__device__ __forceinline__ int candidate_level(const float* __restrict__ levels, const int32_t* __restrict__ protect, int cell, int t) {
-    const int drop = protect ? max(t - min(max(protect[cell], 0), 48), 0) : t;
-    return max((int)imp_symbol(levels[cell]) - drop, 0);
-}
-
-// candidate j (blockIdx.y) of lic360_imp_levels_to_mask_protected: the candidate level of every cell (candidate_level) and the
-// (48, 2h, 2w) code mask the decoder derives from it (Imp2mask + Dtow)
-struct LevelOffsets { int k[32]; };
+// candidate j (blockIdx.y) of lic360_imp_levels_to_mask_batch: the candidate level of every cell of source latent off.src[j] at offset
+// off.k[j] (candidate_level) and the (48, 2h, 2w) code mask the decoder derives from it (Imp2mask + Dtow)
+struct LevelOffsets { int k[32]; int src[32]; };
 __global__ void imp_levels_to_mask_kernel(const float* __restrict__ levels, const int32_t* __restrict__ protect, int h, int w,
                                           LevelOffsets off, float* __restrict__ levels_out, float* __restrict__ mask_out) {
     const int j = blockIdx.y, k = off.k[j], hw = h * w, W = 2 * w, n = 48 * 4 * hw;
+    levels += (size_t)off.src[j] * hw;
+    if (protect) protect += (size_t)off.src[j] * hw;
     levels_out += (size_t)j * hw;
     mask_out += (size_t)j * n;
     for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x) {
@@ -959,7 +1013,7 @@ static int grow_buffers(lic360_codec* c, const std::vector<GrowBuf>& bufs, int K
 }
 
 // The buffers that scale with the number of latents an encode or an estimate runs at once: both networks' encoder frames, the bits
-// kernels' partials and the estimate's results.  They only grow.
+// kernels' partials, the estimate's results and the candidate table and levels of estimate_candidates.  They only grow.
 static int batch_reserve(lic360_codec* c, int K) {
     if (K <= c->batch_cap) return LIC360_OK;
     std::vector<GrowBuf> bufs;
@@ -968,6 +1022,8 @@ static int batch_reserve(lic360_codec* c, int K) {
         bufs.push_back({reinterpret_cast<void**>(&n->bits_partial_dev), (size_t)n->bits_blocks * K * sizeof(double), false});
         bufs.push_back({reinterpret_cast<void**>(&n->count_partial_dev), (size_t)n->bits_blocks * K * sizeof(int), false});
     }
+    bufs.push_back({reinterpret_cast<void**>(&c->cand_dev), (size_t)K * sizeof(int2), false});
+    bufs.push_back({reinterpret_cast<void**>(&c->cand_levels_dev), (size_t)K * c->imp.H * c->imp.W * sizeof(float), false});
     bufs.push_back({&c->est_dev, estimate_bytes(K), false});
     bufs.push_back({&c->est_host, estimate_bytes(K), true});
     const int rc = grow_buffers(c, bufs, K);
@@ -1044,6 +1100,7 @@ void lic360_codec_destroy(lic360_codec* c) {
     ctx_free(c->code); ctx_free(c->imp);
     cudaFree(c->levels_dev); cudaFree(c->mask192_dev);
     cudaFree(c->est_dev); cudaFreeHost(c->est_host);
+    cudaFree(c->cand_dev); cudaFree(c->cand_levels_dev);
     if (c->ev_est) cudaEventDestroy(c->ev_est);
     delete c;
 }
@@ -1081,11 +1138,17 @@ int lic360_codec_set_layer(lic360_codec* c, int stream_id, int layer, const floa
 // alike, whatever else is in the batch).
 //   importance stream (lic360_demo.py:173-189): Scale(-1, 2/47) of the levels
 //   code stream (lic360_demo.py:124-131): (code - 3.5) * mask, once for each of the three nets
-static int run_encoder_net(lic360_codec* c, bool is_code, int K, const float* code_dev, const float* mask_dev, const float* imp_dev) {
+// cand: the K latents are candidates (lic360_codec_estimate_candidates): code_dev holds their sources and the masks are derived, imp_dev
+// holds the candidate levels
+static int run_encoder_net(lic360_codec* c, bool is_code, int K, const float* code_dev, const float* mask_dev, const float* imp_dev,
+                           const Candidates* cand = nullptr) {
     NetDesc& n = is_code ? c->code : c->imp;
     if (is_code) {
         const int nel = K * n.G * n.H * n.W;
-        prep_code_kernel<<<stream_grid(nel, 256), 256, 0, n.stream>>>(code_dev, mask_dev, n.frame[0], nel, 3.5f);
+        if (cand)
+            prep_candidate_code_kernel<<<stream_grid(nel, 256), 256, 0, n.stream>>>(code_dev, *cand, n.frame[0], nel, n.G, n.H, n.W, 3.5f);
+        else
+            prep_code_kernel<<<stream_grid(nel, 256), 256, 0, n.stream>>>(code_dev, mask_dev, n.frame[0], nel, 3.5f);
         LAUNCH_CHECK();
     } else {
         const int rc = lic360_scale(imp_dev, n.frame[0], (size_t)K * n.H * n.W, -1.0f, kImpScale, n.stream);
@@ -1144,11 +1207,12 @@ static void code_stream_job(lic360_coder* coder, const uint16_t* rows, int nrows
     out->bytes.assign(b, b + nb);
 }
 
-// appends " (latent k)" to the message of the calling thread's last error
-static void add_latent_suffix(int k) {
+// appends " (<what> k)" to the message of the calling thread's last error
+static void add_index_suffix(const char* what, int k) {
     const std::string msg = lic360_last_error();
-    set_error("%s (latent %d)", msg.c_str(), k);
+    set_error("%s (%s %d)", msg.c_str(), what, k);
 }
+static void add_latent_suffix(int k) { add_index_suffix("latent", k); }
 
 // The host coding of an encode of K latents, every stream into enc_out: the K importance streams as soon as their rows are on the host
 // (the code network may still be running), then the K code streams.  K = 1 codes on the calling thread with the codec's two coders,
@@ -1255,10 +1319,25 @@ int lic360_codec_encode_batch(lic360_codec* c, int K, const float* code_dev, con
     return encode_latents(c, K, code_dev, mask_dev, imp_dev, true);
 }
 
-// the GPU work of an estimate of K latents on the codec's two streams; the code stream ends with the copy of both streams' results
+// the GPU work of an estimate of K latents on the codec's two streams; the code stream ends with the copy of both streams' results.
+// cand (K candidates, lic360_codec_estimate_candidates): its table is uploaded to c->cand_dev first, code_dev holds the sources, and
+// the importance stream's input is the candidate levels, written to c->cand_levels_dev (imp_dev and mask_dev are not read).
 static int enqueue_estimate(lic360_codec* c, int K, const float* code_dev, const float* mask_dev, const float* imp_dev,
-                            float* code_bits_dev, float* imp_bits_dev) {
+                            float* code_bits_dev, float* imp_bits_dev, const int2* cand_host = nullptr, const float* src_levels = nullptr,
+                            const int32_t* protect = nullptr) {
     const EstimateTotals r = estimate_totals(c->est_dev, K);
+    const Candidates cd{c->cand_dev, src_levels, protect};
+    if (cand_host) {
+        // both streams read the table: ev_est marks it and the levels on the device, and is recorded again below for the results
+        cudaStream_t s = c->imp.stream;
+        const int hw = c->imp.H * c->imp.W;
+        LIC360_CUDA(cudaMemcpyAsync(c->cand_dev, cand_host, (size_t)K * sizeof(int2), cudaMemcpyHostToDevice, s));
+        candidate_levels_kernel<<<dim3((hw + 255) / 256, K), 256, 0, s>>>(cd, hw, c->cand_levels_dev);
+        LAUNCH_CHECK();
+        LIC360_CUDA(cudaEventRecord(c->ev_est, s));
+        LIC360_CUDA(cudaStreamWaitEvent(c->code.stream, c->ev_est, 0));
+        imp_dev = c->cand_levels_dev;
+    }
     {
         NetDesc& n = c->imp;
         cudaStream_t s = n.stream;
@@ -1276,11 +1355,16 @@ static int enqueue_estimate(lic360_codec* c, int K, const float* code_dev, const
         NetDesc& n = c->code;
         cudaStream_t s = n.stream;
         LIC360_CUDA(cudaMemsetAsync(r.err, 0xFF, K * sizeof(*r.err), s));
-        int rc = run_encoder_net(c, true, K, code_dev, mask_dev, imp_dev);
+        int rc = run_encoder_net(c, true, K, code_dev, mask_dev, imp_dev, cand_host ? &cd : nullptr);
         if (rc) return rc;
-        gmm_bits_kernel<<<dim3(n.bits_blocks, K), BITS_THREADS, 0, s>>>(n.frame[12], code_dev, mask_dev, n.idx_dev, n.steps_dev,
-                                                                        n.row_off_dev, code_bits_dev, n.bits_partial_dev,
-                                                                        n.count_partial_dev, r.err, n.G, n.H, n.W, kGmmS2);
+        if (cand_host)
+            gmm_bits_kernel<true><<<dim3(n.bits_blocks, K), BITS_THREADS, 0, s>>>(n.frame[12], code_dev, nullptr, cd, n.idx_dev, n.steps_dev,
+                                                                                  n.row_off_dev, code_bits_dev, n.bits_partial_dev,
+                                                                                  n.count_partial_dev, r.err, n.G, n.H, n.W, kGmmS2);
+        else
+            gmm_bits_kernel<false><<<dim3(n.bits_blocks, K), BITS_THREADS, 0, s>>>(n.frame[12], code_dev, mask_dev, cd, n.idx_dev, n.steps_dev,
+                                                                                   n.row_off_dev, code_bits_dev, n.bits_partial_dev,
+                                                                                   n.count_partial_dev, r.err, n.G, n.H, n.W, kGmmS2);
         LAUNCH_CHECK();
         bits_sum_kernel<<<K, BITS_THREADS, 0, s>>>(n.bits_partial_dev, n.count_partial_dev, n.bits_blocks, r.bits, r.count);
         LAUNCH_CHECK();
@@ -1290,14 +1374,16 @@ static int enqueue_estimate(lic360_codec* c, int K, const float* code_dev, const
     return LIC360_OK;
 }
 
-// lic360_codec_estimate (K = 1, latent_suffix false) and lic360_codec_estimate_batch; the maps may be NULL
+// lic360_codec_estimate (K = 1, no suffix), lic360_codec_estimate_batch (suffix "latent") and lic360_codec_estimate_candidates (suffix
+// "candidate", the table in cand_host); the maps may be NULL
 static int estimate_latents(lic360_codec* c, int K, const float* code_dev, const float* mask_dev, const float* imp_dev,
-                            float* code_bits_dev, float* imp_bits_dev, double* bits_host, long long* counts_host, bool latent_suffix) {
+                            float* code_bits_dev, float* imp_bits_dev, double* bits_host, long long* counts_host, const char* suffix,
+                            const int2* cand_host = nullptr, const int32_t* protect = nullptr) {
     DeviceGuard guard(c->device);
     int rc = begin_latents(c, guard, K);
     if (rc) return rc;
     const auto t0 = clk::now();
-    rc = enqueue_estimate(c, K, code_dev, mask_dev, imp_dev, code_bits_dev, imp_bits_dev);
+    rc = enqueue_estimate(c, K, code_dev, mask_dev, imp_dev, code_bits_dev, imp_bits_dev, cand_host, imp_dev, protect);
     // both streams are drained on every path: the caller may reuse the inputs and the maps as soon as the call returns
     const auto tw = clk::now();
     const cudaError_t e_imp = cudaStreamSynchronize(c->imp.stream);
@@ -1314,7 +1400,7 @@ static int estimate_latents(lic360_codec* c, int K, const float* code_dev, const
             const unsigned long long e = r.err[sid * K + k];
             if (e == kNoError) continue;
             coder_row_error(sid, (int)(e >> 32), (unsigned)e);
-            if (latent_suffix) add_latent_suffix(k);
+            if (suffix) add_index_suffix(suffix, k);
             return LIC360_ERR_CODER;
         }
     for (int k = 0; k < K; k++)
@@ -1328,7 +1414,7 @@ static int estimate_latents(lic360_codec* c, int K, const float* code_dev, const
 int lic360_codec_estimate(lic360_codec* c, const float* code_dev, const float* mask_dev, const float* imp_dev, float* code_bits_dev,
                           float* imp_bits_dev, double* bits_host) {
     LIC360_CHECK_ARG(c && code_dev && mask_dev && imp_dev && code_bits_dev && imp_bits_dev && bits_host, "bad arguments");
-    return estimate_latents(c, 1, code_dev, mask_dev, imp_dev, code_bits_dev, imp_bits_dev, bits_host, nullptr, false);
+    return estimate_latents(c, 1, code_dev, mask_dev, imp_dev, code_bits_dev, imp_bits_dev, bits_host, nullptr, nullptr);
 }
 
 int lic360_codec_estimate_batch(lic360_codec* c, int K, const float* code_dev, const float* mask_dev, const float* imp_dev,
@@ -1336,12 +1422,45 @@ int lic360_codec_estimate_batch(lic360_codec* c, int K, const float* code_dev, c
     LIC360_CHECK_ARG(K >= 1, "K must be at least 1");
     LIC360_CHECK_ARG(c && code_dev && mask_dev && imp_dev && bits_host && counts_host, "bad arguments");
     LIC360_CHECK_BATCH(c, K);
-    return estimate_latents(c, K, code_dev, mask_dev, imp_dev, code_bits_dev, imp_bits_dev, bits_host, counts_host, true);
+    return estimate_latents(c, K, code_dev, mask_dev, imp_dev, code_bits_dev, imp_bits_dev, bits_host, counts_host, "latent");
+}
+
+int lic360_codec_estimate_candidates(lic360_codec* c, int K, const float* code_dev, const float* imp_dev, const int32_t* protect_dev, int J,
+                                     const int* cand_latent_host, const int* cand_offset_host, double* bits_host, long long* counts_host) {
+    LIC360_CHECK_ARG(K >= 1, "K must be at least 1");
+    LIC360_CHECK_ARG(J >= 1, "J must be at least 1");
+    LIC360_CHECK_ARG(c && code_dev && imp_dev && cand_latent_host && cand_offset_host && bits_host && counts_host, "bad arguments");
+    LIC360_CHECK_BATCH(c, J);
+    std::vector<int2> tab(J);
+    for (int j = 0; j < J; j++) {
+        LIC360_CHECK_ARG(cand_latent_host[j] >= 0 && cand_latent_host[j] < K, "cand_latent must lie in [0, K)");
+        LIC360_CHECK_ARG(cand_offset_host[j] >= 0, "offsets must not be negative");
+        tab[j] = make_int2(cand_latent_host[j], cand_offset_host[j]);
+    }
+    return estimate_latents(c, J, code_dev, nullptr, imp_dev, nullptr, nullptr, bits_host, counts_host, "candidate", tab.data(), protect_dev);
 }
 
 int lic360_imp_levels_to_mask(const float* levels_dev, int h, int w, const int* offsets_host, int K, float* levels_out_dev,
                               float* mask_out_dev, void* stream) {
     return lic360_imp_levels_to_mask_protected(levels_dev, h, w, offsets_host, K, nullptr, levels_out_dev, mask_out_dev, stream);
+}
+
+// the launches of the candidate maps: candidate j is source latent src_host[j] (0 when src_host is NULL) at offset offsets_host[j]
+static int enqueue_levels_to_mask(const float* levels_dev, int h, int w, const int32_t* protect_dev, int J, const int* src_host,
+                                  const int* offsets_host, float* levels_out_dev, float* mask_out_dev, void* stream) {
+    const int n = 48 * 4 * h * w;
+    for (int j0 = 0; j0 < J; j0 += 32) {  // 32 candidates per launch (the table travels as a kernel parameter)
+        LevelOffsets off;
+        const int nj = std::min(32, J - j0);
+        for (int j = 0; j < nj; j++) {
+            off.k[j] = offsets_host[j0 + j];
+            off.src[j] = src_host ? src_host[j0 + j] : 0;
+        }
+        imp_levels_to_mask_kernel<<<dim3(std::max(1, stream_grid(n, 256) / nj), nj), 256, 0, as_stream(stream)>>>(
+            levels_dev, protect_dev, h, w, off, levels_out_dev + (size_t)j0 * h * w, mask_out_dev + (size_t)j0 * n);
+        LAUNCH_CHECK();
+    }
+    return LIC360_OK;
 }
 
 int lic360_imp_levels_to_mask_protected(const float* levels_dev, int h, int w, const int* offsets_host, int K, const int32_t* protect_dev,
@@ -1350,16 +1469,22 @@ int lic360_imp_levels_to_mask_protected(const float* levels_dev, int h, int w, c
     LIC360_CHECK_ARG(levels_dev && offsets_host && levels_out_dev && mask_out_dev, "bad arguments");
     LIC360_CHECK_ARG(h > 0 && w > 0 && (long long)48 * 4 * h * w <= 0x7fffffffLL, "bad importance map size");
     for (int j = 0; j < K; j++) LIC360_CHECK_ARG(offsets_host[j] >= 0, "offsets must not be negative");
-    const int n = 48 * 4 * h * w;
-    for (int j0 = 0; j0 < K; j0 += 32) {  // 32 candidates per launch (the offsets travel as a kernel parameter)
-        LevelOffsets off;
-        const int nj = std::min(32, K - j0);
-        for (int j = 0; j < nj; j++) off.k[j] = offsets_host[j0 + j];
-        imp_levels_to_mask_kernel<<<dim3(std::max(1, stream_grid(n, 256) / nj), nj), 256, 0, as_stream(stream)>>>(
-            levels_dev, protect_dev, h, w, off, levels_out_dev + (size_t)j0 * h * w, mask_out_dev + (size_t)j0 * n);
-        LAUNCH_CHECK();
+    return enqueue_levels_to_mask(levels_dev, h, w, protect_dev, K, nullptr, offsets_host, levels_out_dev, mask_out_dev, stream);
+}
+
+int lic360_imp_levels_to_mask_batch(const float* levels_dev, int K, int h, int w, const int32_t* protect_dev, int J,
+                                    const int* cand_latent_host, const int* cand_offset_host, float* levels_out_dev, float* mask_out_dev,
+                                    void* stream) {
+    LIC360_CHECK_ARG(K >= 1, "K must be at least 1");
+    LIC360_CHECK_ARG(J >= 1, "J must be at least 1");
+    LIC360_CHECK_ARG(levels_dev && cand_latent_host && cand_offset_host && levels_out_dev && mask_out_dev, "bad arguments");
+    LIC360_CHECK_ARG(h > 0 && w > 0 && (long long)48 * 4 * h * w <= 0x7fffffffLL, "bad importance map size");
+    for (int j = 0; j < J; j++) {
+        LIC360_CHECK_ARG(cand_latent_host[j] >= 0 && cand_latent_host[j] < K, "cand_latent must lie in [0, K)");
+        LIC360_CHECK_ARG(cand_offset_host[j] >= 0, "offsets must not be negative");
     }
-    return LIC360_OK;
+    return enqueue_levels_to_mask(levels_dev, h, w, protect_dev, J, cand_latent_host, cand_offset_host, levels_out_dev, mask_out_dev,
+                                  stream);
 }
 
 // stream stream_id of latent k of the last encode (none before the first encode and after a failed one)

@@ -30,12 +30,12 @@ def make_codec_params(device, seed=2024):
 
 
 def _protect_map(protect, imap_quant):
-    """protect as lic360_imp_levels_to_mask_protected reads it: a (1,1,h,w) integer tensor on imap_quant's device with values in
-    [0, 48], converted to contiguous int32"""
+    """protect as lic360_imp_levels_to_mask_protected reads it: a (K,1,h,w) integer tensor on imap_quant's device with values in
+    [0, 48], converted to contiguous int32 (K = 1 for one latent)"""
     if not (isinstance(protect, torch.Tensor) and protect.device == imap_quant.device and not protect.dtype.is_floating_point
             and not protect.dtype.is_complex and protect.dtype != torch.bool and tuple(protect.shape) == tuple(imap_quant.shape)):
-        raise RuntimeError("levels_to_mask: protect must be a (1,1,h,w) integer tensor on %s, like the importance map"
-                           % imap_quant.device)
+        raise RuntimeError("levels_to_mask: protect must be a (%d,1,h,w) integer tensor on %s, like the importance map"
+                           % (imap_quant.shape[0], imap_quant.device))
     p = protect.to(torch.int32).contiguous()
     lo, hi = int(p.min()), int(p.max())
     if lo < 0 or hi > 48:
@@ -69,6 +69,30 @@ def levels_to_mask(imap_quant, offsets, protect=None):
             p = _protect_map(protect, imap_quant)
             check(LIB.lic360_imp_levels_to_mask_protected(lv.data_ptr(), h, w, offs_c, K, p.data_ptr(), levels.data_ptr(),
                                                           masks.data_ptr(), cstream(lv)))
+    return levels, masks
+
+
+def levels_to_mask_batch(imap_quant, cand_latent, cand_offset, protect=None):
+    """levels_to_mask of J candidates of K importance maps (lic360_imp_levels_to_mask_batch): imap_quant (K,1,h,w) float32 CUDA;
+    candidate j is map cand_latent[j] in [0, K) at offset cand_offset[j] >= 0; protect: None or a (K,1,h,w) integer map per latent,
+    checked as levels_to_mask checks it.  Returns (levels (J,1,h,w), masks (J,48,2h,2w)); entry j is bit-identical to
+    levels_to_mask(imap_quant[k:k+1], [t], protect[k:k+1]) of its latent k and offset t."""
+    if not (isinstance(imap_quant, torch.Tensor) and imap_quant.is_cuda and imap_quant.dtype == torch.float32
+            and imap_quant.dim() == 4 and imap_quant.shape[1] == 1):
+        raise RuntimeError("levels_to_mask_batch: expected a (K,1,h,w) float32 CUDA tensor")
+    lat, offs = [int(k) for k in cand_latent], [int(t) for t in cand_offset]
+    if len(lat) != len(offs):
+        raise RuntimeError("levels_to_mask_batch: %d latents for %d offsets" % (len(lat), len(offs)))
+    (K, _, h, w), J = imap_quant.shape, len(lat)
+    dev = imap_quant.device
+    levels = torch.empty((J, 1, h, w), dtype=torch.float32, device=dev)
+    masks = torch.empty((J, 48, 2 * h, 2 * w), dtype=torch.float32, device=dev)
+    with torch.cuda.device(dev):
+        lv = imap_quant.contiguous()
+        p = None if protect is None else _protect_map(protect, imap_quant)
+        check(LIB.lic360_imp_levels_to_mask_batch(lv.data_ptr(), K, h, w, None if p is None else p.data_ptr(), J,
+                                                  (ctypes.c_int * max(J, 1))(*lat), (ctypes.c_int * max(J, 1))(*offs),
+                                                  levels.data_ptr(), masks.data_ptr(), cstream(lv)))
     return levels, masks
 
 
@@ -143,30 +167,98 @@ def budget_bound(est):
     return stream_bytes_bound(est['imp_bits'], est['imp_symbols']) + stream_bytes_bound(est['code_bits'], est['code_symbols'])
 
 
-def select_budget_offset(estimate, max_bytes, max_offset=48):
-    """The level offset encode_to_budget codes: `estimate(offsets)` returns one estimate dict per offset; an offset fits when its
-    budget_bound is at most max_bytes.  Stage 1 evaluates offsets 0, 8, 16, ... up to max_offset, and max_offset itself when it
-    is not on that grid; if the smallest that fits, k1, is not 0, stage 2 evaluates the offsets strictly between the stage-1
-    offset before k1 and k1 (the seven offsets k1 - 7 .. k1 - 1 on the grid).  The answer is the smallest evaluated offset that
-    fits; the rate is not assumed to fall monotonically with the offset.  Returns (offset, {offset: bound in bytes} of every
-    offset evaluated); RuntimeError if no offset of stage 1 fits."""
-    bounds = {}
+def _stage1_offsets(max_offset):
+    """stage 1 of select_budget_offset: 0, 8, 16, ... up to max_offset, and max_offset itself when it is not on that grid"""
+    return list(range(0, max_offset + 1, 8)) + ([max_offset] if max_offset % 8 else [])
 
-    def run(offsets):
-        offsets = list(offsets)
-        for k, est in zip(offsets, estimate(offsets)):
-            bounds[k] = budget_bound(est)
 
-    stage1 = list(range(0, max_offset + 1, 8)) + ([max_offset] if max_offset % 8 else [])
-    run(stage1)
+def _stage2_offsets(stage1, bounds, max_bytes, max_offset):
+    """stage 2 of select_budget_offset from the stage-1 bounds: the offsets strictly between the stage-1 offset before the first
+    that fits, k1, and k1 (none when k1 is 0); RuntimeError if no stage-1 offset fits"""
     fit = [j for j, k in enumerate(stage1) if bounds[k] <= max_bytes]
     if not fit:
         raise RuntimeError("encode_to_budget: no level offset up to %d fits %d bytes (bound at offset %d: %d bytes)"
                            % (max_offset, max_bytes, max_offset, bounds[max_offset]))
     j = fit[0]
-    if j > 0 and stage1[j] - stage1[j - 1] > 1:
-        run(range(stage1[j - 1] + 1, stage1[j]))
-    return min(k for k, b in bounds.items() if b <= max_bytes), bounds
+    return list(range(stage1[j - 1] + 1, stage1[j])) if j > 0 and stage1[j] - stage1[j - 1] > 1 else []
+
+
+def _smallest_fit(bounds, max_bytes):
+    return min(k for k, b in bounds.items() if b <= max_bytes)
+
+
+def select_budget_offset(estimate, max_bytes, max_offset=48, bound=budget_bound):
+    """The level offset encode_to_budget codes: `estimate(offsets)` returns one estimate per offset; an offset fits when its bound
+    (`bound(estimate)`, budget_bound by default) is at most max_bytes.  Stage 1 evaluates offsets 0, 8, 16, ... up to max_offset, and
+    max_offset itself when it is not on that grid; if the smallest that fits, k1, is not 0, stage 2 evaluates the offsets strictly
+    between the stage-1 offset before k1 and k1 (the seven offsets k1 - 7 .. k1 - 1 on the grid).  The answer is the smallest
+    evaluated offset that fits; the rate is not assumed to fall monotonically with the offset.  Returns (offset, {offset: bound in
+    bytes} of every offset evaluated); RuntimeError if no offset of stage 1 fits."""
+    bounds = {}
+
+    def run(offsets):
+        for k, est in zip(offsets, estimate(offsets)):
+            bounds[k] = bound(est)
+
+    stage1 = _stage1_offsets(max_offset)
+    run(stage1)
+    stage2 = _stage2_offsets(stage1, bounds, max_bytes, max_offset)
+    if stage2:
+        run(stage2)
+    return _smallest_fit(bounds, max_bytes), bounds
+
+
+def _chunked(estimate, items, max_batch):
+    """estimate(items) in calls of at most max_batch items (None: one call), concatenated"""
+    step = len(items) if max_batch is None else int(max_batch)
+    out = []
+    for i in range(0, len(items), max(step, 1)):
+        out += estimate(items[i:i + step])
+    return out
+
+
+def select_budget_offsets(estimate, max_bytes, max_offsets, max_batch=None):
+    """select_budget_offset of K latents side by side, each with its own budget max_bytes[k] and max_offset max_offsets[k]:
+    `estimate(pairs)` returns one estimate per (latent, offset) pair and is called with at most max_batch pairs.  Stage 1 of every
+    latent runs first, then stage 2 of every latent that needs one; latent k evaluates exactly the offsets select_budget_offset
+    evaluates for it alone, so its result is the same.  Returns [(offset, bounds)] per latent; RuntimeError with
+    select_budget_offset's message followed by ' (latent k)' for the lowest latent where no stage-1 offset fits."""
+    K = len(max_offsets)
+    bounds = [{} for _ in range(K)]
+
+    def run(pairs):
+        for (k, t), est in zip(pairs, _chunked(estimate, pairs, max_batch)):
+            bounds[k][t] = budget_bound(est)
+
+    stage1 = [_stage1_offsets(m) for m in max_offsets]
+    run([(k, t) for k in range(K) for t in stage1[k]])
+    stage2 = []
+    for k in range(K):
+        try:
+            stage2 += [(k, t) for t in _stage2_offsets(stage1[k], bounds[k], max_bytes[k], max_offsets[k])]
+        except RuntimeError as e:
+            raise RuntimeError("%s (latent %d)" % (e, k)) from None
+    if stage2:
+        run(stage2)
+    return [(_smallest_fit(b, m), b) for b, m in zip(bounds, max_bytes)]
+
+
+def select_shared_offset(estimate, max_bytes, K, max_offset, max_batch=None):
+    """One offset for K latents together in max_bytes bytes: select_budget_offset whose bound of an offset t is the sum over the
+    latents of budget_bound(estimate of (k, t)), each stream's bound floored on its own.  `estimate(pairs)` as in
+    select_budget_offsets, at most max_batch pairs per call.  Returns (offset, {t: summed bound}, {t: [bound of latent k]});
+    RuntimeError (select_budget_offset's message) when no offset fits."""
+    per = {}
+
+    def estimate_offsets(offsets):
+        ests = _chunked(estimate, [(k, t) for t in offsets for k in range(K)], max_batch)
+        out = [ests[i * K:(i + 1) * K] for i in range(len(offsets))]
+        for t, e in zip(offsets, out):
+            per[t] = [budget_bound(x) for x in e]
+        return out
+
+    offset, bounds = select_budget_offset(estimate_offsets, max_bytes, max_offset, bound=lambda ests: sum(map(budget_bound, ests)))
+    return offset, bounds, per
 
 
 class PerOpCodec(object):
@@ -380,6 +472,96 @@ class FusedCodec(object):
                                % (offset, len(imp_bytes) + len(code_bytes), bounds[offset], max_bytes))
         return {'imp_bytes': imp_bytes, 'code_bytes': code_bytes, 'offset': offset, 'levels': levels, 'mask': mask,
                 'bound': bounds[offset], 'bounds': bounds}
+
+    def _candidates(self, code, imp, protect, pairs):
+        """lic360_codec_estimate_candidates on checked inputs: one estimate dict (estimate_batch's keys, no maps) per (latent, offset)"""
+        J = len(pairs)
+        lat = (ctypes.c_int * max(J, 1))(*[int(k) for k, _ in pairs])
+        off = (ctypes.c_int * max(J, 1))(*[int(t) for _, t in pairs])
+        totals = (ctypes.c_double * max(2 * J, 1))()
+        counts = (ctypes.c_longlong * max(2 * J, 1))()
+        check(LIB.lic360_codec_estimate_candidates(self._h, int(code.shape[0]), code.data_ptr(), imp.data_ptr(),
+                                                   None if protect is None else protect.data_ptr(), J, lat, off, totals, counts))
+        return [{'code_bits': totals[2 * j], 'imp_bits': totals[2 * j + 1], 'code_symbols': counts[2 * j],
+                 'imp_symbols': counts[2 * j + 1], 'code_map': None, 'imp_map': None} for j in range(J)]
+
+    def _budget_inputs(self, code, imap_quant, protect):
+        K = int(code.shape[0]) if code.dim() == 4 else -1
+        code, _, imp = self._latents(K, code, None, imap_quant)
+        if protect is not None:
+            protect = _protect_map(protect, imp)
+        return K, code, imp, protect
+
+    def estimate_candidates(self, code, imap_quant, cand_latent, cand_offset, protect=None):
+        """estimate_batch(maps=False) of J rate-control candidates given as (latent, offset) pairs, without materialising them
+        (lic360_codec_estimate_candidates): code (K,48,H,W), imap_quant (K,1,H/2,W/2) and protect None or (K,1,H/2,W/2) as in
+        levels_to_mask_batch.  Candidate j is latent cand_latent[j] lowered by cand_offset[j]; its dict is bit-identical to
+        estimate_batch of the candidate's levels and mask (levels_to_mask) with its latent's code.  A candidate encode would refuse
+        raises encode's message followed by ' (candidate j)', for the first such j."""
+        K, code, imp, protect = self._budget_inputs(code, imap_quant, protect)
+        lat, offs = list(cand_latent), list(cand_offset)
+        if len(lat) != len(offs):
+            raise RuntimeError("estimate_candidates: %d latents for %d offsets" % (len(lat), len(offs)))
+        return self._candidates(code, imp, protect, list(zip(lat, offs)))
+
+    def encode_batch_to_budget(self, code, imap_quant, max_bytes, protect=None, shared=False, max_batch=16):
+        """encode_to_budget of K latents, with batched estimates and one encode_batch: code (K,48,H,W), imap_quant (K,1,H/2,W/2),
+        protect None or an integer (K,1,H/2,W/2) map per latent (as encode_to_budget's).  Candidates are estimated as (latent,
+        offset) pairs (estimate_candidates), at most max_batch per pass: max_batch bounds the encoder buffers, which grow with the
+        batch, and does not change the result.
+
+        shared=False: max_bytes is one int for every latent or a list of K.  Stage 1 of every latent runs in as few passes as
+        max_batch allows, then stage 2 of every latent that needs one, then one encode_batch of the K chosen candidates
+        (select_budget_offsets).  Returns K dicts; dict k equals encode_to_budget(code[k:k+1], imap_quant[k:k+1], max_bytes[k],
+        protect[k:k+1]) exactly, streams included.
+
+        shared=True: max_bytes is one int for all 2K streams, and one offset t is applied to every latent, so all are lowered alike.
+        t fits when the sum over the latents of budget_bound(estimate of latent k at t) is at most max_bytes (select_shared_offset,
+        offsets up to the largest 48 + max P_k).  Returns {'results': K dicts with encode_to_budget's keys, 'bound' and 'bounds'
+        being the latent's own, 'offset': t, 'bound': the summed bound at t, 'bounds': {t: summed bound} of every offset
+        evaluated}.  K = 1 gives encode_to_budget's offset, bounds and streams.
+
+        RuntimeError, with nothing returned, when no offset fits or the written bytes exceed their budget: encode_to_budget's
+        message, followed by ' (latent k)' for the lowest such latent in the per-latent mode."""
+        K, code, imp, protect = self._budget_inputs(code, imap_quant, protect)
+        if isinstance(max_batch, bool) or not isinstance(max_batch, int) or max_batch < 1:
+            raise RuntimeError("encode_batch_to_budget: max_batch must be a positive int (got %r)" % (max_batch,))
+        tops = [48] * K if protect is None else [48 + int(m) for m in protect.amax(dim=(1, 2, 3)).tolist()]
+
+        def estimate(pairs):
+            return self._candidates(code, imp, protect, pairs)
+
+        if shared:
+            if isinstance(max_bytes, (list, tuple)):
+                raise RuntimeError("encode_batch_to_budget: shared=True takes one budget for all latents")
+            budget = int(max_bytes)
+            offset, bounds, per = select_shared_offset(estimate, budget, K, max(tops), max_batch)
+            offsets, budgets = [offset] * K, None
+        else:
+            budgets = [int(b) for b in max_bytes] if isinstance(max_bytes, (list, tuple)) else [int(max_bytes)] * K
+            if len(budgets) != K:
+                raise RuntimeError("encode_batch_to_budget: %d budgets for %d latents" % (len(budgets), K))
+            picks = select_budget_offsets(estimate, budgets, tops, max_batch)
+            offsets = [o for o, _ in picks]
+        levels, masks = levels_to_mask_batch(imp, range(K), offsets, protect)
+        streams = self.encode_batch(code, masks, levels)
+        results = []
+        for k, (imp_bytes, code_bytes) in enumerate(streams):
+            own = {t: per[t][k] for t in bounds} if shared else picks[k][1]
+            results.append({'imp_bytes': imp_bytes, 'code_bytes': code_bytes, 'offset': offsets[k], 'levels': levels[k:k + 1],
+                            'mask': masks[k:k + 1], 'bound': own[offsets[k]], 'bounds': own})
+        if not shared:
+            for k, r in enumerate(results):
+                size = len(r['imp_bytes']) + len(r['code_bytes'])
+                if size > budgets[k]:
+                    raise RuntimeError("encode_to_budget: offset %d encoded to %d bytes, above its bound of %d and the budget of %d "
+                                       "bytes (latent %d)" % (r['offset'], size, r['bound'], budgets[k], k))
+            return results
+        size = sum(len(r['imp_bytes']) + len(r['code_bytes']) for r in results)
+        if size > budget:
+            raise RuntimeError("encode_to_budget: offset %d encoded to %d bytes, above its bound of %d and the budget of %d bytes"
+                               % (offset, size, bounds[offset], budget))
+        return {'results': results, 'offset': offset, 'bound': bounds[offset], 'bounds': bounds}
 
     def decode(self, imp_bytes, code_bytes, h=None, w=None, name=None):
         code = torch.empty((1, 48, self.H, self.W), dtype=torch.float32, device=self.dev)

@@ -178,6 +178,33 @@ class BandCodec(object):
         """-> the container (identical on every rank)."""
         return pack_band_streams(self.H, self.W, exchange_band_streams(self.encode_local(code, mask, imap), self.nbands))
 
+    def encode_to_budget(self, code, imap, max_bytes, protect=None):
+        """The container in at most max_bytes bytes, its header (16 + 8 * nbands bytes) included: the bands, split as split_bands
+        splits them (protect rows too), are coded by one FusedCodec of the band size in its shared budget mode
+        (FusedCodec.encode_batch_to_budget(..., shared=True)), so every band is lowered by the same level offset.  code (1,48,H,W),
+        imap (1,1,H/2,W/2), protect None or an integer (1,1,H/2,W/2) map.  decode reads the container as any other.  world == 1
+        only: the bands' bounds are not gathered across ranks.
+        -> {'container': bytes, 'offset': the shared offset, 'bound': the container's bound at it, 'bounds': {offset: container
+        bound} of every offset evaluated, 'results': the per-band dicts of encode_batch_to_budget}"""
+        if self.world != 1:
+            raise RuntimeError("BandCodec.encode_to_budget: needs world == 1 (got %d); the bands' bounds are not gathered across ranks"
+                               % self.world)
+        hi = self.H // 2
+        if tuple(code.shape) != (1, code.shape[1], self.H, self.W) or tuple(imap.shape) != (1, 1, hi, self.W // 2):
+            raise RuntimeError("BandCodec.encode_to_budget: expected a (1,C,%d,%d) latent and a (1,1,%d,%d) importance map"
+                               % (self.H, self.W, hi, self.W // 2))
+        if protect is not None and (not isinstance(protect, torch.Tensor) or tuple(protect.shape) != tuple(imap.shape)):
+            raise RuntimeError("BandCodec.encode_to_budget: protect must be a (1,1,%d,%d) integer tensor, like the importance map"
+                               % (hi, self.W // 2))
+        head = 16 + 8 * self.nbands
+        codes = torch.cat([code[:, :, r0:r1] for r0, r1 in self.rows])
+        imaps = torch.cat([imap[:, :, r0 // 2:r1 // 2] for r0, r1 in self.rows])
+        prot = None if protect is None else torch.cat([protect[:, :, r0 // 2:r1 // 2] for r0, r1 in self.rows])
+        r = self.codecs[0].encode_batch_to_budget(codes, imaps, int(max_bytes) - head, protect=prot, shared=True)
+        blob = pack_band_streams(self.H, self.W, [(x["imp_bytes"], x["code_bytes"]) for x in r["results"]])
+        return {"container": blob, "offset": r["offset"], "bound": r["bound"] + head,
+                "bounds": {t: b + head for t, b in r["bounds"].items()}, "results": r["results"]}
+
     def decode_local(self, blob):
         """Decodes this rank's bands -> {band: (code_b, mask_b)}."""
         H, W, streams = unpack_band_streams(blob)

@@ -243,6 +243,21 @@ int lic360_codec_estimate(lic360_codec* c, const float* code_dev, const float* m
  * limits (3K <= 65535 and 3 * K * 48 * H * W < 2^31), is an argument error. */
 int lic360_codec_estimate_batch(lic360_codec* c, int K, const float* code_dev, const float* mask_dev, const float* imp_dev,
                                 float* code_bits_dev, float* imp_bits_dev, double* bits_host, long long* counts_host);
+/* lic360_codec_estimate_batch of J rate-control candidates given as (source latent, offset) pairs, without materialising them.
+ *   code_dev (K,48,H,W), imp_dev (K,1,H/2,W/2): K source latents; protect_dev: NULL or (K,1,H/2,W/2) int32 protection maps
+ *   candidate j: source cand_latent_host[j] in [0, K) lowered by offset cand_offset_host[j] >= 0, cell by cell as
+ *   lic360_imp_levels_to_mask_protected lowers it (P clamped to [0, 48]; NULL: no map)
+ *   bits_host[2j + stream_id], counts_host[2j + stream_id]: totals and coded symbols of candidate j
+ * The outputs are bit-identical to lic360_codec_estimate_batch run on the candidates' levels and masks from
+ * lic360_imp_levels_to_mask_protected with the source's code.  No candidate's code or (48,H,W) mask is stored: the code network's input
+ * (code - 3.5) * mask is built from the source code and each symbol's mask bit, which the code stream's bits kernel derives again; the
+ * candidates' levels (H/2 x W/2 floats each) live in a codec buffer that grows with J.  J has the limits of K in
+ * lic360_codec_estimate_batch.  A candidate lic360_codec_encode would refuse fails the call with encode's status and message followed
+ * by " (candidate j)", for the lowest such j; validity is judged on the candidate (lowering can bring a level into range, and a
+ * masked-out code symbol is never checked).  K < 1, J < 1, a source outside [0, K) or a negative offset is an argument error. */
+int lic360_codec_estimate_candidates(lic360_codec* c, int K, const float* code_dev, const float* imp_dev, const int32_t* protect_dev,
+                                     int J, const int* cand_latent_host, const int* cand_offset_host, double* bits_host,
+                                     long long* counts_host);
 /* lic360_codec_encode of K latents of the codec's size in one pass: both networks run once at batch K, as in
  * lic360_codec_estimate_batch, the row kernels once with the latent in blockIdx.y, and each stream's rows come back with one copy.
  * The host codes the K importance streams as soon as their rows are on the host, while the code network still runs, then the K
@@ -282,6 +297,13 @@ int lic360_imp_levels_to_mask(const float* levels_dev, int h, int w, const int* 
  * bit for bit.  Same argument checks and messages as lic360_imp_levels_to_mask. */
 int lic360_imp_levels_to_mask_protected(const float* levels_dev, int h, int w, const int* offsets_host, int K, const int32_t* protect_dev,
                                         float* levels_out_dev, float* mask_out_dev, void* stream);
+/* lic360_imp_levels_to_mask_protected of J candidates of K source maps: levels_dev (K,1,h,w), protect_dev NULL or (K,1,h,w) int32;
+ * candidate j is source cand_latent_host[j] in [0, K) at offset cand_offset_host[j] >= 0.  levels_out_dev (J,1,h,w) and mask_out_dev
+ * (J,48,2h,2w): entry j is bit-identical to lic360_imp_levels_to_mask_protected of its source's map and protection at its offset.
+ * Enqueued on `stream`; a source outside [0, K) or a negative offset is an argument error. */
+int lic360_imp_levels_to_mask_batch(const float* levels_dev, int K, int h, int w, const int32_t* protect_dev, int J,
+                                    const int* cand_latent_host, const int* cand_offset_host, float* levels_out_dev, float* mask_out_dev,
+                                    void* stream);
 long lic360_codec_stream_size(lic360_codec* c, int stream_id);
 long lic360_codec_stream_copy(lic360_codec* c, int stream_id, uint8_t* out, long cap);
 /* -> code_out_dev (1,48,H,W) = symbols where mask == 1, else 0 (lic360_demo.py:236-237); mask_out_dev (1,48,H,W) */
