@@ -59,6 +59,7 @@ SIGNATURES = {
     "lic360_projects_update": (_I, [_P, _P, _I, _I, _I, _I, _P]),
     "lic360_projects_forward": (_I, [_P, _P, _P, _I, _I, _I, _I, _I, _I, _P]),
     "lic360_projects_backward": (_I, [_P, _P, _P, _P, _I, _I, _I, _I, _I, _I, _P]),
+    "lic360_view_footprint": (_I, [_I, _I, _I, _P, _P, _P, _P, _P]),
     "lic360_coder_create": (_P, [ctypes.c_char_p, _F]),
     "lic360_coder_destroy": (None, [_P]),
     "lic360_coder_reset_fname": (_I, [_P, ctypes.c_char_p]),

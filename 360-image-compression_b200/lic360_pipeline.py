@@ -150,6 +150,42 @@ def viewport_protection(h, w, views, levels, fov=0.6, device=None):
     return (weight > 0).to(torch.int32) * levels
 
 
+def view_footprint(h, w, thetas, phis, fov, device=None):
+    """Exact footprints of V rectilinear views on an h x w ERP grid (lic360_view_footprint): a (V,1,h,w) int32 tensor on `device` (a
+    CUDA device, default the current one), 1 where the cell intersects the view's field, 0 elsewhere.  thetas, phis: V view
+    directions in units of pi, as MultiProject's (view (0, 0) is its front view 1); fov: one field of view in units of pi for all
+    views, or V of them, each in (0, 1).  Cells follow ProjectsOp's grid convention (include/lic360_b200.h); h and w even."""
+    th = [float(x) for x in thetas]
+    ph = [float(x) for x in phis]
+    fovs = [float(x) for x in fov] if isinstance(fov, (list, tuple)) else [float(fov)] * len(th)
+    if not th or len(ph) != len(th) or len(fovs) != len(th):
+        raise RuntimeError("view_footprint: need V >= 1 thetas, V phis and one or V fovs (got %d, %d, %d)" % (len(th), len(ph), len(fovs)))
+    device = torch.device('cuda') if device is None else torch.device(device)
+    if device.type != 'cuda':
+        raise RuntimeError("view_footprint: the footprint is computed on a CUDA device (got %s)" % device)
+    V = len(th)
+    out = torch.empty((V, 1, int(h), int(w)), dtype=torch.int32, device=device)
+    arr = ctypes.c_float * V
+    with torch.cuda.device(out.device):
+        check(LIB.lic360_view_footprint(int(h), int(w), V, arr(*th), arr(*ph), arr(*fovs), out.data_ptr(), cstream(out)))
+    return out
+
+
+def view_protection(h, w, thetas, phis, fov, levels, margin=0, device=None):
+    """Protection map (1,1,h,w) int32 for encode_to_budget / encode_batch_to_budget at any head orientation: `levels` on the union of
+    the views' footprints (view_footprint), dilated by `margin` cells (longitude wraps round the seam, latitude stops at the poles),
+    0 elsewhere.  Combine maps with torch.maximum, as viewport_protection's."""
+    levels = _preset_levels(levels)
+    if isinstance(margin, bool) or not isinstance(margin, int) or margin < 0:
+        raise RuntimeError("view_protection: margin must be an int >= 0 (got %r)" % (margin,))
+    fp = view_footprint(h, w, thetas, phis, fov, device).amax(dim=0, keepdim=True)
+    if margin:
+        mw = min(margin, int(w))  # a wider margin wraps onto columns already covered
+        wide = torch.nn.functional.pad(fp.float(), (mw, mw, 0, 0), mode='circular')
+        fp = torch.nn.functional.max_pool2d(wide, (2 * margin + 1, 2 * mw + 1), stride=1, padding=(margin, 0)).to(torch.int32)
+    return fp * levels
+
+
 def _preset_levels(levels):
     if int(levels) != levels or not 0 <= levels <= 48:
         raise RuntimeError("protection levels must be an integer in [0, 48] (got %r)" % (levels,))

@@ -70,7 +70,7 @@ def band_rows(H, nbands):
 
 
 def rank_bands(nbands, world, rank):
-    """Bands of rank `rank`: round-robin, so that neighbouring bands (similar content, similar cost) land on different GPUs."""
+    """Bands (or tiles) of rank `rank`: round-robin, so that neighbouring parts (similar content, similar cost) land on different GPUs."""
     if world <= 0 or not (0 <= rank < world):
         raise ValueError("rank_bands: bad world/rank %r/%r" % (world, rank))
     return list(range(rank, nbands, world))
@@ -110,8 +110,8 @@ def unpack_band_streams(blob):
     return H, W, out
 
 
-def exchange_band_streams(local, nbands):
-    """local: {band: (imp_bytes, code_bytes)} of this rank -> the full list on every rank (bookkeeping traffic only)."""
+def exchange_streams(local, nparts, kind="band"):
+    """local: {part: (imp_bytes, code_bytes)} of this rank -> the full list on every rank (bookkeeping traffic only)."""
     table = dict(local)
     if dist.is_available() and dist.is_initialized() and dist.get_world_size() > 1:
         parts = [None] * dist.get_world_size()
@@ -120,27 +120,28 @@ def exchange_band_streams(local, nbands):
         for p in parts:
             for k, v in p.items():
                 if k in table:
-                    raise RuntimeError("exchange_band_streams: band %d coded by two ranks" % k)
+                    raise RuntimeError("exchange_%s_streams: %s %d coded by two ranks" % (kind, kind, k))
                 table[k] = v
-    if sorted(table) != list(range(nbands)):
-        raise RuntimeError("exchange_band_streams: bands %s of %d present" % (sorted(table), nbands))
-    return [table[b] for b in range(nbands)]
+    if sorted(table) != list(range(nparts)):
+        raise RuntimeError("exchange_%s_streams: %ss %s of %d present" % (kind, kind, sorted(table), nparts))
+    return [table[b] for b in range(nparts)]
 
 
-class BandCodec(object):
-    """One image as `nbands` independently coded latitude bands, dealt round-robin to the ranks of the process group (or all on
-    this process without one).  `make_codec(h, w)` builds the per-band codec (FusedCodec on a GPU box; the tests pass the CPU
-    rendition): anything with encode(code, mask, imap) -> (imp_bytes, code_bytes) and decode(imp_bytes, code_bytes) -> (code, mask)."""
+def exchange_band_streams(local, nbands):
+    return exchange_streams(local, nbands, "band")
 
-    def __init__(self, make_codec, H, W, nbands, world=1, rank=0, in_flight=1):
-        self.H, self.W, self.nbands, self.world, self.rank = H, W, nbands, world, rank
-        self.rows = band_rows(H, nbands)
-        self.mine = rank_bands(nbands, world, rank)
-        hb = H // nbands
-        self.codecs = [make_codec(hb, W) for _ in range(max(1, min(in_flight, len(self.mine))))]
+
+class _PartCodec(object):
+    """What BandCodec and TileCodec share: the parts dealt round-robin to the ranks (rank_bands), `in_flight` codecs of the part size
+    with one worker thread each, and the exchange of decoded parts between ranks."""
+
+    def __init__(self, make_codec, part_hw, nparts, world, rank, in_flight):
+        self.world, self.rank = world, rank
+        self.mine = rank_bands(nparts, world, rank)
+        self.codecs = [make_codec(*part_hw) for _ in range(max(1, min(in_flight, len(self.mine))))]
 
     def _map(self, fn, items):
-        """fn(codec, item) over this rank's items, one worker thread per codec (each codec = one band in flight)."""
+        """fn(codec, item) over this rank's items, one worker thread per codec (each codec = one part in flight)."""
         if len(self.codecs) == 1 or len(items) <= 1:
             return [fn(self.codecs[0], it) for it in items]
         import threading
@@ -159,7 +160,7 @@ class BandCodec(object):
                     errs.append(e)
                     return
 
-        th = [threading.Thread(target=worker, args=(cd,)) for cd in self.codecs]
+        th = [threading.Thread(target=worker, args=(cd,)) for cd in self.codecs[:len(items)]]
         for t in th:
             t.start()
         for t in th:
@@ -167,6 +168,28 @@ class BandCodec(object):
         if errs:
             raise errs[0]
         return out
+
+    def _gather(self, local):
+        """{part: (code_p, mask_p)} decoded by this rank -> the parts decoded by every rank (assembly, not coding)."""
+        if not (self.world > 1 and dist.is_available() and dist.is_initialized()):
+            return local
+        parts = [None] * self.world
+        dist.all_gather_object(parts, {b: (c.cpu(), m.cpu()) if hasattr(c, "cpu") else (c, m) for b, (c, m) in local.items()})
+        table = {}
+        for p in parts:
+            table.update(p)
+        return table
+
+
+class BandCodec(_PartCodec):
+    """One image as `nbands` independently coded latitude bands, dealt round-robin to the ranks of the process group (or all on
+    this process without one).  `make_codec(h, w)` builds the per-band codec (FusedCodec on a GPU box; the tests pass the CPU
+    rendition): anything with encode(code, mask, imap) -> (imp_bytes, code_bytes) and decode(imp_bytes, code_bytes) -> (code, mask)."""
+
+    def __init__(self, make_codec, H, W, nbands, world=1, rank=0, in_flight=1):
+        self.H, self.W, self.nbands = H, W, nbands
+        self.rows = band_rows(H, nbands)
+        _PartCodec.__init__(self, make_codec, (H // nbands, W), nbands, world, rank, in_flight)
 
     def encode_local(self, code, mask, imap):
         """Codes this rank's bands of the full-size inputs -> {band: (imp_bytes, code_bytes)}."""
@@ -176,7 +199,7 @@ class BandCodec(object):
 
     def encode(self, code, mask, imap):
         """-> the container (identical on every rank)."""
-        return pack_band_streams(self.H, self.W, exchange_band_streams(self.encode_local(code, mask, imap), self.nbands))
+        return pack_band_streams(self.H, self.W, exchange_streams(self.encode_local(code, mask, imap), self.nbands))
 
     def encode_to_budget(self, code, imap, max_bytes, protect=None):
         """The container in at most max_bytes bytes, its header (16 + 8 * nbands bytes) included: the bands, split as split_bands
@@ -216,14 +239,7 @@ class BandCodec(object):
     def decode(self, blob, like=None):
         """-> (code, mask) of the whole image on every rank (the decoded bands are exchanged: assembly, not coding)."""
         local = self.decode_local(blob)
-        if self.world > 1 and dist.is_available() and dist.is_initialized():
-            parts = [None] * self.world
-            dist.all_gather_object(parts, {b: (c.cpu(), m.cpu()) if hasattr(c, "cpu") else (c, m) for b, (c, m) in local.items()})
-            table = {}
-            for p in parts:
-                table.update(p)
-        else:
-            table = local
+        table = self._gather(local)
         cat = torch.cat if isinstance(next(iter(table.values()))[0], torch.Tensor) else None
         if cat is None:
             import numpy as np
@@ -232,3 +248,179 @@ class BandCodec(object):
         dev = like.device if like is not None else next(iter(local.values()))[0].device
         return (torch.cat([table[b][0].to(dev) for b in range(self.nbands)], dim=2),
                 torch.cat([table[b][1].to(dev) for b in range(self.nbands)], dim=2))
+
+
+# ---------------------------------------------------------------------------------------------------------------------
+# Tiles of ONE image: random access for viewers.
+#
+# A viewer shows one viewport of a 360-degree image, yet a single stream (or a latitude band) must be decoded whole.  The same
+# format extension as the bands, in two dimensions: the latent is cut into rows x cols tiles of equal size and every tile is coded
+# as an independent sub-image with its own two bitstreams (zero context at the tile's edges, as at the image's).  Each tile is
+# exactly what the codec produces for that tile as an image of its own (the parity statement, per tile); a viewer decodes only the
+# tiles its view touches (TileCodec.decode_views, with the exact footprint of lic360_pipeline.view_footprint).  Equal tiles make the
+# whole image one batch for FusedCodec.encode_batch and its budget searches.
+# ---------------------------------------------------------------------------------------------------------------------
+TILE_MAGIC = b"L3T1"
+
+
+def tile_grid(H, W, rows, cols):
+    """[(r0, r1, c0, c1)] of the rows x cols tiles of an H x W latent, row-major.  One importance cell covers 2 x 2 latent cells, so
+    the tiles, H / rows by W / cols, must have an even positive number of rows and columns."""
+    if rows < 1 or cols < 1 or H < 1 or W < 1 or H % rows or W % cols or (H // rows) % 2 or (W // cols) % 2:
+        raise ValueError("tile_grid: a %dx%d latent does not split into %dx%d tiles of an even number of rows and columns"
+                         % (H, W, rows, cols))
+    ht, wt = H // rows, W // cols
+    return [(r * ht, (r + 1) * ht, c * wt, (c + 1) * wt) for r in range(rows) for c in range(cols)]
+
+
+def pack_tile_streams(rows, cols, H, W, streams):
+    """streams: [(imp_bytes, code_bytes)] in tile order -> one container: magic, rows, cols, H, W, the 2 * rows * cols lengths, the
+    payloads."""
+    tile_grid(H, W, rows, cols)
+    if len(streams) != rows * cols:
+        raise ValueError("pack_tile_streams: %d stream pairs for %dx%d tiles" % (len(streams), rows, cols))
+    head = TILE_MAGIC + struct.pack("<IIII", rows, cols, H, W)
+    head += b"".join(struct.pack("<II", len(a), len(b)) for a, b in streams)
+    return head + b"".join(a + b for a, b in streams)
+
+
+def tile_header_bytes(ntiles):
+    return 20 + 8 * ntiles
+
+
+def unpack_tile_streams(blob):
+    """-> (rows, cols, H, W, [(imp_bytes, code_bytes)]); raises ValueError on a malformed container."""
+    if len(blob) < 20 or blob[:4] != TILE_MAGIC:
+        raise ValueError("unpack_tile_streams: not a tile container")
+    rows, cols, H, W = struct.unpack_from("<IIII", blob, 4)
+    tile_grid(H, W, rows, cols)  # ValueError when the grid does not divide the latent
+    n = rows * cols
+    off = tile_header_bytes(n)
+    if len(blob) < off:
+        raise ValueError("unpack_tile_streams: truncated header")
+    lens = [struct.unpack_from("<II", blob, 20 + 8 * k) for k in range(n)]
+    if off + sum(a + b for a, b in lens) != len(blob):
+        raise ValueError("unpack_tile_streams: payload size does not match the header")
+    out = []
+    for a, b in lens:
+        out.append((bytes(blob[off:off + a]), bytes(blob[off + a:off + a + b])))
+        off += a + b
+    return rows, cols, H, W, out
+
+
+def split_tiles(x, rows, cols):
+    """(1,C,h,w) -> (rows*cols, C, h/rows, w/cols): the tiles in row-major order, one contiguous batch"""
+    _, C, h, w = x.shape
+    return x.reshape(C, rows, h // rows, cols, w // cols).permute(1, 3, 0, 2, 4).reshape(rows * cols, C, h // rows, w // cols)
+
+
+class TileCodec(_PartCodec):
+    """One image as rows x cols independently coded tiles, dealt round-robin to the ranks of the process group (or all on this
+    process without one), decodable tile by tile.  `make_codec(h_t, w_t)` builds the per-tile codec: FusedCodec on a GPU, whose
+    encode_batch codes all of a rank's tiles in one pass; anything with BandCodec's encode / decode methods is coded tile by tile.
+    `in_flight` codecs decode tiles concurrently, one worker thread each."""
+
+    def __init__(self, make_codec, H, W, rows, cols, world=1, rank=0, in_flight=1):
+        self.H, self.W, self.rows, self.cols = H, W, rows, cols
+        self.tiles = tile_grid(H, W, rows, cols)
+        self.ht, self.wt = H // rows, W // cols
+        _PartCodec.__init__(self, make_codec, (self.ht, self.wt), rows * cols, world, rank, in_flight)
+        self.device = getattr(self.codecs[0], "dev", torch.device("cpu"))
+
+    def _check(self, code, imap, who):
+        hi, wi = self.H // 2, self.W // 2
+        if (code.dim() != 4 or tuple(code.shape) != (1, code.shape[1], self.H, self.W) or imap.dim() != 4
+                or tuple(imap.shape) != (1, 1, hi, wi)):
+            raise RuntimeError("TileCodec.%s: expected a (1,C,%d,%d) latent and a (1,1,%d,%d) importance map" % (who, self.H, self.W, hi, wi))
+
+    def encode_local(self, code, mask, imap):
+        """Codes this rank's tiles of the full-size inputs -> {tile: (imp_bytes, code_bytes)}."""
+        self._check(code, imap, "encode")
+        if not self.mine:
+            return {}
+        codes, masks, imaps = (split_tiles(x, self.rows, self.cols)[self.mine] for x in (code, mask, imap))
+        if hasattr(self.codecs[0], "encode_batch"):
+            res = self.codecs[0].encode_batch(codes, masks, imaps)
+        else:
+            res = self._map(lambda cd, k: cd.encode(codes[k:k + 1], masks[k:k + 1], imaps[k:k + 1]), list(range(len(self.mine))))
+        return dict(zip(self.mine, res))
+
+    def encode(self, code, mask, imap):
+        """code, mask (1,48,H,W), imap (1,1,H/2,W/2) -> the container (identical on every rank)."""
+        streams = exchange_streams(self.encode_local(code, mask, imap), len(self.tiles), "tile")
+        return pack_tile_streams(self.rows, self.cols, self.H, self.W, streams)
+
+    def encode_to_budget(self, code, imap, max_bytes, protect=None):
+        """The container within a byte budget, by FusedCodec.encode_batch_to_budget on the tiles (protect split as the importance map).
+
+        max_bytes an int: the whole container, its header (20 + 8 * rows * cols bytes) included, with one level offset shared by all
+        tiles (shared mode).  -> {'container', 'offset', 'bound': the container's bound at the offset, 'bounds': {offset: container
+        bound} of every offset evaluated, 'results': the per-tile dicts}.
+        max_bytes a list of rows * cols ints: each tile's two streams within its own budget (per-latent mode), e.g. more bytes for the
+        tiles a viewer is likely to see.  -> {'container', 'offsets': per tile, 'results': the per-tile dicts}.
+        world == 1 only: the tiles' bounds are not gathered across ranks."""
+        if self.world != 1:
+            raise RuntimeError("TileCodec.encode_to_budget: needs world == 1 (got %d); the tiles' bounds are not gathered across ranks"
+                               % self.world)
+        self._check(code, imap, "encode_to_budget")
+        if protect is not None and (not isinstance(protect, torch.Tensor) or tuple(protect.shape) != tuple(imap.shape)):
+            raise RuntimeError("TileCodec.encode_to_budget: protect must be a (1,1,%d,%d) integer tensor, like the importance map"
+                               % (self.H // 2, self.W // 2))
+        T = len(self.tiles)
+        codes, imaps = split_tiles(code, self.rows, self.cols), split_tiles(imap, self.rows, self.cols)
+        prot = None if protect is None else split_tiles(protect, self.rows, self.cols)
+        cd = self.codecs[0]
+        if isinstance(max_bytes, (list, tuple)):
+            if len(max_bytes) != T:
+                raise RuntimeError("TileCodec.encode_to_budget: %d budgets for %d tiles" % (len(max_bytes), T))
+            res = cd.encode_batch_to_budget(codes, imaps, [int(b) for b in max_bytes], protect=prot)
+            blob = pack_tile_streams(self.rows, self.cols, self.H, self.W, [(x["imp_bytes"], x["code_bytes"]) for x in res])
+            return {"container": blob, "offsets": [x["offset"] for x in res], "results": res}
+        head = tile_header_bytes(T)
+        r = cd.encode_batch_to_budget(codes, imaps, int(max_bytes) - head, protect=prot, shared=True)
+        blob = pack_tile_streams(self.rows, self.cols, self.H, self.W, [(x["imp_bytes"], x["code_bytes"]) for x in r["results"]])
+        return {"container": blob, "offset": r["offset"], "bound": r["bound"] + head,
+                "bounds": {t: b + head for t, b in r["bounds"].items()}, "results": r["results"]}
+
+    def tiles_for_views(self, thetas, phis, fov, margin=0):
+        """Sorted indices of the tiles that hold a cell of the views' footprints (lic360_pipeline.view_protection on the importance
+        grid, dilated by `margin` cells), by a max over each tile on the codec's device."""
+        import lic360_pipeline as pl
+        fp = pl.view_protection(self.H // 2, self.W // 2, thetas, phis, fov, 1, margin, self.device)
+        hit = split_tiles(fp, self.rows, self.cols).amax(dim=(1, 2, 3))
+        return [int(k) for k in torch.nonzero(hit).flatten().tolist()]
+
+    def decode_tiles(self, blob, tiles):
+        """Decodes only `tiles` (indices into tile_grid's order), this rank's share of them on up to in_flight codecs at once, and
+        assembles them on every rank -> (code, mask, decoded): code and mask (1,48,H,W), zero outside the decoded tiles (mask 0: not
+        coded), decoded (1,1,H,W) int32, 1 on the latent cells decoded."""
+        rows, cols, H, W, streams = unpack_tile_streams(blob)
+        if (rows, cols, H, W) != (self.rows, self.cols, self.H, self.W):
+            raise ValueError("TileCodec.decode: container is %dx%d in %dx%d tiles, codec is %dx%d in %dx%d"
+                             % (H, W, rows, cols, self.H, self.W, self.rows, self.cols))
+        want = sorted(set(int(k) for k in tiles))
+        if want and not (0 <= want[0] and want[-1] < len(self.tiles)):
+            raise ValueError("TileCodec.decode_tiles: tile indices must lie in [0, %d) (got %s)" % (len(self.tiles), want))
+        mine = [k for k in want if k in set(self.mine)]
+        local = dict(zip(mine, self._map(lambda cd, k: cd.decode(*streams[k]), mine)))
+        table = self._gather(local)
+        dev = self.device
+        code = torch.zeros((1, 48, H, W), dtype=torch.float32, device=dev)
+        mask = torch.zeros((1, 48, H, W), dtype=torch.float32, device=dev)
+        decoded = torch.zeros((1, 1, H, W), dtype=torch.int32, device=dev)
+        for k in want:
+            r0, r1, c0, c1 = self.tiles[k]
+            c, m = table[k]
+            code[:, :, r0:r1, c0:c1] = torch.as_tensor(c).to(dev)
+            mask[:, :, r0:r1, c0:c1] = torch.as_tensor(m).to(dev)
+            decoded[:, :, r0:r1, c0:c1] = 1
+        return code, mask, decoded
+
+    def decode_views(self, blob, thetas, phis, fov, margin=0):
+        """decode_tiles of the tiles the views need (tiles_for_views) -> (code, mask, decoded)."""
+        return self.decode_tiles(blob, self.tiles_for_views(thetas, phis, fov, margin))
+
+    def decode(self, blob):
+        """-> (code, mask) of the whole image on every rank."""
+        code, mask, _ = self.decode_tiles(blob, range(len(self.tiles)))
+        return code, mask

@@ -172,6 +172,17 @@ int lic360_projects_forward(const float* in_dev, const float* tf_dev, float* out
 int lic360_projects_backward(const float* top_diff_dev, const float* tf_dev, float* bottom_diff_dev, float* count_dev, int NC, int H,
                              int W, int h_out, int w_out, int nearest, void* stream);
 
+/* ---- View footprint: the cells of an h x w ERP grid that a rectilinear view of any direction touches --------------------------
+ * Cell (i, j) is the closed spherical rectangle x in [j - 1/2, j + 1/2], y in [i - 1/2, i + 1/2] of ProjectsOp's ERP coordinates
+ * (x = theta / pi * hx + hx, y = -2 lat / pi * hy + hy, hx = (w - 1) / 2, hy = (h - 1) / 2), clamped to the sphere: columns 0 and
+ * w - 1 are the half cells beside the +-pi seam, rows 0 and h - 1 end in a pole.  View v is (theta, phi, fov) in units of pi, as
+ * MultiProject's: its axes (f, r, u) are the columns of the rotation lic360_projects_init builds (view (0, 0) looks along +x), and its
+ * field is the closed frustum {d : |d.r| <= tan(a) d.f, |d.u| <= tan(a) d.f}, a = fov * pi / 2.  out_dev (nviews, h, w) int32:
+ * 1 exactly where the cell and the field intersect (float64 predicate: a corner of one inside the other, or a field edge across a
+ * cell edge), else 0.  h, w even and positive; 0 < fov < 1; finite angles.                                                          */
+int lic360_view_footprint(int h, int w, int nviews, const float* theta_host, const float* phi_host, const float* fov_host,
+                          int32_t* out_dev, void* stream);
+
 /* ---- Coder (main.cpp:132-143, coder.h:10-63, coder.cpp:30-114; ArithmeticCoder.cpp, BitIoStream.cpp) -----
  * Same bitstream format (32-bit state range coder, MSB-first bits, `1` terminator + zero padding).
  * Tables are int32 rows of ncode+1 cumulative counts, total = row[ncode].                                   */
