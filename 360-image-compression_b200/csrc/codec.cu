@@ -254,8 +254,8 @@ struct lic360_codec {
     void* est_dev = nullptr;            // estimate: totals, error keys and counts of both streams (EstimateTotals layout)
     void* est_host = nullptr;           // pinned copy of est_dev
     cudaEvent_t ev_est = nullptr;                // estimate: the importance stream's results are in est_dev
-    int2* cand_dev = nullptr;           // estimate_candidates: the (source latent, offset) table, batch_cap entries
-    float* cand_levels_dev = nullptr;   // estimate_candidates: the candidates' levels (batch_cap,1,H/2,W/2), the importance net's input
+    int2* cand_dev = nullptr;           // estimate_ / encode_candidates: the (source latent, offset) table, batch_cap entries
+    float* cand_levels_dev = nullptr;   // estimate_ / encode_candidates: the candidates' levels (batch_cap,1,H/2,W/2), the importance net's input
     int rows_cap = 1;                   // latents the encoder's row buffers (rows_dev / rows_host of both streams) hold (grown on demand)
     int enc_k = 0;                      // latents of the last successful encode / encode_batch (0 after a failure or a decode)
     std::vector<lic360::EncodedStream> enc_out = std::vector<lic360::EncodedStream>(2);  // [2k + stream_id]: the streams of the last encode (empty after a failed one)
@@ -361,9 +361,9 @@ __device__ __forceinline__ int candidate_level(const float* __restrict__ levels,
     return max((int)imp_symbol(levels[cell]) - drop, 0);
 }
 
-// Candidates of lic360_codec_estimate_candidates: candidate j (the batch's latent j) is source latent tab[j].x lowered by offset
-// tab[j].y (candidate_level), with the levels, code and protection map of that source; the mask bit of a code symbol is
-// code_mask_from_level of its cell's candidate level, the bit lic360_imp_levels_to_mask_protected stores.
+// Candidates of lic360_codec_estimate_candidates and lic360_codec_encode_candidates: candidate j (the batch's latent j) is source latent
+// tab[j].x lowered by offset tab[j].y (candidate_level), with the levels, code and protection map of that source; the mask bit of a code
+// symbol is code_mask_from_level of its cell's candidate level, the bit lic360_imp_levels_to_mask_protected stores.
 struct Candidates {
     const int2* tab;
     const float* levels;     // (S,1,h,w) source levels
@@ -445,13 +445,22 @@ __device__ __forceinline__ void imp_symbol_row(const float* y, int H, int W, int
     entropy_row(o, 49, 65536.f);
 }
 
-// code stream: one thread = one symbol (tc = i / HW, k = i % HW in plan order); its packed row (8 u16) at its coding-order row
+// code stream: one thread = one symbol (tc = i / HW, k = i % HW in plan order); its packed row (8 u16) at its coding-order row.
+// CAND: latent blockIdx.y is candidate blockIdx.y of `cd`, as in gmm_bits_kernel<true>; `mask` is not read.
+template <bool CAND>
 __global__ void gmm_rows_kernel(const float* __restrict__ y, const float* __restrict__ code, const float* __restrict__ mask,
-                                const int32_t* __restrict__ idx, const StepDesc* __restrict__ steps,
+                                Candidates cd, const int32_t* __restrict__ idx, const StepDesc* __restrict__ steps,
                                 const int* __restrict__ row_off, uint16_t* __restrict__ rows, int G, int H, int W, float s2) {
     const int HW = H * W;
     const size_t lat = gmm_latent(y, G, HW);
-    code += lat; mask += lat; rows += lat * 8;
+    int2 cand = make_int2(0, 0);
+    if constexpr (CAND) {
+        cand = cd.tab[blockIdx.y];
+        code += (size_t)cand.x * G * HW;
+    } else {
+        code += lat; mask += lat;
+    }
+    rows += lat * 8;
     const int i = blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= G * HW) return;
     const int k = i % HW, tc = i / HW;
@@ -460,7 +469,10 @@ __global__ void gmm_rows_kernel(const float* __restrict__ y, const float* __rest
     const size_t pos = ((size_t)tc * H + th) * W + tw;
     // NaN and anything outside [0, 8) become the out-of-range marker of the row.  Symbol and mask bit are read before the row is built:
     // it keeps the kernel at 32 registers.
-    const int sym = code_symbol(code[pos]), maskbit = code_mask_bit(mask[pos]);
+    const int sym = code_symbol(code[pos]);
+    int maskbit;
+    if constexpr (CAND) maskbit = candidate_mask_bit(cd, cand.x, cand.y, tc, th, tw, H, W);
+    else maskbit = code_mask_bit(mask[pos]);
     float o[9];
     gmm_symbol_row(y, G, H, W, tc, th, tw, s2, o);
     pack_gmm_row(o, sym, maskbit, rows);
@@ -1013,7 +1025,7 @@ static int grow_buffers(lic360_codec* c, const std::vector<GrowBuf>& bufs, int K
 }
 
 // The buffers that scale with the number of latents an encode or an estimate runs at once: both networks' encoder frames, the bits
-// kernels' partials, the estimate's results and the candidate table and levels of estimate_candidates.  They only grow.
+// kernels' partials, the estimate's results and the candidate table and levels of estimate_ / encode_candidates.  They only grow.
 static int batch_reserve(lic360_codec* c, int K) {
     if (K <= c->batch_cap) return LIC360_OK;
     std::vector<GrowBuf> bufs;
@@ -1138,8 +1150,8 @@ int lic360_codec_set_layer(lic360_codec* c, int stream_id, int layer, const floa
 // alike, whatever else is in the batch).
 //   importance stream (lic360_demo.py:173-189): Scale(-1, 2/47) of the levels
 //   code stream (lic360_demo.py:124-131): (code - 3.5) * mask, once for each of the three nets
-// cand: the K latents are candidates (lic360_codec_estimate_candidates): code_dev holds their sources and the masks are derived, imp_dev
-// holds the candidate levels
+// cand: the K latents are candidates (lic360_codec_estimate_candidates, lic360_codec_encode_candidates): code_dev holds their sources
+// and the masks are derived, imp_dev holds the candidate levels
 static int run_encoder_net(lic360_codec* c, bool is_code, int K, const float* code_dev, const float* mask_dev, const float* imp_dev,
                            const Candidates* cand = nullptr) {
     NetDesc& n = is_code ? c->code : c->imp;
@@ -1157,9 +1169,40 @@ static int run_encoder_net(lic360_codec* c, bool is_code, int K, const float* co
     return run_ec_net(n, K, n.stream);
 }
 
+// The candidates of an estimate or an encode of K candidates: the table cand_host goes to c->cand_dev (cd.tab) and their levels to
+// c->cand_levels_dev, on the importance stream; both streams read the table, so the code stream waits for it (ev_est).
+static int enqueue_candidates(lic360_codec* c, int K, const int2* cand_host, const Candidates& cd) {
+    cudaStream_t s = c->imp.stream;
+    const int hw = c->imp.H * c->imp.W;
+    LIC360_CUDA(cudaMemcpyAsync(c->cand_dev, cand_host, (size_t)K * sizeof(int2), cudaMemcpyHostToDevice, s));
+    candidate_levels_kernel<<<dim3((hw + 255) / 256, K), 256, 0, s>>>(cd, hw, c->cand_levels_dev);
+    LAUNCH_CHECK();
+    LIC360_CUDA(cudaEventRecord(c->ev_est, s));
+    LIC360_CUDA(cudaStreamWaitEvent(c->code.stream, c->ev_est, 0));
+    return LIC360_OK;
+}
+
+// the (source latent, offset) table of J candidates of K sources; a source outside [0, K) or a negative offset is an argument error of
+// the entry point fn
+static int candidate_table(const char* fn, int K, int J, const int* cand_latent_host, const int* cand_offset_host, std::vector<int2>& tab) {
+    tab.resize(J);
+    for (int j = 0; j < J; j++) {
+        const char* bad = cand_latent_host[j] < 0 || cand_latent_host[j] >= K ? "cand_latent must lie in [0, K)"
+                        : cand_offset_host[j] < 0                            ? "offsets must not be negative" : nullptr;
+        if (bad) {
+            set_error("%s: %s", fn, bad);
+            return LIC360_ERR_ARG;
+        }
+        tab[j] = make_int2(cand_latent_host[j], cand_offset_host[j]);
+    }
+    return LIC360_OK;
+}
+
 // the GPU work of an encode of K latents on the codec's two streams: both networks at batch K, the CDF rows of every latent in coding
-// order (latent k's rows at k * total_rows) and their copy to the host, one per stream
-static int enqueue_encode(lic360_codec* c, int K, const float* code_dev, const float* mask_dev, const float* imp_dev, clk::time_point t0) {
+// order (latent k's rows at k * total_rows) and their copy to the host, one per stream.  cand (K candidates, enqueue_candidates done):
+// code_dev holds the sources, imp_dev the candidate levels, and the code stream's mask bits are derived (mask_dev is not read).
+static int enqueue_encode(lic360_codec* c, int K, const float* code_dev, const float* mask_dev, const float* imp_dev, clk::time_point t0,
+                          const Candidates* cand = nullptr) {
     // The two bitstreams are independent: both networks are enqueued on their own CUDA streams first, then the host
     // codes the (small) importance stream while the code-stream network is still running.
     // ---- importance stream: net -> rows of all symbols
@@ -1180,10 +1223,15 @@ static int enqueue_encode(lic360_codec* c, int K, const float* code_dev, const f
         cudaStream_t s = n.stream;
         const auto tq0 = clk::now();
         const int nel = n.G * n.H * n.W;
-        int rc = run_encoder_net(c, true, K, code_dev, mask_dev, imp_dev);
+        int rc = run_encoder_net(c, true, K, code_dev, mask_dev, imp_dev, cand);
         if (rc) return rc;
-        gmm_rows_kernel<<<dim3((nel + 127) / 128, K), 128, 0, s>>>(n.frame[12], code_dev, mask_dev, n.idx_dev, n.steps_dev, n.row_off_dev,
-                                                                   n.rows_dev, n.G, n.H, n.W, kGmmS2);
+        const dim3 grid((nel + 127) / 128, K);
+        if (cand)
+            gmm_rows_kernel<true><<<grid, 128, 0, s>>>(n.frame[12], code_dev, nullptr, *cand, n.idx_dev, n.steps_dev, n.row_off_dev,
+                                                       n.rows_dev, n.G, n.H, n.W, kGmmS2);
+        else
+            gmm_rows_kernel<false><<<grid, 128, 0, s>>>(n.frame[12], code_dev, mask_dev, Candidates{}, n.idx_dev, n.steps_dev,
+                                                        n.row_off_dev, n.rows_dev, n.G, n.H, n.W, kGmmS2);
         LAUNCH_CHECK();
         LIC360_CUDA(cudaMemcpyAsync(n.rows_host, n.rows_dev, (size_t)K * n.total_rows * 16, cudaMemcpyDeviceToHost, s));
         c->t_gpu_steps = ms_since(tq0);  // host time spent enqueueing the code-stream work
@@ -1212,12 +1260,11 @@ static void add_index_suffix(const char* what, int k) {
     const std::string msg = lic360_last_error();
     set_error("%s (%s %d)", msg.c_str(), what, k);
 }
-static void add_latent_suffix(int k) { add_index_suffix("latent", k); }
 
 // The host coding of an encode of K latents, every stream into enc_out: the K importance streams as soon as their rows are on the host
 // (the code network may still be running), then the K code streams.  K = 1 codes on the calling thread with the codec's two coders,
-// K > 1 on the coder pool.  Both CUDA streams are drained on every path.
-static int code_streams(lic360_codec* c, int K, bool latent_suffix, clk::time_point t0) {
+// K > 1 on the coder pool.  Both CUDA streams are drained on every path.  suffix: NULL, or the word of the " (<suffix> k)" an error gets
+static int code_streams(lic360_codec* c, int K, const char* suffix, clk::time_point t0) {
     const bool pooled = K > 1;
     if (pooled) {
         const unsigned hw = std::thread::hardware_concurrency();
@@ -1265,7 +1312,7 @@ static int code_streams(lic360_codec* c, int K, bool latent_suffix, clk::time_po
             const EncodedStream& r = c->enc_out[2 * (size_t)k + sid];
             if (r.rc == LIC360_OK) continue;
             set_error("%s", r.err.c_str());
-            if (latent_suffix) add_latent_suffix(k);
+            if (suffix) add_index_suffix(suffix, k);
             rc = r.rc;
             break;
         }
@@ -1286,17 +1333,22 @@ static int begin_latents(lic360_codec* c, const DeviceGuard& guard, int K) {
     return LIC360_OK;
 }
 
-// lic360_codec_encode (K = 1, latent_suffix false) and lic360_codec_encode_batch
-static int encode_latents(lic360_codec* c, int K, const float* code_dev, const float* mask_dev, const float* imp_dev, bool latent_suffix) {
+// lic360_codec_encode (K = 1, no suffix), lic360_codec_encode_batch (suffix "latent") and lic360_codec_encode_candidates (suffix
+// "candidate", the table in cand_host, imp_dev the sources' levels); protect may be NULL
+static int encode_latents(lic360_codec* c, int K, const float* code_dev, const float* mask_dev, const float* imp_dev, const char* suffix,
+                          const int2* cand_host = nullptr, const int32_t* protect = nullptr) {
     DeviceGuard guard(c->device);
     c->enc_k = 0;
     int rc = begin_latents(c, guard, K);
     if (rc == LIC360_OK) rc = rows_reserve(c, K);
     if (rc) return rc;
     const auto t0 = clk::now();
-    rc = enqueue_encode(c, K, code_dev, mask_dev, imp_dev, t0);
+    const Candidates cd{c->cand_dev, imp_dev, protect};
+    if (cand_host) rc = enqueue_candidates(c, K, cand_host, cd);
+    if (rc == LIC360_OK && cand_host) rc = enqueue_encode(c, K, code_dev, nullptr, c->cand_levels_dev, t0, &cd);
+    else if (rc == LIC360_OK) rc = enqueue_encode(c, K, code_dev, mask_dev, imp_dev, t0);
     if (rc) { drain(c); return rc; }
-    rc = code_streams(c, K, latent_suffix, t0);
+    rc = code_streams(c, K, suffix, t0);
     c->t_total = ms_since(t0);
     if (rc == LIC360_OK) c->enc_k = K;
     return rc;
@@ -1309,14 +1361,26 @@ static int encode_latents(lic360_codec* c, int K, const float* code_dev, const f
 
 int lic360_codec_encode(lic360_codec* c, const float* code_dev, const float* mask_dev, const float* imp_dev) {
     LIC360_CHECK_ARG(c && code_dev && mask_dev && imp_dev, "bad arguments");
-    return encode_latents(c, 1, code_dev, mask_dev, imp_dev, false);
+    return encode_latents(c, 1, code_dev, mask_dev, imp_dev, nullptr);
 }
 
 int lic360_codec_encode_batch(lic360_codec* c, int K, const float* code_dev, const float* mask_dev, const float* imp_dev) {
     LIC360_CHECK_ARG(K >= 1, "K must be at least 1");
     LIC360_CHECK_ARG(c && code_dev && mask_dev && imp_dev, "bad arguments");
     LIC360_CHECK_BATCH(c, K);
-    return encode_latents(c, K, code_dev, mask_dev, imp_dev, true);
+    return encode_latents(c, K, code_dev, mask_dev, imp_dev, "latent");
+}
+
+int lic360_codec_encode_candidates(lic360_codec* c, int K, const float* code_dev, const float* imp_dev, const int32_t* protect_dev, int J,
+                                   const int* cand_latent_host, const int* cand_offset_host) {
+    LIC360_CHECK_ARG(K >= 1, "K must be at least 1");
+    LIC360_CHECK_ARG(J >= 1, "J must be at least 1");
+    LIC360_CHECK_ARG(c && code_dev && imp_dev && cand_latent_host && cand_offset_host, "bad arguments");
+    LIC360_CHECK_BATCH(c, J);
+    std::vector<int2> tab;
+    const int rc = candidate_table(__func__, K, J, cand_latent_host, cand_offset_host, tab);
+    if (rc) return rc;
+    return encode_latents(c, J, code_dev, nullptr, imp_dev, "candidate", tab.data(), protect_dev);
 }
 
 // the GPU work of an estimate of K latents on the codec's two streams; the code stream ends with the copy of both streams' results.
@@ -1328,14 +1392,8 @@ static int enqueue_estimate(lic360_codec* c, int K, const float* code_dev, const
     const EstimateTotals r = estimate_totals(c->est_dev, K);
     const Candidates cd{c->cand_dev, src_levels, protect};
     if (cand_host) {
-        // both streams read the table: ev_est marks it and the levels on the device, and is recorded again below for the results
-        cudaStream_t s = c->imp.stream;
-        const int hw = c->imp.H * c->imp.W;
-        LIC360_CUDA(cudaMemcpyAsync(c->cand_dev, cand_host, (size_t)K * sizeof(int2), cudaMemcpyHostToDevice, s));
-        candidate_levels_kernel<<<dim3((hw + 255) / 256, K), 256, 0, s>>>(cd, hw, c->cand_levels_dev);
-        LAUNCH_CHECK();
-        LIC360_CUDA(cudaEventRecord(c->ev_est, s));
-        LIC360_CUDA(cudaStreamWaitEvent(c->code.stream, c->ev_est, 0));
+        const int rc = enqueue_candidates(c, K, cand_host, cd);  // ev_est is recorded again below for the results
+        if (rc) return rc;
         imp_dev = c->cand_levels_dev;
     }
     {
@@ -1431,12 +1489,9 @@ int lic360_codec_estimate_candidates(lic360_codec* c, int K, const float* code_d
     LIC360_CHECK_ARG(J >= 1, "J must be at least 1");
     LIC360_CHECK_ARG(c && code_dev && imp_dev && cand_latent_host && cand_offset_host && bits_host && counts_host, "bad arguments");
     LIC360_CHECK_BATCH(c, J);
-    std::vector<int2> tab(J);
-    for (int j = 0; j < J; j++) {
-        LIC360_CHECK_ARG(cand_latent_host[j] >= 0 && cand_latent_host[j] < K, "cand_latent must lie in [0, K)");
-        LIC360_CHECK_ARG(cand_offset_host[j] >= 0, "offsets must not be negative");
-        tab[j] = make_int2(cand_latent_host[j], cand_offset_host[j]);
-    }
+    std::vector<int2> tab;
+    const int rc = candidate_table(__func__, K, J, cand_latent_host, cand_offset_host, tab);
+    if (rc) return rc;
     return estimate_latents(c, J, code_dev, nullptr, imp_dev, nullptr, nullptr, bits_host, counts_host, "candidate", tab.data(), protect_dev);
 }
 

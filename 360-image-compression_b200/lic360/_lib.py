@@ -85,6 +85,7 @@ SIGNATURES = {
     "lic360_codec_encode_batch": (_I, [_P, _I, _P, _P, _P]),
     "lic360_codec_batch_stream_size": (_L, [_P, _I, _I]),
     "lic360_codec_batch_stream_copy": (_L, [_P, _I, _I, _P, _L]),
+    "lic360_codec_encode_candidates": (_I, [_P, _I, _P, _P, _P, _I, _P, _P]),
     "lic360_imp_levels_to_mask": (_I, [_P, _I, _I, _P, _I, _P, _P, _P]),
     "lic360_imp_levels_to_mask_protected": (_I, [_P, _I, _I, _P, _I, _P, _P, _P, _P]),
     "lic360_codec_estimate_candidates": (_I, [_P, _I, _P, _P, _P, _I, _P, _P, _P, _P]),

@@ -297,6 +297,37 @@ def select_shared_offset(estimate, max_bytes, K, max_offset, max_batch=None):
     return offset, bounds, per
 
 
+def select_shared_offsets(estimate, budgets, K, max_offset, max_batch=None):
+    """select_shared_offset for R budgets at once, e.g. the rungs of a quality ladder: stage 1 runs once for all budgets, then the
+    stage 2 of every budget, with each (latent, offset) pair estimated once in calls of at most max_batch pairs.  Budget r evaluates
+    exactly the offsets select_shared_offset evaluates for it alone, and its fit is the smallest over those offsets only (the rate is
+    not assumed to fall monotonically with the offset, so an offset another budget evaluated could change the answer).  Returns
+    [(offset, {t: summed bound}, {t: [bound of latent k]})] per budget, each equal to select_shared_offset(estimate, budgets[r], K,
+    max_offset); RuntimeError with select_budget_offset's message followed by ' (rung r)' for the lowest budget no offset fits."""
+    per, summed = {}, {}
+
+    def run(offsets):
+        ests = _chunked(estimate, [(k, t) for t in offsets for k in range(K)], max_batch)
+        for i, t in enumerate(offsets):
+            per[t] = [budget_bound(x) for x in ests[i * K:(i + 1) * K]]
+            summed[t] = sum(per[t])
+
+    stage1 = _stage1_offsets(max_offset)
+    run(stage1)
+    stage2 = []
+    for r, b in enumerate(budgets):
+        try:
+            stage2.append(_stage2_offsets(stage1, summed, b, max_offset))
+        except RuntimeError as e:
+            raise RuntimeError("%s (rung %d)" % (e, r)) from None
+    run(sorted(set(t for s in stage2 for t in s)))
+    out = []
+    for b, s in zip(budgets, stage2):
+        own = {t: summed[t] for t in stage1 + s}
+        out.append((_smallest_fit(own, b), own, {t: per[t] for t in own}))
+    return out
+
+
 class PerOpCodec(object):
     def __init__(self, backend, params, gid=0, workdir=None):
         self.backend, self.gid = backend, gid
@@ -539,6 +570,20 @@ class FusedCodec(object):
         if len(lat) != len(offs):
             raise RuntimeError("estimate_candidates: %d latents for %d offsets" % (len(lat), len(offs)))
         return self._candidates(code, imp, protect, list(zip(lat, offs)))
+
+    def encode_candidates(self, code, imap_quant, cand_latent, cand_offset, protect=None):
+        """encode_batch of J rate-control candidates given as (latent, offset) pairs, without materialising them
+        (lic360_codec_encode_candidates): the inputs as in estimate_candidates.  Returns J pairs (imp_bytes, code_bytes); pair j is
+        byte-identical to encode_batch of the candidate's levels and mask (levels_to_mask_batch) with its latent's code.  A candidate
+        encode would refuse raises encode's message followed by ' (candidate j)', for the first such j."""
+        K, code, imp, protect = self._budget_inputs(code, imap_quant, protect)
+        lat, offs = [int(k) for k in cand_latent], [int(t) for t in cand_offset]
+        if len(lat) != len(offs):
+            raise RuntimeError("encode_candidates: %d latents for %d offsets" % (len(lat), len(offs)))
+        J = len(lat)
+        check(LIB.lic360_codec_encode_candidates(self._h, K, code.data_ptr(), imp.data_ptr(), None if protect is None else protect.data_ptr(),
+                                                 J, (ctypes.c_int * max(J, 1))(*lat), (ctypes.c_int * max(J, 1))(*offs)))
+        return [(self._batch_stream_bytes(j, 1), self._batch_stream_bytes(j, 0)) for j in range(J)]
 
     def encode_batch_to_budget(self, code, imap_quant, max_bytes, protect=None, shared=False, max_batch=16):
         """encode_to_budget of K latents, with batched estimates and one encode_batch: code (K,48,H,W), imap_quant (K,1,H/2,W/2),

@@ -308,6 +308,76 @@ def unpack_tile_streams(blob):
     return rows, cols, H, W, out
 
 
+# A quality ladder of a tiled image: every tile coded at R rates (rungs), so that a server can cut, per viewer, an ordinary tile
+# container that sends the tiles in view from a high rung and the rest from a low one (ladder_to_tiles).  Rung r of tile k is an
+# ordinary stream pair, coded with the rung's level offset.
+LADDER_MAGIC = b"L3L1"
+
+
+def ladder_header_bytes(nrungs, ntiles):
+    return 24 + 4 * nrungs + 8 * nrungs * ntiles
+
+
+def pack_ladder_streams(rows, cols, H, W, offsets, rungs):
+    """offsets: the R rungs' level offsets; rungs: R lists of rows * cols (imp_bytes, code_bytes) in tile order -> one container: magic,
+    rows, cols, H, W, R, the R offsets, the R * rows * cols stream-length pairs rung-major, the payloads in the same order."""
+    tile_grid(H, W, rows, cols)
+    T, R = rows * cols, len(rungs)
+    if R < 1 or len(offsets) != R:
+        raise ValueError("pack_ladder_streams: %d offsets for %d rungs (need at least one rung)" % (len(offsets), R))
+    if any(isinstance(t, bool) or not isinstance(t, int) or not 0 <= t < 2 ** 32 for t in offsets):
+        raise ValueError("pack_ladder_streams: offsets must be non-negative ints (got %r)" % (list(offsets),))
+    if any(len(r) != T for r in rungs):
+        raise ValueError("pack_ladder_streams: rungs of %s stream pairs for %dx%d tiles" % ([len(r) for r in rungs], rows, cols))
+    head = LADDER_MAGIC + struct.pack("<IIIII", rows, cols, H, W, R) + struct.pack("<%dI" % R, *offsets)
+    head += b"".join(struct.pack("<II", len(a), len(b)) for r in rungs for a, b in r)
+    return head + b"".join(a + b for r in rungs for a, b in r)
+
+
+def unpack_ladder_streams(blob):
+    """-> (rows, cols, H, W, offsets, rungs), rungs[r][k] = (imp_bytes, code_bytes) of tile k at rung r; raises ValueError on a
+    malformed container."""
+    if len(blob) < 24 or blob[:4] != LADDER_MAGIC:
+        raise ValueError("unpack_ladder_streams: not a ladder container")
+    rows, cols, H, W, R = struct.unpack_from("<IIIII", blob, 4)
+    tile_grid(H, W, rows, cols)  # ValueError when the grid does not divide the latent
+    T = rows * cols
+    if R < 1:
+        raise ValueError("unpack_ladder_streams: a ladder needs at least one rung")
+    off = ladder_header_bytes(R, T)
+    if len(blob) < off:
+        raise ValueError("unpack_ladder_streams: truncated header")
+    offsets = list(struct.unpack_from("<%dI" % R, blob, 24))
+    lens = struct.unpack_from("<%dI" % (2 * R * T), blob, 24 + 4 * R)
+    if off + sum(lens) != len(blob):
+        raise ValueError("unpack_ladder_streams: payload size does not match the header")
+    rungs = []
+    for r in range(R):
+        rung = []
+        for k in range(T):
+            a, b = lens[2 * (r * T + k)], lens[2 * (r * T + k) + 1]
+            rung.append((bytes(blob[off:off + a]), bytes(blob[off + a:off + a + b])))
+            off += a + b
+        rungs.append(rung)
+    return rows, cols, H, W, offsets, rungs
+
+
+def ladder_to_tiles(blob, rungs):
+    """Cuts a tile container from a ladder: tile k from rung rungs[k] (rungs: one rung index for every tile, or a list of rows * cols
+    indices, e.g. TileCodec.rungs_for_views).  The result is an ordinary L3T1 container, equal to pack_tile_streams of the chosen
+    streams, which TileCodec.decode / decode_tiles / decode_views read as any other.  ValueError on a malformed ladder, a wrongly
+    sized list or a rung outside [0, R)."""
+    rows, cols, H, W, offsets, ladder = unpack_ladder_streams(blob)
+    T, R = rows * cols, len(offsets)
+    if isinstance(rungs, int) and not isinstance(rungs, bool):
+        rungs = [rungs] * T
+    if not isinstance(rungs, (list, tuple)) or len(rungs) != T:
+        raise ValueError("ladder_to_tiles: need one rung index or a list of %d (got %r)" % (T, rungs))
+    if any(isinstance(r, bool) or not isinstance(r, int) or not 0 <= r < R for r in rungs):
+        raise ValueError("ladder_to_tiles: rung indices must be ints in [0, %d) (got %r)" % (R, rungs))
+    return pack_tile_streams(rows, cols, H, W, [ladder[r][k] for k, r in enumerate(rungs)])
+
+
 def split_tiles(x, rows, cols):
     """(1,C,h,w) -> (rows*cols, C, h/rows, w/cols): the tiles in row-major order, one contiguous batch"""
     _, C, h, w = x.shape
@@ -381,6 +451,73 @@ class TileCodec(_PartCodec):
         blob = pack_tile_streams(self.rows, self.cols, self.H, self.W, [(x["imp_bytes"], x["code_bytes"]) for x in r["results"]])
         return {"container": blob, "offset": r["offset"], "bound": r["bound"] + head,
                 "bounds": {t: b + head for t, b in r["bounds"].items()}, "results": r["results"]}
+
+    def encode_ladder(self, code, imap, budgets=None, offsets=None, protect=None, max_batch=16):
+        """Every tile at R rates in one ladder container (pack_ladder_streams), from which ladder_to_tiles cuts ordinary tile containers.
+        Give exactly one of:
+          budgets: R container budgets in bytes, header included.  Rung r is encode_to_budget(code, imap, budgets[r], protect)'s
+            shared mode, one offset for all tiles, found for all rungs by one select_shared_offsets over estimate_candidates, so the
+            stage-1 estimates are shared and no (tile, offset) pair is estimated twice; ladder_to_tiles(ladder, r) equals that call's
+            container byte for byte.
+          offsets: R fixed level offsets, no search; rung r is encode() of the tiles lowered by offsets[r] (levels_to_mask).
+        Each distinct (tile, offset) pair is coded once by FusedCodec.encode_candidates, at most max_batch per pass (it bounds the
+        encoder buffers and does not change the result).  code (1,48,H,W), imap (1,1,H/2,W/2), protect None or an integer (1,1,H/2,W/2)
+        map, split as encode_to_budget splits it.
+        -> {'ladder': bytes, 'offsets': per rung, 'bounds': per rung encode_to_budget's {offset: container bound} (None with offsets),
+        'sizes': bytes of each rung's cut}.  RuntimeError, with nothing returned, when no offset fits a budget (encode_to_budget's
+        message followed by ' (rung r)') or a cut exceeds its budget.  world == 1 only."""
+        if self.world != 1:
+            raise RuntimeError("TileCodec.encode_ladder: needs world == 1 (got %d); the tiles' bounds are not gathered across ranks"
+                               % self.world)
+        self._check(code, imap, "encode_ladder")
+        if protect is not None and (not isinstance(protect, torch.Tensor) or tuple(protect.shape) != tuple(imap.shape)):
+            raise RuntimeError("TileCodec.encode_ladder: protect must be a (1,1,%d,%d) integer tensor, like the importance map"
+                               % (self.H // 2, self.W // 2))
+        if (budgets is None) == (offsets is None):
+            raise RuntimeError("TileCodec.encode_ladder: give exactly one of budgets and offsets")
+        rungs = [int(x) for x in (budgets if offsets is None else offsets)]
+        if not rungs:
+            raise RuntimeError("TileCodec.encode_ladder: a ladder needs at least one rung")
+        if isinstance(max_batch, bool) or not isinstance(max_batch, int) or max_batch < 1:
+            raise RuntimeError("TileCodec.encode_ladder: max_batch must be a positive int (got %r)" % (max_batch,))
+        import lic360_pipeline as pl
+        T, head = len(self.tiles), tile_header_bytes(len(self.tiles))
+        codes, imaps = split_tiles(code, self.rows, self.cols), split_tiles(imap, self.rows, self.cols)
+        prot = None if protect is None else split_tiles(protect, self.rows, self.cols)
+        cd = self.codecs[0]
+        bounds = None
+        if offsets is None:
+            top = 48 if prot is None else 48 + int(prot.max())
+
+            def estimate(pairs):
+                return cd.estimate_candidates(codes, imaps, [k for k, _ in pairs], [t for _, t in pairs], prot)
+
+            picks = pl.select_shared_offsets(estimate, [b - head for b in rungs], T, top, max_batch)
+            offs = [o for o, _, _ in picks]
+            bounds = [{t: b + head for t, b in own.items()} for _, own, _ in picks]
+        else:
+            offs = rungs
+            if any(t < 0 for t in offs):
+                raise RuntimeError("TileCodec.encode_ladder: offsets must not be negative (got %r)" % (offs,))
+        pairs = [(k, t) for t in sorted(set(offs)) for k in range(T)]
+        coded = {}
+        for i in range(0, len(pairs), max_batch):
+            part = pairs[i:i + max_batch]
+            coded.update(zip(part, cd.encode_candidates(codes, imaps, [k for k, _ in part], [t for _, t in part], prot)))
+        streams = [[coded[(k, t)] for k in range(T)] for t in offs]
+        sizes = [head + sum(len(a) + len(b) for a, b in s) for s in streams]
+        if budgets is not None:
+            for r, (size, budget) in enumerate(zip(sizes, rungs)):
+                if size > budget:
+                    raise RuntimeError("TileCodec.encode_ladder: rung %d (offset %d) encoded to %d bytes, above its bound of %d and the "
+                                       "budget of %d bytes" % (r, offs[r], size, bounds[r][offs[r]], budget))
+        return {"ladder": pack_ladder_streams(self.rows, self.cols, self.H, self.W, offs, streams), "offsets": offs, "bounds": bounds,
+                "sizes": sizes}
+
+    def rungs_for_views(self, thetas, phis, fov, inside, outside, margin=0):
+        """Rung indices for ladder_to_tiles: `inside` for the tiles the views need (tiles_for_views), `outside` for the others."""
+        need = set(self.tiles_for_views(thetas, phis, fov, margin))
+        return [inside if k in need else outside for k in range(len(self.tiles))]
 
     def tiles_for_views(self, thetas, phis, fov, margin=0):
         """Sorted indices of the tiles that hold a cell of the views' footprints (lic360_pipeline.view_protection on the importance

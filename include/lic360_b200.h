@@ -291,6 +291,19 @@ int lic360_codec_encode_batch(lic360_codec* c, int K, const float* code_dev, con
  * them to out and returns the stream's size.  -1 (and a message) when k is not a latent of the last successful encode. */
 long lic360_codec_batch_stream_size(lic360_codec* c, int k, int stream_id);
 long lic360_codec_batch_stream_copy(lic360_codec* c, int k, int stream_id, uint8_t* out, long cap);
+/* lic360_codec_encode_batch of J rate-control candidates given as (source latent, offset) pairs, without materialising them: the
+ * arguments and their limits are those of lic360_codec_estimate_candidates.  Candidate j's two streams are byte-identical to
+ * lic360_codec_encode_batch run on the source's code with the candidate's levels and mask from lic360_imp_levels_to_mask_batch.  No
+ * candidate's code or (48,H,W) mask is stored: the code network's input is built as in lic360_codec_estimate_candidates, and the code
+ * stream's row kernel reads the source code and derives each mask bit again; the importance stream codes the candidate levels.
+ * Results: candidate j's streams are read with lic360_codec_batch_stream_size / _copy (k = j) and stay valid until the next encode,
+ * encode_batch, encode_candidates or decode.  Buffers and lic360_codec_last_timing are those of lic360_codec_encode_batch at K = J.
+ * Errors: a candidate lic360_codec_encode would refuse fails the whole call with encode's status and message followed by
+ * " (candidate j)", for the lowest such j; within a candidate the importance stream's error comes first; validity is judged on the
+ * candidate, as the estimate judges it (a masked-out code symbol is never checked).  A failed call returns no streams.  K < 1, J < 1,
+ * J beyond the launch limits, a source outside [0, K) or a negative offset is an argument error. */
+int lic360_codec_encode_candidates(lic360_codec* c, int K, const float* code_dev, const float* imp_dev, const int32_t* protect_dev,
+                                   int J, const int* cand_latent_host, const int* cand_offset_host);
 /* Candidate importance maps and the code masks the decoder derives from them, for rate control.  levels_dev (h,w) are importance
  * levels as lic360_codec_encode reads them: s = the symbol it codes for a level ((int) of it).  For each offsets_host[j] >= 0:
  *   levels_out_dev[j] (K,1,h,w) = max(s - offsets_host[j], 0)
